@@ -64,7 +64,10 @@ def parse():
     p.add_argument("--variant", type=int, default=0, help="K3 variant: 0 TMA ring, 1 LDG/STG, 2 TMA full staging, 3 TMA two CTAs per transition")
     p.add_argument("--cpu-entries", type=int, default=1_000_000, help="entries in the CPU arm's lz4 deque (replay.py:18: 1 M)")
     p.add_argument("--cpu-distinct", type=int, default=16384, help="distinct lz4 blobs behind those entries (the deque holds references)")
-    p.add_argument("--min-seconds", type=float, default=0.25, help="repeat the --steps block until this much device time (value) / wall clock (e2e)")
+    p.add_argument("--min-seconds", type=float, default=0.25, help="secondary measurements (not value, not e2e.value): repeat their "
+                   "blocks until this much time")
+    p.add_argument("--dump-outputs", metavar="DIR", default=None, help="after the timed steps, write what the last timed step computed "
+                   "(indices, IS weights, losses, gradients, the gathered batch) as DIR/<name>.npy (--impl ours)")
     p.add_argument("--gather-waves", default="auto", help="gather schedule of the step: auto (waves on a side stream, K4 of batch k waits "
                    "for its wave only), none (one gather launch before the first K4), or wave sizes in batches, e.g. 1,1,2,4,12")
     p.add_argument("--gather-window", default="auto", help="ordered fetch inside the gather waves: draws in flight beyond the completed ones (auto | 0 = no limit | n)")
@@ -73,7 +76,12 @@ def parse():
     p.add_argument("--no-k4-priority", action="store_true", help="K4 + K2b on the caller's stream instead of the loop's high-priority stream")
     p.add_argument("--no-pdl-at-joins", action="store_true", help="the K4 that joins a gather wave is launched without its programmatic-launch attribute")
     p.add_argument("--cpu-workers", type=int, default=-1, help="--impl reference DataLoader workers (-1: all cores)")
-    return p.parse_args()
+    a = p.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        p.error("--steps must be >= 1 and --warmup >= 0")
+    if a.dump_outputs and a.impl != "ours":
+        p.error("--dump-outputs writes what the CUDA path computed: --impl ours only")
+    return a
 
 
 # ------------------------------------------------------------------------------------------ clocks
@@ -201,9 +209,10 @@ def HotPath(rp, wl, L, A, torch, variant=0, waves=None):
 
 def time_graphed(hp, steps, warmup, torch, use_graph, barrier, step_fn=None, min_seconds=0.0, reduce_max=None, stats=None):
     """Device time of ONE block of exactly ``steps`` steps (CUDA events on the launching stream, barrier +
-    synchronize on both sides).  The block is repeated until ``min_seconds`` of device time have been measured
-    -- 20 steps of the batch-32 workload are 1.4 ms, too little for one number -- and the MEDIAN block is
-    returned; ``stats`` receives every block's seconds.  ``reduce_max(t)``: max over ranks of one block's time
+    synchronize on both sides), after SETTLE + ``warmup`` untimed steps.  With ``min_seconds`` > 0 (the secondary
+    measurements) the block is repeated until that much device time has been measured and the MEDIAN block is
+    returned; the headline ``value`` times one block, so that --steps is the number of timed steps and the state
+    after them (--dump-outputs) is fixed by the arguments.  ``stats`` receives every block's seconds.  ``reduce_max(t)``: max over ranks of one block's time
     (so every rank sees the same totals and runs the same number of blocks)."""
     step_fn = step_fn or hp.step
     hp.rp.push_dynamic()
@@ -216,7 +225,7 @@ def time_graphed(hp, steps, warmup, torch, use_graph, barrier, step_fn=None, min
         with torch.cuda.graph(g):
             step_fn()
         runner = g.replay
-    for _ in range(warmup):
+    for _ in range(SETTLE + warmup):
         runner()
     torch.cuda.synchronize()
     blocks, total = [], 0.0
@@ -241,16 +250,53 @@ def time_graphed(hp, steps, warmup, torch, use_graph, barrier, step_fn=None, min
     return float(np.median(blocks))
 
 
+def _sample_rows(total, row_bytes, budget, seed):
+    """All rows, or a fixed seeded sample of them that fits ``budget`` bytes."""
+    n = max(1, min(total, budget // row_bytes))
+    return np.arange(total) if n == total else np.sort(np.random.default_rng(seed).choice(total, n, replace=False))
+
+
+def dump_outputs(hp, out_dir, torch):
+    """--dump-outputs: what the last step of ``hp`` computed, as out_dir/<name>.npy in float32 / float64 (integers as
+    float64, exact): the drawn indices and IS weights, per-sample losses, gradients w.r.t. the online output, the
+    gathered batch and the priorities K2b wrote.  Under 64 MB in all: the gradients are cut to a seeded row sample above
+    32 MB, the gathered frame stacks (8 x 84 x 84 u8 per transition) to a seeded sample of 16 MB (*_rows.npy: which)."""
+    torch.cuda.synchronize()
+    T = hp.total
+    f64 = lambda t: t.cpu().numpy().astype(np.float64)
+    f32 = lambda t: t.cpu().numpy().astype(np.float32)
+    out = {"indices": f64(hp.idx), "weights": f32(hp.w), "loss": f32(hp.loss), "actions": f64(hp.act),
+           "returns": f64(hp.r64), "terminals": f32(hp.d32), "bootstrap": f64(hp.boot),
+           "priorities": f32(hp.rp.priority.leaves()[hp.idx]), "max_priority": f32(hp.rp.max_p_tensor)}
+    grad = hp.grad.view(T, -1)
+    g_rows = _sample_rows(T, grad.shape[1] * 4, 32 << 20, 1)
+    out["grad"] = f32(grad[torch.from_numpy(g_rows).to(grad.device)].view(-1, *hp.grad.shape[1:]))
+    if len(g_rows) < T:
+        out["grad_rows"] = g_rows.astype(np.float64)
+    if hp.frac is not None:                                   # FQF: fraction-loss outputs
+        out["fraction_loss"], out["fraction_grad"] = f32(hp.frac), f32(hp.gtau)
+    fr_rows = _sample_rows(T, hp.frames.shape[1] * 4, 16 << 20, 2)
+    out["frames"] = f32(hp.frames[torch.from_numpy(fr_rows).to(hp.frames.device)])
+    out["frames_rows"] = fr_rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def block_stats(blocks, units_per_block):
-    """median / p10 / p90 of the per-block rates."""
+    """median / p10 / p90 of the per-block rates (p10 / p90 only when there is more than one block)."""
     r = np.sort(units_per_block / np.asarray(blocks, dtype=np.float64))
     q = lambda p: float(r[min(len(r) - 1, int(round(p * (len(r) - 1))))])
-    return {"blocks": len(r), "timed_region_s": round(float(np.sum(blocks)), 4), "rate_median": round(float(np.median(r)), 1),
-            "rate_p10": round(q(0.1), 1), "rate_p90": round(q(0.9), 1)}
+    out = {"blocks": len(r), "timed_region_s": round(float(np.sum(blocks)), 4), "rate_median": round(float(np.median(r)), 1)}
+    if len(r) > 1:
+        out.update(rate_p10=round(q(0.1), 1), rate_p90=round(q(0.9), 1))
+    return out
 
 
 EMIT = print
 INNER = 20
+SETTLE = 200             # untimed steps before the --warmup ones: the first ~150 replays of a freshly captured step run 1-2 %
+                         # slower (profiles/settle_first_replays.txt); a fixed count keeps the state deterministic
 GATHER_WAVES = "auto"    # --gather-waves
 PDL_AT_JOINS = True      # --no-pdl-at-joins
 GATHER_WINDOW = "auto"   # --gather-window
@@ -578,9 +624,10 @@ def run_ours(args):
     hp = HotPath(rp, wl, L, A, torch, variant=args.variant)
 
     blocks = []
-    with ClockSampler(local) as clk:
-        secs = time_graphed(hp, args.steps, args.warmup, torch, not args.no_graph, barrier, min_seconds=args.min_seconds,
-                            reduce_max=reduce_max, stats=blocks)
+    with ClockSampler(local) as clk:     # exactly --steps timed steps: one block
+        secs = time_graphed(hp, args.steps, args.warmup, torch, not args.no_graph, barrier, reduce_max=reduce_max, stats=blocks)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(hp, args.dump_outputs, torch)
     total = hp.total
     value = total * args.steps * world / secs
     timing = block_stats(blocks, total * args.steps * world)
@@ -614,8 +661,8 @@ def run_ours(args):
     # ---- e2e through the public API -----------------------------------------------------------------
     barrier()
     e2e_blocks = []
-    e2e_v, h2d, d2h = e2e_cabi(hp, args.steps, 5, torch, graph=not args.no_graph, depth=2, copy_stream=True,
-                               min_seconds=args.min_seconds, stats=e2e_blocks)
+    e2e_v, h2d, d2h = e2e_cabi(hp, args.steps, SETTLE + 5, torch, graph=not args.no_graph, depth=2, copy_stream=True,
+                               stats=e2e_blocks)   # its graphs are freshly captured too
     e2e_timing = block_stats(e2e_blocks, total * args.steps)
     side = [0.0, 0.0, 0.0, 0.0]
     if not args.no_extra:
@@ -686,7 +733,7 @@ def run_ours(args):
             "scaling": "weak", "vs_baseline": None, "dtype": "u8 frames / f32 targets / f64 n-step returns",
             "data": "synthetic",
             "config": shared_config(wl, L, A, ring, args),
-            "timing": dict(timing, note=f"the block of --steps {args.steps} steps was repeated until {args.min_seconds} s of device time; value = median block"),
+            "timing": dict(timing, note=f"one block of exactly --steps {args.steps} steps after {SETTLE} + --warmup {args.warmup} untimed steps"),
             "timed_region_s": timing["timed_region_s"],
             "run": {"frame_ring_GB_per_gpu": round((ring * 1.0625 + 65536) * F_BYTES / 1e9, 2), "cuda_graph": not args.no_graph,
                     "uniforms": "torch uniform_ launch" if RNG_SEED is None else "Philox4x32-10 inside K2a (a0_pt_sample_rng)",
@@ -1090,7 +1137,7 @@ def run_reference(args):
     from oracle import ref_arm as RA
     B, algo = wl["B"], wl["algo"]
     entries = cpu_entries_for(wl, args)
-    steps = max(1, min(args.steps, 200))
+    steps = args.steps
     warm = max(1, min(args.warmup, 5))
     # ---- the port, all intra-op threads, in-process fetch and the reference's 2 workers: cross-check ----------------
     torch.set_num_threads(cores)

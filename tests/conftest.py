@@ -23,9 +23,13 @@ def golden():
 
 
 def pytest_sessionfinish(session, exitstatus):
-    """Worst relative errors seen by the GPU parity tests (tests/parity.py) -> profiles/parity_r02.json."""
+    """Worst relative errors seen by the GPU parity tests (tests/parity.py) -> the JSON file A0_PARITY_RECORD names.
+    Unset (the default), nothing is written: a test run leaves the tree as it found it."""
+    path = os.environ.get("A0_PARITY_RECORD")
+    if not path:
+        return
     try:
         from tests import parity
-        parity.dump(ROOT)
+        parity.dump(path)
     except Exception:
         pass

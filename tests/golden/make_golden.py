@@ -17,6 +17,8 @@ Fixtures:
   loss_<algo>_<dq>.npz  train_step inputs/outputs/autograd grads, six algos
   static_fns.npz      huber_qr_loss / log_softmax_stable known answers
   act.npz             Actor.act epsilon-greedy selection (python tests/golden/make_golden.py --only act)
+  model_parity.npz    DeepQNet per algo x {plain, dueling, dueling+noisy}: tests/model_record.py's record
+                      (python tests/golden/make_golden.py --only model_parity)
 """
 import os
 import sys
@@ -463,6 +465,23 @@ def gen_act():
     print("act ok:", {k: v.shape for k, v in out.items()})
 
 
+def gen_model_parity():
+    """The reference's agent0.deepq.model.DeepQNet, recorded by tests/model_record.py (what
+    tests/test_model_parity.py compares agent0_b200.model against), six algorithms x three head variants."""
+    from agent0.deepq.model import DeepQNet
+    from tests.model_record import ALGOS, VARIANTS, key, record
+    out = {}
+    for algo in ALGOS:
+        for dueling, noisy in VARIANTS:
+            cfg = ExpConfig()
+            cfg.obs_shape, cfg.action_dim = (4, 84, 84), 6
+            cfg.learner.algo, cfg.learner.dueling_head, cfg.learner.noisy_net = AlgoEnum[algo], dueling, noisy
+            for k, v in record(lambda: DeepQNet(cfg), algo).items():
+                out[f"{key(algo, dueling, noisy)}/{k}"] = v
+    np.savez_compressed(os.path.join(HERE, "model_parity.npz"), **out)
+    print(f"model_parity: {len(out)} arrays")
+
+
 if __name__ == "__main__":
     np.random.seed(0)
     torch.manual_seed(0)
@@ -485,3 +504,4 @@ if __name__ == "__main__":
     for algo, dq, du in (("dqn", True, False), ("mdqn", False, True), ("c51", True, True), ("qr", False, False),
                          ("iqn", True, True), ("fqf", True, False)):
         gen_learner(algo, dq, du)
+    gen_model_parity()

@@ -156,7 +156,7 @@ def test_duplicates_per_batch_against_the_reference_draw_without_replacement(sha
     replay.py:41-43: no index twice in a batch, at the price of a law that is no longer P(i) ~ p_i once a heavy
     record has been taken); the stratified tree descent draws WITH replacement and keeps the law.  The figure
     that separates the two is the duplicate rate inside a batch of 512, measured here on three priority
-    vectors and written to profiles/parity_r02.json:
+    vectors and recorded by tests/parity.py:
       spread   |N(0,1)|-shaped priorities (the shard as built): no stratum is narrower than a leaf
       peaked   1 % of the records at 100x the rest
       extreme  100 records hold 90 % of the mass (each spans ~4.6 strata: those draws MUST repeat)

@@ -2,7 +2,7 @@
 golden outputs of the unmodified reference and (b) the numpy oracle on larger seeded inputs.
 Tolerance: 1e-5 RELATIVE in fp32 (north_star) with an explicit denominator floor -- tests/parity.py:
 |got - ref| <= 1e-5 * max(|ref|, 1e-2 * max|ref|) -- no absolute ``atol``; argmax/indices exact.  The worst
-relative error per quantity is written to profiles/parity_r02.json."""
+relative error per quantity is recorded by tests/parity.py."""
 import numpy as np
 import pytest
 import torch
