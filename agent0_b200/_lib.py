@@ -81,6 +81,7 @@ SIGNATURES = {
     "a0_pt_sample": (_i32, [_vp, _vp, _i32, _i32, _f32, _f32, _f32, _i32, _vp, _vp, _vp, _vp]),
     "a0_pt_sample_rng": (_i32, [_vp, C.c_uint64, _i64, _i32, _i32, _f32, _f32, _f32, _i32, _vp, _vp, _vp, _vp, _vp]),
     "a0_pt_rng_seek": (_i32, [_vp, C.c_uint64, _vp]),
+    "a0_pt_sample_unique": (_i32, [_vp, C.c_uint64, _i64, _i32, _i32, _f32, _f32, _f32, _i32, _vp, _vp, _vp, _vp, _vp]),
     "a0_rb_gather": (_i32, [_vp, _vp, _i32, _i32, _f64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _vp]),
     "a0_rb_sample_gather": (_i32, [_vp, _vp, C.c_uint64, _i64, _i32, _i32, _f32, _f32, _f32, _i32, _vp, _vp, _vp, _i32, _f64,
                                    _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),

@@ -85,7 +85,8 @@ int a0_check_fault(a0_replay* h, const char* who) {
     *(volatile int32_t*)h->fault_host = 0;
     a0_set_error("%s: an earlier launch on this shard reported device fault %d (%s)", who, code,
                  code == 1 ? "a gather CTA of a0_rb_sample_gather timed out waiting for its sampler: its outputs are invalid"
-                           : "unknown");
+                 : code == 2 ? "a0_pt_sample_unique found fewer than B records with positive priority: the batch's last rows repeat its first record"
+                             : "unknown");
     return A0_EFAULT;
   }
   return A0_OK;

@@ -509,6 +509,245 @@ extern "C" int a0_pt_rng_seek(a0_replay_t* h, uint64_t call, a0_stream_t stream_
 }
 
 // ------------------------------------------------------------------------------------------------
+// K2a-unique.  Prioritized batches WITHOUT replacement, the law of the reference's
+// torch.multinomial(priority[:top], B, replacement=False) (agent0/deepq/replay.py:41-43).  Defined
+// exactly by oracle/sample_unique.py, which this kernel matches bit for bit (indices, priorities, stats):
+//   * a batch is the first B DISTINCT records of a stream of independent descents; candidate j of batch k
+//     in call c takes u = ((x0 >> 5) * 2^26 + (x1 >> 6)) * 2^-53 (float64) from
+//     Philox4x32-10(counter {j, 0x80000000 | k, c_lo, c_hi}, key {seed_lo, seed_hi});
+//   * round r draws B - |F| candidates that descend in float64 against the accepted set F as it stood at
+//     the start of the round: m(v) = max(0, tree[v] - (Pre[hi_v] - Pre[lo_v])) with Pre the sequential
+//     float64 prefix sums of F's priorities in position order; t = u * m(1); go left iff
+//     t < m(2v) || !(m(2v+1) > 0), else t -= m(2v).  A leaf in F or with p <= 0 is void.  The non-void
+//     candidates are accepted in j order, each record once; the rows are F in acceptance order;
+//   * m(1) <= 0 at the start of a round, or 8 consecutive rounds accepting nothing: fewer than B records
+//     with positive priority.  The remaining rows repeat F[0] and the handle's fault word gets code 2.
+// One CTA per batch owns the whole batch: thread c descends candidate c (float2 loads below the
+// shared-memory top levels), a bitonic sort of (position, ordinal) keeps each record's first occurrence,
+// a block scan turns acceptances into rows, and the IS-weight epilogue (trainer.py:91-94) needs no
+// cross-CTA ticket.  A further round re-sorts F and forms Pre (one thread: the order of the sum is part
+// of the law), and each level of its descents binary-searches F's range below the current node.
+// ------------------------------------------------------------------------------------------------
+constexpr int KU_MAX_BATCH = 1024;
+constexpr int KU_MAX_IDLE = 8;
+constexpr int KU_FAULT_SHORTFALL = 2;
+
+// ascending sort of s_key[0, n) (n a power of two, n <= blockDim.x), every thread of the CTA calls it
+__device__ __forceinline__ void a0_ku_bitonic(unsigned long long* s_key, int n) {
+  for (int k = 2; k <= n; k <<= 1)
+    for (int j = k >> 1; j > 0; j >>= 1) {
+      const int i = threadIdx.x;
+      const int x = i ^ j;
+      if (i < n && x > i) {
+        const unsigned long long a = s_key[i], b = s_key[x];
+        if ((a > b) == ((i & k) == 0)) { s_key[i] = b; s_key[x] = a; }
+      }
+      __syncthreads();
+    }
+}
+
+// exclusive prefix sum of v over the CTA; *total = the sum (every thread)
+__device__ __forceinline__ int a0_ku_scan(int v, int* s_warp, int* total) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+  int x = v;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int y = __shfl_up_sync(0xffffffffu, x, o);
+    if (lane >= o) x += y;
+  }
+  if (lane == 31) s_warp[warp] = x;
+  __syncthreads();
+  if (warp == 0) {
+    int w = lane < nw ? s_warp[lane] : 0;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int y = __shfl_up_sync(0xffffffffu, w, o);
+      if (lane >= o) w += y;
+    }
+    if (lane < nw) s_warp[lane] = w;          // inclusive over warps
+  }
+  __syncthreads();
+  const int before = (warp > 0 ? s_warp[warp - 1] : 0) + x - v;
+  *total = s_warp[nw - 1];
+  __syncthreads();                            // s_warp is reused by the next scan
+  return before;
+}
+
+__global__ void __launch_bounds__(KU_MAX_BATCH)
+a0_k2a_unique(const float* __restrict__ tree, int32_t P, int32_t D, int32_t batch, int32_t nbatches, float top, float beta,
+              float sum_offset, int32_t uniform, int64_t* __restrict__ idx_out, float* __restrict__ prio_out,
+              float* __restrict__ weight_out, int32_t* __restrict__ stats_out, const float* __restrict__ dyn, const A0Rng rng,
+              int32_t* fault, int32_t top_levels) {
+  __shared__ __align__(16) float s_top[2 << K2A_TOP];
+  __shared__ unsigned long long s_key[KU_MAX_BATCH];
+  __shared__ int32_t s_apos[KU_MAX_BATCH];          // F in acceptance order
+  __shared__ float s_apri[KU_MAX_BATCH];
+  __shared__ int32_t s_fpos[KU_MAX_BATCH];          // F in position order
+  __shared__ double s_pre[KU_MAX_BATCH + 1];        // its prefix sums
+  __shared__ int32_t s_flag[KU_MAX_BATCH];
+  __shared__ int s_warp[32];
+  __shared__ unsigned long long s_call;
+  A0_T0();
+  A0_PDL_PROLOGUE();
+  A0_TMID();
+  if (dyn) {
+    top = __ldcg(dyn);
+    beta = __ldcg(dyn + 1);
+    sum_offset = __ldcg(dyn + 2);
+  }
+  const int tid = threadIdx.x;
+  const int k = blockIdx.x;
+  const bool rng_dev = rng.call < 0;
+  if (tid == 0) {
+    s_call = rng_dev ? __ldcg(rng.call_dev) : (unsigned long long)rng.call;
+    s_pre[0] = 0.0;
+  }
+  const int n4 = (2 << top_levels) >> 2;
+  for (int i = tid; i < n4; i += blockDim.x) reinterpret_cast<float4*>(s_top)[i] = __ldcg(reinterpret_cast<const float4*>(tree) + i);
+  __syncthreads();
+  const unsigned long long call = s_call;
+  const float root = s_top[1];
+  int nF = 0, rounds = 0, cand = 0, idle = 0;
+  bool shortfall = false;
+  while (nF < batch) {
+    const double m1 = fmax(0.0, __dsub_rn((double)root, s_pre[nF]));
+    if (!(m1 > 0.0)) { shortfall = true; break; }
+    const int need = batch - nF;
+    int pos = -1;
+    float leaf = 0.0f;
+    if (tid < need) {
+      const uint32_t j = (uint32_t)(cand + tid);
+      uint32_t c0 = j, c1 = 0x80000000u | (uint32_t)k, c2 = (uint32_t)call, c3 = (uint32_t)(call >> 32);
+      uint32_t k0 = (uint32_t)rng.seed, k1 = (uint32_t)(rng.seed >> 32);
+#pragma unroll
+      for (int r = 0; r < 10; ++r) {
+        const uint32_t hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
+        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
+        const uint32_t n0 = hi1 ^ c1 ^ k0, n2 = hi0 ^ c3 ^ k1;
+        c0 = n0; c1 = lo1; c2 = n2; c3 = lo0;
+        k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
+      }
+      const unsigned long long bits = ((unsigned long long)(c0 >> 5) << 26) | (unsigned long long)(c1 >> 6);
+      double t = __dmul_rn(__dmul_rn(__ull2double_rn(bits), 1.1102230246251565e-16), m1);      // * 2^-53: exact
+      int v = 1, a = 0, b = nF;
+      leaf = root;
+      for (int d = 0; d < D; ++d) {
+        const int mid = ((2 * v + 1) << (D - d - 1)) - P;
+        int lo = a, hi = b;                                   // first F position >= mid inside [a, b)
+        while (lo < hi) {
+          const int m = (lo + hi) >> 1;
+          if (s_fpos[m] < mid) lo = m + 1; else hi = m;
+        }
+        float L, R;
+        if (d < top_levels) { L = s_top[2 * v]; R = s_top[2 * v + 1]; }
+        else { const float2 lr = __ldcg(reinterpret_cast<const float2*>(tree + 2 * v)); L = lr.x; R = lr.y; }
+        const double mL = fmax(0.0, __dsub_rn((double)L, __dsub_rn(s_pre[lo], s_pre[a])));
+        const double mR = fmax(0.0, __dsub_rn((double)R, __dsub_rn(s_pre[b], s_pre[lo])));
+        if (t < mL || !(mR > 0.0)) { v = 2 * v; b = lo; leaf = L; }
+        else { t = __dsub_rn(t, mL); v = 2 * v + 1; a = lo; leaf = R; }
+      }
+      if (b - a != 1 && leaf > 0.0f) pos = v - P;             // void: already accepted, or an empty leaf
+    }
+    // first occurrence of every record among this round's candidates, in draw order
+    int n2 = 1;
+    while (n2 < need) n2 <<= 1;
+    if (tid < n2) s_key[tid] = pos >= 0 ? ((unsigned long long)pos << 32) | (unsigned)tid : ~0ull;
+    if (tid < need) s_flag[tid] = 0;
+    __syncthreads();
+    a0_ku_bitonic(s_key, n2);
+    if (tid < need) {
+      const unsigned long long key = s_key[tid];
+      if (key != ~0ull && (tid == 0 || (s_key[tid - 1] >> 32) != (key >> 32))) s_flag[(int)(key & 0xffffffffu)] = 1;
+    }
+    __syncthreads();
+    const int acc = tid < need ? s_flag[tid] : 0;
+    int accepted;
+    const int row = nF + a0_ku_scan(acc, s_warp, &accepted);
+    if (acc) { s_apos[row] = pos; s_apri[row] = leaf; }
+    nF += accepted;
+    rounds += 1;
+    cand += need;
+    idle = accepted ? 0 : idle + 1;
+    if (nF == batch) break;
+    if (idle == KU_MAX_IDLE) { shortfall = true; break; }
+    // F in position order and its prefix sums for the next round's masked descents
+    n2 = 1;
+    while (n2 < nF) n2 <<= 1;
+    __syncthreads();                                          // s_apos / s_apri complete
+    if (tid < n2) s_key[tid] = tid < nF ? ((unsigned long long)s_apos[tid] << 32) | __float_as_uint(s_apri[tid]) : ~0ull;
+    __syncthreads();
+    a0_ku_bitonic(s_key, n2);
+    if (tid < nF) s_fpos[tid] = (int32_t)(s_key[tid] >> 32);
+    if (tid == 0) {
+      double s = 0.0;
+      for (int i = 0; i < nF; ++i) {
+        s = __dadd_rn(s, (double)__uint_as_float((unsigned)(s_key[i] & 0xffffffffu)));
+        s_pre[i + 1] = s;
+      }
+    }
+    __syncthreads();
+  }
+  __syncthreads();
+  if (tid == 0 && shortfall && fault) { *reinterpret_cast<volatile int32_t*>(fault) = KU_FAULT_SHORTFALL; __threadfence_system(); }
+  if (tid == 0 && stats_out) { stats_out[2 * k] = rounds; stats_out[2 * k + 1] = cand; }
+  // rows [nF, batch) of a shortfall repeat F[0]: every row is a valid position for the gather
+  const int fill_pos = nF > 0 ? s_apos[0] : 0;
+  const float fill_pri = nF > 0 ? s_apri[0] : __ldcg(tree + P);
+  float p = 0.0f;
+  if (tid < batch) {
+    const int q = tid < nF ? s_apos[tid] : fill_pos;
+    p = tid < nF ? s_apri[tid] : fill_pri;
+    idx_out[(size_t)k * batch + tid] = q;
+    prio_out[(size_t)k * batch + tid] = p;
+  }
+  if (weight_out) {
+    float* w = weight_out + (size_t)k * batch;
+    if (uniform) {
+      if (tid < batch) w[tid] = 1.0f;                         // ReplayEnum.uniform: weights = 1 (trainer.py:95-96)
+    } else {
+      const float denom = __fadd_rn(root, sum_offset);
+      const float wj = tid < batch ? powf(__fmul_rn(top, __fdiv_rn(p, denom)), -beta) : 0.0f;
+      const float mx = a0_warp_max(wj);
+      if ((tid & 31) == 0) reinterpret_cast<float*>(s_warp)[tid >> 5] = mx;
+      __syncthreads();
+      float bm = reinterpret_cast<float*>(s_warp)[0];
+      for (int i = 1; i < (int)(blockDim.x >> 5); ++i) bm = fmaxf(bm, reinterpret_cast<float*>(s_warp)[i]);
+      if (tid < batch) w[tid] = __fdiv_rn(wj, __fadd_rn(bm, 1e-8f));
+    }
+  }
+  if (tid == 0) {
+    A0_TEND(6);
+    if (rng_dev) a0_rng_done(rng, call, (unsigned)nbatches);   // this CTA read the counter before it arrives
+  }
+}
+
+extern "C" int a0_pt_sample_unique(a0_replay_t* h, uint64_t seed, int64_t call, int32_t total, int32_t batch, float top,
+                                   float beta, float sum_offset, int32_t uniform, int64_t* idx_out, float* prio_out,
+                                   float* weight_out, int32_t* stats_out, a0_stream_t stream_) {
+  // the shape of the draw is checked before the handle: a malformed request is reported without a shard
+  A0_REQUIRE(batch > 0 && batch <= KU_MAX_BATCH, "a0_pt_sample_unique: batch %d outside [1, %d]", batch, KU_MAX_BATCH);
+  A0_REQUIRE(total >= 0 && total % batch == 0, "a0_pt_sample_unique: total %d must be a multiple of batch %d", total, batch);
+  A0_REQUIRE(total / batch <= A0_MAX_BATCHES, "a0_pt_sample_unique: %d batches, at most %d per call", total / batch, A0_MAX_BATCHES);
+  A0_REQUIRE(h != nullptr, "a0_pt_sample_unique: handle is NULL");
+  if (total == 0) return A0_OK;
+  A0_REQUIRE(idx_out && prio_out, "a0_pt_sample_unique: NULL argument");
+  { int frc = a0_check_fault(h, "a0_pt_sample_unique"); if (frc) return frc; }
+  A0DeviceGuard guard(h->device);
+  A0Rng rng;
+  rng.seed = seed;
+  rng.call = call;
+  rng.call_dev = reinterpret_cast<unsigned long long*>(h->counter + K2A_RNG_CALL);
+  rng.ticket = h->counter + K2A_RNG_TICKET;
+  rng.u_out = nullptr;
+  int threads = 32;
+  while (threads < batch) threads <<= 1;
+  A0_LAUNCH(a0_k2a_unique, (unsigned)(total / batch), (unsigned)threads, 0, (cudaStream_t)stream_, 1, A0_PDL_K2, h->tree,
+            (int32_t)h->P, h->D, batch, total / batch, top, beta, sum_offset, uniform, idx_out, prio_out, weight_out, stats_out,
+            (const float*)(top < 0.0f ? h->dyn : nullptr), rng, h->fault_dev, (int32_t)(h->D < K2A_TOP ? h->D : K2A_TOP));
+  return A0_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
 // K2b.  Leaves are written with a deterministic last-writer-wins rule:
 //        mode 0: value = (loss+eps)^alpha, skipped when the leaf is 0; max_p = max(max_p, max loss)
 //        mode 1: pos >= 0 -> max_p^alpha;  pos < 0 -> leaf ~pos = 0

@@ -63,8 +63,9 @@ def wave_plan(L, B, frame_bytes, spec="auto"):
 class ReplayTargetLoop:
     def __init__(self, replay, algo, batch_size, learner_steps, action_dim, outputs, n_step=None, double_q=True,
                  per=None, variant=0, discount=None, alpha=0.5, eps=0.01, c51=(51, -10.0, 10.0), mdqn=(0.03, -1.0),
-                 frames=None, rng_seed=None, overlap_sample_gather=True, want_prio=False, early_update=True,
-                 gather_waves="auto", pdl_at_joins=True, gather_window="auto", k4_priority=True, waves_when_eager=False):
+                 frames=None, rng_seed=None, overlap_sample_gather=None, want_prio=False, early_update=True,
+                 gather_waves="auto", pdl_at_joins=True, gather_window="auto", k4_priority=True, waves_when_eager=False,
+                 replacement=True):
         """replay: ReplayDataset (native_nstep=True when n_step > 1).  outputs: dict of STATIC f32 device
         tensors holding the network outputs of all L*B sampled transitions, batch k in rows
         [k*B, (k+1)*B): ``online``, ``tgt_next`` (+ ``qsel`` [L*B,A] under double_q / for iqn, fqf;
@@ -95,13 +96,29 @@ class ReplayTargetLoop:
         ``step()`` issues the single gather launch unless this is set (the tests set it).
         pdl_at_joins: the K4 that waits for a wave keeps its programmatic-launch attribute (it executes griddepcontrol.wait
         before it reads anything, so every predecessor is complete whichever way the edge is typed): 67.2 against 68.2 us
-        per batch-32 step.  False: those K4 launches are plain stream-ordered launches."""
+        per batch-32 step.  False: those K4 launches are plain stream-ordered launches.
+        replacement=False: every batch holds B distinct records, drawn by a0_pt_sample_unique (the law of the
+        reference's torch.multinomial(priority[:top], B, replacement=False), replay.py:41-43) from the sampler's own
+        Philox stream (``rng_seed``; drawn from torch's default generator when None), and gathered by one plain K3
+        launch: the overlapped and waved schedules (``overlap_sample_gather``, default on only with replacement)
+        are for the stratified draw."""
         assert algo in ALGOS, algo
         self.lib = _lib.load()
         self.rp, self.algo, self.B, self.L, self.A = replay, algo, int(batch_size), int(learner_steps), int(action_dim)
         self.total = T = self.L * self.B
         self.dev = dev = replay.device
         self.variant = int(variant)
+        self.replacement = bool(replacement)
+        if not self.replacement:
+            if overlap_sample_gather:
+                raise ValueError("ReplayTargetLoop(replacement=False) gathers with one plain launch: the overlapped / waved "
+                                 "sample-gather schedules draw with replacement only")
+            if self.B > 1024:
+                raise ValueError(f"ReplayTargetLoop(replacement=False) takes batches of at most 1024 records, not {self.B}")
+            if rng_seed is None:
+                rng_seed = int(torch.randint(-2 ** 63, 2 ** 63 - 1, (1,), dtype=torch.int64).item())
+        elif overlap_sample_gather is None:
+            overlap_sample_gather = True
         self.overlap_sg = bool(overlap_sample_gather) and int(variant) == 0
         self.early_update = bool(early_update)      # step(): K2b starts under the last K4 (a0_pt_update_overlapped)
         self.rng_seed = None if rng_seed is None else int(rng_seed) & 0xFFFFFFFFFFFFFFFF
@@ -152,6 +169,11 @@ class ReplayTargetLoop:
     def sample(self):
         """K2a: L stratified batches + IS weights (top/beta from the device: push_dynamic first)."""
         rp = self.rp
+        if not self.replacement:
+            _lib.check(self.lib.a0_pt_sample_unique(rp.h, self.rng_seed, -1, self.total, self.B, -1.0, float(rp.beta), 0.0,
+                                                    0 if self.per else 1, self.idx.data_ptr(), self.prio.data_ptr(),
+                                                    self.w.data_ptr(), None, self._st()), "a0_pt_sample_unique")
+            return
         if self.rng_seed is not None:
             _lib.check(self.lib.a0_pt_sample_rng(rp.h, self.rng_seed, -1, self.total, self.B, -1.0, float(rp.beta), 0.0,
                                                  0 if self.per else 1, self.idx.data_ptr(), self.prio.data_ptr(),

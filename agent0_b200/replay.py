@@ -367,7 +367,7 @@ class ReplayDataset:
                                                   _lib.stream_ptr(self.device)), "a0_rb_set_dynamic")
 
     def sample(self, batch_size=None, k_batches=1, u=None, indices=None, generator=None, out=None, dynamic=False,
-               normalized=None, seed=None, call=-1, u_out=None, obs_dtype=None):
+               normalized=None, seed=None, call=-1, u_out=None, obs_dtype=None, replacement=True, stats_out=None):
         """Draw ``k_batches`` stratified batches (K2a) and gather them (K3).  ``u`` (f32 device
         tensor of k*B uniforms) or ``indices`` (i64, explicit record positions) make the draw
         reproducible for parity tests; otherwise uniforms come from torch's CUDA generator.
@@ -378,12 +378,32 @@ class ReplayDataset:
         ``obs_dtype=torch.bfloat16`` writes them as bf16(f32 value) for a mixed-precision CNN.
         ``seed`` (int): the sampler draws its own uniforms (Philox4x32-10 inside K2a, no separate RNG
         launch); ``call`` >= 0 names the call number, < 0 uses the shard's device-resident counter,
-        which every launch -- or graph replay -- advances; ``u_out`` receives the uniforms."""
+        which every launch -- or graph replay -- advances; ``u_out`` receives the uniforms.
+        ``replacement=False``: no record twice in a batch, with the law of the reference's
+        torch.multinomial(priority[:top], B, replacement=False) (replay.py:41-43; a0_pt_sample_unique, rows in draw
+        order).  It takes its uniforms from the sampler's own Philox stream: without ``seed``, a 64-bit seed is drawn
+        once from ``generator`` (or torch's default generator) and kept for the shard.  ``stats_out`` (i32 device
+        tensor [k_batches, 2]) receives {rounds, candidates drawn} per batch."""
         B = int(batch_size or self.cfg.learner.batch_size)
         total = B * int(k_batches)
         dev = self.device
         if self.index.top <= 0:
             raise RuntimeError("sample() on an empty replay shard")
+        if not replacement:
+            if u is not None or indices is not None:
+                raise ValueError("sample(replacement=False) draws its own uniforms: u= and indices= are not accepted")
+            if B > 1024:
+                raise ValueError(f"sample(replacement=False) takes batches of at most 1024 records, not {B}")
+            if self.index.top < B:
+                raise ValueError(f"sample(replacement=False): {B} distinct records asked of a shard that holds {self.index.top}")
+            if stats_out is not None and stats_out.numel() < 2 * int(k_batches):
+                raise ValueError("stats_out needs room for {rounds, candidates} of every batch")
+            if seed is None:
+                if getattr(self, "_unique_seed", None) is None:
+                    gd = generator.device if generator is not None else "cpu"
+                    self._unique_seed = int(torch.randint(-2 ** 63, 2 ** 63 - 1, (1,), dtype=torch.int64, device=gd,
+                                                          generator=generator).item()) & 0xFFFFFFFFFFFFFFFF
+                seed = self._unique_seed
         with torch.cuda.device(dev):
             stream = _lib.stream_ptr(dev)
             weights = out.weights if out is not None else torch.empty(total, dtype=torch.float32, device=dev)
@@ -392,7 +412,12 @@ class ReplayDataset:
                 idx = out.indices if out is not None else torch.empty(total, dtype=torch.int64, device=dev)
                 sum_offset = float(self.size - self.index.top) if self.compat_sum else 0.0
                 top = -1.0 if dynamic else float(self.index.top)
-                if u is None and seed is not None:
+                if not replacement:
+                    _lib.check(self.lib.a0_pt_sample_unique(
+                        self.h, int(seed) & 0xFFFFFFFFFFFFFFFF, int(call), total, B, top, float(self.beta), sum_offset,
+                        0 if self.prioritize else 1, _lib.ptr(idx), _lib.ptr(prio), _lib.ptr(weights),
+                        _lib.ptr(stats_out, torch.int32), stream), "a0_pt_sample_unique")
+                elif u is None and seed is not None:
                     _lib.check(self.lib.a0_pt_sample_rng(
                         self.h, int(seed) & 0xFFFFFFFFFFFFFFFF, int(call), total, B, top, float(self.beta), sum_offset,
                         0 if self.prioritize else 1, _lib.ptr(idx), _lib.ptr(prio), _lib.ptr(weights),

@@ -33,7 +33,8 @@ class GraphedUpdates:
     replay.  The first call runs eagerly (it is also the warm-up) and captures; later calls replay.
     At batch 32 the eager loop is bound by ~150 kernel launches per update; the replay is not."""
 
-    def __init__(self, learner, replay, batch_size, learner_steps, normalized=None, sampler_seed=None, obs_dtype=None):
+    def __init__(self, learner, replay, batch_size, learner_steps, normalized=None, sampler_seed=None, obs_dtype=None,
+                 replacement=True):
         import torch
         assert learner.capturable, "construct the learner with capturable=True"
         freq = learner.cfg.learner.target_update_freq
@@ -43,12 +44,13 @@ class GraphedUpdates:
         self.normalized = normalized
         self.sampler_seed = sampler_seed
         self.obs_dtype = obs_dtype
+        self.replacement = bool(replacement)
         self.static = replay.alloc_batch(self.B * self.L, normalized=normalized, obs_dtype=obs_dtype or torch.float32)
         self.graph, self.outs = None, None
 
     def _updates(self):
         self.replay.sample(self.B, k_batches=self.L, out=self.static, dynamic=True, normalized=self.normalized,
-                           seed=self.sampler_seed, obs_dtype=self.obs_dtype)
+                           seed=self.sampler_seed, obs_dtype=self.obs_dtype, replacement=self.replacement)
         outs = []
         for b in split_batches(self.static, self.B):
             result = self.learner.update(_learner_data(b))
@@ -77,7 +79,7 @@ class GraphedUpdates:
 
 class Trainer:
     def __init__(self, cfg, process_group=None, native_nstep=False, graph=False, fused_input=False, sampler_seed=None,
-                 global_is_max=False, amp=False, channels_last=None, **replay_kw):
+                 global_is_max=False, amp=False, channels_last=None, replacement=True, **replay_kw):
         """graph=True: the learner updates of a step run as one CUDA-graph replay (GraphedUpdates).
         fused_input=True: K3 writes the learner's normalised f32 obs / next_obs directly
         (a0_rb_gather_f32) instead of u8 frames that torch then casts, divides and splits
@@ -92,11 +94,15 @@ class Trainer:
         (BaseLearner(amp_dtype=)).  Not the reference's arithmetic, so outside the parity contract.  C51, batch 512,
         graphed: 2.61 ms per update in fp32, 2.33 with bf16, 1.79 with bf16 + channels-last.
         global_is_max (with process_group): the IS weights of every draw are normalised by the maximum over the
-        GLOBAL batch of all ranks (one all-reduce(MAX) of learner_steps floats per draw) instead of per shard."""
+        GLOBAL batch of all ranks (one all-reduce(MAX) of learner_steps floats per draw) instead of per shard.
+        replacement=False: every batch holds B distinct records, with the law of the reference's
+        torch.multinomial(priority[:top], B, replacement=False) (replay.py:41-43; ReplayDataset.sample), eagerly and
+        in the graphed updates."""
         self.pg = process_group
         self.global_is_max = bool(global_is_max) and process_group is not None
         self.cfg = cfg
         self.sampler_seed = sampler_seed
+        self.replacement = bool(replacement)
         self.amp = bool(amp)
         self.obs_dtype = torch.bfloat16 if self.amp else None
         self.normalized = NORM_RECIP if (fused_input or self.amp) else None
@@ -123,10 +129,12 @@ class Trainer:
         if self.graph:
             if self._graphed is None or self._graphed.L != L:
                 self._graphed = GraphedUpdates(self.learner, self.replay, B, L, normalized=self.normalized,
-                                               sampler_seed=self.sampler_seed, obs_dtype=self.obs_dtype)
+                                               sampler_seed=self.sampler_seed, obs_dtype=self.obs_dtype,
+                                               replacement=self.replacement)
             return self._graphed.run()
         out = []
-        drawn = self.replay.sample(B, k_batches=L, normalized=self.normalized, seed=self.sampler_seed, obs_dtype=self.obs_dtype)
+        drawn = self.replay.sample(B, k_batches=L, normalized=self.normalized, seed=self.sampler_seed, obs_dtype=self.obs_dtype,
+                                   replacement=self.replacement)
         if self.global_is_max and self.replay.prioritize:
             drawn = drawn._replace(weights=self.replay.global_is_weights(drawn.priorities, B, self.pg))
         for b in split_batches(drawn, B):

@@ -347,6 +347,20 @@ int a0_pt_sample_rng(a0_replay_t* h, uint64_t seed, int64_t call, int32_t total,
                      float* prio_out, float* weight_out, float* u_out, a0_stream_t stream);
 int a0_pt_rng_seek(a0_replay_t* h, uint64_t call, a0_stream_t stream);
 
+/* Batches WITHOUT replacement (K2a-unique): the law of the reference's torch.multinomial(priority[:top], B,
+ * replacement=False) (agent0/deepq/replay.py:41-43), no record twice in a batch.  A batch is the first B
+ * distinct records of a stream of descents; later rounds descend with the records already taken masked out.
+ * Candidate j of batch k in call c under `seed` uses u = ((x0 >> 5) * 2^26 + (x1 >> 6)) * 2^-53 from
+ * Philox4x32-10(counter {j, 0x80000000 | k, c_lo, c_hi}, key {seed_lo, seed_hi}); the arithmetic is defined by
+ * oracle/sample_unique.py.  Rows are in draw order.  call, top (< 0: device-resident values), uniform and the
+ * IS weights as a0_pt_sample_rng; batch <= 1024.  stats_out (optional, dev i32 [total / batch][2]) receives
+ * {rounds, candidates drawn} per batch.  A batch with fewer than `batch` records of positive priority fills
+ * its remaining rows with its first record and sets device fault code 2, which the next call on the handle
+ * that checks faults (this one included) reports as A0_EFAULT.                                           */
+int a0_pt_sample_unique(a0_replay_t* h, uint64_t seed, int64_t call, int32_t total, int32_t batch,
+                        float top, float beta, float sum_offset, int32_t uniform, int64_t* idx_out,
+                        float* prio_out, float* weight_out, int32_t* stats_out, a0_stream_t stream);
+
 /* ---- K3: fused gather ---------------------------------------------------------------------------------
  * For each sampled record position: walk n_step-1 successor links, rebuild the two 4-frame stacks
  * (each distinct frame is read from HBM once and written to every place it appears), and compute
