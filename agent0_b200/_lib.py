@@ -17,6 +17,8 @@ A0_MAX_ACTIONS = 32
 A0_MAX_QUANTILES = 256
 PTR_FRAMES, PTR_REC_SLOTS, PTR_REC_INFO, PTR_TREE, PTR_MAX_P = range(5)
 OPT_PDL = 1          # include/agent0_b200.h: A0_OPT_PDL (mask of kernel classes launched programmatically; bit 0 = K4)
+K2B_PLAN_MAX = 1024  # include/agent0_b200.h: A0_K2B_PLAN_MAX (largest index count of a0_pt_update_plan / _apply)
+K2B_PLAN_BYTES = 90176  # A0_K2B_PLAN_BYTES (the plan buffer)
 
 _vp, _i32, _i64, _f32, _f64 = C.c_void_p, C.c_int32, C.c_int64, C.c_float, C.c_double
 
@@ -75,6 +77,8 @@ SIGNATURES = {
     "a0_pt_update": (_i32, [_vp, _vp, _vp, _i32, _f32, _f32, _vp]),
     "a0_pt_update_report": (_i32, [_vp, _vp, _vp, _i32, _f32, _f32, _vp, _vp, _vp]),
     "a0_pt_update_overlapped": (_i32, [_vp, _vp, _vp, _i32, _f32, _f32, _vp, _vp, _vp]),
+    "a0_pt_update_plan": (_i32, [_vp, _vp, _i32, _vp, _vp]),
+    "a0_pt_update_apply": (_i32, [_vp, _vp, _vp, _i32, _f32, _f32, _vp, _vp, _vp, _vp]),
     "a0_host_map": (_i32, [_vp, C.POINTER(_vp)]),
     "a0_pt_set": (_i32, [_vp, _vp, _vp, _i32, _vp]),
     "a0_rb_set_dynamic": (_i32, [_vp, _f32, _f32, _f32, _vp]),

@@ -1652,6 +1652,184 @@ a0_k2b_chunks(float* __restrict__ tree, int64_t P, int32_t D, int64_t N, const i
   if (tid == 0) A0_TEND(5);
 }
 
+// ------------------------------------------------------------------------------------------------
+// K2b in two halves, for the end of a training step (a0_pt_update_plan + a0_pt_update_apply).
+// Everything the write-back needs but the losses is known once the draw has run: the positions, the
+// duplicate winners, the paths and the values of the off-path siblings (nothing else writes the tree
+// during a step).  a0_k2b_plan works that out in one CTA off the critical path; a0_k2b_apply runs under
+// the step's last K4, reads the plan before griddepcontrol.wait and after it only reads the losses, forms
+// the leaves and climbs.  The climb is short arithmetic; in one CTA it is bound by issuing the ~5 800
+// scattered node stores of 640 paths on 1 M leaves from one SM (device timeline: 5 100 cycles).  So each of
+// K2Q_APPLY_CTAS CTAs runs the whole apply and stores only its share of the nodes (slots d with
+// d % K2Q_APPLY_CTAS == cta, and a slice of the dense top): the CTAs need nothing from each other, so there
+// is no fence and no grid ticket.
+//
+// The tree splits at level t = min(D, 12): the 2^t level-t nodes are the inputs of a dense top (as in
+// a0_k2b_chunks, two block barriers), the s = D - t levels below are climbed path by path.  Slot d holds
+// the d-th distinct valid leaf in ascending order.  Paths d-1 and d of one level-t subtree meet at height
+// lca = bit length of (p[d-1] ^ p[d]); slot d owns its path up to height top = lca - 1 and hands that value
+// to the slot r that owns the left child there (the last slot before d whose own path joins above that
+// height) -- r's right neighbour at that level is on a path, every other neighbour is an off-path sibling
+// the plan has read.  The first slot of a subtree owns its path up to level t.  Hand-overs inside a warp
+// need a warp barrier; the plan marks the heights where one crosses warps (xmask), and only those take a
+// block barrier.  Every node is fl32(left + right) of its children: the tree a0_pt_update writes, bit for bit.
+// ------------------------------------------------------------------------------------------------
+constexpr int K2Q_THREADS = A0_K2B_PLAN_MAX;                  // indices (and so distinct leaves) of one planned update
+constexpr int K2Q_TOP = 12;                                   // dense top from up to 4096 level-t nodes
+constexpr int K2Q_SMAX = 16;                                  // levels climbed below it: trees of up to 2^28 leaves
+struct A0K2bPlan {
+  int32_t nd, s, xmask, pad_[13];
+  int32_t pos[K2Q_THREADS];                                  // distinct valid leaves, ascending
+  int32_t k[K2Q_THREADS];                                    // each one's winning index (the highest k of its duplicates)
+  float old[K2Q_THREADS];                                    // the leaf before the update (0: evicted, stays)
+  int32_t top[K2Q_THREADS];                                  // height up to which the slot owns its path
+  int32_t recv[K2Q_THREADS];                                 // slot that receives the value at `top` (top < s)
+  int32_t rmask[K2Q_THREADS];                                // heights at which the slot receives its right child
+  float sib[K2Q_SMAX][K2Q_THREADS];                          // off-path sibling at heights 0 .. top-1
+};
+static_assert(sizeof(A0K2bPlan) == A0_K2B_PLAN_BYTES, "A0_K2B_PLAN_BYTES");
+constexpr int K2Q_ROOT = 1 << 30;                            // lca of a subtree's first slot
+constexpr int K2Q_APPLY_CTAS = 8;                            // power of two
+
+__global__ void __launch_bounds__(K2Q_THREADS)
+a0_k2b_plan(const float* __restrict__ tree, int64_t P, int32_t D, int64_t N, const int64_t* __restrict__ idx, int32_t count,
+            A0K2bPlan* __restrict__ plan) {
+  __shared__ unsigned long long s_key[K2Q_THREADS];
+  __shared__ int s_pos[K2Q_THREADS];
+  __shared__ int s_lca[K2Q_THREADS];
+  __shared__ unsigned s_rmask[K2Q_THREADS];
+  __shared__ int s_warp[32];
+  __shared__ unsigned s_xmask;
+  A0_T0();
+  A0_PDL_PROLOGUE();
+  A0_TMID();
+  const int tid = threadIdx.x;
+  const int s = D - (D < K2Q_TOP ? D : K2Q_TOP);
+  unsigned long long key = ~0ull;                            // (leaf << 10 | k); invalid positions sort last
+  if (tid < count) {
+    const int64_t p = idx[tid];
+    if (p >= 0 && p < N) key = ((unsigned long long)p << 10) | (unsigned)tid;
+  }
+  s_key[tid] = key;
+  s_rmask[tid] = 0u;
+  if (tid == 0) s_xmask = 0u;
+  __syncthreads();
+  a0_ku_bitonic(s_key, K2Q_THREADS);
+  A0_TX(0);
+  key = s_key[tid];
+  const unsigned long long nxt = tid + 1 < K2Q_THREADS ? s_key[tid + 1] : ~0ull;
+  const bool win = key != ~0ull && (nxt == ~0ull || (nxt >> 10) != (key >> 10));     // last of its run: highest k
+  int nd;
+  const int d = a0_ku_scan(win ? 1 : 0, s_warp, &nd);
+  const int p = (int)(key >> 10);
+  if (win) s_pos[d] = p;
+  __syncthreads();
+  int lca = K2Q_ROOT;
+  if (win && d > 0) {
+    const int q = s_pos[d - 1];
+    if ((q >> s) == (p >> s)) lca = 32 - __clz(q ^ p);
+  }
+  if (win) s_lca[d] = lca;
+  __syncthreads();
+  A0_TX(1);
+  if (win) {
+    const int top = lca == K2Q_ROOT ? s : lca - 1;
+    if (lca != K2Q_ROOT) {
+      int r = d - 1;
+      while (s_lca[r] <= top) --r;                           // stops at the subtree's first slot at the latest
+      atomicOr(&s_rmask[r], 1u << top);
+      if ((r >> 5) != (d >> 5)) atomicOr(&s_xmask, 1u << top);
+      plan->recv[d] = r;
+    }
+    const int64_t leaf = P + p;
+    for (int h = 0; h < top; ++h) plan->sib[h][d] = __ldcg(tree + ((leaf >> h) ^ 1));
+    plan->pos[d] = p;
+    plan->k[d] = (int)(key & 1023u);
+    plan->old[d] = __ldcg(tree + leaf);
+    plan->top[d] = top;
+  }
+  __syncthreads();
+  if (win) plan->rmask[d] = (int)s_rmask[d];
+  if (tid == 0) { plan->nd = nd; plan->s = s; plan->xmask = (int)s_xmask; }
+  A0_TX(2);
+  if (tid == 0) A0_TEND(7);
+}
+
+__global__ void __launch_bounds__(K2Q_THREADS)
+a0_k2b_apply(float* __restrict__ tree, int64_t P, int32_t D, int64_t N, const int64_t* __restrict__ idx,
+             const float* __restrict__ vals, int32_t count, float alpha, float eps, float* __restrict__ max_p,
+             const A0K2bPlan* __restrict__ plan, const A0Report rep) {
+  extern __shared__ __align__(16) float a0_k2q_smem[];
+  A0_T0();
+#ifdef A0_TRACE
+  const long long _c0 = clock64();
+#endif
+  const int tid = threadIdx.x, lane = tid & 31, cta = blockIdx.x;
+  const bool mine = (tid & (K2Q_APPLY_CTAS - 1)) == cta;      // this CTA stores slot tid's nodes
+  const int t = D < K2Q_TOP ? D : K2Q_TOP;
+  const int n = 1 << t;
+  float* heap = a0_k2q_smem;                                 // heap[i] = node i of the top, level t in [n, 2n)
+  float* xch = a0_k2q_smem + (2 << K2Q_TOP);                // xch[h * K2Q_THREADS + r]: r's right child at height h
+  // ---- before the wait: the plan, the positions and the level-t nodes (written by launches older than the last K4)
+  const int nd = __ldcg(&plan->nd), s = __ldcg(&plan->s);
+  const unsigned xmask = (unsigned)__ldcg(&plan->xmask);
+  for (int i = tid; i < n; i += K2Q_THREADS) heap[n + i] = __ldcg(tree + n + i);
+  __syncthreads();                                           // the heap is final before the climb overlays its paths
+  const bool live = tid < nd;
+  int p = 0, k = 0, top = -1, recv = 0;
+  unsigned rmask = 0u;
+  float old = 0.0f, sib[K2Q_SMAX];
+  if (live) {
+    p = __ldcg(&plan->pos[tid]); k = __ldcg(&plan->k[tid]); old = __ldcg(&plan->old[tid]);
+    top = __ldcg(&plan->top[tid]); recv = __ldcg(&plan->recv[tid]); rmask = (unsigned)__ldcg(&plan->rmask[tid]);
+  }
+#pragma unroll
+  for (int h = 0; h < K2Q_SMAX; ++h) sib[h] = h < top ? __ldcg(&plan->sib[h][tid]) : 0.0f;
+  const int64_t pos_k = tid < count ? idx[tid] : -1;
+  A0_TX(0);
+  A0_PDL_PROLOGUE();                                         // the last K4 is complete: the losses
+  A0_TMID();
+  A0_TX(1);
+  const float loss_k = tid < count ? __ldcg(vals + tid) : 0.0f;
+  const float loss_w = live ? __ldcg(vals + k) : 0.0f;
+  if (cta == 0) {
+    if (rep.idx && tid < count) { rep.idx[tid] = pos_k; rep.loss[tid] = loss_k; }
+    float mx = pos_k >= 0 && pos_k < N ? fmaxf(0.0f, loss_k) : 0.0f;
+    mx = a0_warp_max(mx);
+    if (lane == 0) a0_atomic_max_pos(max_p, mx);            // max_p = max(max_p, max loss), replay.py:59
+  }
+  const int64_t leaf = P + p;
+  float v = old;
+  if (live && old > 0.0f && a0_loss_ok(loss_w)) {            // evicted since it was sampled / NaN loss: the leaf stays
+    v = a0_priority(loss_w, eps, alpha);
+    if (mine) __stcg(tree + leaf, v);
+  }
+  A0_TX(2);
+#pragma unroll
+  for (int h = 0; h < K2Q_SMAX; ++h) {
+    if (h >= s) break;
+    if (live && top == h && h < s) xch[h * K2Q_THREADS + recv] = v;
+    if ((xmask >> h) & 1u) __syncthreads(); else __syncwarp();
+    if (live && h < top) {
+      const float o = ((rmask >> h) & 1u) ? xch[h * K2Q_THREADS + tid] : sib[h];
+      v = ((p >> h) & 1) ? __fadd_rn(o, v) : __fadd_rn(v, o);
+      if (mine) __stcg(tree + (leaf >> (h + 1)), v);
+    }
+  }
+  if (live && top == s) heap[n + (p >> s)] = v;
+  __syncthreads();
+  A0_TX(3);
+  a0_heap_reduce<K2Q_THREADS>(heap, t);
+  const int share = (n + K2Q_APPLY_CTAS - 1) / K2Q_APPLY_CTAS;
+  for (int i = cta * share + tid; i < n && i < (cta + 1) * share; i += K2Q_THREADS)
+    if (i >= 1) tree[i] = heap[i];
+  A0_TX(4);
+#ifdef A0_TRACE
+  _tx[7] = (unsigned long long)_c0;
+#endif
+  if (tid == 0) A0_TEND(8);
+}
+
 static int g_k2b_chunk_max = -1;   // largest index list the one-launch chunk schedule takes (A0_K2B_CHUNK_MAX)
 static int a0_option_k2b_chunk_max() {
   if (g_k2b_chunk_max < 0) {
@@ -1796,4 +1974,40 @@ extern "C" int a0_pt_set(a0_replay_t* h, const int64_t* idx, const float* value,
   A0_REQUIRE(h != nullptr && count >= 0, "a0_pt_set: bad handle or count");
   A0_REQUIRE(count == 0 || (idx && value), "a0_pt_set: NULL argument");
   return a0_launch_update(h, idx, nullptr, value, count, 2, 1.0f, 0.0f, stream);
+}
+
+// The planned write-back (see a0_k2b_plan): idx must not change, and nothing may write the tree, between the two calls.
+extern "C" int a0_pt_update_plan(a0_replay_t* h, const int64_t* idx, int32_t count, void* plan, a0_stream_t stream) {
+  A0_REQUIRE(h != nullptr && count >= 0 && count <= A0_K2B_PLAN_MAX, "a0_pt_update_plan: bad handle or count (at most %d)",
+             A0_K2B_PLAN_MAX);
+  A0_REQUIRE(idx && plan, "a0_pt_update_plan: NULL argument");
+  A0_REQUIRE(h->D >= 1 && h->D <= K2Q_TOP + K2Q_SMAX, "a0_pt_update_plan: tree depth %d outside 1..%d", (int)h->D,
+             K2Q_TOP + K2Q_SMAX);
+  { int frc = a0_check_fault(h, "a0_pt_update_plan"); if (frc) return frc; }
+  A0DeviceGuard guard(h->device);
+  A0_LAUNCH(a0_k2b_plan, 1, K2Q_THREADS, 0, (cudaStream_t)stream, 1, A0_PDL_K2, (const float*)h->tree, h->P, h->D, h->N, idx,
+            count, (A0K2bPlan*)plan);
+  return A0_OK;
+}
+extern "C" int a0_pt_update_apply(a0_replay_t* h, const int64_t* idx, const float* loss, int32_t count, float alpha, float eps,
+                                  const void* plan, int64_t* idx_report, float* loss_report, a0_stream_t stream) {
+  A0_REQUIRE(h != nullptr && count >= 0 && count <= A0_K2B_PLAN_MAX, "a0_pt_update_apply: bad handle or count (at most %d)",
+             A0_K2B_PLAN_MAX);
+  A0_REQUIRE(idx && loss && plan, "a0_pt_update_apply: NULL argument");
+  A0_REQUIRE((idx_report == nullptr) == (loss_report == nullptr), "a0_pt_update_apply: give both report buffers or none");
+  A0_REQUIRE(h->D >= 1 && h->D <= K2Q_TOP + K2Q_SMAX, "a0_pt_update_apply: tree depth %d outside 1..%d", (int)h->D,
+             K2Q_TOP + K2Q_SMAX);
+  { int frc = a0_check_fault(h, "a0_pt_update_apply"); if (frc) return frc; }
+  A0DeviceGuard guard(h->device);
+  const int s = h->D - (h->D < K2Q_TOP ? h->D : K2Q_TOP);
+  const size_t smem = ((size_t)(2 << K2Q_TOP) + (size_t)s * K2Q_THREADS) * sizeof(float);
+  static thread_local bool attr[64] = {false};
+  if (h->device < 64 && !attr[h->device]) {
+    A0_CUDA(cudaFuncSetAttribute(a0_k2b_apply, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 (int)(((size_t)(2 << K2Q_TOP) + (size_t)K2Q_SMAX * K2Q_THREADS) * sizeof(float))));
+    attr[h->device] = true;
+  }
+  A0_LAUNCH(a0_k2b_apply, K2Q_APPLY_CTAS, K2Q_THREADS, smem, (cudaStream_t)stream, 1, A0_PDL_FORCE, h->tree, h->P, h->D, h->N, idx, loss, count,
+            alpha, eps, h->max_p, (const A0K2bPlan*)plan, A0Report{idx_report, loss_report});
+  return A0_OK;
 }

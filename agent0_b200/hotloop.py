@@ -154,6 +154,15 @@ class ReplayTargetLoop:
             # batch-512 step's K4 launches on pace with the waves at 216 us (no limit: 238, 320: 233, 480: 223)
             self.window = (400 if per_batch else 128) if gather_window == "auto" else int(gather_window or 0)
         n_gather = len(self.waves) if self.waves else 1
+        # the waved step writes its priorities back in two halves when the count fits one CTA: a0_pt_update_plan on the side
+        # stream after the last wave, and a0_pt_update_apply under the last K4 (a0_pt_update_overlapped's chunk
+        # schedule otherwise).  The plan starts when the last wave is complete; the K4 that waits for it comes at least one
+        # link after the one that waits for that wave, and 4 links before the end.  (launches_per_step leaves the plan out.)
+        self._plan_join = max(self.waves[-1][0] + 1, self.L - 4) if self.waves else self.L
+        self._use_plan = self._use_plan_default = self.per and self.early_update and T <= _lib.K2B_PLAN_MAX and self._plan_join < self.L
+        if self._use_plan:
+            self.plan = torch.empty(_lib.K2B_PLAN_BYTES, dtype=torch.uint8, device=dev)
+            self.plan_ev = torch.cuda.Event()
         self.launches_per_step = 1 + n_gather + self.L + (1 if self.per else 0)     # our kernels (uniform_ is torch's)
         self._k4 = None
         self._k4_all = None
@@ -202,9 +211,10 @@ class ReplayTargetLoop:
     def _wave_plan(self, spec):
         return wave_plan(self.L, self.B, self.rp.F, spec)
 
-    def sample_gather_waves(self):
+    def sample_gather_waves(self, plan=False):
         """K2a + the gather in waves on the side stream (a0_rb_sample_mail, a0_rb_gather_mail per wave, an event after
-        each): same outputs as sample_gather().  The caller's stream joins wave by wave (``_wait_wave``)."""
+        each): same outputs as sample_gather().  The caller's stream joins wave by wave (``_wait_wave``).  plan: then the
+        first half of the write-back (a0_pt_update_plan) on the same stream, and ``plan_ev`` after it."""
         rp, lib = self.rp, self.lib
         main = torch.cuda.current_stream(self.dev)
         self.side.wait_stream(main)           # everything before this step (the previous write-back, the ingest)
@@ -218,6 +228,9 @@ class ReplayTargetLoop:
                                                  self.r64.data_ptr(), self.r32.data_ptr(), self.d8.data_ptr(), self.d32.data_ptr(),
                                                  self.boot.data_ptr(), st), "a0_rb_gather_mail")
                 self.wave_ev[j].record(self.side)
+            if plan:
+                _lib.check(lib.a0_pt_update_plan(rp.h, self.idx.data_ptr(), self.total, self.plan.data_ptr(), st), "a0_pt_update_plan")
+                self.plan_ev.record(self.side)
 
     def _wait_wave(self, j):
         torch.cuda.current_stream(self.dev).wait_event(self.wave_ev[j])
@@ -313,9 +326,17 @@ class ReplayTargetLoop:
             self.report[slot][0].copy_(self.idx, non_blocking=True)
             self.report[slot][1].copy_(self.loss, non_blocking=True)
 
+    def _apply(self, slot=None):
+        """Second half of the planned write-back (a0_pt_update_apply), launched right after the step's last K4."""
+        ri, rl = self._report_dev[slot] if slot is not None else (None, None)
+        _lib.check(self.lib.a0_pt_update_apply(self.rp.h, self.idx.data_ptr(), self.loss.data_ptr(), self.total, self.alpha,
+                                               self.eps, self.plan.data_ptr(), ri, rl, self._st()), "a0_pt_update_apply")
+
     # ------------------------------------------------------------------ whole steps
-    def _targets_and_update(self, fused_k4, slot, update=True):
-        """The K4 launches of a step whose gather runs in waves (each waits for the wave that holds its batch), then K2b."""
+    def _targets_and_update(self, fused_k4, slot, update=True, planned=False):
+        """The K4 launches of a step whose gather runs in waves (each waits for the wave that holds its batch), then K2b.
+        planned: the K4 ``_plan_join`` also waits for the plan (it executes griddepcontrol.wait before anything else, so the
+        plan is complete when the apply, launched under the last K4, starts), and the apply is the write-back."""
         if fused_k4:
             for j in range(len(self.waves)):
                 self._wait_wave(j)
@@ -325,14 +346,18 @@ class ReplayTargetLoop:
             return
         for k in range(self.L):
             j = self._join.get(k)
-            if j is None or self.pdl_at_joins:
+            join_plan = planned and k == self._plan_join
+            if join_plan:
+                torch.cuda.current_stream(self.dev).wait_event(self.plan_ev)
+            if (j is None and not join_plan) or self.pdl_at_joins:
                 if j is not None:
                     self._wait_wave(j)
                 self.target_loss(k)
             else:
-                # the K4 that joins wave j has TWO predecessors (the previous K4, the wave): launched without the
+                # the K4 that joins wave j (or the plan) has more than one predecessor: launched without the
                 # programmatic attribute unless pdl_at_joins
-                self._wait_wave(j)
+                if j is not None:
+                    self._wait_wave(j)
                 mask = C.c_int64(0)
                 _lib.check(self.lib.a0_get_option(_lib.OPT_PDL, C.byref(mask)), "a0_get_option")
                 self.lib.a0_set_option(_lib.OPT_PDL, mask.value & ~1)
@@ -340,7 +365,9 @@ class ReplayTargetLoop:
                     self.target_loss(k)
                 finally:
                     self.lib.a0_set_option(_lib.OPT_PDL, mask.value)
-        if update:
+        if planned:
+            self._apply(slot)
+        elif update:
             self.update(slot, after_k4=True)
 
     def step(self, fused_k4=False, slot=None, update=True):
@@ -348,14 +375,15 @@ class ReplayTargetLoop:
         if self.rng_seed is None:
             self.u.uniform_()
         if self.waves and (self.waves_when_eager or torch.cuda.is_current_stream_capturing()):
-            self.sample_gather_waves()
+            planned = update and self._use_plan and not fused_k4
+            self.sample_gather_waves(plan=planned)
             if self.fast is None:
-                self._targets_and_update(fused_k4, slot, update)
+                self._targets_and_update(fused_k4, slot, update, planned)
                 return
             main = torch.cuda.current_stream(self.dev)
             self.fast.wait_stream(main)           # the network outputs, the previous step
             with torch.cuda.stream(self.fast):
-                self._targets_and_update(fused_k4, slot, update)
+                self._targets_and_update(fused_k4, slot, update, planned)
             main.wait_stream(self.fast)
             return
         if self.overlap_sg:

@@ -315,6 +315,21 @@ int a0_pt_update_report(a0_replay_t* h, const int64_t* idx /* dev */, const floa
 int a0_pt_update_overlapped(a0_replay_t* h, const int64_t* idx /* dev */, const float* loss /* dev */,
                             int32_t count, float alpha, float eps, int64_t* idx_report, float* loss_report,
                             a0_stream_t stream);
+/* The write-back of a Trainer.step in two halves, for counts up to A0_K2B_PLAN_MAX.  a0_pt_update_plan reads idx and
+ * the tree (one CTA; run it any time after the draw) and writes into `plan` (A0_K2B_PLAN_BYTES of device memory owned
+ * by the caller) the distinct valid leaves with their winning index (the highest k of each leaf's duplicates), the old
+ * leaves, the off-path siblings of every path and where the paths meet.  a0_pt_update_apply (8 CTAs) is launched
+ * programmatically under its predecessor on `stream`, like a0_pt_update_overlapped: it reads the plan before it waits
+ * and after the wait only the losses.  THE CALLER GUARANTEES that idx and the tree do not change between the two
+ * calls, and that the plan and idx were written by launches older than the one immediately preceding the apply.
+ * Same tree, same max_p, same reports as a0_pt_update_report / a0_pt_update.  Trees of 2 .. 2^28 leaves.        */
+#define A0_K2B_PLAN_MAX 1024
+#define A0_K2B_PLAN_BYTES 90176
+int a0_pt_update_plan(a0_replay_t* h, const int64_t* idx /* dev */, int32_t count, void* plan /* dev */,
+                      a0_stream_t stream);
+int a0_pt_update_apply(a0_replay_t* h, const int64_t* idx /* dev */, const float* loss /* dev */, int32_t count,
+                       float alpha, float eps, const void* plan /* dev */, int64_t* idx_report, float* loss_report,
+                       a0_stream_t stream);
 /* Device-visible alias of page-locked host memory (cudaHostAlloc / cudaHostRegister with mapping,
  * torch's pin_memory); fails for pageable memory.  Not a stream operation: call it once per
  * buffer, outside CUDA-graph capture.                                                          */

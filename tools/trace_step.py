@@ -71,10 +71,10 @@ t0, t1, t2, kid = t0[sel], t1[sel], t2[sel], kid[sel]
 xs = rec[sel][:, 4:12]
 base = t0.min()
 rows = []
-names = {2: "K2a", 3: "K3", 4: "K4", 5: "K2b"}
+names = {2: "K2a", 3: "K3", 4: "K4", 5: "K2b", 7: "K2b plan", 8: "K2b apply"}
 if (kid == 4).any():
     t2 = np.where(kid == 4, t0, t2)          # K4's t2 holds cycles, not time
-for k in (2, 3, 5):
+for k in (2, 3, 5, 7, 8):
     m = kid == k
     if m.any():
         rows.append((names[k], int(m.sum()), (t0[m].min() - base) / 1e3, (np.median(t2[m]) - base) / 1e3, (t2[m].max() - base) / 1e3,
@@ -132,6 +132,16 @@ if m5.any():
     pts = [c0] + [x5[i] for i in range(7)]
     print("K2b (one CTA) phases, SM cycles: " + " | ".join(f"{l} {int(pts[i + 1] - pts[i])}" for i, l in enumerate(lab5)
                                                                  if pts[i + 1] and pts[i]) + f" | total {int(x5[6] - c0)}")
+m8 = kid == 8
+if m8.any():
+    x8 = xs[m8][0]
+    lab8 = ["plan + leaves read (before the wait)", "wait", "losses + report + leaves", "climb", "dense top"]
+    pts = [x8[7]] + [x8[i] for i in range(5)]
+    print("K2b apply, phases of one of its CTAs, SM cycles: " + " | ".join(f"{l} {int(pts[i + 1] - pts[i])}" for i, l in enumerate(lab8))
+          + f" | after the wait {int(x8[4] - x8[1])}")
+    m4 = kid == 4
+    if m4.any():
+        print(f"end of the last K4 -> end of the apply: {(t1[m8].max() - t1[m4].max()) / 1e3:.2f} us")
 print(f"B={B} L={L} overlap={overlap} gather waves (batches)={[w[1] for w in hp.waves] if hp.waves else None} records={n}; times in us from the first traced entry; globaltimer tick = "
       f"{int(np.min(np.diff(np.unique(np.concatenate([t0, t1])))))} ns")
 print(f"{'kernel':8s} {'ctas':>5s} {'first entry':>12s} {'median ready':>13s} {'last ready':>11s} {'last exit':>10s}")
