@@ -353,6 +353,8 @@ __device__ __forceinline__ float a0_priority(float loss, float eps, float alpha)
 // A priority update with a loss that is NaN, infinite or negative leaves the old leaf in place: the
 // reference skips the whole update when the loss is NaN (agent.py:150-152, SURVEY Q15); inside a captured
 // CUDA graph there is no host guard, and one NaN leaf would poison every ancestor up to the root.
+// The write-back's max_p takes only the losses that pass this test, filtered one by one before any reduction:
+// a warp maximum that met an infinite loss would otherwise be dropped whole, finite losses beside it included.
 __device__ __forceinline__ bool a0_loss_ok(float x) { return x >= 0.0f && x < __int_as_float(0x7f800000); }
 __device__ __forceinline__ void a0_atomic_max_pos(float* addr, float v) {
   // valid for non-negative floats: the int ordering equals the float ordering

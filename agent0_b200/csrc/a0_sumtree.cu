@@ -799,7 +799,7 @@ a0_k2b_write(float* __restrict__ tree, int64_t P, int32_t chunk_log, int64_t N, 
     if (rep.idx) { rep.idx[k] = pos; rep.loss[k] = vals[k]; }
     if (pos < 0 || pos >= N) continue;
     atomicMax(winner + pos, k);
-    if (mode == 0) local_max = fmaxf(local_max, vals[k]);
+    if (mode == 0 && a0_loss_ok(vals[k])) local_max = fmaxf(local_max, vals[k]);
   }
   __syncthreads();
   for (int k = tid; k < count; k += K2B_THREADS) {          // write
@@ -1090,7 +1090,7 @@ a0_paths_body(float* __restrict__ tree, int64_t P, int32_t D, int64_t N, const i
   if (mode == 0) {
     float mx = 0.0f;
 #pragma unroll
-    for (int s = 0; s < K2P_PER_THREAD; ++s) mx = fmaxf(mx, pos[s] >= 0 ? val[s] : 0.0f);
+    for (int s = 0; s < K2P_PER_THREAD; ++s) mx = fmaxf(mx, pos[s] >= 0 && a0_loss_ok(val[s]) ? val[s] : 0.0f);
     mx = a0_warp_max(mx);
     if ((threadIdx.x & 31) == 0) a0_atomic_max_pos(max_p, mx);   // max_p = max(max_p, max loss), replay.py:59
   }
@@ -1278,7 +1278,7 @@ a0_small_body(float* __restrict__ tree, int64_t P, int32_t D, int64_t N, const i
       if (s < S) sib[s] = a0_ld_now(tree + ((leaf >> s) ^ 1u));
   }
   if (mode == 0) {
-    const float mx = a0_warp_max(valid ? val : 0.0f);
+    const float mx = a0_warp_max(valid && a0_loss_ok(val) ? val : 0.0f);
     if ((tid & 31) == 0) a0_atomic_max_pos(max_p, mx);      // max_p = max(max_p, max loss), replay.py:59
   }
   __syncthreads();                                          // the map is empty
@@ -1575,7 +1575,7 @@ a0_k2b_chunks(float* __restrict__ tree, int64_t P, int32_t D, int64_t N, const i
       bool set;
       const int64_t p = position(k, set);
       if (rep.idx) { rep.idx[k] = p; rep.loss[k] = vals[k]; }
-      if (mode == 0 && p >= 0 && p < N) mx = fmaxf(mx, vals[k]);
+      if (mode == 0 && p >= 0 && p < N && a0_loss_ok(vals[k])) mx = fmaxf(mx, vals[k]);
     }
     if (mode == 0) {
       mx = a0_warp_max(mx);
@@ -1792,12 +1792,7 @@ a0_k2b_apply(float* __restrict__ tree, int64_t P, int32_t D, int64_t N, const in
   A0_TX(1);
   const float loss_k = tid < count ? __ldcg(vals + tid) : 0.0f;
   const float loss_w = live ? __ldcg(vals + k) : 0.0f;
-  if (cta == 0) {
-    if (rep.idx && tid < count) { rep.idx[tid] = pos_k; rep.loss[tid] = loss_k; }
-    float mx = pos_k >= 0 && pos_k < N ? fmaxf(0.0f, loss_k) : 0.0f;
-    mx = a0_warp_max(mx);
-    if (lane == 0) a0_atomic_max_pos(max_p, mx);            // max_p = max(max_p, max loss), replay.py:59
-  }
+  if (cta == 0 && rep.idx && tid < count) { rep.idx[tid] = pos_k; rep.loss[tid] = loss_k; }
   const int64_t leaf = P + p;
   float v = old;
   if (live && old > 0.0f && a0_loss_ok(loss_w)) {            // evicted since it was sampled / NaN loss: the leaf stays
@@ -1823,6 +1818,11 @@ a0_k2b_apply(float* __restrict__ tree, int64_t P, int32_t D, int64_t N, const in
   const int share = (n + K2Q_APPLY_CTAS - 1) / K2Q_APPLY_CTAS;
   for (int i = cta * share + tid; i < n && i < (cta + 1) * share; i += K2Q_THREADS)
     if (i >= 1) tree[i] = heap[i];
+  if (cta == 0) {                                            // off the climb's path: nothing here waits for max_p
+    float mx = pos_k >= 0 && pos_k < N && a0_loss_ok(loss_k) ? loss_k : 0.0f;
+    mx = a0_warp_max(mx);
+    if (lane == 0) a0_atomic_max_pos(max_p, mx);            // max_p = max(max_p, max loss), replay.py:59
+  }
   A0_TX(4);
 #ifdef A0_TRACE
   _tx[7] = (unsigned long long)_c0;

@@ -73,6 +73,64 @@ class SumTree:
             idx[b] = self.descend(f32(t))
         return idx, self.nodes[self.P + idx].copy()
 
+    # ---- bulk forms: the same float32 operations as set / sample_stratified, one numpy operation per tree level,
+    #      so that trees of up to 2^24 leaves can be built and descended in well under a second
+    def build(self, leaves):
+        """set(arange(len(leaves)), leaves) on an empty tree: every node recomputed, level by level."""
+        leaves = np.asarray(leaves, dtype=f32)
+        self.nodes[:] = 0
+        self.nodes[self.P:self.P + leaves.size] = leaves
+        n = self.P // 2
+        while n >= 1:
+            self.nodes[n:2 * n] = self.nodes[2 * n:4 * n:2] + self.nodes[2 * n + 1:4 * n:2]
+            n //= 2
+
+    def _recompute(self, leaf_pos):
+        level = np.unique((self.P + np.asarray(leaf_pos, dtype=np.int64)) >> 1)
+        while level.size:
+            self.nodes[level] = self.nodes[2 * level] + self.nodes[2 * level + 1]
+            level = np.unique(level[level > 1] >> 1)
+
+    def update(self, idx, loss, eps, alpha, max_p):
+        """The priority write-back (a0_pt_update and every K2b schedule); returns the new max_p.
+          * positions outside [0, capacity) are ignored;
+          * of several entries for one position the last one wins;
+          * a winner whose loss is NaN, infinite or negative leaves the old leaf (no fall-back to an earlier entry);
+          * a leaf that is 0 (evicted since it was sampled) stays 0;
+          * max_p = max(max_p, every finite loss at a position in range) (replay.py:59)."""
+        idx = np.asarray(idx, dtype=np.int64)
+        loss = np.asarray(loss, dtype=f32)
+        ok = (idx >= 0) & (idx < self.capacity)
+        finite = ok & np.isfinite(loss)
+        if finite.any():
+            max_p = max(f32(max_p), f32(loss[finite].max()))
+        pos, k = idx[ok], np.flatnonzero(ok)
+        if pos.size == 0:
+            return f32(max_p)
+        rev_first = np.unique(pos[::-1], return_index=True)[1]
+        win = k[pos.size - 1 - rev_first]                        # the last entry of every distinct position
+        p, x = idx[win], loss[win]
+        good = (x >= 0) & np.isfinite(x) & (self.nodes[self.P + p] > 0)
+        self.nodes[self.P + p[good]] = new_priority(x[good], eps, alpha)
+        self._recompute(p)
+        return f32(max_p)
+
+    def sample(self, u, batch):
+        """sample_stratified over consecutive batches of ``batch`` uniforms (draw g is stratum g % batch),
+        all draws descending together: t = fl32(fl32(fl32(b + u) / B) * root); go left iff t < L or not (R > 0);
+        going right, t = fl32(t - L)."""
+        u = np.asarray(u, dtype=f32)
+        b = (np.arange(u.size) % batch).astype(f32)
+        t = ((b + u) / f32(batch)) * self.root
+        node = np.ones(u.size, dtype=np.int64)
+        for _ in range(self.P.bit_length() - 1):
+            L, R = self.nodes[2 * node], self.nodes[2 * node + 1]
+            right = ~((t < L) | ~(R > 0))
+            t = np.where(right, t - L, t).astype(f32)
+            node = 2 * node + right
+        idx = node - self.P
+        return idx, self.nodes[node].copy()
+
 
 def new_priority(loss, eps, alpha):
     """replay.py:56-58: (loss+eps)^alpha; sqrt when alpha == 0.5 as torch's CPU pow does."""

@@ -1,12 +1,14 @@
 """Parity at BASELINE.json's full sizes (2 M-transition shard, 20 x 512 draws) through
-size-independent properties -- the oracle's Python loops cannot run there, so the checker is an
-independent torch formulation over the raw device state (frames/slots/info/tree views):
+size-independent properties -- the oracle's scalar Python loops cannot run there, so besides the vectorised
+sum-tree oracle the checker is an independent torch formulation over the raw device state (frames/slots/info/tree
+views):
 
   * gather == frames[slots] rebuilt with torch indexing along the record links (bit-exact),
     n-step returns in float64 with the reference's operation order (bit-exact);
   * every sum-tree node == fl32(left + right); root == what a pairwise fp32 reduction gives;
   * every sampled index is sampleable, its priority is its leaf, the stratified target of draw b
-    falls inside the index's prefix interval (float64 check with fp32 slack);
+    falls inside the index's prefix interval (float64 check with fp32 slack), and the draw is the vectorised
+    oracle's descent of the host copy of the tree, bit for bit;
   * IS weights follow trainer.py:91-94 and max to 1;
   * update_priority is idempotent and order independent; checksum of gathered frames equals the
     checksum of the source frames."""
@@ -17,6 +19,7 @@ import torch
 from agent0_b200 import _lib
 from agent0_b200.config import make_config
 from agent0_b200.synth import fill_shard_synthetic
+from oracle.sumtree import SumTree, philox_uniform
 
 pytestmark = pytest.mark.gpu
 N, E, n, B, K = 2_000_000, 16, 3, 512, 20
@@ -78,6 +81,11 @@ def test_sample_gather_properties_20x512(shard):
     lo_, hi_ = cum[idx] - leaves[idx].double(), cum[idx]
     slack = 2e-6 * root
     assert bool(((tgt >= lo_ - slack) & (tgt <= hi_ + slack)).all())
+    ref = SumTree(N)
+    ref.build(leaves.cpu().numpy())
+    assert np.array_equal(rp.tree.cpu().numpy().view(np.int32), ref.nodes.view(np.int32))
+    ref_idx, ref_prio = ref.sample(u.cpu().numpy(), B)
+    assert np.array_equal(idx.cpu().numpy(), ref_idx) and np.array_equal(b.priorities.cpu().numpy(), ref_prio)
     # IS weights (trainer.py:91-94) per batch
     w = (rp.top * (b.priorities / rp.tree[1])).pow(-rp.beta).view(K, B)
     w = (w / (w.max(dim=1, keepdim=True)[0] + 1e-8)).view(-1)
@@ -231,6 +239,8 @@ def test_waved_graphed_step_at_full_size(shard):
     gr = torch.cuda.CUDAGraph()
     with torch.cuda.graph(gr):
         lb.step(update=False)
+    ref = SumTree(N)
+    ref.build(rp.priority.leaves().cpu().numpy())
     for call in (700, 701):
         rp.rng_seek(call)
         la.step(update=False)
@@ -240,6 +250,8 @@ def test_waved_graphed_step_at_full_size(shard):
         torch.cuda.synchronize()
         for f in ("idx", "prio", "w", "frames", "act", "r64", "r32", "d8", "d32", "boot", "loss", "grad"):
             assert torch.equal(getattr(la, f), getattr(lb, f)), f
+        ref_idx, ref_prio = ref.sample(philox_uniform(33, call, T), B)         # the mailbox sampler at depth 21
+        assert np.array_equal(lb.idx.cpu().numpy(), ref_idx) and np.array_equal(lb.prio.cpu().numpy(), ref_prio)
     p0 = lb.idx
     p2 = info[info[p0, 3].long(), 3].long()
     sl = torch.cat((slots[p0, :4], slots[p2, 4:]), dim=1).long()

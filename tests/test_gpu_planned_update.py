@@ -1,5 +1,5 @@
 """The planned priority write-back (a0_pt_update_plan + a0_pt_update_apply) against a0_pt_update_report on twin shards:
-every node of the tree, max_p and the report buffers must be identical -- over tree depths 1 to 22, index counts up to
+every node of the tree, max_p and the report buffers must be identical -- over tree depths 1 to 24, index counts up to
 A0_K2B_PLAN_MAX, duplicates, bad losses, evicted leaves, out-of-range positions and clustered paths.  Then the captured
 flagship loop (which takes the planned path at 640 indices) against the same loop forced onto the chunk schedule."""
 import pytest
@@ -59,7 +59,7 @@ def _losses(n, seed, bad=True):
     return loss
 
 
-@pytest.mark.parametrize("D", [1, 3, 11, 12, 17, 20, 22])
+@pytest.mark.parametrize("D", [1, 3, 11, 12, 17, 20, 21, 22, 23, 24])
 @pytest.mark.parametrize("count", [1, 31, 32, 33, 640, CAP])
 def test_plan_apply_equals_pt_update(D, count):
     """Random positions over [-2, P + 2) on a shard of N = P - P/8 records (out-of-range on both sides and between N and

@@ -346,16 +346,16 @@ def test_sampler_own_generator_other_launch_shapes(per, Bn):
             assert np.allclose(w.max(axis=1), 1.0, atol=1e-6)
 
 
-@pytest.mark.parametrize("N", [2, 5, 2048, 4096, 70000, 3_000_000])
+@pytest.mark.parametrize("N", [2, 5, 2048, 4096, 70000, 3_000_000, 1 << 24])
 def test_sumtree_update_paths_all_depths_and_sizes(N):
-    """K2b at tree depths 1, 3, 11, 12, 17 and 22 and at every launch shape: one CTA with the shared-memory
+    """K2b at tree depths 1, 3, 11, 12, 17, 22 and 24 and at every launch shape: one CTA with the shared-memory
     node map (<= 1024 indices), a cluster of up to 8 CTAs climbing the paths, the cluster leaf write + chunk rebuild on all SMs (from 2048 indices
     with >= 4 per chunk), and the one-CTA write + rebuild above 16384 indices -- always the oracle's tree."""
     rp = _replay(N, per=True, **({"frame_capacity": 65536} if N > 1_000_000 else {}))     # 3 M leaves: depth 22, 10 sparse levels
     rng = np.random.RandomState(N)
     ref = SumTree(N)
     pr = (rng.rand(N).astype(np.float32) + 0.1)
-    ref.set(np.arange(N), pr)
+    ref.build(pr)
     for lo in range(0, N, 30000):                      # > 16384 per call: write + rebuild kernels
         hi = min(N, lo + 30000)
         rp.set_priorities(torch.arange(lo, hi), torch.as_tensor(pr[lo:hi]))

@@ -16,7 +16,7 @@ pytestmark = pytest.mark.gpu
 
 
 class RawShard:
-    """A shard handle used only for its sum-tree (16-byte frames, 8 of them): tree depths up to 22 cost no frame ring."""
+    """A shard handle used only for its sum-tree (16-byte frames, 8 of them): tree depths up to 24 cost no frame ring."""
 
     def __init__(self, capacity):
         self.lib = _lib.load()
@@ -88,7 +88,7 @@ def _check_oracle(sh, seed, call, K, B, top, beta=0.4, sum_offset=0.0, uniform=0
     return ri, rs
 
 
-@pytest.mark.parametrize("D,B,K", [(1, 2, 3), (3, 4, 5), (11, 64, 6), (17, 512, 4), (22, 512, 20)])
+@pytest.mark.parametrize("D,B,K", [(1, 2, 3), (3, 4, 5), (11, 64, 6), (17, 512, 4), (22, 512, 20), (24, 512, 20)])
 @pytest.mark.parametrize("kind", ["spread", "peaked", "extreme"])
 def test_bit_exact_against_the_oracle(D, B, K, kind):
     sh = RawShard(1 << D)
