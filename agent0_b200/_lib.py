@@ -20,6 +20,12 @@ OPT_PDL = 1          # include/agent0_b200.h: A0_OPT_PDL (mask of kernel classes
 K2B_PLAN_MAX = 1024  # include/agent0_b200.h: A0_K2B_PLAN_MAX (largest index count of a0_pt_update_plan / _apply)
 K2B_PLAN_BYTES = 90176  # A0_K2B_PLAN_BYTES (the plan buffer)
 
+
+def lz4_stride(frame_bytes):
+    """include/agent0_b200.h: A0_LZ4_STRIDE -- bytes between the groups of a0_lz4_encode's output."""
+    n = 8 * int(frame_bytes)
+    return (n + n // 255 + 20 + 15) // 16 * 16
+
 _vp, _i32, _i64, _f32, _f64 = C.c_void_p, C.c_int32, C.c_int64, C.c_float, C.c_double
 
 
@@ -69,6 +75,12 @@ SIGNATURES = {
     "a0_ex_decode": (_i32, [_vp, _vp, _vp, _i32, _vp, _vp, _vp]),
     "a0_ex_resolve": (_i32, [_vp, _vp, _vp, _i32, _vp, _vp, C.POINTER(_i32)]),
     "a0_ex_last_timing": (_i32, [_vp, _vp]),
+    "a0_lz4_encode": (_i32, [_vp, _i32, _i32, _vp, _vp, _vp, _vp]),
+    "a0_ix_serialize": (_i32, [_vp, _vp, _i64, C.POINTER(_i64)]),
+    "a0_ix_deserialize": (_i32, [_vp, _vp, _i64]),
+    "a0_ckpt_save": (_i32, [_vp, _vp, _vp, C.c_char_p, _vp, _i64, _vp]),
+    "a0_ckpt_load": (_i32, [_vp, _vp, _vp, C.c_char_p, _vp, _i64, C.POINTER(_i64), _vp]),
+    "a0_ckpt_last_timing": (_i32, [_vp]),
     "a0_rb_ingest_plan": (_i32, [_vp, C.POINTER(Plan), _vp, _vp, _i32, _f32, _vp]),
     "a0_rb_ingest_steps": (_i32, [_vp, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _i32, _f32, _vp]),
     "a0_rb_ingest_steps_dyn": (_i32, [_vp, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _i32, _f32, _f32, _i32, _vp]),

@@ -5,6 +5,8 @@
 #include <stdio.h>
 #include <string.h>
 
+#include <vector>
+
 #include "../../include/agent0_b200.h"
 
 // Per-record side data (16 B, one vector load).  Rewards stay float64 because the reference
@@ -269,6 +271,18 @@ int a0_gather_launch_mail(a0_replay* h, const int64_t* idx, long long* mail, int
 constexpr int A0_K3_PROGRESS = 2 * A0_MAX_BATCHES + 40;      // counter[] word: completed draws of the current windowed gather
 int a0_mail_reserve(a0_replay* h, int32_t total, cudaStream_t stream);
 
+// a0_ckpt.cu's access to the other modules' state: the ring index (a0_ingest.cu) and the reference-tuple ingest
+// (a0_extend.cu: the K6a decode of one batch of at most 2048 blobs into its scratch, and the stream tails)
+void a0_ix_clear(a0_index* ix);
+int a0_ex_decode_dev(a0_extend* ex, const uint8_t* blobs, const int64_t* blob_len, int32_t mb, cudaStream_t cs,
+                     const uint8_t** dec, const unsigned long long** hash, const int32_t** status);
+int a0_ex_tails_save(a0_extend* ex, std::vector<uint8_t>& out);
+int a0_ex_tails_check(int32_t F, const uint8_t* p, int64_t len, int64_t head_fs);
+int a0_ex_tails_load(a0_extend* ex, const uint8_t* p, int64_t len, cudaStream_t cs);
+void a0_ex_tails_clear(a0_extend* ex);
+a0_replay* a0_ex_shard(a0_extend* ex);
+constexpr int A0_RNG_CALL_WORD = 2 * A0_MAX_BATCHES + 34;   // counter[] words of the sampler's 64-bit call counter
+
 __device__ __forceinline__ uint32_t a0_smem_u32(const void* p) {
   return (uint32_t)__cvta_generic_to_shared(p);
 }
@@ -317,6 +331,38 @@ __device__ __forceinline__ void a0_bulk_load_hint(uint32_t smem_dst, const void*
 __device__ __forceinline__ void a0_bulk_store_hint(void* gdst, uint32_t smem_src, uint32_t bytes, uint64_t pol) {
   asm volatile("cp.async.bulk.global.shared::cta.bulk_group.L2::cache_hint [%0], [%1], %2, %3;"
                ::"l"(gdst), "r"(smem_src), "r"(bytes), "l"(pol) : "memory");
+}
+
+// ---- 64-bit frame content hash of K6a / K7 ---------------------------------------------------------
+__device__ __forceinline__ uint32_t a0_k6_rotl(uint32_t x, int r) { return (x << r) | (x >> (32 - r)); }
+__device__ __forceinline__ uint32_t a0_k6_mix32(uint32_t h) {
+  h ^= h >> 16; h *= 0x85EBCA6Bu; h ^= h >> 13; h *= 0xC2B2AE35u; h ^= h >> 16;
+  return h;
+}
+// 64-bit content hash of one frame held in shared memory (K6a computes it while decoding, K7 while
+// encoding, and K6b uses it as a gate in front of the byte compare).  Four independent 32-bit multiply-rotate streams over 16-byte
+// vector loads -- three instructions per word (the first version's 64-bit multiplies were a fifth of the
+// kernel's instructions).  Lanes are seeded differently, so equal words in different places do not cancel
+// in the final xor across the warp.
+__device__ __forceinline__ unsigned long long a0_k6_frame_hash(const uint8_t* frame, int nvec, int lane) {
+  uint32_t h0 = 0x9E3779B1u * (uint32_t)(lane + 1), h1 = 0x85EBCA77u * (uint32_t)(lane + 33);
+  uint32_t h2 = 0xC2B2AE3Du * (uint32_t)(lane + 65), h3 = 0x27D4EB2Fu * (uint32_t)(lane + 97);
+  const uint4* v4 = reinterpret_cast<const uint4*>(frame);
+#pragma unroll 2
+  for (int i = lane; i < nvec; i += 32) {
+    const uint4 v = v4[i];
+    h0 = a0_k6_rotl((h0 ^ v.x) * 0x9E3779B1u, 13);
+    h1 = a0_k6_rotl((h1 ^ v.y) * 0x85EBCA77u, 15);
+    h2 = a0_k6_rotl((h2 ^ v.z) * 0xC2B2AE3Du, 17);
+    h3 = a0_k6_rotl((h3 ^ v.w) * 0x27D4EB2Fu, 11);
+  }
+  uint32_t lo = a0_k6_mix32(h0 + 0x165667B1u * h2), hi = a0_k6_mix32(h1 + 0x9E3779B1u * h3);
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    lo ^= __shfl_xor_sync(0xffffffffu, lo, o);
+    hi ^= __shfl_xor_sync(0xffffffffu, hi, o);
+  }
+  return ((unsigned long long)a0_k6_mix32(hi ^ 0x5bd1e995u) << 32) | a0_k6_mix32(lo);
 }
 
 // ---- small device helpers ------------------------------------------------------------------------

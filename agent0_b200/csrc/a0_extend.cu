@@ -148,37 +148,6 @@ __device__ __forceinline__ void a0_k6_copy_match(uint8_t* gout, int op, int off,
   }
 }
 
-__device__ __forceinline__ uint32_t a0_k6_rotl(uint32_t x, int r) { return (x << r) | (x >> (32 - r)); }
-__device__ __forceinline__ uint32_t a0_k6_mix32(uint32_t h) {
-  h ^= h >> 16; h *= 0x85EBCA6Bu; h ^= h >> 13; h *= 0xC2B2AE35u; h ^= h >> 16;
-  return h;
-}
-// 64-bit content hash of one frame held in shared memory (a gate in front of the byte compare: nothing
-// depends on its value outside this file).  Four independent 32-bit multiply-rotate streams over 16-byte
-// vector loads -- three instructions per word (the first version's 64-bit multiplies were a fifth of the
-// kernel's instructions).  Lanes are seeded differently, so equal words in different places do not cancel
-// in the final xor across the warp.
-__device__ __forceinline__ unsigned long long a0_k6_frame_hash(const uint8_t* frame, int nvec, int lane) {
-  uint32_t h0 = 0x9E3779B1u * (uint32_t)(lane + 1), h1 = 0x85EBCA77u * (uint32_t)(lane + 33);
-  uint32_t h2 = 0xC2B2AE3Du * (uint32_t)(lane + 65), h3 = 0x27D4EB2Fu * (uint32_t)(lane + 97);
-  const uint4* v4 = reinterpret_cast<const uint4*>(frame);
-#pragma unroll 2
-  for (int i = lane; i < nvec; i += 32) {
-    const uint4 v = v4[i];
-    h0 = a0_k6_rotl((h0 ^ v.x) * 0x9E3779B1u, 13);
-    h1 = a0_k6_rotl((h1 ^ v.y) * 0x85EBCA77u, 15);
-    h2 = a0_k6_rotl((h2 ^ v.z) * 0xC2B2AE3Du, 17);
-    h3 = a0_k6_rotl((h3 ^ v.w) * 0x27D4EB2Fu, 11);
-  }
-  uint32_t lo = a0_k6_mix32(h0 + 0x165667B1u * h2), hi = a0_k6_mix32(h1 + 0x9E3779B1u * h3);
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    lo ^= __shfl_xor_sync(0xffffffffu, lo, o);
-    hi ^= __shfl_xor_sync(0xffffffffu, hi, o);
-  }
-  return ((unsigned long long)a0_k6_mix32(hi ^ 0x5bd1e995u) << 32) | a0_k6_mix32(lo);
-}
-
 // ------------------------------------------------------------------------------------------------
 // K6a: LZ4 block decode, one warp per reference entry
 // ------------------------------------------------------------------------------------------------
@@ -723,3 +692,97 @@ extern "C" int a0_ex_last_timing(a0_extend_t* ex, float* out6) {
   for (int i = 0; i < 6; ++i) out6[i] = ex->timing[i];
   return A0_OK;
 }
+
+// ------------------------------------------------------------------------------------------------
+// checkpoints (a0_ckpt.cu): the decode kernel on one batch of blobs, and the stream tails.
+// TAILS layout: count i64, then per stream in ascending id order {id i64, seq i64[8], cls u8[8], frames u8[8][F],
+// hash u64[8]}.
+// ------------------------------------------------------------------------------------------------
+int a0_ex_decode_dev(a0_extend* ex, const uint8_t* blobs, const int64_t* blob_len, int32_t mb, cudaStream_t cs,
+                     const uint8_t** dec, const unsigned long long** hash, const int32_t** status) {
+  int rc = a0_ex_run_batch(ex, blobs, nullptr, blob_len, nullptr, mb, false, cs, "a0_ckpt_load");
+  if (rc) return rc;
+  *dec = ex->d_dec;
+  *hash = ex->d_hash;
+  *status = reinterpret_cast<const int32_t*>(ex->h_back + (size_t)ex->cap * A0_SLOTS);
+  return A0_OK;
+}
+
+static inline size_t a0_ex_tail_bytes(int32_t F) { return 8 + 64 + 8 + (size_t)A0_SLOTS * F + 64; }
+
+int a0_ex_tails_save(a0_extend* ex, std::vector<uint8_t>& out) {
+  std::vector<int64_t> ids;
+  for (auto& kv : ex->tail)
+    if (kv.second.valid) ids.push_back(kv.first);
+  std::sort(ids.begin(), ids.end());
+  const size_t each = a0_ex_tail_bytes(ex->F);
+  out.assign(8 + ids.size() * each, 0);
+  const int64_t count = (int64_t)ids.size();
+  memcpy(out.data(), &count, 8);
+  uint8_t* p = out.data() + 8;
+  for (int64_t id : ids) {
+    const A0ExTail& tl = ex->tail[id];
+    memcpy(p, &id, 8);
+    memcpy(p + 8, tl.seq, 64);
+    memcpy(p + 72, tl.cls, 8);
+    A0_CUDA(cudaMemcpy(p + 80, ex->d_tail_frames + (size_t)tl.slot * A0_SLOTS * ex->F, (size_t)A0_SLOTS * ex->F, cudaMemcpyDeviceToHost));
+    A0_CUDA(cudaMemcpy(p + 80 + (size_t)A0_SLOTS * ex->F, ex->d_tail_hash + (size_t)tl.slot * A0_SLOTS, 64, cudaMemcpyDeviceToHost));
+    p += each;
+  }
+  return A0_OK;
+}
+
+// structure only: called before the shard is touched
+int a0_ex_tails_check(int32_t F, const uint8_t* p, int64_t len, int64_t head_fs) {
+  int64_t count = 0;
+  A0_REQUIRE(len >= 8, "a0_ckpt_load: TAILS section truncated");
+  memcpy(&count, p, 8);
+  const size_t each = a0_ex_tail_bytes(F);
+  A0_REQUIRE(count >= 0 && (uint64_t)count <= (uint64_t)(len - 8) / each && 8 + (int64_t)(count * each) == len,
+             "a0_ckpt_load: TAILS section has the wrong length");
+  int64_t prev = 0;
+  for (int64_t i = 0; i < count; ++i) {
+    const uint8_t* e = p + 8 + i * each;
+    int64_t id, seq[A0_SLOTS];
+    memcpy(&id, e, 8);
+    memcpy(seq, e + 8, 64);
+    A0_REQUIRE(i == 0 || id > prev, "a0_ckpt_load: TAILS stream ids out of order");
+    prev = id;
+    for (int j = 0; j < A0_SLOTS; ++j)
+      A0_REQUIRE(seq[j] >= 0 && seq[j] < head_fs && e[72 + j] < 2 * A0_SLOTS, "a0_ckpt_load: TAILS entry of stream %lld is inconsistent",
+                 (long long)id);
+  }
+  return A0_OK;
+}
+
+void a0_ex_tails_clear(a0_extend* ex) {
+  ex->tail.clear();
+  ex->n_slots = 0;
+}
+
+int a0_ex_tails_load(a0_extend* ex, const uint8_t* p, int64_t len, cudaStream_t cs) {
+  (void)len;
+  a0_ex_tails_clear(ex);
+  int64_t count = 0;
+  memcpy(&count, p, 8);
+  int rc = a0_ex_reserve(ex, 0, 0, (int32_t)count);
+  if (rc) return rc;
+  const size_t each = a0_ex_tail_bytes(ex->F), entry = (size_t)A0_SLOTS * ex->F;
+  for (int64_t i = 0; i < count; ++i) {
+    const uint8_t* e = p + 8 + i * each;
+    int64_t id;
+    memcpy(&id, e, 8);
+    A0ExTail& tl = ex->tail[id];
+    memcpy(tl.seq, e + 8, 64);
+    memcpy(tl.cls, e + 72, 8);
+    tl.slot = (int32_t)i;
+    tl.valid = true;
+    A0_CUDA(cudaMemcpyAsync(ex->d_tail_frames + (size_t)i * entry, e + 80, entry, cudaMemcpyHostToDevice, cs));
+    A0_CUDA(cudaMemcpyAsync(ex->d_tail_hash + (size_t)i * A0_SLOTS, e + 80 + entry, 64, cudaMemcpyHostToDevice, cs));
+  }
+  ex->n_slots = (int32_t)count;
+  A0_CUDA(cudaStreamSynchronize(cs));
+  return A0_OK;
+}
+
+a0_replay* a0_ex_shard(a0_extend* ex) { return ex->h; }

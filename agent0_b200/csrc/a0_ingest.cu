@@ -529,3 +529,132 @@ extern "C" int a0_rb_ingest_steps_dyn(a0_replay_t* h, a0_index_t* ix, const int6
   return a0_ingest_steps_impl(h, ix, stream, n_new, new_frames, flags, action, reward, done, m, alpha, &beta, compat_sum,
                               cuda_stream, "a0_rb_ingest_steps_dyn");
 }
+
+// ------------------------------------------------------------------------------------------------
+// serialization of the ring index (checkpoints: a0_ckpt_save / a0_ckpt_load)
+// ------------------------------------------------------------------------------------------------
+// Layout, little-endian i64 words unless noted: magic "A0IX" u32, version u32, N, NF, n_step, age_limit, head_q,
+// tail_q, head_fs, top, fs_at_append[N], sampleable u8[N], streams, per stream in ascending id order {id, last_pos,
+// last_seq, has_stack, stack[4], pending count, pending[...]}, stale count, stale[...] ascending.
+static constexpr uint32_t A0_IX_MAGIC = 0x58493041u;   // "A0IX"
+static constexpr uint32_t A0_IX_VERSION = 1;
+
+namespace {
+struct A0IxWriter {
+  uint8_t* out; int64_t cap, len = 0;
+  void put(const void* p, size_t k) { if (out && len + (int64_t)k <= cap) memcpy(out + len, p, k); len += (int64_t)k; }
+  void i64(int64_t v) { put(&v, 8); }
+};
+struct A0IxReader {
+  const uint8_t* p; int64_t len, at = 0;
+  bool get(void* d, size_t k) { if (at + (int64_t)k > len) return false; memcpy(d, p + at, k); at += (int64_t)k; return true; }
+  bool i64(int64_t& v) { return get(&v, 8); }
+};
+}  // namespace
+
+extern "C" int a0_ix_serialize(a0_index_t* ix, uint8_t* out, int64_t cap, int64_t* len_out) {
+  A0_REQUIRE(ix && len_out, "a0_ix_serialize: NULL argument");
+  A0IxWriter w{out, out ? cap : 0};
+  const uint32_t hdr[2] = {A0_IX_MAGIC, A0_IX_VERSION};
+  w.put(hdr, 8);
+  for (int64_t v : {ix->N, ix->NF, ix->n, ix->age_limit, ix->head_q, ix->tail_q, ix->head_fs, ix->top}) w.i64(v);
+  w.put(ix->fs_at_append.data(), (size_t)ix->N * 8);
+  w.put(ix->sampleable.data(), (size_t)ix->N);
+  std::vector<int64_t> ids;
+  for (auto& kv : ix->streams) ids.push_back(kv.first);
+  std::sort(ids.begin(), ids.end());
+  w.i64((int64_t)ids.size());
+  for (int64_t id : ids) {
+    const A0Stream& st = ix->streams[id];
+    w.i64(id); w.i64(st.last_pos); w.i64(st.last_seq); w.i64(st.has_stack ? 1 : 0);
+    for (int j = 0; j < A0_STACK; ++j) w.i64(st.stack[j]);
+    w.i64((int64_t)st.pending.size());
+    w.put(st.pending.data(), st.pending.size() * 8);
+  }
+  std::vector<int64_t> stale(ix->stale.begin(), ix->stale.end());
+  std::sort(stale.begin(), stale.end());
+  w.i64((int64_t)stale.size());
+  w.put(stale.data(), stale.size() * 8);
+  *len_out = w.len;
+  A0_REQUIRE(out && cap >= w.len, "a0_ix_serialize: the index needs %lld bytes", (long long)w.len);
+  return A0_OK;
+}
+
+extern "C" int a0_ix_deserialize(a0_index_t* ix, const uint8_t* blob, int64_t len) {
+  A0_REQUIRE(ix && blob && len >= 0, "a0_ix_deserialize: NULL argument");
+  A0IxReader r{blob, len};
+  uint32_t hdr[2];
+  A0_REQUIRE(r.get(hdr, 8) && hdr[0] == A0_IX_MAGIC && hdr[1] == A0_IX_VERSION, "a0_ix_deserialize: not a ring index (bad magic or version)");
+  int64_t N, NF, n, age, hq, tq, hfs, top;
+  A0_REQUIRE(r.i64(N) && r.i64(NF) && r.i64(n) && r.i64(age) && r.i64(hq) && r.i64(tq) && r.i64(hfs) && r.i64(top),
+             "a0_ix_deserialize: truncated header");
+  A0_REQUIRE(N == ix->N && NF == ix->NF && n == ix->n && age == ix->age_limit,
+             "a0_ix_deserialize: saved for N=%lld NF=%lld n_step=%lld age_limit=%lld, this index has %lld %lld %lld %lld",
+             (long long)N, (long long)NF, (long long)n, (long long)age, (long long)ix->N, (long long)ix->NF, (long long)ix->n,
+             (long long)ix->age_limit);
+  A0_REQUIRE(0 <= tq && tq <= hq && hq - tq <= N && hfs >= 0 && 0 <= top && top <= hq - tq,
+             "a0_ix_deserialize: inconsistent counters (head_q %lld, tail_q %lld, head_fs %lld, top %lld)", (long long)hq,
+             (long long)tq, (long long)hfs, (long long)top);
+  a0_index t;
+  t.N = N; t.NF = NF; t.n = n; t.age_limit = age; t.head_q = hq; t.tail_q = tq; t.head_fs = hfs; t.top = top;
+  t.fs_at_append.resize((size_t)N);
+  t.sampleable.resize((size_t)N);
+  A0_REQUIRE(r.get(t.fs_at_append.data(), (size_t)N * 8) && r.get(t.sampleable.data(), (size_t)N), "a0_ix_deserialize: truncated");
+  int64_t count = 0;
+  for (int64_t q = 0; q < N; ++q) {
+    const bool live = (q - tq % N + N) % N < hq - tq;      // ring position of a record in [tail_q, head_q)
+    A0_REQUIRE(t.sampleable[q] <= 1 && (live || t.sampleable[q] == 0), "a0_ix_deserialize: record %lld is sampleable but not live",
+               (long long)q);
+    A0_REQUIRE(!live || (t.fs_at_append[q] >= 0 && t.fs_at_append[q] <= hfs), "a0_ix_deserialize: record %lld has a bad frame key",
+               (long long)q);
+    count += t.sampleable[q];
+  }
+  A0_REQUIRE(count == top, "a0_ix_deserialize: %lld sampleable records, top says %lld", (long long)count, (long long)top);
+  int64_t ns;
+  A0_REQUIRE(r.i64(ns) && ns >= 0 && ns <= (len - r.at) / 72, "a0_ix_deserialize: truncated stream table");
+  int64_t prev_id = 0;
+  for (int64_t i = 0; i < ns; ++i) {
+    int64_t id, lp, ls, hs, k;
+    A0Stream st;
+    A0_REQUIRE(r.i64(id) && r.i64(lp) && r.i64(ls) && r.i64(hs) && r.get(st.stack, sizeof(st.stack)) && r.i64(k),
+               "a0_ix_deserialize: truncated stream %lld", (long long)i);
+    A0_REQUIRE(i == 0 || id > prev_id, "a0_ix_deserialize: stream ids out of order");
+    prev_id = id;
+    A0_REQUIRE(ls >= -1 && ls < hq && (ls < 0 ? lp == -1 : lp == ls % N) && (hs == 0 || hs == 1),
+               "a0_ix_deserialize: stream %lld has an inconsistent last record", (long long)id);
+    A0_REQUIRE(k >= 0 && k < n && k <= (len - r.at) / 8, "a0_ix_deserialize: stream %lld has %lld pending records", (long long)id,
+               (long long)k);
+    st.pending.resize((size_t)k);
+    A0_REQUIRE(r.get(st.pending.data(), (size_t)k * 8), "a0_ix_deserialize: truncated");
+    for (int64_t j = 0; j < k; ++j)
+      A0_REQUIRE(st.pending[j] >= 0 && st.pending[j] < hq && (j == 0 || st.pending[j] > st.pending[j - 1]),
+                 "a0_ix_deserialize: stream %lld has a bad pending record", (long long)id);
+    st.last_pos = (int32_t)lp; st.last_seq = ls; st.has_stack = hs != 0;
+    t.streams.emplace(id, std::move(st));
+  }
+  int64_t nst;
+  A0_REQUIRE(r.i64(nst) && nst >= 0 && nst <= (len - r.at) / 8, "a0_ix_deserialize: truncated stale set");
+  for (int64_t i = 0; i < nst; ++i) {
+    int64_t s;
+    r.i64(s);
+    A0_REQUIRE(s >= 0 && s < hq, "a0_ix_deserialize: stale record %lld out of range", (long long)s);
+    t.stale.insert(s);
+  }
+  A0_REQUIRE(r.at == len, "a0_ix_deserialize: %lld trailing bytes", (long long)(len - r.at));
+  ix->head_q = t.head_q; ix->tail_q = t.tail_q; ix->head_fs = t.head_fs; ix->top = t.top;
+  ix->fs_at_append.swap(t.fs_at_append);
+  // in place: a0_ix_sampleable hands out a pointer into this vector
+  memcpy(ix->sampleable.data(), t.sampleable.data(), (size_t)N);
+  ix->streams.swap(t.streams);
+  ix->stale.swap(t.stale);
+  return A0_OK;
+}
+
+// back to the state of a0_ix_create (a checkpoint load that failed after it touched the index)
+void a0_ix_clear(a0_index* ix) {
+  ix->head_q = ix->tail_q = ix->head_fs = ix->top = 0;
+  std::fill(ix->fs_at_append.begin(), ix->fs_at_append.end(), 0);
+  std::fill(ix->sampleable.begin(), ix->sampleable.end(), 0);
+  ix->streams.clear();
+  ix->stale.clear();
+}

@@ -358,7 +358,7 @@ extern "C" int a0_pt_sample(a0_replay_t* h, const float* u, int32_t total, int32
 
 // counter[] words used by the sampler's own generator (the rest of the layout is in a0_common.cuh)
 constexpr int K2A_RNG_TICKET = 2 * A0_MAX_BATCHES + 32;  // past the per-batch maxima at [MAXB+16, 2*MAXB+16)
-constexpr int K2A_RNG_CALL = 2 * A0_MAX_BATCHES + 34;    // two words, 8-byte aligned
+constexpr int K2A_RNG_CALL = A0_RNG_CALL_WORD;           // two words, 8-byte aligned (a0_common.cuh)
 
 extern "C" int a0_pt_sample_rng(a0_replay_t* h, uint64_t seed, int64_t call, int32_t total, int32_t batch, float top,
                                 float beta, float sum_offset, int32_t uniform, int64_t* idx_out, float* prio_out,

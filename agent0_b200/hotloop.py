@@ -456,7 +456,10 @@ class StaleByOneLoop:
     replays), duplicates keep last-writer-wins, the tree stays node == fl32(left + right) at every replay
     boundary.  A draw that races with a write-back can see a parent that is newer or older than its children:
     every decision of the descent still moves to a child whose mass was positive when it was read, and K2b never
-    zeroes a leaf, so every drawn index is a live record (tested)."""
+    zeroes a leaf, so every drawn index is a live record (tested).
+
+    Call ``flush()`` before ``ReplayDataset.save``: until then the last step's priority write-back is still pending
+    and the checkpoint would miss it."""
 
     def __init__(self, replay, algo, batch_size, learner_steps, action_dim, outputs, **kw):
         kw = dict(kw)

@@ -15,6 +15,8 @@ fallback.
 from __future__ import annotations
 
 import ctypes as C
+import json
+import os
 from collections import namedtuple
 
 import numpy as np
@@ -514,6 +516,35 @@ class ReplayDataset:
         with torch.cuda.device(dev):
             _lib.check(self.lib.a0_pt_update(self.h, ids.data_ptr(), loss.data_ptr(), ids.numel(), self.alpha,
                                              self.eps, _lib.stream_ptr(dev)), "a0_pt_update")
+
+    # ------------------------------------------------------------------ checkpoint
+    def save(self, path):
+        """Write the whole shard to ``path`` (a0_ckpt_save): frames of the resident window as K7 LZ4 blobs, records,
+        priorities, max_p, the sampler's scalars and call counter, the ring index and the reference-tuple ingest's
+        stream tails, plus beta, the beta schedule's position and the draw-without-replacement seed.  Synchronises
+        the current stream; refused during a CUDA-graph capture.  A ``StaleByOneLoop`` must be ``flush()``ed first."""
+        user = json.dumps(dict(beta=self.beta, beta_current=getattr(getattr(self, "beta_schedule", None), "current", None),
+                               unique_seed=getattr(self, "_unique_seed", None))).encode()
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.a0_ckpt_save(self.h, self.index.h, self._ex, os.fsencode(os.fspath(path)), user, len(user),
+                                             _lib.stream_ptr(self.device)), "a0_ckpt_save")
+
+    def load(self, path):
+        """Replace this shard's contents with a checkpoint written by ``save`` for a shard of the same config
+        (a0_ckpt_load, into the buffers the shard already owns: CUDA graphs captured on it stay valid).  Raises
+        RuntimeError on a mismatched or corrupt file; a file rejected before the frames are decoded leaves the shard
+        as it was, a failure while they are decoded leaves it empty."""
+        buf = C.create_string_buffer(1 << 16)
+        n = C.c_int64(0)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.a0_ckpt_load(self.h, self.index.h, self._ex, os.fsencode(os.fspath(path)), buf, len(buf),
+                                             C.byref(n), _lib.stream_ptr(self.device)), "a0_ckpt_load")
+        user = json.loads(buf.raw[:n.value].decode()) if n.value else {}
+        if "beta" in user:
+            self.beta = user["beta"]
+        if user.get("beta_current") is not None and getattr(self, "beta_schedule", None) is not None:
+            self.beta_schedule.current = user["beta_current"]
+        self._unique_seed = user.get("unique_seed")
 
     def rng_seek(self, call):
         """Set the device-resident call counter of the sampler's own generator (stream-ordered)."""

@@ -368,6 +368,19 @@ class NativeRingIndex:
                 last4[sid] = self.get_stack(sid)
         return fs8
 
+    def serialize(self):
+        """The whole index state as bytes (a0_ix_serialize; the INDEX section of a shard checkpoint)."""
+        n = self._C.c_int64(0)
+        self.lib.a0_ix_serialize(self.h, None, 0, self._C.byref(n))
+        buf = (self._C.c_uint8 * n.value)()
+        self._L.check(self.lib.a0_ix_serialize(self.h, buf, n.value, self._C.byref(n)), "a0_ix_serialize")
+        return bytes(buf)
+
+    def deserialize(self, blob):
+        """Replace the state with ``serialize()`` output of an index with the same parameters (a0_ix_deserialize)."""
+        blob = bytes(blob)
+        self._L.check(self.lib.a0_ix_deserialize(self.h, blob, len(blob)), "a0_ix_deserialize")
+
     def plan_native(self, stream, fs8, n_new, action, reward, done):
         """a0_ix_plan; returns the ctypes a0_plan_t (arrays owned by the index until its next call)."""
         stream = np.ascontiguousarray(stream, dtype=np.int64)

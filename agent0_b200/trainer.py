@@ -10,8 +10,10 @@ sample several batches ahead with a fork-time snapshot of the priorities (SURVEY
 """
 from __future__ import annotations
 
+import os
 from collections import deque
 
+import numpy as np
 import torch
 
 from .learner import make_learner
@@ -166,3 +168,51 @@ class Trainer:
         frac = vals.pop(0) if self.FLs else None
         return dict(frames=self.frame_count, fraction_loss=frac, loss=loss, return_train=hmean(self.Rs),
                     return_train_max=self.R_max, qmax=hmean(self.Qs))
+
+    # ------------------------------------------------------------------ checkpoint
+    def _replay_file(self, directory):
+        name = "replay.a0ckpt" if self.pg is None else f"replay.rank{torch.distributed.get_rank(self.pg)}.a0ckpt"
+        return os.path.join(directory, name)
+
+    def save(self, directory):
+        """Checkpoint the run into ``directory``: the shard (``replay.a0ckpt``, ``replay.rank{r}.a0ckpt`` per rank with a
+        process group) and ``learner.pt`` -- online and target models, optimizers, update_steps, frame_count, the
+        logging deques, R_max and the torch CPU / CUDA and numpy RNG states."""
+        os.makedirs(directory, exist_ok=True)
+        self.replay.save(self._replay_file(directory))
+        if self.pg is not None and torch.distributed.get_rank(self.pg) != 0:
+            return
+        ln = self.learner
+        state = dict(model=ln.model.state_dict(), model_target=ln.model_target.state_dict(), optimizer=ln.optimizer.state_dict(),
+                     update_steps=ln.update_steps, frame_count=self.frame_count,
+                     logs={k: [float(x) for x in getattr(self, k)] for k in ("Ls", "FLs", "Rs", "Qs")}, R_max=self.R_max,
+                     rng_cpu=torch.get_rng_state(), rng_cuda=torch.cuda.get_rng_state(self.replay.device),
+                     rng_numpy=np.random.get_state())
+        if getattr(ln, "fqf_optimizer", None) is not None:
+            state["fqf_optimizer"] = ln.fqf_optimizer.state_dict()
+        torch.save(state, os.path.join(directory, "learner.pt"))
+
+    def load(self, directory):
+        """Resume from ``save``: into a Trainer built with the same config.  Captured graphs are dropped (the next
+        ``learn`` captures again): Adam's state tensors are replaced, and a graph captured before would keep updating
+        the old ones."""
+        self.replay.load(self._replay_file(directory))
+        state = torch.load(os.path.join(directory, "learner.pt"), map_location=self.replay.device, weights_only=False)
+        ln = self.learner
+        ln.model.load_state_dict(state["model"])
+        ln.model_target.load_state_dict(state["model_target"])
+        ln.optimizer.load_state_dict(state["optimizer"])
+        if "fqf_optimizer" in state:
+            ln.fqf_optimizer.load_state_dict(state["fqf_optimizer"])
+        ln.update_steps = state["update_steps"]
+        self.frame_count = state["frame_count"]
+        dev = self.replay.device
+        for k, vals in state["logs"].items():
+            d = getattr(self, k)
+            d.clear()
+            d.extend(torch.tensor(v, device=dev) if k in ("Ls", "FLs") else v for v in vals)
+        self.R_max = state["R_max"]
+        torch.set_rng_state(state["rng_cpu"].cpu())
+        torch.cuda.set_rng_state(state["rng_cuda"].cpu(), dev)
+        np.random.set_state(state["rng_numpy"])
+        self._graphed = None

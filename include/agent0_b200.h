@@ -252,6 +252,61 @@ int a0_ex_resolve(a0_extend_t* ex, const int64_t* stream, const uint8_t* labels,
  * host resolve + plan, append launches, device time of decode + label (CUDA events), entries}       */
 int a0_ex_last_timing(a0_extend_t* ex, float* out6);
 
+/* ---- K7: LZ4 encode of 8-frame groups on the device ---------------------------------------------------
+ * frames dev u8[m][8][frame_bytes] (16-byte aligned); group g becomes one python-lz4 block (4-byte little-endian
+ * decoded size + one raw LZ4 block, no dictionary shared across groups) at out + g * A0_LZ4_STRIDE(frame_bytes),
+ * or the 8 * frame_bytes input bytes themselves when that block would not be shorter (K6a takes a blob of exactly
+ * the decoded size as uncompressed).  out_len dev i32[m]: blob lengths; frame_hash dev u64[m][8]: the 64-bit content
+ * hash K6a computes for each decoded frame.  The parse is the greedy one defined by oracle/lz4_encode.py
+ * (encode_greedy), byte for byte: one warp per group, the group in shared memory.                              */
+#define A0_LZ4_STRIDE(frame_bytes) \
+  ((((int64_t)8 * (frame_bytes) + (int64_t)8 * (frame_bytes) / 255 + 20) + 15) / 16 * 16)
+int a0_lz4_encode(const uint8_t* frames /* dev */, int32_t m, int32_t frame_bytes, uint8_t* out /* dev */,
+                  int32_t* out_len /* dev */, uint64_t* frame_hash /* dev */, a0_stream_t stream);
+
+/* ---- checkpoint: one shard (+ its ring index and reference-ingest state) to a file and back ---------------
+ * a0_ix_serialize writes the ring index's whole state (head_q, tail_q, head_fs, top, fs_at_append, sampleable,
+ * per stream last_pos / last_seq / pending / stack / has_stack, the stale set) into out[cap]; *len_out receives
+ * the length (also when out is NULL or cap is too small, which then fails with A0_EINVAL).  a0_ix_deserialize
+ * replaces the state of an index created with the same capacities, n_step and age limit; a blob that is
+ * truncated, inconsistent or made for other parameters is rejected with A0_EINVAL and the index is unchanged.
+ * Host code only.                                                                                          */
+int a0_ix_serialize(a0_index_t* ix, uint8_t* out, int64_t cap, int64_t* len_out);
+int a0_ix_deserialize(a0_index_t* ix, const uint8_t* blob, int64_t len);
+/* a0_ckpt_save synchronises `stream`, refuses during a CUDA-graph capture and on a shard whose fault word is set,
+ * and writes the shard h, its index ix and (ex != NULL) the stream tails of the reference-tuple ingest to `path`
+ * (through path + ".tmp", renamed when complete), with `user` (user_len bytes) stored alongside.  Frames leave as
+ * K7 blobs.  File format (little-endian; section hash: the 64-bit streaming hash of a0_ckpt.cu):
+ *   header   "A0CKPT01" magic (8 B), version u32 (= 1), 0 u32, N i64, NF i64, F i64, P i64, n_step i64, age_limit i64
+ *   sections {tag u32, 0 u32, length u64, hash u64 of the payload} + payload, in this order:
+ *   INDEX    (1) a0_ix_serialize
+ *   RECORDS  (2) rec_slots i32[N][8], then rec_info {reward f64, action|done<<31 i32, link i32}[N]
+ *   LEAVES   (3) f32[N] tree leaves (the inner nodes are rebuilt on load: node = fl32(left + right))
+ *   SCALARS  (4) max_p f32, dyn {top, beta, sum_offset} f32[3], sampler call counter u64, stride_hint i64
+ *   TAILS    (5) count i64, then per stream {id i64, seq i64[8], cls u8[8], frames u8[8][F], hash u64[8]}
+ *   USER     (6) the caller's bytes
+ *   FRAMES   (7) lo i64 (first frame seq: max(0, head_fs - NF)), frames i64 (head_fs - lo), groups i64, then
+ *                {first ring position i64, blob length i64}[groups] and the frame hashes u64[groups][8].  Group g
+ *                holds seqs lo + 8g .. lo + 8g + 7 (the last group padded with zero frames)
+ *   BLOBS    (8) the groups' K7 blobs, back to back
+ * a0_ckpt_load reads such a file into an existing shard + index (+ ex, or NULL) of the same N, NF, F, n_step and
+ * age limit, into the buffers they already own (CUDA graphs captured on the shard stay valid).  It validates
+ * everything it can before touching the shard (header, section hashes, index invariants, finite non-negative
+ * leaves that are 0 where a record is not sampleable, slots and links of live records, the group table); a file
+ * that fails there leaves shard and index unchanged.  Frames are then decoded by K6a into the ring and every
+ * frame's hash is compared with the saved one; a failure from there on leaves shard, index and tails as freshly
+ * created.  Both return A0_EINVAL with a message for a bad file.  user_out[user_cap] receives the USER bytes and
+ * *user_len_out their length (NULLs allowed).                                                              */
+int a0_ckpt_save(a0_replay_t* h, a0_index_t* ix, a0_extend_t* ex, const char* path, const uint8_t* user,
+                 int64_t user_len, a0_stream_t stream);
+int a0_ckpt_load(a0_replay_t* h, a0_index_t* ix, a0_extend_t* ex, const char* path, uint8_t* user_out,
+                 int64_t user_cap, int64_t* user_len_out, a0_stream_t stream);
+/* Phases of the last a0_ckpt_save / a0_ckpt_load of the process.  Save: {total us, K7 device us (CUDA events),
+ * blob compaction + device-to-host copy device us (CUDA events), file write us, raw frame bytes, blob bytes, host
+ * wait for the copies us, 0}.  Load: {total us, header + small sections + validation us, blob file read us,
+ * decode + hash check + restore us (host clock, K6a included), raw frame bytes, blob bytes, 0, 0}.               */
+int a0_ckpt_last_timing(double* out8);
+
 /* ---- staged ingest: execute a plan on the device ------------------------------------------------
  * One pinned H2D copy of {frames, positions, record metadata, marks} from a double-buffered
  * staging area owned by the handle, then a0_pt_mark and a0_rb_append on `stream`.  frames:
