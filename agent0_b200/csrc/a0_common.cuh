@@ -149,6 +149,7 @@ void a0_set_k2b_chunks(int on);
 void a0_set_k2b_sparse(int max_paths);
 void a0_set_k2a_rounds(int on);
 void a0_set_qh_sorted(int on);
+void a0_set_qh_spec(int on);
 void a0_set_k6_global(int on);
 
 // (Measured alternative: launch_dependents BEFORE the wait lets a whole chain of dependent kernels

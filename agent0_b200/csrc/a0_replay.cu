@@ -127,6 +127,7 @@ extern "C" int a0_set_option(int32_t option, int64_t value) {
     return A0_OK;
   }
   if (option == A0_OPT_K6_GLOBAL) { a0_set_k6_global(value != 0); return A0_OK; }
+  if (option == A0_OPT_QH_SPEC) { a0_set_qh_spec(value != 0); return A0_OK; }
   if (option == A0_OPT_QH_SORTED) {
     A0_REQUIRE(value >= 0 && value <= 2, "a0_set_option: A0_OPT_QH_SORTED must be 0, 1 or 2");
     a0_set_qh_sorted((int)value);

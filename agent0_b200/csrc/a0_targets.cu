@@ -344,7 +344,10 @@ a0_k4_c51(const A0Common c, const float* __restrict__ logits, const float* __res
       int lo_ = (int)floorf(base), up_ = (int)ceilf(base);
       if (up_ > 0 && lo_ == up_) lo_ -= 1;
       if (lo_ < M - 1 && lo_ == up_) up_ += 1;
-      lo[k] = lo_; up[k] = up_;
+      // delta is rounded to fp32, so an atom clamped at vmax can get a base just above M-1 (M = 128, vmin = -10,
+      // vmax = 25: 127.0000076) and up_ = M.  That upper term is dropped, as in a0_k4_c51_fast: bin M is past the
+      // sample's row, and at M = 128 it is bin 0 of the next warp's sample.
+      lo[k] = lo_; up[k] = up_ < M ? up_ : -1;
       wlo[k] = __fmul_rn(pj, __fsub_rn((float)up_, base));
       wup[k] = __fmul_rn(pj, __fsub_rn(base, (float)lo_));
     }
@@ -418,8 +421,8 @@ __global__ void __launch_bounds__(WARPS * 32)
 a0_k4_c51_fast(const A0Common c, const float* __restrict__ logits, const float* __restrict__ tgt_logits,
                const float* __restrict__ qsel, const float* __restrict__ atoms, int32_t M, float vmin, float vmax,
                float delta, float* __restrict__ grad, float* __restrict__ target_prob) {
-  __shared__ float s_m[WARPS][72];       // projected distribution (bin M may be touched when b rounds above M-1:
-                                             // ignored, as in the reference's clamp), then the taken action's gradient row
+  __shared__ float s_m[WARPS][72];       // projected distribution (bin M may be touched when b rounds above M-1: that
+                                             // upper term is dropped, as in a0_k4_c51 and oracle.losses.c51_project)
   A0_T0();
   A0_PDL_PROLOGUE();
   A0_TMID();
@@ -789,7 +792,9 @@ a0_k4_quantile(const A0Common c, int32_t layout, const float* __restrict__ q, co
 // bitonic networks in registers, then three merge levels in shared memory where every element finds its rank in
 // the sibling run by binary search -- no compare-exchange stages, three barriers), prefix sums of T and T^2, and
 // per online quantile three binary searches plus ~25 flops.  The prefix sums and the polynomial are evaluated in
-// float64: the quadratic ranges subtract numbers of size N*T^2 to get terms of size (q-T)^2 <= 1.  The summation
+// float64 and centred on the median target c (sums of T-c and (T-c)^2, q-c): the quadratic ranges subtract numbers of
+// size N*(T-c)^2 to get terms of size (q-T)^2 <= 1, and uncentred sums of size N*T^2 lost the 1e-5 contract from
+// |T| ~ 1e5 (8e-5 relative; 8e-3 at 1e6).  The summation
 // order differs from the reference's pairwise sum, so this kernel lives under the 1e-5 relative contract (it is
 // closer to the exact sum than the fp32 pairwise form); oracle.losses.huber_qr_sorted is its specification.
 constexpr int QS_MAX = A0_MAX_QUANTILES;         // 256 = 8 sorted runs of one warp each
@@ -936,9 +941,12 @@ a0_k4_quantile_sorted(const A0Common c, int32_t layout, const float* __restrict_
   __syncthreads();
   a0_qs_merge<7>(bufA, bufB, pos, x, x_up);
   __syncthreads();
-  // ---- prefix sums of T and T^2 over the sorted targets (float64) -----------------------------------------
+  // ---- prefix sums of T-c and (T-c)^2 over the sorted targets (float64) --------------------------------------
+  // c = the sorted target at Ni/2.  Centring keeps the sums of size N*(T-c)^2 instead of N*T^2, so the quadratic
+  // ranges lose no precision as |T| grows; T - c and q - c are exact in float64 (T, q and c are fp32).
+  const double cen = (double)bufB[Ni >> 1];
   {
-    const double y = tid < Ni ? (double)bufB[tid] : 0.0;
+    const double y = tid < Ni ? (double)bufB[tid] - cen : 0.0;
     double p1 = y, p2 = y * y;
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) {
@@ -971,7 +979,7 @@ a0_k4_quantile_sorted(const A0Common c, int32_t layout, const float* __restrict_
     ib += (bufB[ib] < qj) ? 1 : 0;
     ic += (bufB[ic] < qp) ? 1 : 0;
     ia = min(ia, Ni); ib = min(max(ib, ia), Ni); ic = min(max(ic, ib), Ni);
-    const double qd = (double)qj, td = (double)tau;
+    const double qd = (double)qj - cen, td = (double)tau;       // the range boundaries above use the uncentred fp32 values
     const double nA = (double)ia, nB = (double)(ib - ia), nC = (double)(ic - ib), nD = (double)(Ni - ic);
     const double s1a = S1[ia], s1b = S1[ib], s1c = S1[ic];
     const double s1B = s1b - s1a, s2B = S2[ib] - S2[ia];
@@ -1076,16 +1084,20 @@ a0_k4_quantile_warp(const A0Common c, int32_t layout, const float* __restrict__ 
     x[i] = e < Ni ? a0_td_target(r, d, c.gamma_n, tb[a_star * sA_t + e * sN_t]) : a0_qs_pad(e);
   }
   a0_qw_sort256(x, lane);
-  // ---- sorted targets and their float64 prefix sums to shared memory -----------------------------------------
+  // ---- sorted targets and their float64 prefix sums, centred on the target at Ni/2 (as a0_k4_quantile_sorted) --
   {
     float4* dst = reinterpret_cast<float4*>(sT + lane * QW_R);
     dst[0] = make_float4(x[0], x[1], x[2], x[3]);
     dst[1] = make_float4(x[4], x[5], x[6], x[7]);
+  }
+  __syncwarp();
+  const double cen = (double)sT[Ni >> 1];
+  {
     double c1[QW_R], c2[QW_R];
     double p1 = 0.0, p2 = 0.0;
 #pragma unroll
     for (int i = 0; i < QW_R; ++i) {
-      const double y = (lane * QW_R + i) < Ni ? (double)x[i] : 0.0;      // sorted position >= Ni: a pad
+      const double y = (lane * QW_R + i) < Ni ? (double)x[i] - cen : 0.0;      // sorted position >= Ni: a pad
       p1 += y;
       p2 += y * y;
       c1[i] = p1;
@@ -1126,7 +1138,7 @@ a0_k4_quantile_warp(const A0Common c, int32_t layout, const float* __restrict__ 
     ib += (sT[ib] < qj) ? 1 : 0;
     ic += (sT[ic] < qp) ? 1 : 0;
     ia = min(ia, Ni); ib = min(max(ib, ia), Ni); ic = min(max(ic, ib), Ni);
-    const double qd = (double)qj, td = (double)tau;
+    const double qd = (double)qj - cen, td = (double)tau;
     const double nA = (double)ia, nB = (double)(ib - ia), nC = (double)(ic - ib), nD = (double)(Ni - ic);
     const double s1a = S1[ia], s1b = S1[ib], s1c = S1[ic];
     const double s1B = s1b - s1a, s2B = S2[ib] - S2[ia];
@@ -1144,7 +1156,7 @@ a0_k4_quantile_warp(const A0Common c, int32_t layout, const float* __restrict__ 
   if (lane == 0) a0_emit(c, b, __fdiv_rn(total, (float)Ni));
 }
 
-static int g_qh_spec = -1;         // A0_QH_SPEC=0: the sorted QR kernel without the all-action fetch (measured alternative)
+static int g_qh_spec = -1;         // A0_OPT_QH_SPEC = 0: the quantile kernels without the all-action fetch (measured alternative)
 static bool a0_option_qh_spec() {
   if (g_qh_spec < 0) {
     const char* e = getenv("A0_QH_SPEC");
@@ -1152,6 +1164,7 @@ static bool a0_option_qh_spec() {
   }
   return g_qh_spec != 0;
 }
+void a0_set_qh_spec(int on) { g_qh_spec = on != 0; }
 static int g_qh_sorted = -1;
 static int a0_option_qh_sorted() {
   if (g_qh_sorted < 0) {
@@ -1198,7 +1211,7 @@ extern "C" int a0_loss_quantile(const a0_loss_common_t* c, int32_t layout, const
                 taus, qsel, Ni, Nj, grad);
     return A0_OK;
   }
-  if (layout == 1 && qsel && c->A <= QH_SPEC_A && threads <= 64)
+  if (layout == 1 && qsel && c->A <= QH_SPEC_A && threads <= 64 && a0_option_qh_spec())
     A0_LAUNCH(a0_k4_quantile<true>, (unsigned)c->B, (unsigned)threads, 0, (cudaStream_t)stream, 1, A0_PDL_K4, a0_unpack(c), layout, q, qt,
               taus, qsel, Ni, Nj, grad, q_bar, taus_full, fraction_loss, grad_taus);
   else

@@ -110,6 +110,11 @@ const char* a0_last_error(void);
  * longer chain, slower at batch 512); 0 forces the O(N^2) pair loop.  All
  * agree to ~1e-6 relative (different summation order), within the 1e-5 contract.                      */
 #define A0_OPT_QH_SORTED 10
+/* A0_OPT_QH_SPEC (default 1; A0_QH_SPEC in the environment): a0_loss_quantile with qsel given and at most 8
+ * actions fetches every action's quantiles and the selection values in one batch of loads and selects in
+ * registers (the sorted form, and the pair loop of IQN / FQF with at most 64 quantiles); 0 selects the
+ * action first and then fetches its row.  Bit-identical outputs.                                          */
+#define A0_OPT_QH_SPEC 14
 /* A0_OPT_K6_GLOBAL (default 0; A0_K6_GLOBAL in the environment): the LZ4 decode of a0_ex_extend / a0_ex_decode
  * writes its output in place in the scratch buffer (matches read back through L1/L2) instead of staging the
  * entry in shared memory: no shared memory, so every entry of a call is resident at once.  Same bytes, hashes

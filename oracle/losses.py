@@ -98,7 +98,10 @@ def c51_project(p_next, r, d, atoms, vmin, vmax, G):
     m = np.zeros((B, M), dtype=f32)
     for b in range(B):       # index_add_ order: all lo terms, then all up terms
         np.add.at(m[b], lo[b], (p_next[b] * (up[b].astype(f32) - base[b])).astype(f32))
-        np.add.at(m[b], up[b], (p_next[b] * (base[b] - lo[b].astype(f32))).astype(f32))
+        # delta is rounded to fp32, so an atom clamped at vmax can get a base just above M-1 and up == M: that
+        # upper term is dropped (DESIGN section 5)
+        keep = up[b] < M
+        np.add.at(m[b], up[b][keep], (p_next[b] * (base[b] - lo[b].astype(f32))).astype(f32)[keep])
     return m
 
 
@@ -167,8 +170,11 @@ def huber_qr_sorted(qj, Ti, tauj, w):
     (loss [B], grad [B,Nj]) = (huber_qr_loss, _huber_qr_grad).  For a fixed q the sorted targets split
     into four ranges of u = q - T:  u >= 1 (linear, weight 1-tau), 0 < u < 1 (quadratic, 1-tau),
     -1 < u <= 0 (quadratic, tau), u <= -1 (linear, tau); over each range the Huber terms are polynomials
-    in q whose coefficients are prefix sums of T and T^2.  The prefix sums are float64: the quadratic
-    ranges subtract numbers of size T^2 to obtain terms of size (q-T)^2."""
+    in q whose coefficients are prefix sums of T and T^2.  The prefix sums are float64 and centred on the
+    sorted target c at position Ni//2 (sums of T-c and (T-c)^2, polynomial in q-c; both differences are exact
+    for fp32 inputs): the quadratic ranges subtract numbers of size N*(T-c)^2 to obtain terms of size
+    (q-T)^2, where uncentred sums of size N*T^2 lose the 1e-5 contract from |T| ~ 1e5.  The ranges are
+    found on the uncentred values."""
     qj = np.asarray(qj, dtype=np.float64)
     B, Nj = qj.shape
     Ni = Ti.shape[1]
@@ -177,12 +183,13 @@ def huber_qr_sorted(qj, Ti, tauj, w):
     grad = np.zeros((B, Nj), dtype=np.float64)
     for b in range(B):
         T = np.sort(np.asarray(Ti[b], dtype=np.float64))
-        S1 = np.concatenate(([0.0], np.cumsum(T)))
-        S2 = np.concatenate(([0.0], np.cumsum(T * T)))
-        q = qj[b]
-        ia = np.searchsorted(T, q - 1.0, side="right")        # T <= q-1          : u >= 1
-        ib = np.searchsorted(T, q, side="left")               # q-1 < T < q       : 0 < u < 1
-        ic = np.searchsorted(T, q + 1.0, side="left")         # q <= T < q+1      : -1 < u <= 0
+        c = T[Ni // 2]
+        S1 = np.concatenate(([0.0], np.cumsum(T - c)))
+        S2 = np.concatenate(([0.0], np.cumsum((T - c) * (T - c))))
+        ia = np.searchsorted(T, qj[b] - 1.0, side="right")    # T <= q-1          : u >= 1
+        ib = np.searchsorted(T, qj[b], side="left")           # q-1 < T < q       : 0 < u < 1
+        ic = np.searchsorted(T, qj[b] + 1.0, side="left")     # q <= T < q+1      : -1 < u <= 0
+        q = qj[b] - c
         nA, nB, nC, nD = ia, ib - ia, ic - ib, Ni - ic
         s1B, s2B = S1[ib] - S1[ia], S2[ib] - S2[ia]
         s1C, s2C = S1[ic] - S1[ib], S2[ic] - S2[ib]

@@ -48,7 +48,7 @@ def test_argument_errors_do_not_need_a_gpu():
     assert lib.a0_rb_gather_bf16(None, None, 4, 3, 0.99, None, None, 0, None, None, None, None, None, None, None) == -1
     for opt, bad in ((6, 9), (3, 0), (2, 5)):
         assert lib.a0_set_option(opt, bad) == -1
-    for opt, ok in ((4, 1), (5, 1), (6, 4), (7, 0), (8, 1)):
+    for opt, ok in ((4, 1), (5, 1), (6, 4), (7, 0), (8, 1), (14, 1)):
         assert lib.a0_set_option(opt, ok) == 0
     assert lib.a0_set_option(99, 0) == -1 and b"unknown option" in lib.a0_last_error()
 
