@@ -60,6 +60,11 @@ struct a0_replay {
 // A0_EFAULT if a kernel of an earlier call on this handle reported a device-side fault
 int a0_check_fault(a0_replay* h, const char* who);
 uint64_t a0_option_mail_timeout_ns();
+// Raises `kernel`'s dynamic shared-memory limit on `device` (the current device) to at least `bytes`, and with
+// `max_carveout` asks for the largest shared-memory carveout.  The attribute belongs to the function for the whole
+// process, so the record of what was set is process-wide too: one kept per shard or per thread would let a shard of
+// small frames lower the limit that a shard of large frames still relies on.
+int a0_smem_at_least(const void* kernel, int device, size_t bytes, bool max_carveout = false);
 
 void a0_set_error(const char* fmt, ...);
 

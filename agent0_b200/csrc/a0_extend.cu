@@ -327,7 +327,6 @@ struct a0_extend {
   uint8_t* h_stage = nullptr;            // page-locked: descriptors, tail lists, compressed blobs
   uint8_t* d_stage = nullptr;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-  bool smem_set = false;
   std::vector<int64_t> fs8, new_src;
   std::vector<int32_t> tail_src, tail_slot;
   float timing[6] = {0, 0, 0, 0, 0, 0};  // last call, microseconds: stage, wait (decode+label on the device), resolve+plan,
@@ -465,12 +464,9 @@ static int a0_ex_reserve(a0_extend* ex, int32_t mb, size_t stage_bytes, int32_t 
     cudaFree(ex->d_tail_frames); cudaFree(ex->d_tail_hash);
     ex->d_tail_frames = nf; ex->d_tail_hash = nh; ex->slot_cap = cap;
   }
-  if (!ex->smem_set) {
-    A0_CUDA(cudaFuncSetAttribute(a0_k6_lz4_decode_t<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)entry));
-    A0_CUDA(cudaFuncSetAttribute(a0_k6_lz4_decode_t<false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    ex->smem_set = true;
-  }
-  return A0_OK;
+  int dev = 0;
+  A0_CUDA(cudaGetDevice(&dev));
+  return a0_smem_at_least((const void*)a0_k6_lz4_decode_t<false>, dev, entry, true);
 }
 
 // Stages mb blobs (16-byte aligned each) behind their descriptors and launches the decode.

@@ -10,6 +10,10 @@
 #include <stdarg.h>
 #include <stdlib.h>
 
+#include <map>
+#include <mutex>
+#include <utility>
+
 #include "a0_common.cuh"
 
 static thread_local char g_err[512] = "";
@@ -20,6 +24,18 @@ void a0_set_error(const char* fmt, ...) {
   va_end(ap);
 }
 extern "C" const char* a0_last_error(void) { return g_err; }
+
+int a0_smem_at_least(const void* kernel, int device, size_t bytes, bool max_carveout) {
+  static std::mutex mu;
+  static std::map<std::pair<const void*, int>, size_t> set;
+  std::lock_guard<std::mutex> lock(mu);
+  size_t& cur = set[{kernel, device}];
+  if (cur >= bytes) return A0_OK;
+  A0_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+  if (max_carveout) A0_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+  cur = bytes;
+  return A0_OK;
+}
 extern "C" int a0_version(void) { return 101; }
 #ifdef A0_TRACE
 A0_TRACE_SETTER(a0_trace_set_replay)
@@ -177,7 +193,8 @@ extern "C" int a0_rb_create(a0_replay_t** out, int64_t rec_capacity, int64_t fra
              (long long)frame_capacity);
   A0_REQUIRE(frame_bytes > 0 && frame_bytes % 16 == 0, "a0_rb_create: frame_bytes %d must be a positive multiple of 16",
              frame_bytes);
-  A0_REQUIRE((int64_t)frame_bytes * A0_SLOTS <= 200 * 1024, "a0_rb_create: frame_bytes %d too large for the smem-staged gather",
+  A0_REQUIRE((int64_t)frame_bytes * A0_SLOTS <= 200 * 1024,
+             "a0_rb_create: frame_bytes %d is above 25 600 (the gather and the LZ4 kernels stage 8 frames in 200 KB of shared memory)",
              frame_bytes);
   A0DeviceGuard guard(device);
   a0_replay* h = new a0_replay();
@@ -1003,11 +1020,8 @@ static int a0_gather_cvt(a0_replay_t* h, const int64_t* idx, int32_t count, int3
   g.progress = nullptr; g.window = 0; g.gbase = 0; g.gtotal = 0;
   g.l2_hints = 0;
   const size_t smem = (size_t)K3_RING * h->F;
-  static thread_local size_t configured[64] = {0};       // one table per OutT instantiation
-  if (h->device < 64 && configured[h->device] < smem) {
-    A0_CUDA(cudaFuncSetAttribute(a0_k3_gather_cvt<OutT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    configured[h->device] = smem;
-  }
+  int rc = a0_smem_at_least((const void*)a0_k3_gather_cvt<OutT>, h->device, smem);
+  if (rc) return rc;
   A0_LAUNCH(a0_k3_gather_cvt<OutT>, (unsigned)count, K3F_THREADS, smem, (cudaStream_t)stream_, 1, A0_PDL_K3, g, obs_out, next_out,
             (int)norm_mode);
   return A0_OK;
@@ -1030,13 +1044,7 @@ extern "C" int a0_rb_gather_bf16(a0_replay_t* h, const int64_t* idx, int32_t cou
 }
 
 static int a0_k3_smem_attr(a0_replay_t* h, size_t smem) {
-  static thread_local size_t configured[64] = {0};
-  if (h->device < 64 && configured[h->device] < smem) {
-    A0_CUDA(cudaFuncSetAttribute(a0_k3_gather_tma, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    A0_CUDA(cudaFuncSetAttribute(a0_k3_gather_tma, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    configured[h->device] = smem;
-  }
-  return A0_OK;
+  return a0_smem_at_least((const void*)a0_k3_gather_tma, h->device, smem, true);
 }
 // The gather half of a0_rb_sample_gather: variant 0 taking its record positions from the mailbox, always
 // launched with programmatic stream serialization so that it becomes resident under the sampler.
@@ -1096,22 +1104,13 @@ extern "C" int a0_rb_gather(a0_replay_t* h, const int64_t* idx, int32_t count, i
   g.l2_hints = a0_option_k3_l2((int64_t)count * 16 * h->F);
   if (variant == 3) {
     const size_t smem = (size_t)K3S_RING * h->F;
-    static thread_local size_t configured3[64] = {0};
-    if (h->device < 64 && configured3[h->device] < smem) {
-      A0_CUDA(cudaFuncSetAttribute(a0_k3_gather_tma_split, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      configured3[h->device] = smem;
-    }
+    int rc = a0_smem_at_least((const void*)a0_k3_gather_tma_split, h->device, smem);
+    if (rc) return rc;
     A0_LAUNCH(a0_k3_gather_tma_split, (unsigned)count * 2, 32, smem, stream, 1, A0_PDL_K3, g);
   } else if (variant == 0 || variant == 2) {
     const size_t smem = (size_t)(variant == 0 ? K3_RING : A0_SLOTS) * h->F;
-    static thread_local size_t configured[64] = {0};
-    if (variant == 0) {
-      int rc = a0_k3_smem_attr(h, smem);
-      if (rc) return rc;
-    } else if (h->device < 64 && configured[h->device] < smem) {
-      A0_CUDA(cudaFuncSetAttribute(a0_k3_gather_tma_full, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      configured[h->device] = smem;
-    }
+    int rc = variant == 0 ? a0_k3_smem_attr(h, smem) : a0_smem_at_least((const void*)a0_k3_gather_tma_full, h->device, smem);
+    if (rc) return rc;
     if (variant == 0) A0_LAUNCH(a0_k3_gather_tma, (unsigned)count, 32, smem, stream, 1, A0_PDL_K3, g);
     else A0_LAUNCH(a0_k3_gather_tma_full, (unsigned)count, 32, smem, stream, 1, A0_PDL_K3, g);
   } else {

@@ -31,8 +31,8 @@ def _stream(E, T, hw, seed, p_new4=0.1, p_static=0.0):
     """obs[k] u8[E,4,h,w]; ordinary step shifts by one new frame, p_new4: whole new stack,
     p_static: nothing changes (n_new = 0, a paused screen)."""
     rng = np.random.RandomState(seed)
-    h, w = hw
-    obs = [rng.randint(0, 256, (E, 4, h, w)).astype(np.uint8)]
+    shape = tuple(hw)                      # any frame shape: (h, w), (h, w, c)
+    obs = [rng.randint(0, 256, (E, 4) + shape).astype(np.uint8)]
     n_new = []
     for k in range(T):
         cur = obs[-1].copy()
@@ -42,10 +42,10 @@ def _stream(E, T, hw, seed, p_new4=0.1, p_static=0.0):
         kk[(r >= p_new4) & (r < p_new4 + p_static)] = 0
         for e in range(E):
             if kk[e] == 4:
-                cur[e] = rng.randint(0, 256, (4, h, w))
+                cur[e] = rng.randint(0, 256, (4,) + shape)
             elif kk[e] == 1:
                 cur[e, :3] = obs[-1][e, 1:]
-                cur[e, 3] = rng.randint(0, 256, (h, w))
+                cur[e, 3] = rng.randint(0, 256, shape)
         obs.append(cur)
         n_new.append(kk)
     act = rng.randint(0, 18, (T, E)).astype(np.int64)
@@ -79,6 +79,49 @@ def test_nstep_limits_frame_sizes_and_static_screens(n, hw, p_static):
         assert np.array_equal(_np(b.rewards).view(np.int64), r_ref[ref_i].view(np.int64))
         assert np.array_equal(_np(b.terminals), d_ref[ref_i]) and np.array_equal(_np(b.actions), a_ref[ref_i])
     assert rp.index.head_fs == 4 * E + int(n_new.sum())    # one stored frame per NEW frame: static steps store none
+
+
+def test_gather_after_a_smaller_frame_shard_in_another_thread():
+    """K3's shared-memory limits are attributes of the kernels for the whole process: a thread that gathers from a
+    shard of 16-byte frames must not lower them under a shard of 84x84 frames another thread gathers from (a per-thread
+    record of the limits did, and the other thread's next gather failed to launch)."""
+    import threading
+    E = 2
+    obs, n_new, act, rew, done = _stream(E, 6, (84, 84), seed=9)
+    fr_ref = OR.pack_nstep(obs, act, rew, done, 1, 0.99)[0]
+    big = _replay(64, 1, E)
+    big.reset_streams(np.arange(E), obs[0])
+    for k in range(6):
+        new = np.concatenate([obs[k + 1][e, 4 - n_new[k][e]:] for e in range(E) if n_new[k][e]])
+        big.append_steps(np.arange(E), n_new[k], new, act[k], rew[k], done[k])
+    idx = torch.arange(12, device="cuda")
+
+    def gathers(rp):
+        for variant in (0, 2, 3):
+            rp.gather_variant = variant
+            yield variant, _np(rp.gather(idx[:rp.top]).frames)
+        yield "f32", _np(rp.gather(idx[:rp.top], normalized=2).obs)
+
+    for _, fr in gathers(big):
+        assert fr.shape[0] == 12
+    err = []
+
+    def small():
+        try:
+            rp = _replay(64, 1, E, (4, 4))
+            o = _stream(E, 2, (4, 4), seed=1)
+            rp.reset_streams(np.arange(E), o[0][0])
+            rp.append_steps(np.arange(E), [1] * E, o[0][1][:, 3], [0] * E, [0.0] * E, [False] * E)
+            list(gathers(rp))
+        except BaseException as e:          # noqa: BLE001 (re-raised in the main thread)
+            err.append(e)
+
+    t = threading.Thread(target=small)
+    t.start(); t.join()
+    assert not err, err
+    for variant, fr in gathers(big):
+        want = fr_ref[:12] if variant != "f32" else fr_ref[:12, :4 * 7056].astype(np.float32)
+        assert np.array_equal(fr.reshape(12, -1), want), variant
 
 
 def test_ragged_and_empty_calls():

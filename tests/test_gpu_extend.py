@@ -93,9 +93,30 @@ def test_decode_equals_the_oracle(hw, k6_kernel):
         assert got[i].tobytes() == w, f"entry {i} differs"
 
 
+def test_decode_keeps_working_after_a_shard_of_smaller_frames():
+    """K6a's shared-memory limit is an attribute of the kernel for the whole process: a shard of 16-byte frames must not
+    lower it under a shard of 84x84 frames created earlier (a per-shard 'already set' flag did, and the earlier
+    shard's next decode failed to launch)."""
+    z = CP.lz4()
+    rng = np.random.RandomState(3)
+    blobs = {}
+    for hw in ((84, 84), (4, 4)):
+        p = rng.randint(0, 4, 8 * hw[0] * hw[1], dtype=np.uint8).tobytes()
+        blobs[hw] = (z.compress(p), p)
+    big = _replay(64, hw=(84, 84))
+    for rp, hw in ((big, (84, 84)), (_replay(64, hw=(4, 4)), (4, 4)), (big, (84, 84))):
+        out, status = rp.decode_entries([blobs[hw][0]])
+        assert (status == 0).all() and _np(out)[0].tobytes() == blobs[hw][1]
+
+
 def test_decode_reports_malformed_blocks(k6_kernel):
-    hw = (8, 8)
-    total = 8 * 64
+    check_malformed_blocks((8, 8))
+
+
+def check_malformed_blocks(hw):
+    """Truncated blocks, a wrong size prefix, offsets past what has been produced or 0, blocks that decode to more or
+    fewer than 8 frames: K6a reports the oracle's status, and extend() refuses the call and commits nothing."""
+    total = 8 * int(np.prod(hw))
     rp = _replay(64, hw=hw)
     rng = np.random.RandomState(2)
     seqs = _random_sequences(rng, total - 12, [1, 5, 40])

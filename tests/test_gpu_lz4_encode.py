@@ -13,13 +13,13 @@ pytestmark = pytest.mark.gpu
 HW = {16: (4, 4), 7056: (84, 84), 9216: (96, 96)}
 
 
-def _groups(F, kind, count, seed):
+def _groups(F, kind, count, seed, hw=None):
     rng = np.random.RandomState(seed)
     if kind == "noise":
         return [rng.randint(0, 256, 8 * F, dtype=np.uint8).tobytes() for _ in range(count)]
     if kind == "constant":
         return [bytes([int(rng.randint(0, 256))]) * (8 * F) for _ in range(count)]
-    syn = synth_groups(count, seed=seed, hw=HW[F])
+    syn = synth_groups(count, seed=seed, hw=hw or HW[F])
     if kind == "synthetic":
         return syn
     out = []                                   # mixed: frames of a group alternate between Atari-like and noise

@@ -10,6 +10,7 @@ from agent0_b200.synth import SyntheticStreams
 from oracle import cpu_path as CP
 from oracle import lz4_block as LZ
 from oracle import lz4_encode as LE
+from tests.frame_cases import far_blocks, frame_bytes, hw2
 
 
 def _liblz4_decode(blob, size):
@@ -150,6 +151,41 @@ def test_offset_limit_above_64k():
     assert all(s != 65540 for s, _, _ in ms)
     assert any(s == 70000 and off == 100 for s, _, off in ms)
     assert _liblz4_decode(len(d).to_bytes(4, "little") + LE.encode_block(d), len(d)) == bytes(d)
+
+
+@pytest.mark.parametrize("shape", [(64, 128), (16, 513), (64, 64, 3), (160, 160)], ids=["F8192", "F8208", "F12288", "F25600"])
+def test_large_groups_round_trip_and_far_offsets_agree_with_liblz4(shape):
+    """The references of the device LZ4 kernels in the large-group regime: 8F = 65 536 (the largest group of K7's u16
+    table), 65 664, 98 304 and 204 800 bytes.  encode_greedy's blocks of Atari-like, noise and mixed groups decode to the
+    input under oracle/lz4_block.py and liblz4; hand-built blocks with offsets up to 65 535 and a match that ends
+    12 bytes before 8F decode identically under both; blocks whose last match ends exactly at 8F (which K6a accepts
+    and liblz4 refuses) decode under the oracle."""
+    F = frame_bytes(shape)
+    n = 8 * F
+    rng = np.random.RandomState(F)
+    groups = synth_groups(2, seed=F, hw=hw2(shape))
+    mixed = np.frombuffer(groups[0], np.uint8).reshape(8, F).copy()
+    mixed[1::2] = rng.randint(0, 256, (4, F), dtype=np.uint8)
+    groups += [mixed.tobytes(), bytes([9]) * n]
+    for g in groups:
+        blob = LE.encode_greedy(g)
+        assert len(blob) < n
+        assert LZ.decode(blob, n) == g
+        assert _liblz4_decode(blob, n) == g
+        assert all(1 <= off <= LE.MAX_OFFSET for _, _, off in _matches(blob)[0])
+    noise = rng.randint(0, 256, n, dtype=np.uint8).tobytes()
+    assert LE.encode_greedy(noise) == noise                     # stored raw
+    offsets = set()
+    for seqs, end_rules in far_blocks(rng, n):
+        blob, want = LZ.encode_sequences(seqs)
+        assert len(want) == n
+        assert LZ.decode(blob, n) == want
+        if end_rules:
+            assert _liblz4_decode(blob, n) == want
+        offsets |= {off for _, _, off in _matches(blob)[0]}
+    assert max(offsets) == min(n - 4, 65535)
+    if n > 65536:
+        assert {65534, 65535} <= offsets
 
 
 def test_size_within_ten_percent_of_liblz4_on_synthetic_groups():
