@@ -42,6 +42,12 @@ class Plan(C.Structure):
                 ("rec_meta", C.POINTER(_i32)), ("marks", C.POINTER(_i32))]
 
 
+class Merge(C.Structure):
+    """a0_merge_t"""
+    _fields_ = [("n_place", _i64), ("place", C.POINTER(_i64)), ("n_rec", _i64), ("record_map", C.POINTER(_i64)),
+                ("n_tail", _i64), ("tails", C.POINTER(_i64)), ("stride_hint", _i64)]
+
+
 IX_HEAD_Q, IX_TAIL_Q, IX_HEAD_FS, IX_TOP, IX_REC_CAPACITY, IX_FRAME_CAPACITY, IX_NSTEP, IX_AGE_LIMIT, \
     IX_MAX_CHUNK, IX_STATE_WORDS = range(10)
 INGEST_FRAMES_ON_DEVICE, INGEST_FRAMES_PINNED, INGEST_COPY_STREAM = 1, 2, 4
@@ -81,6 +87,9 @@ SIGNATURES = {
     "a0_ckpt_save": (_i32, [_vp, _vp, _vp, C.c_char_p, _vp, _i64, _vp]),
     "a0_ckpt_load": (_i32, [_vp, _vp, _vp, C.c_char_p, _vp, _i64, C.POINTER(_i64), _vp]),
     "a0_ckpt_last_timing": (_i32, [_vp]),
+    "a0_ix_merge": (_i32, [_vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.POINTER(Merge)]),
+    "a0_ckpt_info": (_i32, [C.c_char_p, _vp, _vp, _i64]),
+    "a0_ckpt_merge": (_i32, [_vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _i64, _vp, _vp]),
     "a0_rb_ingest_plan": (_i32, [_vp, C.POINTER(Plan), _vp, _vp, _i32, _f32, _vp]),
     "a0_rb_ingest_steps": (_i32, [_vp, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _i32, _f32, _vp]),
     "a0_rb_ingest_steps_dyn": (_i32, [_vp, _vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _i32, _f32, _f32, _i32, _vp]),

@@ -319,30 +319,158 @@ struct CkReader {
   FILE* f;
   const char* path;
   int64_t size;
+  const char* who;
   int section(uint32_t tag, std::vector<uint8_t>& out, bool check_hash = true) {
     CkSection s;
-    A0_REQUIRE(fread(&s, sizeof(s), 1, f) == 1, "a0_ckpt_load: %s is truncated (section %u)", path, tag);
-    A0_REQUIRE(s.tag == tag && s.zero == 0, "a0_ckpt_load: %s: expected section %u, found %u", path, tag, s.tag);
-    A0_REQUIRE(s.len <= (uint64_t)(size - ftell(f)), "a0_ckpt_load: %s is truncated (section %u)", path, tag);
+    A0_REQUIRE(fread(&s, sizeof(s), 1, f) == 1, "%s: %s is truncated (section %u)", who, path, tag);
+    A0_REQUIRE(s.tag == tag && s.zero == 0, "%s: %s: expected section %u, found %u", who, path, tag, s.tag);
+    A0_REQUIRE(s.len <= (uint64_t)(size - ftell(f)), "%s: %s is truncated (section %u)", who, path, tag);
     out.resize((size_t)s.len);
-    A0_REQUIRE(s.len == 0 || fread(out.data(), 1, (size_t)s.len, f) == (size_t)s.len, "a0_ckpt_load: %s is truncated", path);
-    A0_REQUIRE(!check_hash || ck_hash(out.data(), out.size()) == s.hash, "a0_ckpt_load: %s: section %u is corrupt (hash)", path, tag);
+    A0_REQUIRE(s.len == 0 || fread(out.data(), 1, (size_t)s.len, f) == (size_t)s.len, "%s: %s is truncated", who, path);
+    A0_REQUIRE(!check_hash || ck_hash(out.data(), out.size()) == s.hash, "%s: %s: section %u is corrupt (hash)", who, path, tag);
     return A0_OK;
   }
 };
+
+// One checkpoint file, read and validated up to the BLOBS payload (where the file position stays).  a0_ckpt_load,
+// a0_ckpt_merge and a0_ckpt_info share it, so every file is validated by the same code.
+struct CkData {
+  CkFile file;
+  CkReader rd{nullptr, nullptr, 0, nullptr};
+  CkHeader hd;
+  std::vector<uint8_t> index_b, rec_b, leaf_b, sc_b, tail_b, user_b, frames_b;
+  CkSection bs;
+  std::vector<int64_t> tab;
+  std::vector<uint64_t> fh;
+  std::unique_ptr<a0_index_t, int (*)(a0_index_t*)> ix{nullptr, a0_ix_destroy};     // the file's index, validated
+};
+
+// the header: magic and version
+int ck_open(const char* who, const char* path, CkData& d) {
+  d.file.f = fopen(path, "rb");
+  A0_REQUIRE(d.file.f, "%s: cannot open %s", who, path);
+  struct stat sb;
+  A0_REQUIRE(fstat(fileno(d.file.f), &sb) == 0, "%s: cannot stat %s", who, path);
+  d.rd = CkReader{d.file.f, path, (int64_t)sb.st_size, who};
+  CkHeader& hd = d.hd;
+  A0_REQUIRE(fread(&hd, sizeof(hd), 1, d.file.f) == 1, "%s: %s is truncated (header)", who, path);
+  A0_REQUIRE(memcmp(hd.magic, A0_CK_MAGIC, 8) == 0, "%s: %s is not a shard checkpoint (bad magic)", who, path);
+  A0_REQUIRE(hd.version == A0_CK_VERSION && hd.zero == 0, "%s: %s has format version %u, this library reads %u", who, path,
+             hd.version, A0_CK_VERSION);
+  return A0_OK;
+}
+
+// a header read from a file that is not compared with a shard of the same shape: its sizes must at least fit the file
+int ck_plausible(const char* who, CkData& d) {
+  const CkHeader& hd = d.hd;
+  A0_REQUIRE(hd.N >= 2 && hd.NF >= 8 && hd.F > 0 && hd.F % 16 == 0 && hd.n_step >= 1 && hd.n_step <= A0_MAX_NSTEP &&
+                 hd.age_limit >= 0 && hd.N <= d.rd.size / 61,
+             "%s: %s has an implausible header (N=%lld NF=%lld F=%lld n_step=%lld)", who, d.rd.path, (long long)hd.N,
+             (long long)hd.NF, (long long)hd.F, (long long)hd.n_step);
+  return A0_OK;
+}
+
+// the INDEX section into a scratch index of the header's parameters
+int ck_read_index(CkData& d) {
+  const CkHeader& hd = d.hd;
+  int rc = d.rd.section(CK_INDEX, d.index_b);
+  if (rc) return rc;
+  a0_index_t* tix = nullptr;
+  if ((rc = a0_ix_create(&tix, hd.N, hd.NF, (int32_t)hd.n_step, hd.age_limit))) return rc;
+  d.ix.reset(tix);
+  return a0_ix_deserialize(tix, d.index_b.data(), (int64_t)d.index_b.size());
+}
+
+// everything after the header, validated before anything is touched
+int ck_read(const char* who, CkData& d) {
+  const char* path = d.rd.path;
+  FILE* f = d.file.f;
+  CkReader& rd = d.rd;
+  const int64_t N = d.hd.N, NF = d.hd.NF, F = d.hd.F;
+  int rc;
+  if ((rc = rd.section(CK_INDEX, d.index_b)) || (rc = rd.section(CK_RECORDS, d.rec_b)) || (rc = rd.section(CK_LEAVES, d.leaf_b)) ||
+      (rc = rd.section(CK_SCALARS, d.sc_b)) || (rc = rd.section(CK_TAILS, d.tail_b)) || (rc = rd.section(CK_USER, d.user_b)) ||
+      (rc = rd.section(CK_FRAMES, d.frames_b)))
+    return rc;
+  CkSection& bs = d.bs;
+  A0_REQUIRE(fread(&bs, sizeof(bs), 1, f) == 1 && bs.tag == CK_BLOBS && bs.zero == 0, "%s: %s is truncated (blobs)", who, path);
+  A0_REQUIRE(bs.len == (uint64_t)(rd.size - ftell(f)), "%s: %s has %lld blob bytes, the section says %llu", who, path,
+             (long long)(rd.size - ftell(f)), (unsigned long long)bs.len);
+
+  // the index, on a scratch copy
+  a0_index_t* tix = nullptr;
+  if ((rc = a0_ix_create(&tix, N, NF, (int32_t)d.hd.n_step, d.hd.age_limit))) return rc;
+  d.ix.reset(tix);
+  if ((rc = a0_ix_deserialize(tix, d.index_b.data(), (int64_t)d.index_b.size()))) return rc;
+  int64_t ts[A0_IX_STATE_WORDS];
+  a0_ix_state(tix, ts);
+  const uint8_t* samp = a0_ix_sampleable(tix);
+  const int64_t hq = ts[A0_IX_HEAD_Q], tq = ts[A0_IX_TAIL_Q], head_fs = ts[A0_IX_HEAD_FS];
+  A0_REQUIRE(d.rec_b.size() == (size_t)N * (A0_SLOTS * 4 + sizeof(A0RecInfo)) && d.leaf_b.size() == (size_t)N * 4 && d.sc_b.size() == 32,
+             "%s: %s: a section has the wrong size", who, path);
+  const int32_t* slots = reinterpret_cast<const int32_t*>(d.rec_b.data());
+  const A0RecInfo* info = reinterpret_cast<const A0RecInfo*>(d.rec_b.data() + (size_t)N * A0_SLOTS * 4);
+  const int64_t resident = std::min(head_fs, NF);
+  auto live = [&](int64_t pos) { return (pos - tq % N + N) % N < hq - tq; };
+  for (int64_t q = tq; q < hq; ++q) {
+    const int64_t pos = q % N;
+    for (int j = 0; j < A0_SLOTS; ++j)
+      A0_REQUIRE(slots[pos * A0_SLOTS + j] >= 0 && slots[pos * A0_SLOTS + j] < resident,
+                 "%s: %s: record %lld names frame slot %d outside the resident window", who, path, (long long)pos,
+                 slots[pos * A0_SLOTS + j]);
+    const int32_t link = info[pos].link;
+    A0_REQUIRE(link == -1 || (link >= 0 && link < N && live(link)), "%s: %s: record %lld links to %d, not a live record", who, path,
+               (long long)pos, link);
+  }
+  const float* leaves = reinterpret_cast<const float*>(d.leaf_b.data());
+  for (int64_t i = 0; i < N; ++i)
+    A0_REQUIRE(std::isfinite(leaves[i]) && leaves[i] >= 0.0f && (samp[i] || leaves[i] == 0.0f),
+               "%s: %s: priority %lld is %g (finite, >= 0, and 0 for a record that is not sampleable)", who, path, (long long)i,
+               (double)leaves[i]);
+  {
+    float sc[4];
+    int64_t sh;
+    memcpy(sc, d.sc_b.data(), 16);
+    memcpy(&sh, d.sc_b.data() + 24, 8);
+    for (float x : sc) A0_REQUIRE(std::isfinite(x), "%s: %s: a saved scalar is not finite", who, path);
+    A0_REQUIRE(sc[0] >= 0.0f && sh >= 0 && sh < N, "%s: %s: bad max_p or stride hint", who, path);
+  }
+  if ((rc = a0_ex_tails_check((int32_t)F, d.tail_b.data(), (int64_t)d.tail_b.size(), head_fs))) return rc;
+  // the group table
+  A0_REQUIRE(d.frames_b.size() >= 24, "%s: %s: frames section truncated", who, path);
+  std::vector<int64_t>& tab = d.tab;
+  tab.resize(3);
+  memcpy(tab.data(), d.frames_b.data(), 24);
+  const int64_t lo = std::max<int64_t>(0, head_fs - NF), nfr = head_fs - lo, G = (nfr + 7) / 8;
+  A0_REQUIRE(tab[0] == lo && tab[1] == nfr && tab[2] == G && d.frames_b.size() == (size_t)(24 + 16 * G + 64 * G),
+             "%s: %s: the frame table does not match the index", who, path);
+  tab.resize((size_t)(3 + 2 * G));
+  memcpy(tab.data(), d.frames_b.data(), (size_t)(3 + 2 * G) * 8);
+  d.fh.resize((size_t)G * A0_SLOTS);
+  memcpy(d.fh.data(), d.frames_b.data() + (size_t)(3 + 2 * G) * 8, d.fh.size() * 8);
+  const int64_t maxlen = (int64_t)A0_SLOTS * F;
+  uint64_t total = 0;
+  for (int64_t g = 0; g < G; ++g) {
+    A0_REQUIRE(tab[3 + 2 * g] == (lo + 8 * g) % NF && tab[4 + 2 * g] > 4 && tab[4 + 2 * g] <= maxlen,
+               "%s: %s: frame group %lld has a bad table entry", who, path, (long long)g);
+    total += (uint64_t)tab[4 + 2 * g];
+  }
+  A0_REQUIRE(total == bs.len, "%s: %s: the group table covers %llu blob bytes, the file holds %llu", who, path,
+             (unsigned long long)total, (unsigned long long)bs.len);
+  return A0_OK;
+}
 }  // namespace
 
 // everything after the shard was touched: on failure, shard, index and tails go back to freshly created
-static int ck_restore(a0_replay* h, a0_index_t* ix, a0_extend* ex, bool tails, const std::vector<uint8_t>& index_b,
-                      const std::vector<uint8_t>& rec_b, const std::vector<uint8_t>& leaf_b, const std::vector<uint8_t>& sc_b,
-                      const std::vector<uint8_t>& tail_b, const std::vector<int64_t>& tab, const std::vector<uint64_t>& fh,
-                      CkReader& rd, uint64_t blob_len, uint64_t blob_hash, cudaStream_t cs) {
+static int ck_restore(a0_replay* h, a0_index_t* ix, a0_extend* ex, bool tails, CkData& d, cudaStream_t cs) {
   const int64_t N = h->N, F = h->F;
+  CkReader& rd = d.rd;
+  const std::vector<int64_t>& tab = d.tab;
   int rc = a0_rb_reset(h, cs);
   if (rc) return rc;
-  if ((rc = a0_ix_deserialize(ix, index_b.data(), (int64_t)index_b.size()))) return rc;
-  A0_CUDA(cudaMemcpyAsync(h->rec_slots, rec_b.data(), (size_t)N * A0_SLOTS * 4, cudaMemcpyHostToDevice, cs));
-  A0_CUDA(cudaMemcpyAsync(h->rec_info, rec_b.data() + (size_t)N * A0_SLOTS * 4, (size_t)N * sizeof(A0RecInfo), cudaMemcpyHostToDevice, cs));
+  if ((rc = a0_ix_deserialize(ix, d.index_b.data(), (int64_t)d.index_b.size()))) return rc;
+  A0_CUDA(cudaMemcpyAsync(h->rec_slots, d.rec_b.data(), (size_t)N * A0_SLOTS * 4, cudaMemcpyHostToDevice, cs));
+  A0_CUDA(cudaMemcpyAsync(h->rec_info, d.rec_b.data() + (size_t)N * A0_SLOTS * 4, (size_t)N * sizeof(A0RecInfo), cudaMemcpyHostToDevice, cs));
   {
     CkDev d_idx, d_val;
     std::vector<int64_t> idx((size_t)N);
@@ -350,16 +478,16 @@ static int ck_restore(a0_replay* h, a0_index_t* ix, a0_extend* ex, bool tails, c
     A0_CUDA(cudaMalloc(&d_idx.p, (size_t)N * 8));
     A0_CUDA(cudaMalloc(&d_val.p, (size_t)N * 4));
     A0_CUDA(cudaMemcpyAsync(d_idx.p, idx.data(), (size_t)N * 8, cudaMemcpyHostToDevice, cs));
-    A0_CUDA(cudaMemcpyAsync(d_val.p, leaf_b.data(), (size_t)N * 4, cudaMemcpyHostToDevice, cs));
+    A0_CUDA(cudaMemcpyAsync(d_val.p, d.leaf_b.data(), (size_t)N * 4, cudaMemcpyHostToDevice, cs));
     if ((rc = a0_pt_set(h, static_cast<const int64_t*>(d_idx.p), static_cast<const float*>(d_val.p), (int32_t)N, cs))) return rc;
     A0_CUDA(cudaStreamSynchronize(cs));
   }
-  A0_CUDA(cudaMemcpyAsync(h->max_p, sc_b.data(), 4, cudaMemcpyHostToDevice, cs));
-  A0_CUDA(cudaMemcpyAsync(h->dyn, sc_b.data() + 4, 12, cudaMemcpyHostToDevice, cs));
-  A0_CUDA(cudaMemcpyAsync(h->counter + A0_RNG_CALL_WORD, sc_b.data() + 16, 8, cudaMemcpyHostToDevice, cs));
-  memcpy(&h->stride_hint, sc_b.data() + 24, 8);
+  A0_CUDA(cudaMemcpyAsync(h->max_p, d.sc_b.data(), 4, cudaMemcpyHostToDevice, cs));
+  A0_CUDA(cudaMemcpyAsync(h->dyn, d.sc_b.data() + 4, 12, cudaMemcpyHostToDevice, cs));
+  A0_CUDA(cudaMemcpyAsync(h->counter + A0_RNG_CALL_WORD, d.sc_b.data() + 16, 8, cudaMemcpyHostToDevice, cs));
+  memcpy(&h->stride_hint, d.sc_b.data() + 24, 8);
   A0_CUDA(cudaStreamSynchronize(cs));
-  if (tails && (rc = a0_ex_tails_load(ex, tail_b.data(), (int64_t)tail_b.size(), cs))) return rc;
+  if (tails && (rc = a0_ex_tails_load(ex, d.tail_b.data(), (int64_t)d.tail_b.size(), cs))) return rc;
   // frames: K6a straight into the ring, batch by batch, every frame's hash compared with the saved one
   const int64_t lo = tab[0], nfr = tab[1], G = tab[2], head_fs = lo + nfr;
   CkHash bh;
@@ -382,7 +510,7 @@ static int ck_restore(a0_replay* h, a0_index_t* ix, a0_extend* ex, bool tails, c
       A0_REQUIRE(status[i] == 0, "a0_ckpt_load: %s: frame group %lld does not decode (status %d)", rd.path, (long long)(g0 + i), status[i]);
     A0_CUDA(cudaMemcpyAsync(got.data(), dh, (size_t)mb * A0_SLOTS * 8, cudaMemcpyDeviceToHost, cs));
     A0_CUDA(cudaStreamSynchronize(cs));
-    A0_REQUIRE(memcmp(got.data(), fh.data() + (size_t)g0 * A0_SLOTS, (size_t)mb * A0_SLOTS * 8) == 0,
+    A0_REQUIRE(memcmp(got.data(), d.fh.data() + (size_t)g0 * A0_SLOTS, (size_t)mb * A0_SLOTS * 8) == 0,
                "a0_ckpt_load: %s: a decoded frame of groups %lld.. differs from the saved one (hash)", rd.path, (long long)g0);
     const int64_t s0 = lo + 8 * g0, s1 = std::min<int64_t>(s0 + 8 * (int64_t)mb, head_fs);
     if ((rc = ck_ring_copy(h, const_cast<uint8_t*>(dec), s0, s1, true, cs))) return rc;
@@ -391,10 +519,22 @@ static int ck_restore(a0_replay* h, a0_index_t* ix, a0_extend* ex, bool tails, c
     g_timing[3] += ck_us(b, ck_clock::now());
     g_timing[5] += (double)bytes;
   }
-  A0_REQUIRE(bh.final() == blob_hash && bh.total == blob_len, "a0_ckpt_load: %s: the frame blobs are corrupt (hash)", rd.path);
+  A0_REQUIRE(bh.final() == d.bs.hash && bh.total == d.bs.len, "a0_ckpt_load: %s: the frame blobs are corrupt (hash)", rd.path);
   g_timing[4] = (double)nfr * F;
-  (void)F;
   return A0_OK;
+}
+
+// a failure after the shard was touched: shard, index and tails back to freshly created
+static int ck_reset_all(a0_replay* h, a0_index_t* ix, a0_extend* ex, cudaStream_t cs) {
+  const std::string msg = a0_last_error();
+  cudaStreamSynchronize(cs);
+  a0_rb_reset(h, cs);
+  cudaStreamSynchronize(cs);
+  h->stride_hint = 0;
+  a0_ix_clear(ix);
+  if (ex) a0_ex_tails_clear(ex);
+  a0_set_error("%s (the shard was reset to empty)", msg.c_str());
+  return A0_EINVAL;
 }
 
 extern "C" int a0_ckpt_load(a0_replay_t* h, a0_index_t* ix, a0_extend_t* ex, const char* path, uint8_t* user_out,
@@ -413,114 +553,266 @@ extern "C" int a0_ckpt_load(a0_replay_t* h, a0_index_t* ix, a0_extend_t* ex, con
   int rc = a0_ix_state(ix, st);
   if (rc) return rc;
   A0_REQUIRE(st[A0_IX_REC_CAPACITY] == h->N && st[A0_IX_FRAME_CAPACITY] == h->NF, "a0_ckpt_load: index and shard capacities differ");
-  CkFile file;
-  file.f = fopen(path, "rb");
-  A0_REQUIRE(file.f, "a0_ckpt_load: cannot open %s", path);
-  struct stat sb;
-  A0_REQUIRE(fstat(fileno(file.f), &sb) == 0, "a0_ckpt_load: cannot stat %s", path);
-  CkReader rd{file.f, path, (int64_t)sb.st_size};
-  CkHeader hd;
-  A0_REQUIRE(fread(&hd, sizeof(hd), 1, file.f) == 1, "a0_ckpt_load: %s is truncated (header)", path);
-  A0_REQUIRE(memcmp(hd.magic, A0_CK_MAGIC, 8) == 0, "a0_ckpt_load: %s is not a shard checkpoint (bad magic)", path);
-  A0_REQUIRE(hd.version == A0_CK_VERSION && hd.zero == 0, "a0_ckpt_load: %s has format version %u, this library reads %u", path,
-             hd.version, A0_CK_VERSION);
+  CkData d;
+  if ((rc = ck_open("a0_ckpt_load", path, d))) return rc;
+  const CkHeader& hd = d.hd;
   const int64_t N = h->N, NF = h->NF, F = h->F;
   A0_REQUIRE(hd.N == N && hd.NF == NF && hd.F == F && hd.P == h->P && hd.n_step == st[A0_IX_NSTEP] && hd.age_limit == st[A0_IX_AGE_LIMIT],
              "a0_ckpt_load: %s holds a shard of N=%lld NF=%lld F=%lld n_step=%lld age_limit=%lld; this one has %lld %lld %lld %lld %lld",
              path, (long long)hd.N, (long long)hd.NF, (long long)hd.F, (long long)hd.n_step, (long long)hd.age_limit, (long long)N,
              (long long)NF, (long long)F, (long long)st[A0_IX_NSTEP], (long long)st[A0_IX_AGE_LIMIT]);
-  std::vector<uint8_t> index_b, rec_b, leaf_b, sc_b, tail_b, user_b, frames_b;
-  if ((rc = rd.section(CK_INDEX, index_b)) || (rc = rd.section(CK_RECORDS, rec_b)) || (rc = rd.section(CK_LEAVES, leaf_b)) ||
-      (rc = rd.section(CK_SCALARS, sc_b)) || (rc = rd.section(CK_TAILS, tail_b)) || (rc = rd.section(CK_USER, user_b)) ||
-      (rc = rd.section(CK_FRAMES, frames_b)))
-    return rc;
-  CkSection bs;
-  A0_REQUIRE(fread(&bs, sizeof(bs), 1, file.f) == 1 && bs.tag == CK_BLOBS && bs.zero == 0, "a0_ckpt_load: %s is truncated (blobs)", path);
-  A0_REQUIRE(bs.len == (uint64_t)(rd.size - ftell(file.f)), "a0_ckpt_load: %s has %lld blob bytes, the section says %llu", path,
-             (long long)(rd.size - ftell(file.f)), (unsigned long long)bs.len);
-
-  // ---- validation, before anything is touched
-  // the index, on a scratch copy
-  a0_index_t* tix = nullptr;
-  if ((rc = a0_ix_create(&tix, N, NF, (int32_t)st[A0_IX_NSTEP], st[A0_IX_AGE_LIMIT]))) return rc;
-  std::unique_ptr<a0_index_t, int (*)(a0_index_t*)> tix_owner(tix, a0_ix_destroy);
-  if ((rc = a0_ix_deserialize(tix, index_b.data(), (int64_t)index_b.size()))) return rc;
-  int64_t ts[A0_IX_STATE_WORDS];
-  a0_ix_state(tix, ts);
-  const uint8_t* samp = a0_ix_sampleable(tix);
-  const int64_t hq = ts[A0_IX_HEAD_Q], tq = ts[A0_IX_TAIL_Q], head_fs = ts[A0_IX_HEAD_FS];
-  A0_REQUIRE(rec_b.size() == (size_t)N * (A0_SLOTS * 4 + sizeof(A0RecInfo)) && leaf_b.size() == (size_t)N * 4 && sc_b.size() == 32,
-             "a0_ckpt_load: %s: a section has the wrong size", path);
-  const int32_t* slots = reinterpret_cast<const int32_t*>(rec_b.data());
-  const A0RecInfo* info = reinterpret_cast<const A0RecInfo*>(rec_b.data() + (size_t)N * A0_SLOTS * 4);
-  const int64_t resident = std::min(head_fs, NF);
-  auto live = [&](int64_t pos) { return (pos - tq % N + N) % N < hq - tq; };
-  for (int64_t q = tq; q < hq; ++q) {
-    const int64_t pos = q % N;
-    for (int j = 0; j < A0_SLOTS; ++j)
-      A0_REQUIRE(slots[pos * A0_SLOTS + j] >= 0 && slots[pos * A0_SLOTS + j] < resident,
-                 "a0_ckpt_load: %s: record %lld names frame slot %d outside the resident window", path, (long long)pos,
-                 slots[pos * A0_SLOTS + j]);
-    const int32_t link = info[pos].link;
-    A0_REQUIRE(link == -1 || (link >= 0 && link < N && live(link)), "a0_ckpt_load: %s: record %lld links to %d, not a live record", path,
-               (long long)pos, link);
-  }
-  const float* leaves = reinterpret_cast<const float*>(leaf_b.data());
-  for (int64_t i = 0; i < N; ++i)
-    A0_REQUIRE(std::isfinite(leaves[i]) && leaves[i] >= 0.0f && (samp[i] || leaves[i] == 0.0f),
-               "a0_ckpt_load: %s: priority %lld is %g (finite, >= 0, and 0 for a record that is not sampleable)", path, (long long)i,
-               (double)leaves[i]);
-  {
-    float sc[4];
-    int64_t sh;
-    memcpy(sc, sc_b.data(), 16);
-    memcpy(&sh, sc_b.data() + 24, 8);
-    for (float x : sc) A0_REQUIRE(std::isfinite(x), "a0_ckpt_load: %s: a saved scalar is not finite", path);
-    A0_REQUIRE(sc[0] >= 0.0f && sh >= 0 && sh < N, "a0_ckpt_load: %s: bad max_p or stride hint", path);
-  }
-  if ((rc = a0_ex_tails_check((int32_t)F, tail_b.data(), (int64_t)tail_b.size(), head_fs))) return rc;
-  // the group table
-  A0_REQUIRE(frames_b.size() >= 24, "a0_ckpt_load: %s: frames section truncated", path);
-  std::vector<int64_t> tab(3);
-  memcpy(tab.data(), frames_b.data(), 24);
-  const int64_t lo = std::max<int64_t>(0, head_fs - NF), nfr = head_fs - lo, G = (nfr + 7) / 8;
-  A0_REQUIRE(tab[0] == lo && tab[1] == nfr && tab[2] == G && frames_b.size() == (size_t)(24 + 16 * G + 64 * G),
-             "a0_ckpt_load: %s: the frame table does not match the index", path);
-  tab.resize((size_t)(3 + 2 * G));
-  memcpy(tab.data(), frames_b.data(), (size_t)(3 + 2 * G) * 8);
-  std::vector<uint64_t> fh((size_t)G * A0_SLOTS);
-  memcpy(fh.data(), frames_b.data() + (size_t)(3 + 2 * G) * 8, fh.size() * 8);
-  const int64_t maxlen = (int64_t)A0_SLOTS * F;
-  uint64_t total = 0;
-  for (int64_t g = 0; g < G; ++g) {
-    A0_REQUIRE(tab[3 + 2 * g] == (lo + 8 * g) % NF && tab[4 + 2 * g] > 4 && tab[4 + 2 * g] <= maxlen,
-               "a0_ckpt_load: %s: frame group %lld has a bad table entry", path, (long long)g);
-    total += (uint64_t)tab[4 + 2 * g];
-  }
-  A0_REQUIRE(total == bs.len, "a0_ckpt_load: %s: the group table covers %llu blob bytes, the file holds %llu", path,
-             (unsigned long long)total, (unsigned long long)bs.len);
-  A0_REQUIRE(user_b.empty() || (user_out && user_cap >= (int64_t)user_b.size()), "a0_ckpt_load: the user buffer needs %lld bytes",
-             (long long)user_b.size());
+  if ((rc = ck_read("a0_ckpt_load", d))) return rc;
+  A0_REQUIRE(d.user_b.empty() || (user_out && user_cap >= (int64_t)d.user_b.size()), "a0_ckpt_load: the user buffer needs %lld bytes",
+             (long long)d.user_b.size());
   g_timing[1] = ck_us(t0, ck_clock::now());
 
   // ---- restore; from here a failure leaves everything as freshly created
   a0_extend_t* own = nullptr;
   if (!ex && (rc = a0_ex_create(&own, h, ix))) return rc;
   std::unique_ptr<a0_extend_t, int (*)(a0_extend_t*)> own_owner(own, a0_ex_destroy);
-  rc = ck_restore(h, ix, ex ? ex : own, ex != nullptr, index_b, rec_b, leaf_b, sc_b, tail_b, tab, fh, rd, bs.len, bs.hash, cs);
-  if (rc) {
-    const std::string msg = a0_last_error();
-    cudaStreamSynchronize(cs);
-    a0_rb_reset(h, cs);
-    cudaStreamSynchronize(cs);
-    h->stride_hint = 0;
-    a0_ix_clear(ix);
-    if (ex) a0_ex_tails_clear(ex);
-    a0_set_error("%s (the shard was reset to empty)", msg.c_str());
-    return A0_EINVAL;
+  rc = ck_restore(h, ix, ex ? ex : own, ex != nullptr, d, cs);
+  if (rc) return ck_reset_all(h, ix, ex, cs);
+  if (user_len_out) *user_len_out = (int64_t)d.user_b.size();
+  if (!d.user_b.empty()) memcpy(user_out, d.user_b.data(), d.user_b.size());
+  g_timing[0] = ck_us(t0, ck_clock::now());
+  return A0_OK;
+}
+
+extern "C" int a0_ckpt_info(const char* path, int64_t* out8, int64_t* ids_out, int64_t ids_cap) {
+  A0_REQUIRE(path && out8 && (ids_cap == 0 || ids_out), "a0_ckpt_info: NULL argument");
+  CkData d;
+  int rc = ck_open("a0_ckpt_info", path, d);
+  if (rc || (rc = ck_plausible("a0_ckpt_info", d)) || (rc = ck_read_index(d))) return rc;
+  int64_t st[A0_IX_STATE_WORDS];
+  a0_ix_state(d.ix.get(), st);
+  std::vector<int64_t> ids;
+  a0_ix_stream_ids(d.ix.get(), ids);
+  const int64_t v[8] = {d.hd.N, d.hd.NF, d.hd.F, d.hd.n_step, d.hd.age_limit, st[A0_IX_HEAD_Q] - st[A0_IX_TAIL_Q], st[A0_IX_TOP],
+                        (int64_t)ids.size()};
+  memcpy(out8, v, sizeof(v));
+  A0_REQUIRE(ids_cap >= (int64_t)ids.size(), "a0_ckpt_info: %s has %lld streams, the id buffer takes %lld", path, (long long)ids.size(),
+             (long long)ids_cap);
+  if (!ids.empty()) memcpy(ids_out, ids.data(), ids.size() * 8);
+  return A0_OK;
+}
+
+// ---- a0_ckpt_merge ---------------------------------------------------------------------------------------------
+// the placed frames of one file: its BLOBS section read once, sequentially, and hashed whole; of each batch of
+// CK_BATCH groups only those holding a placed frame are decoded (K6a into the ingest scratch), their hashes checked,
+// and the placed frames copied to their target slots by K1's source-indexed copy
+static int ck_place_file(a0_replay* h, a0_extend* ex, CkData& d, const std::vector<std::pair<int64_t, int32_t>>& place,
+                         cudaStream_t cs, cudaEvent_t e0, cudaEvent_t e1) {
+  const std::vector<int64_t>& tab = d.tab;
+  const int64_t lo = tab[0], G = tab[2];
+  CkHash bh;
+  std::vector<uint8_t> raw, blobs;
+  std::vector<int64_t> lens, src;
+  std::vector<int32_t> pos, gsel;
+  std::vector<unsigned long long> got((size_t)CK_BATCH * A0_SLOTS);
+  size_t pi = 0;             // place: (source seq, target slot), ascending source seq
+  for (int64_t g0 = 0; g0 < G; g0 += CK_BATCH) {
+    const int32_t mb = (int32_t)std::min<int64_t>(CK_BATCH, G - g0);
+    std::vector<size_t> off((size_t)mb + 1, 0);
+    for (int32_t i = 0; i < mb; ++i) off[i + 1] = off[i] + (size_t)tab[4 + 2 * (g0 + i)];
+    raw.resize(off[mb]);
+    const auto a = ck_clock::now();
+    A0_REQUIRE(fread(raw.data(), 1, raw.size(), d.rd.f) == raw.size(), "a0_ckpt_merge: %s is truncated (blobs)", d.rd.path);
+    bh.update(raw.data(), raw.size());
+    g_timing[7] += ck_us(a, ck_clock::now());
+    // the groups of this batch that hold a placed frame
+    gsel.clear(); blobs.clear(); lens.clear(); src.clear(); pos.clear();
+    const int64_t s_end = lo + 8 * (g0 + mb);
+    while (pi < place.size() && place[pi].first < s_end) {
+      const int64_t g = (place[pi].first - lo) / 8 - g0;
+      if (gsel.empty() || gsel.back() != (int32_t)g) {
+        gsel.push_back((int32_t)g);
+        blobs.insert(blobs.end(), raw.begin() + off[g], raw.begin() + off[g + 1]);
+        lens.push_back((int64_t)(off[g + 1] - off[g]));
+      }
+      src.push_back((int64_t)(gsel.size() - 1) * A0_SLOTS + (place[pi].first - lo) % 8);
+      pos.push_back(place[pi].second);
+      ++pi;
+    }
+    if (gsel.empty()) continue;
+    const int32_t nd = (int32_t)gsel.size();
+    A0_CUDA(cudaEventRecord(e0, cs));
+    const uint8_t* dec; const unsigned long long* dh; const int32_t* status;
+    int rc = a0_ex_decode_dev(ex, blobs.data(), lens.data(), nd, cs, &dec, &dh, &status);
+    if (rc) return rc;
+    for (int32_t i = 0; i < nd; ++i)
+      A0_REQUIRE(status[i] == 0, "a0_ckpt_merge: %s: frame group %lld does not decode (status %d)", d.rd.path, (long long)(g0 + gsel[i]),
+                 status[i]);
+    A0_CUDA(cudaMemcpyAsync(got.data(), dh, (size_t)nd * A0_SLOTS * 8, cudaMemcpyDeviceToHost, cs));
+    A0_CUDA(cudaStreamSynchronize(cs));
+    for (int32_t i = 0; i < nd; ++i)
+      A0_REQUIRE(memcmp(got.data() + (size_t)i * A0_SLOTS, d.fh.data() + (size_t)(g0 + gsel[i]) * A0_SLOTS, A0_SLOTS * 8) == 0,
+                 "a0_ckpt_merge: %s: a decoded frame of group %lld differs from the saved one (hash)", d.rd.path, (long long)(g0 + gsel[i]));
+    a0_plan_t plan = {0, (int32_t)pos.size(), 0, pos.data(), nullptr, nullptr};
+    const A0Dyn none = {nullptr, 0.0f, 0.0f, 0.0f};
+    if ((rc = a0_ingest_plan_impl(h, &plan, dec, src.data(), A0_INGEST_FRAMES_ON_DEVICE, 0.0f, (a0_stream_t)cs, none))) return rc;
+    A0_CUDA(cudaEventRecord(e1, cs));
+    A0_CUDA(cudaStreamSynchronize(cs));
+    float ms = 0.0f;
+    cudaEventElapsedTime(&ms, e0, e1);
+    g_timing[3] += ms * 1e3;
+    g_timing[5] += (double)nd * A0_SLOTS * h->F;
+    g_timing[6] += (double)pos.size() * h->F;
   }
-  if (user_len_out) *user_len_out = (int64_t)user_b.size();
-  if (!user_b.empty()) memcpy(user_out, user_b.data(), user_b.size());
+  A0_REQUIRE(pi == place.size(), "a0_ckpt_merge: %s: a placed frame lies outside the file's frame groups", d.rd.path);
+  A0_REQUIRE(bh.final() == d.bs.hash && bh.total == d.bs.len, "a0_ckpt_merge: %s: the frame blobs are corrupt (hash)", d.rd.path);
+  return A0_OK;
+}
+
+extern "C" int a0_ckpt_merge(a0_replay_t* h, a0_index_t* ix, a0_extend_t* ex, const char* const* paths, int32_t k,
+                             const int64_t* map_old, const int64_t* map_new, const int64_t* map_len, uint8_t* user_out,
+                             int64_t user_cap, int64_t* user_len_out, a0_stream_t stream_) {
+  A0_REQUIRE(h && ix && paths && k >= 1 && map_len, "a0_ckpt_merge: NULL argument");
+  A0_REQUIRE(!ex || a0_ex_shard(ex) == h, "a0_ckpt_merge: the ingest handle belongs to another shard");
+  const auto t0 = ck_clock::now();
+  for (double& x : g_timing) x = 0.0;
+  A0DeviceGuard guard(h->device);
+  cudaStream_t cs = (cudaStream_t)stream_;
+  cudaStreamCaptureStatus cst = cudaStreamCaptureStatusNone;
+  A0_CUDA(cudaStreamIsCapturing(cs, &cst));
+  A0_REQUIRE(cst == cudaStreamCaptureStatusNone, "a0_ckpt_merge: the stream is being captured into a CUDA graph");
+  A0_CUDA(cudaStreamSynchronize(cs));
+  { int frc = a0_check_fault(h, "a0_ckpt_merge"); if (frc) return frc; }
+  int64_t st[A0_IX_STATE_WORDS];
+  int rc = a0_ix_state(ix, st);
+  if (rc) return rc;
+  A0_REQUIRE(st[A0_IX_REC_CAPACITY] == h->N && st[A0_IX_FRAME_CAPACITY] == h->NF, "a0_ckpt_merge: index and shard capacities differ");
+  // ---- every file validated before anything is touched
+  std::vector<std::unique_ptr<CkData>> files;
+  int64_t user_total = 0;
+  for (int32_t j = 0; j < k; ++j) {
+    A0_REQUIRE(paths[j], "a0_ckpt_merge: path %d is NULL", j);
+    files.emplace_back(new CkData());
+    CkData& d = *files.back();
+    if ((rc = ck_open("a0_ckpt_merge", paths[j], d)) || (rc = ck_plausible("a0_ckpt_merge", d))) return rc;
+    A0_REQUIRE(d.hd.F == h->F && d.hd.n_step == st[A0_IX_NSTEP],
+               "a0_ckpt_merge: %s holds frames of F=%lld gathered with n_step=%lld; this shard has F=%lld n_step=%lld", paths[j],
+               (long long)d.hd.F, (long long)d.hd.n_step, (long long)h->F, (long long)st[A0_IX_NSTEP]);
+    if ((rc = ck_read("a0_ckpt_merge", d))) return rc;
+    user_total += (int64_t)d.user_b.size();
+  }
+  A0_REQUIRE(user_total == 0 || (user_out && user_cap >= user_total), "a0_ckpt_merge: the user buffer needs %lld bytes",
+             (long long)user_total);
+  g_timing[1] = ck_us(t0, ck_clock::now());
+  // ---- the merge plan on a scratch index of the target's parameters
+  const auto t1 = ck_clock::now();
+  a0_index_t* tix = nullptr;
+  if ((rc = a0_ix_create(&tix, h->N, h->NF, (int32_t)st[A0_IX_NSTEP], st[A0_IX_AGE_LIMIT]))) return rc;
+  std::unique_ptr<a0_index_t, int (*)(a0_index_t*)> tix_owner(tix, a0_ix_destroy);
+  std::vector<a0_index_t*> six;
+  std::vector<const uint8_t*> recs;
+  std::vector<const float*> leaves;
+  std::vector<int64_t> tail_count, tail_ids, tail_seq;
+  const size_t tail_each = 8 + 64 + 8 + (size_t)A0_SLOTS * h->F + 64;      // a0_ex_tails_check verified the layout
+  for (auto& dp : files) {
+    six.push_back(dp->ix.get());
+    recs.push_back(dp->rec_b.data());
+    leaves.push_back(reinterpret_cast<const float*>(dp->leaf_b.data()));
+    int64_t cnt;
+    memcpy(&cnt, dp->tail_b.data(), 8);
+    tail_count.push_back(cnt);
+    for (int64_t e = 0; e < cnt; ++e) {
+      const uint8_t* p = dp->tail_b.data() + 8 + (size_t)e * tail_each;
+      int64_t v[1 + A0_SLOTS];
+      memcpy(v, p, sizeof(v));
+      tail_ids.push_back(v[0]);
+      tail_seq.insert(tail_seq.end(), v + 1, v + 1 + A0_SLOTS);
+    }
+  }
+  std::vector<uint8_t> rec_out((size_t)h->N * (A0_SLOTS * 4 + sizeof(A0RecInfo)));
+  std::vector<float> leaf_out((size_t)h->N);
+  a0_merge_t mg;
+  if ((rc = a0_ix_merge(tix, k, six.data(), recs.data(), leaves.data(), map_old, map_new, map_len, tail_count.data(),
+                        tail_ids.data(), tail_seq.data(), rec_out.data(), leaf_out.data(), &mg)))
+    return rc;
+  std::vector<uint8_t> index_b;
+  {
+    int64_t len = 0;
+    a0_ix_serialize(tix, nullptr, 0, &len);
+    index_b.resize((size_t)len);
+    if ((rc = a0_ix_serialize(tix, index_b.data(), len, &len))) return rc;
+  }
+  // scalars: max_p and the call counter the maxima over the files, dyn {top, file 0's beta, 0}
+  float max_p = 0.0f, dyn[3];
+  uint64_t calls = 0;
+  for (auto& dp : files) {
+    float mp;
+    uint64_t c;
+    memcpy(&mp, dp->sc_b.data(), 4);
+    memcpy(&c, dp->sc_b.data() + 16, 8);
+    max_p = std::max(max_p, mp);
+    calls = std::max(calls, c);
+  }
+  int64_t tst[A0_IX_STATE_WORDS];
+  a0_ix_state(tix, tst);
+  dyn[0] = (float)tst[A0_IX_TOP];
+  memcpy(&dyn[1], files[0]->sc_b.data() + 8, 4);
+  dyn[2] = 0.0f;
+  // tails: new ids and remapped seqs, the rest of each entry as saved
+  std::vector<uint8_t> tails_b(8 + (size_t)mg.n_tail * tail_each);
+  memcpy(tails_b.data(), &mg.n_tail, 8);
+  for (int64_t i = 0; i < mg.n_tail; ++i) {
+    const int64_t* o = mg.tails + i * (3 + A0_SLOTS);
+    uint8_t* p = tails_b.data() + 8 + (size_t)i * tail_each;
+    memcpy(p, files[(size_t)o[1]]->tail_b.data() + 8 + (size_t)o[2] * tail_each, tail_each);
+    memcpy(p, &o[0], 8);
+    memcpy(p + 8, o + 3, 64);
+  }
+  // placements per file, ascending source seq
+  std::vector<std::vector<std::pair<int64_t, int32_t>>> place((size_t)k);
+  for (int64_t i = 0; i < mg.n_place; ++i) place[(size_t)mg.place[3 * i]].push_back({mg.place[3 * i + 1], (int32_t)mg.place[3 * i + 2]});
+  for (auto& p : place) std::sort(p.begin(), p.end());
+  g_timing[2] = ck_us(t1, ck_clock::now());
+
+  // ---- from here a failure leaves everything as freshly created
+  a0_extend_t* own = nullptr;
+  if (!ex && (rc = a0_ex_create(&own, h, ix))) return rc;
+  std::unique_ptr<a0_extend_t, int (*)(a0_extend_t*)> own_owner(own, a0_ex_destroy);
+  a0_extend* dx = ex ? ex : own;
+  CkEvents ev;
+  rc = [&]() -> int {
+    const auto t2 = ck_clock::now();
+    const int64_t N = h->N;
+    int r = a0_rb_reset(h, cs);
+    if (r) return r;
+    if ((r = a0_ix_deserialize(ix, index_b.data(), (int64_t)index_b.size()))) return r;
+    A0_CUDA(cudaMemcpyAsync(h->rec_slots, rec_out.data(), (size_t)N * A0_SLOTS * 4, cudaMemcpyHostToDevice, cs));
+    A0_CUDA(cudaMemcpyAsync(h->rec_info, rec_out.data() + (size_t)N * A0_SLOTS * 4, (size_t)N * sizeof(A0RecInfo), cudaMemcpyHostToDevice, cs));
+    {
+      CkDev d_idx, d_val;
+      std::vector<int64_t> idx((size_t)N);
+      for (int64_t i = 0; i < N; ++i) idx[i] = i;
+      A0_CUDA(cudaMalloc(&d_idx.p, (size_t)N * 8));
+      A0_CUDA(cudaMalloc(&d_val.p, (size_t)N * 4));
+      A0_CUDA(cudaMemcpyAsync(d_idx.p, idx.data(), (size_t)N * 8, cudaMemcpyHostToDevice, cs));
+      A0_CUDA(cudaMemcpyAsync(d_val.p, leaf_out.data(), (size_t)N * 4, cudaMemcpyHostToDevice, cs));
+      if ((r = a0_pt_set(h, static_cast<const int64_t*>(d_idx.p), static_cast<const float*>(d_val.p), (int32_t)N, cs))) return r;
+      A0_CUDA(cudaStreamSynchronize(cs));
+    }
+    A0_CUDA(cudaMemcpyAsync(h->max_p, &max_p, 4, cudaMemcpyHostToDevice, cs));
+    A0_CUDA(cudaMemcpyAsync(h->dyn, dyn, 12, cudaMemcpyHostToDevice, cs));
+    A0_CUDA(cudaMemcpyAsync(h->counter + A0_RNG_CALL_WORD, &calls, 8, cudaMemcpyHostToDevice, cs));
+    h->stride_hint = mg.stride_hint;
+    A0_CUDA(cudaStreamSynchronize(cs));
+    if (ex && (r = a0_ex_tails_load(ex, tails_b.data(), (int64_t)tails_b.size(), cs))) return r;
+    g_timing[4] = ck_us(t2, ck_clock::now());
+    for (auto& x : ev.e) A0_CUDA(cudaEventCreate(&x));
+    for (int32_t j = 0; j < k; ++j)
+      if ((r = ck_place_file(h, dx, *files[(size_t)j], place[(size_t)j], cs, ev.e[0], ev.e[1]))) return r;
+    return A0_OK;
+  }();
+  if (rc) return ck_reset_all(h, ix, ex, cs);
+  int64_t at = 0;
+  for (int32_t j = 0; j < k; ++j) {
+    const std::vector<uint8_t>& u = files[(size_t)j]->user_b;
+    if (user_len_out) user_len_out[j] = (int64_t)u.size();
+    if (!u.empty()) memcpy(user_out + at, u.data(), u.size());
+    at += (int64_t)u.size();
+  }
   g_timing[0] = ck_us(t0, ck_clock::now());
   return A0_OK;
 }

@@ -280,6 +280,7 @@ int a0_mail_reserve(a0_replay* h, int32_t total, cudaStream_t stream);
 // a0_ckpt.cu's access to the other modules' state: the ring index (a0_ingest.cu) and the reference-tuple ingest
 // (a0_extend.cu: the K6a decode of one batch of at most 2048 blobs into its scratch, and the stream tails)
 void a0_ix_clear(a0_index* ix);
+void a0_ix_stream_ids(a0_index* ix, std::vector<int64_t>& out);      // ascending
 int a0_ex_decode_dev(a0_extend* ex, const uint8_t* blobs, const int64_t* blob_len, int32_t mb, cudaStream_t cs,
                      const uint8_t** dec, const unsigned long long** hash, const int32_t** status);
 int a0_ex_tails_save(a0_extend* ex, std::vector<uint8_t>& out);

@@ -41,6 +41,8 @@ struct a0_index {
   std::vector<int32_t> new_frame_pos, rec_meta, marks;
   std::vector<int32_t> order;
   std::vector<int64_t> fs8, ready;
+  // a0_ix_merge output, valid until the next merge into this index
+  std::vector<int64_t> merge_place, merge_rmap, merge_tails;
 
   int64_t max_chunk() const {
     const int64_t a = N / 2, b = (NF - 2 * age_limit) / (2 * A0_SLOTS);
@@ -657,4 +659,259 @@ void a0_ix_clear(a0_index* ix) {
   std::fill(ix->sampleable.begin(), ix->sampleable.end(), 0);
   ix->streams.clear();
   ix->stale.clear();
+}
+
+// ------------------------------------------------------------------------------------------------
+// a0_ix_merge: k shard checkpoints into one empty index of any capacity (rules: ring_index.merge, which stays the
+// executable specification; tests/test_ix_merge.py requires identical output)
+// ------------------------------------------------------------------------------------------------
+namespace {
+struct MergeRec {
+  int64_t age_key;        // q - head_q of its file (oldest first)
+  int32_t file;
+  int64_t q, pos, stream;
+  bool stale;
+};
+}  // namespace
+
+void a0_ix_stream_ids(a0_index* ix, std::vector<int64_t>& out) {
+  out.clear();
+  for (auto& kv : ix->streams) out.push_back(kv.first);
+  std::sort(out.begin(), out.end());
+}
+
+extern "C" int a0_ix_merge(a0_index_t* t, int32_t k, a0_index_t* const* src, const uint8_t* const* records,
+                           const float* const* leaves, const int64_t* map_old, const int64_t* map_new, const int64_t* map_len,
+                           const int64_t* tail_count, const int64_t* tail_ids, const int64_t* tail_seq, uint8_t* records_out,
+                           float* leaves_out, a0_merge_t* out) {
+  A0_REQUIRE(t && k >= 1 && src && records && leaves && map_len && records_out && leaves_out && out, "a0_ix_merge: NULL argument");
+  A0_REQUIRE(t->head_q == 0 && t->head_fs == 0 && t->streams.empty(), "a0_ix_merge: the target index is not empty");
+  for (int32_t j = 0; j < k; ++j) {
+    A0_REQUIRE(src[j] && records[j] && leaves[j], "a0_ix_merge: NULL source %d", j);
+    A0_REQUIRE(src[j]->n == t->n, "a0_ix_merge: file %d gathers n_step=%lld, the target %lld", j, (long long)src[j]->n,
+               (long long)t->n);
+  }
+  // ---- rule 5: stream maps (old id -> new id per file), collisions refused before anything changes
+  std::vector<std::unordered_map<int64_t, int64_t>> maps((size_t)k);
+  {
+    std::vector<std::unordered_set<int64_t>> present((size_t)k);
+    int64_t S = 0;
+    const int64_t* tid = tail_ids;
+    for (int32_t j = 0; j < k; ++j) {
+      for (auto& kv : src[j]->streams) present[j].insert(kv.first);
+      const int64_t nt = tail_count ? tail_count[j] : 0;
+      for (int64_t e = 0; e < nt; ++e) present[j].insert(tid[e]);
+      tid += nt;
+      for (int64_t id : present[j]) S = std::max(S, id + 1);
+    }
+    const int64_t* mo = map_old;
+    const int64_t* mn = map_new;
+    std::unordered_set<int64_t> seen;
+    for (int32_t j = 0; j < k; ++j) {
+      if (map_len[j] < 0) {
+        for (int64_t id : present[j]) maps[j][id] = id + (int64_t)j * S;
+      } else {
+        A0_REQUIRE(map_len[j] == 0 || (mo && mn), "a0_ix_merge: NULL stream map");
+        for (int64_t e = 0; e < map_len[j]; ++e)
+          if (present[j].count(mo[e])) maps[j][mo[e]] = mn[e];
+        mo += map_len[j];
+        mn += map_len[j];
+      }
+      for (auto& kv : maps[j]) {
+        A0_REQUIRE(seen.insert(kv.second).second, "a0_ix_merge: two kept streams would both become stream %lld", (long long)kv.second);
+      }
+    }
+  }
+  // ---- rule 1: live records of the kept streams; a record's stream by walking the links backwards
+  std::vector<MergeRec> recs;
+  for (int32_t j = 0; j < k; ++j) {
+    const a0_index* s = src[j];
+    const int64_t N = s->N, hq = s->head_q, tq = s->tail_q;
+    const A0RecInfo* info = reinterpret_cast<const A0RecInfo*>(records[j] + (size_t)N * A0_SLOTS * 4);
+    std::vector<int64_t> pred((size_t)N, -1), owner((size_t)N, INT64_MIN);
+    for (int64_t q = tq; q < hq; ++q) {
+      const int32_t link = info[q % N].link;
+      if (link < 0) continue;
+      A0_REQUIRE(link < N && pred[link] < 0, "a0_ix_merge: file %d: two records link to record %d", j, link);
+      pred[link] = q % N;
+    }
+    std::unordered_set<int64_t> pending;
+    int64_t reached = 0;
+    for (auto& kv : s->streams) {
+      for (int64_t p : kv.second.pending) pending.insert(p);
+      for (int64_t p = kv.second.last_seq >= tq ? kv.second.last_pos : -1; p >= 0; p = pred[p]) {
+        A0_REQUIRE(owner[p] == INT64_MIN && reached < hq - tq, "a0_ix_merge: file %d: record %lld is reached twice", j, (long long)p);
+        owner[p] = kv.first;
+        ++reached;
+      }
+    }
+    A0_REQUIRE(reached == hq - tq, "a0_ix_merge: file %d: %lld live records belong to no stream", j, (long long)(hq - tq - reached));
+    for (int64_t q = tq; q < hq; ++q) {
+      const int64_t pos = q % N;
+      auto it = maps[j].find(owner[pos]);
+      if (it == maps[j].end()) continue;
+      const bool stale = !s->sampleable[pos] && (!pending.count(q) || s->stale.count(q));
+      recs.push_back({q - hq, j, q, pos, it->second, stale});
+    }
+  }
+  // ---- rule 2: oldest first, ties by file
+  std::stable_sort(recs.begin(), recs.end(), [](const MergeRec& a, const MergeRec& b) {
+    return a.age_key != b.age_key ? a.age_key < b.age_key : a.file < b.file;
+  });
+  // ---- rule 3: the target is fed the merged sequence through a0_ix_plan
+  struct Ident {
+    int32_t file;
+    int64_t seq;
+    bool operator==(const Ident& o) const { return file == o.file && seq == o.seq; }
+  };
+  struct IdentHash {
+    size_t operator()(const Ident& x) const { return std::hash<int64_t>()(x.seq * 131 + x.file); }
+  };
+  std::unordered_map<Ident, int64_t, IdentHash> newest;
+  struct Alloc { int64_t t; int32_t file; int64_t seq; };
+  std::vector<Alloc> alloc;
+  auto resolve = [&](const Ident& id, int64_t& next_fs, int64_t hf) -> int64_t {
+    auto it = newest.find(id);
+    if (it != newest.end() && it->second >= hf - t->NF && next_fs - it->second < t->age_limit) return it->second;
+    const int64_t f = next_fs++;
+    newest[id] = f;
+    alloc.push_back({f, id.file, id.seq});
+    return f;
+  };
+  auto src_seq = [&](int32_t j, int64_t pos) {
+    const a0_index* s = src[j];
+    const int64_t lo = std::max<int64_t>(0, s->head_fs - s->NF);
+    return lo + ((pos - lo % s->NF) % s->NF + s->NF) % s->NF;
+  };
+  const int64_t N2 = t->N;
+  int32_t* slots2 = reinterpret_cast<int32_t*>(records_out);
+  A0RecInfo* info2 = reinterpret_cast<A0RecInfo*>(records_out + (size_t)N2 * A0_SLOTS * 4);
+  memset(slots2, 0, (size_t)N2 * A0_SLOTS * 4);
+  memset(info2, 0xff, (size_t)N2 * sizeof(A0RecInfo));
+  int64_t hint = 0;
+  const int64_t chunk = t->max_chunk();
+  std::vector<int64_t> stream, fs8, action, tq_of(recs.size());
+  std::vector<double> reward;
+  std::vector<uint8_t> done;
+  for (size_t c0 = 0; c0 < recs.size(); c0 += (size_t)chunk) {
+    const int32_t m = (int32_t)std::min<size_t>((size_t)chunk, recs.size() - c0);
+    const int64_t hf = t->head_fs, q0 = t->head_q;
+    int64_t next_fs = hf;
+    stream.resize((size_t)m); fs8.resize((size_t)m * A0_SLOTS); action.resize((size_t)m); reward.resize((size_t)m);
+    done.resize((size_t)m);
+    for (int32_t i = 0; i < m; ++i) {
+      const MergeRec& r = recs[c0 + i];
+      const int32_t* sl = reinterpret_cast<const int32_t*>(records[r.file]) + (size_t)r.pos * A0_SLOTS;
+      for (int c = 0; c < A0_SLOTS; ++c) fs8[(size_t)i * A0_SLOTS + c] = resolve({r.file, src_seq(r.file, sl[c])}, next_fs, hf);
+      const A0RecInfo& in = reinterpret_cast<const A0RecInfo*>(records[r.file] + (size_t)src[r.file]->N * A0_SLOTS * 4)[r.pos];
+      stream[i] = r.stream;
+      action[i] = in.action_done & 0x7fffffff;
+      done[i] = in.action_done < 0;
+      reward[i] = in.reward;
+      if (r.stale) t->stale.insert(q0 + i);
+      tq_of[c0 + i] = q0 + i;
+    }
+    a0_plan_t plan;
+    int rc = a0_ix_plan(t, stream.data(), fs8.data(), m, (int32_t)(next_fs - hf), action.data(), reward.data(), done.data(), &plan);
+    if (rc) return rc;
+    int64_t stride = -1;
+    for (int32_t i = 0; i < m; ++i) {
+      const int32_t* mt = plan.rec_meta + (size_t)i * A0_REC_META_I32;
+      const int32_t pos = mt[0];
+      memcpy(slots2 + (size_t)pos * A0_SLOTS, mt + 4, A0_SLOTS * 4);
+      memcpy(&info2[pos].reward, mt + 12, 8);
+      info2[pos].action_done = mt[3];
+      info2[pos].link = mt[2];
+      if (mt[1] >= 0) info2[mt[1]].link = pos;
+      if (stride == 0 || mt[1] < 0) continue;
+      int64_t dlt = (int64_t)mt[0] - mt[1];
+      if (dlt <= 0) dlt += N2;
+      stride = (stride < 0 || stride == dlt) ? dlt : 0;
+    }
+    if (stride >= 0) hint = stride;
+  }
+  // ---- rule 6: stacks (frames-only plans, ascending new id), then the tails
+  struct Todo { int64_t id; int32_t file; const int64_t* stack; };
+  std::vector<Todo> todo;
+  for (int32_t j = 0; j < k; ++j) {
+    const a0_index* s = src[j];
+    const int64_t lo = std::max<int64_t>(0, s->head_fs - s->NF);
+    for (auto& kv : s->streams) {
+      auto it = maps[j].find(kv.first);
+      if (it == maps[j].end() || !kv.second.has_stack) continue;
+      bool ok = true;
+      for (int c = 0; c < A0_STACK; ++c) ok = ok && kv.second.stack[c] >= lo && kv.second.stack[c] < s->head_fs;
+      if (ok) todo.push_back({it->second, j, kv.second.stack});
+    }
+  }
+  std::sort(todo.begin(), todo.end(), [](const Todo& a, const Todo& b) { return a.id < b.id; });
+  const size_t per = (size_t)std::max<int64_t>(1, 2 * chunk);
+  for (size_t g0 = 0; g0 < todo.size(); g0 += per) {
+    const size_t g1 = std::min(todo.size(), g0 + per);
+    const int64_t hf = t->head_fs;
+    int64_t next_fs = hf;
+    std::vector<int64_t> seqs;
+    for (size_t g = g0; g < g1; ++g)
+      for (int c = 0; c < A0_STACK; ++c) seqs.push_back(resolve({todo[g].file, todo[g].stack[c]}, next_fs, hf));
+    a0_plan_t plan;
+    int rc = a0_ix_plan(t, nullptr, nullptr, 0, (int32_t)(next_fs - hf), nullptr, nullptr, nullptr, &plan);
+    if (rc) return rc;
+    for (size_t g = g0; g < g1; ++g) {
+      A0Stream& st = t->streams[todo[g].id];
+      for (int c = 0; c < A0_STACK; ++c) st.stack[c] = seqs[(g - g0) * A0_STACK + c];
+      st.has_stack = true;
+    }
+  }
+  const int64_t final_lo = t->head_fs - t->NF;
+  t->merge_tails.clear();
+  {
+    struct TailOut { int64_t id; int32_t file; int64_t entry; int64_t seq[A0_SLOTS]; };
+    std::vector<TailOut> tl;
+    const int64_t* tid = tail_ids;
+    const int64_t* tsq = tail_seq;
+    for (int32_t j = 0; j < k; ++j) {
+      const int64_t nt = tail_count ? tail_count[j] : 0;
+      for (int64_t e = 0; e < nt; ++e) {
+        auto it = maps[j].find(tid[e]);
+        if (it == maps[j].end()) continue;
+        TailOut o{it->second, j, e, {}};
+        bool ok = true;
+        for (int c = 0; c < A0_SLOTS && ok; ++c) {
+          auto f = newest.find({j, tsq[e * A0_SLOTS + c]});
+          ok = f != newest.end() && f->second >= final_lo;
+          if (ok) o.seq[c] = f->second;
+        }
+        if (ok) tl.push_back(o);
+      }
+      tid += nt;
+      tsq += nt * A0_SLOTS;
+    }
+    std::sort(tl.begin(), tl.end(), [](const TailOut& a, const TailOut& b) { return a.id < b.id; });
+    for (const TailOut& o : tl) {
+      t->merge_tails.push_back(o.id); t->merge_tails.push_back(o.file); t->merge_tails.push_back(o.entry);
+      t->merge_tails.insert(t->merge_tails.end(), o.seq, o.seq + A0_SLOTS);
+    }
+  }
+  // ---- rule 4: leaves of the records the target holds sampleable; the record map and the placements
+  memset(leaves_out, 0, (size_t)N2 * 4);
+  t->merge_rmap.clear();
+  for (size_t i = 0; i < recs.size(); ++i) {
+    const int64_t q = tq_of[i];
+    const int64_t dst = q >= t->tail_q ? q % N2 : -1;
+    if (dst >= 0 && t->sampleable[dst]) leaves_out[dst] = leaves[recs[i].file][recs[i].pos];
+    t->merge_rmap.push_back(recs[i].file); t->merge_rmap.push_back(recs[i].pos); t->merge_rmap.push_back(dst);
+  }
+  t->merge_place.clear();
+  for (const Alloc& a : alloc) {
+    if (a.t < final_lo) continue;
+    t->merge_place.push_back(a.file); t->merge_place.push_back(a.seq); t->merge_place.push_back(a.t % t->NF);
+  }
+  out->n_place = (int64_t)t->merge_place.size() / 3;
+  out->place = t->merge_place.data();
+  out->n_rec = (int64_t)t->merge_rmap.size() / 3;
+  out->record_map = t->merge_rmap.data();
+  out->n_tail = (int64_t)t->merge_tails.size() / (3 + A0_SLOTS);
+  out->tails = t->merge_tails.data();
+  out->stride_hint = hint;
+  return A0_OK;
 }

@@ -23,7 +23,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from .ring_index import NativeRingIndex, stack_delta
+from .ring_index import NativeRingIndex, stack_delta, stream_map_arrays
 
 Batch = namedtuple("Batch", ["frames", "actions", "rewards", "terminals", "priorities", "indices",
                              "weights", "rewards_f32", "terminals_f32", "boot_indices", "obs", "next_obs"],
@@ -539,12 +539,58 @@ class ReplayDataset:
         with torch.cuda.device(self.device):
             _lib.check(self.lib.a0_ckpt_load(self.h, self.index.h, self._ex, os.fsencode(os.fspath(path)), buf, len(buf),
                                              C.byref(n), _lib.stream_ptr(self.device)), "a0_ckpt_load")
-        user = json.loads(buf.raw[:n.value].decode()) if n.value else {}
+        self._apply_user(json.loads(buf.raw[:n.value].decode()) if n.value else {})
+
+    def _apply_user(self, user):
         if "beta" in user:
             self.beta = user["beta"]
         if user.get("beta_current") is not None and getattr(self, "beta_schedule", None) is not None:
             self.beta_schedule.current = user["beta_current"]
         self._unique_seed = user.get("unique_seed")
+
+    def load_merged(self, paths, streams=None):
+        """Fill this shard from one or more checkpoints written by ``save`` for shards of any capacity, frame capacity
+        and age limit (the same frame size and n-step gathering), merging them stream by stream (a0_ckpt_merge; the
+        rule: ring_index.merge).  Every file's live records are taken oldest first; when this shard is smaller, the
+        newest suffix stays.  Each kept record keeps its frames, action, reward, done, n-step window and priority bit
+        for bit; record positions and frame seqs are renumbered, so this is not ``load``'s exact resume.
+        ``streams=None`` takes every stream, file j's ids offset by j * S (S = 1 + the largest id of any file; file
+        0's ids unchanged); otherwise one {old id: new id} dict per file names the streams taken.  max_p and the
+        sampler's call counter are the maxima over the files; beta, the beta schedule's position and the
+        draw-without-replacement seed come from file 0.  A stream whose observation stack is no longer in its file
+        needs ``reset_streams`` before ``append_steps``.  Returns the files' user dicts.  Raises RuntimeError on a
+        mismatched or corrupt file or colliding stream ids: a file rejected before the frames are decoded leaves the
+        shard as it was, a failure while they are decoded leaves it empty.  CUDA graphs captured on the shard stay
+        valid."""
+        paths = [os.fsencode(os.fspath(p)) for p in paths]
+        k = len(paths)
+        map_old, map_new, map_len = stream_map_arrays(streams, k)
+        cap = sum(os.path.getsize(p) for p in paths) if k else 0
+        buf = C.create_string_buffer(max(1, min(cap, 1 << 16) * k))
+        lens = np.zeros(k, dtype=np.int64)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib.a0_ckpt_merge(self.h, self.index.h, self._ex, (C.c_char_p * k)(*paths), k, map_old.ctypes.data,
+                                              map_new.ctypes.data, map_len.ctypes.data, buf, len(buf), lens.ctypes.data,
+                                              _lib.stream_ptr(self.device)), "a0_ckpt_merge")
+        users, at = [], 0
+        for n in lens.tolist():
+            users.append(json.loads(buf.raw[at:at + n].decode()) if n else {})
+            at += n
+        self._apply_user(users[0])
+        self.push_dynamic()
+        return users
+
+    @staticmethod
+    def checkpoint_info(path):
+        """Header and INDEX section of a checkpoint (a0_ckpt_info; the frames are not read): dict(N, NF, F, n_step,
+        age_limit, live, sampleable, streams=[ids])."""
+        lib = _lib.load()
+        out = np.zeros(8, dtype=np.int64)
+        ids = np.zeros(1 << 16, dtype=np.int64)
+        _lib.check(lib.a0_ckpt_info(os.fsencode(os.fspath(path)), out.ctypes.data, ids.ctypes.data, len(ids)), "a0_ckpt_info")
+        d = dict(zip(("N", "NF", "F", "n_step", "age_limit", "live", "sampleable"), out[:7].tolist()))
+        d["streams"] = ids[:int(out[7])].tolist()
+        return d
 
     def rng_seek(self, call):
         """Set the device-resident call counter of the sampler's own generator (stream-ordered)."""

@@ -296,6 +296,260 @@ def stack_delta(prev_stack, next_stack):
     return k
 
 
+# ------------------------------------------------------------------------------------------------------------------
+# merging shard checkpoints into a shard of another shape (a0_ix_merge specification)
+# ------------------------------------------------------------------------------------------------------------------
+IX_MAGIC, IX_VERSION = 0x58493041, 1
+REC_BYTES = SLOTS * 4 + 16           # one record of a RECORDS section: slots i32[8] + {reward f64, action|done i32, link i32}
+
+
+def parse_index(blob):
+    """The fields of an ``a0_ix_serialize`` blob (the INDEX section of a shard checkpoint) as a dict."""
+    b = memoryview(bytes(blob))
+    magic, ver = np.frombuffer(b[:8], dtype="<u4")
+    assert magic == IX_MAGIC and ver == IX_VERSION, "not a ring index"
+    N, NF, n, age, hq, tq, hfs, top = (int(x) for x in np.frombuffer(b[8:72], dtype="<i8"))
+    at = 72
+    d = dict(N=N, NF=NF, n=n, age_limit=age, head_q=hq, tail_q=tq, head_fs=hfs, top=top)
+    d["fs_at_append"] = np.frombuffer(b[at:at + 8 * N], dtype="<i8").copy()
+    at += 8 * N
+    d["sampleable"] = np.frombuffer(b[at:at + N], dtype=np.uint8).astype(np.bool_)
+    at += N
+    i64 = lambda k: np.frombuffer(b[at:at + 8 * k], dtype="<i8").astype(np.int64)
+    ns = int(i64(1)[0])
+    at += 8
+    streams = {}
+    for _ in range(ns):
+        sid, lp, ls, hs, s0, s1, s2, s3, k = (int(x) for x in i64(9))
+        at += 72
+        streams[sid] = dict(last_pos=lp, last_seq=ls, has_stack=bool(hs), stack=[s0, s1, s2, s3], pending=i64(k).tolist())
+        at += 8 * k
+    d["streams"] = streams
+    nst = int(i64(1)[0])
+    at += 8
+    d["stale"] = set(i64(nst).tolist())
+    return d
+
+
+def serialize_index(ix, stacks=None):
+    """``RingIndex`` state in the byte layout of ``a0_ix_serialize``; ``stacks``: stream -> i64[4] current stack."""
+    stacks = stacks or {}
+    out = [np.array([IX_MAGIC, IX_VERSION], dtype="<u4").tobytes(),
+           np.array([ix.N, ix.NF, ix.n, ix.age_limit, ix.head_q, ix.tail_q, ix.head_fs, ix.top], dtype="<i8").tobytes(),
+           np.asarray(ix.fs_at_append, dtype="<i8").tobytes(), np.asarray(ix.sampleable, dtype=np.uint8).tobytes()]
+    ids = sorted(set(ix.streams) | set(stacks))
+    out.append(np.array([len(ids)], dtype="<i8").tobytes())
+    for sid in ids:
+        st = ix.streams.get(sid, dict(last_pos=-1, last_seq=-1, pending=[]))
+        stack = stacks.get(sid)
+        words = [sid, st["last_pos"], st["last_seq"], 1 if stack is not None else 0] + \
+            (list(stack) if stack is not None else [0, 0, 0, 0]) + [len(st["pending"])] + list(st["pending"])
+        out.append(np.array(words, dtype="<i8").tobytes())
+    stale = sorted(ix.stale)
+    out.append(np.array([len(stale)] + stale, dtype="<i8").tobytes())
+    return b"".join(out)
+
+
+def empty_records(N):
+    """RECORDS of a freshly reset shard: slots 0, info bytes 0xff (a0_rb_reset)."""
+    slots = np.zeros((N, SLOTS), dtype=np.int32)
+    info = np.full((N, 4), -1, dtype=np.int32)          # reward (2 words), action|done, link
+    return slots, info
+
+
+def apply_rec_meta(slots, info, meta):
+    """What K1 writes for the records of one plan (a0_k1_write_record): slots, {reward, action|done, link} and the
+    predecessor's link word.  Inside one plan no record is both written and named as a predecessor."""
+    for mt in np.asarray(meta, dtype=np.int32):
+        pos = int(mt[0])
+        slots[pos] = mt[4:12]
+        info[pos, 0:2] = mt[12:14]
+        info[pos, 2] = mt[3]
+        info[pos, 3] = mt[2]
+        if mt[1] >= 0:
+            info[int(mt[1]), 3] = pos
+
+
+def stride_rule(meta, N, hint):
+    """The successor stride a0_rb_ingest_plan keeps for K3 after one plan's records (csrc/a0_ingest.cu)."""
+    stride = -1
+    for mt in meta:
+        if stride == 0:
+            break
+        if mt[1] < 0:
+            continue
+        dlt = int(mt[0]) - int(mt[1])
+        if dlt <= 0:
+            dlt += N
+        stride = dlt if (stride < 0 or stride == dlt) else 0
+    return stride if stride >= 0 else hint
+
+
+def merge_stream_maps(sources, streams):
+    """Rule 5: one {old id: new id} dict per file.  ``streams=None``: every stream, file j's ids offset by j * S
+    (S = 1 + the largest id of any file).  Raises ValueError when two kept streams would share a new id."""
+    present = [set(s["index"]["streams"]) | {t[0] for t in s.get("tails", ())} for s in sources]
+    if streams is None:
+        S = 1 + max((max(p) for p in present if p), default=-1)
+        maps = [{sid: sid + j * S for sid in p} for j, p in enumerate(present)]
+    else:
+        assert len(streams) == len(sources), "one stream map per file"
+        maps = [{int(a): int(b) for a, b in dict(m).items() if int(a) in p} for m, p in zip(streams, present)]
+    seen = set()
+    for m in maps:
+        for new in m.values():
+            if new in seen:
+                raise ValueError(f"two kept streams would both become stream {new}")
+            seen.add(new)
+    return maps
+
+
+def merge(target, sources, streams=None):
+    """Specification of a0_ix_merge: fill the empty ``RingIndex`` ``target`` from k shard checkpoints.
+
+    ``sources``: one dict per file, {index: parse_index(INDEX section), slots: i32[N,8], info: i32[N,4] (the RECORDS
+    section), leaves: f32[N], tails: [(stream id, seq[8])] of its TAILS section}.  Returns dict(slots, info, leaves)
+    of the target, ``stacks`` {new id: i64[4]}, ``placements`` i64[P,3] {file, source frame seq, target ring slot},
+    ``record_map`` i64[R,3] {file, source position, target position or -1 when the target evicted it}, ``tails``
+    [(new id, file, tail entry, seq[8])] in ascending new id, and ``stride_hint``.
+
+      1. From each file the live records of the kept streams; a record's stream is found by walking the ``link`` words
+         backwards from the stream's last record.
+      2. Age head_q - 1 - q inside the file; all records oldest first, ties by file index.
+      3. Fed to ``target.plan`` in chunks of ``target.max_chunk``.  A frame is (file, source seq); it reuses its newest
+         target seq t when t is resident and next_fs - t < age_limit (ContentDeduper's rule), otherwise it gets the
+         next new seq, in (record, slot) order.  The target's eviction rule keeps the newest suffix.
+      4. A sampleable record keeps its source leaf; a record that was stale in its file (live, neither sampleable nor
+         pending, or pending and in the stale set) enters the target's stale set, so it never becomes sampleable.
+      5. Stream ids: see ``merge_stream_maps``.
+      6. The kept streams' stacks whose frames are resident in their file are placed after the records (frames-only
+         plans, ascending new id, the same reuse rule); TAILS entries take the newest target seq of each frame and
+         are dropped when one of their frames is not resident in the target at the end.
+    """
+    k = len(sources)
+    for s in sources:
+        if s["index"]["n"] != target.n:
+            raise ValueError(f"a file gathers n_step={s['index']['n']}, the target {target.n}")
+    if target.head_q or target.head_fs or target.streams:
+        raise ValueError("the target index is not empty")
+    maps = merge_stream_maps(sources, streams)
+    recs = []                          # (q - head_q, file, q, pos, stream, stale)
+    for j, s in enumerate(sources):
+        ix, slots, info = s["index"], s["slots"], s["info"]
+        N, hq, tq = ix["N"], ix["head_q"], ix["tail_q"]
+        seq_of = lambda pos: tq + (pos - tq % N) % N
+        pred = {}
+        for q in range(tq, hq):
+            link = int(info[q % N, 3])
+            if link >= 0:
+                if link in pred:
+                    raise ValueError(f"file {j}: two records link to record {link}")
+                pred[link] = q % N
+        pending = {p for st in ix["streams"].values() for p in st["pending"]}
+        owner = {}
+        for sid, st in ix["streams"].items():
+            p = st["last_pos"] if st["last_seq"] >= tq else -1
+            while p >= 0:
+                if p in owner:
+                    raise ValueError(f"file {j}: record {p} is reached twice")
+                owner[p] = sid
+                p = pred.get(p, -1)
+        if len(owner) != hq - tq:
+            raise ValueError(f"file {j}: {hq - tq - len(owner)} live records belong to no stream")
+        for pos, sid in owner.items():
+            if sid in maps[j]:
+                q = seq_of(pos)
+                stale = not ix["sampleable"][pos] and (q not in pending or q in ix["stale"])
+                recs.append((q - hq, j, q, pos, maps[j][sid], stale))
+    recs.sort()
+
+    def src_seq(j, pos):
+        ix = sources[j]["index"]
+        lo = max(0, ix["head_fs"] - ix["NF"])
+        return lo + (pos - lo % ix["NF"]) % ix["NF"]
+
+    newest = {}                        # (file, source seq) -> newest target seq
+    alloc = []                         # (target seq, file, source seq) in allocation order
+
+    def resolve(idents, next_fs, hf):
+        out = []
+        for ident in idents:
+            t = newest.get(ident)
+            if t is None or t < hf - target.NF or next_fs - t >= target.age_limit:
+                t = next_fs
+                next_fs += 1
+                newest[ident] = t
+                alloc.append((t,) + ident)
+            out.append(t)
+        return out, next_fs
+
+    N2 = target.N
+    slots2, info2 = empty_records(N2)
+    hint = 0
+    tq_of = []                         # target seq of every merged record
+    chunk = target.max_chunk
+    for c0 in range(0, len(recs), chunk):
+        part = recs[c0:c0 + chunk]
+        m = len(part)
+        hf = target.head_fs
+        idents = [(r[1], src_seq(r[1], int(p))) for r in part for p in sources[r[1]]["slots"][r[3]]]
+        fs, nxt = resolve(idents, hf, hf)
+        fs8 = np.asarray(fs, dtype=np.int64).reshape(m, SLOTS)
+        q0 = target.head_q
+        target.stale.update(q0 + i for i, r in enumerate(part) if r[5])
+        infos = [sources[r[1]]["info"][r[3]] for r in part]
+        ad = np.array([int(x[2]) for x in infos], dtype=np.int64)
+        reward = np.ascontiguousarray(np.array([x[0:2] for x in infos], dtype=np.int32)).view(np.float64).reshape(m)
+        stream = np.array([r[4] for r in part], dtype=np.int64)
+        p = target.plan(stream, fs8, np.arange(nxt - hf), ad & 0x7fffffff, reward, ad < 0)
+        apply_rec_meta(slots2, info2, p.rec_meta)
+        hint = stride_rule(p.rec_meta, N2, hint)
+        tq_of.extend(range(q0, q0 + m))
+
+    stacks = {}
+    todo = []
+    for j, s in enumerate(sources):
+        ix = s["index"]
+        lo = max(0, ix["head_fs"] - ix["NF"])
+        for sid, st in ix["streams"].items():
+            if sid in maps[j] and st["has_stack"] and all(lo <= f < ix["head_fs"] for f in st["stack"]):
+                todo.append((maps[j][sid], j, st["stack"]))
+    todo.sort(key=lambda x: x[0])
+    per = max(1, 2 * chunk)            # streams per frames-only plan: at most 8 * max_chunk new frames
+    for g0 in range(0, len(todo), per):
+        hf = target.head_fs
+        group = todo[g0:g0 + per]
+        fs, nxt = resolve([(j, int(f)) for _, j, st in group for f in st], hf, hf)
+        z = np.zeros(0, dtype=np.int64)
+        target.plan(z, np.zeros((0, SLOTS), dtype=np.int64), np.arange(nxt - hf), z, z.astype(np.float64), z.astype(np.bool_))
+        for i, (new, _, _) in enumerate(group):
+            stacks[new] = np.asarray(fs[4 * i:4 * i + 4], dtype=np.int64)
+            target.streams.setdefault(new, dict(last_pos=-1, last_seq=-1, pending=[]))
+
+    final_lo = target.head_fs - target.NF
+    tails = []
+    for j, s in enumerate(sources):
+        for e, (sid, seq8) in enumerate(s.get("tails", ())):
+            if sid not in maps[j]:
+                continue
+            t = [newest.get((j, int(f)), -1) for f in seq8]
+            if all(x >= 0 and x >= final_lo for x in t):
+                tails.append((maps[j][sid], j, e, np.asarray(t, dtype=np.int64)))
+    tails.sort(key=lambda x: x[0])
+
+    leaves2 = np.zeros(N2, dtype=np.float32)
+    rmap = []
+    for r, q in zip(recs, tq_of):
+        live = q >= target.tail_q
+        dst = q % N2 if live else -1
+        if live and target.sampleable[dst]:
+            leaves2[dst] = sources[r[1]]["leaves"][r[3]]
+        rmap.append((r[1], r[3], dst))
+    place = np.array([(j, f, t % target.NF) for t, j, f in alloc if t >= final_lo], dtype=np.int64).reshape(-1, 3)
+    return dict(slots=slots2, info=info2, leaves=leaves2, stacks=stacks, placements=place,
+                record_map=np.array(rmap, dtype=np.int64).reshape(-1, 3), tails=tails, stride_hint=hint)
+
+
 class NativeRingIndex:
     """The same index, implemented in C++ inside libagent0_b200.so (csrc/a0_ingest.cu) so that an
     append costs microseconds of host time instead of ~0.6 ms of numpy; this is the one
@@ -399,3 +653,47 @@ class NativeRingIndex:
         arr = lambda ptr, k: np.ctypeslib.as_array(ptr, shape=(k,)).copy() if k else np.zeros(0, dtype=np.int32)
         return AppendPlan(new_src, arr(p.new_frame_pos, p.n_new), arr(p.rec_meta, p.m * META_I32).reshape(p.m, META_I32),
                           arr(p.marks, p.n_marks), p.m)
+
+    def merge(self, sources, records, leaves, streams=None, tails=None):
+        """a0_ix_merge into this (empty) index: ``sources`` NativeRingIndex of the files, ``records`` their RECORDS
+        sections (bytes or u8/i32 arrays of N*48 bytes), ``leaves`` f32[N] each, ``streams`` as ``merge``, ``tails``
+        one [(stream id, seq[8])] list per file (or None).  Returns what ``merge`` returns except ``stacks``
+        (``get_stack`` reads them)."""
+        C = self._C
+        k = len(sources)
+        recs = [np.frombuffer(bytes(r) if not isinstance(r, np.ndarray) else r.tobytes(), dtype=np.uint8) for r in records]
+        lvs = [np.ascontiguousarray(x, dtype=np.float32) for x in leaves]
+        for s, r, x in zip(sources, recs, lvs):
+            assert r.size == s.N * REC_BYTES and x.size == s.N
+        map_old, map_new, map_len = stream_map_arrays(streams, k)
+        tails = tails or [[] for _ in range(k)]
+        tcount = np.array([len(t) for t in tails], dtype=np.int64)
+        tids = np.array([int(e[0]) for t in tails for e in t], dtype=np.int64)
+        tseq = np.array([np.asarray(e[1], dtype=np.int64) for t in tails for e in t], dtype=np.int64).reshape(-1, SLOTS)
+        ptrs = lambda arrs, T: (T * k)(*[C.cast(a.ctypes.data, T) for a in arrs])
+        rec_out = np.zeros(self.N * REC_BYTES, dtype=np.uint8)
+        leaf_out = np.zeros(self.N, dtype=np.float32)
+        out = self._L.Merge()
+        self._L.check(self.lib.a0_ix_merge(self.h, k, (C.c_void_p * k)(*[s.h.value for s in sources]), ptrs(recs, C.c_void_p),
+                                           ptrs(lvs, C.c_void_p), map_old.ctypes.data, map_new.ctypes.data, map_len.ctypes.data,
+                                           tcount.ctypes.data, tids.ctypes.data, tseq.ctypes.data, rec_out.ctypes.data,
+                                           leaf_out.ctypes.data, C.byref(out)), "a0_ix_merge")
+        arr = lambda p, n, w: np.ctypeslib.as_array(p, shape=(n * w,)).reshape(n, w).copy() if n else np.zeros((0, w), np.int64)
+        tl = arr(out.tails, out.n_tail, 3 + SLOTS)
+        slots = rec_out[:self.N * SLOTS * 4].view(np.int32).reshape(self.N, SLOTS).copy()
+        info = rec_out[self.N * SLOTS * 4:].view(np.int32).reshape(self.N, 4).copy()
+        return dict(slots=slots, info=info, leaves=leaf_out, placements=arr(out.place, out.n_place, 3),
+                    record_map=arr(out.record_map, out.n_rec, 3),
+                    tails=[(int(r[0]), int(r[1]), int(r[2]), r[3:].copy()) for r in tl], stride_hint=int(out.stride_hint))
+
+
+def stream_map_arrays(streams, k):
+    """(map_old, map_new, map_len) of the C ABI for ``streams`` = None (every stream of every file, rule 5) or one
+    {old id: new id} dict per file."""
+    if streams is None:
+        return np.zeros(1, np.int64), np.zeros(1, np.int64), np.full(k, -1, dtype=np.int64)
+    assert len(streams) == k, "one stream map per file"
+    old = [int(a) for m in streams for a in dict(m)]
+    new = [int(b) for m in streams for b in dict(m).values()]
+    return (np.array(old + [0], dtype=np.int64), np.array(new + [0], dtype=np.int64),
+            np.array([len(dict(m)) for m in streams], dtype=np.int64))

@@ -192,11 +192,36 @@ class Trainer:
             state["fqf_optimizer"] = ln.fqf_optimizer.state_dict()
         torch.save(state, os.path.join(directory, "learner.pt"))
 
-    def load(self, directory):
+    def load(self, directory, rank=None, world=None):
         """Resume from ``save``: into a Trainer built with the same config.  Captured graphs are dropped (the next
         ``learn`` captures again): Adam's state tensors are replaced, and a graph captured before would keep updating
-        the old ones."""
-        self.replay.load(self._replay_file(directory))
+        the old ones.
+
+        ``directory`` may hold ``replay.a0ckpt`` or ``replay.rank0..G-1.a0ckpt`` of a run on G ranks.  When G equals
+        this run's world size (``world``, default: the process group's, else 1) and this rank's file (``rank``, default:
+        the process group's, else 0) has the shape of its shard, the shard resumes bit for bit (``ReplayDataset.load``).
+        Otherwise the files are resharded: this rank merges the streams ``reshard_assignment`` gives it
+        (``ReplayDataset.load_merged``), and every Adam param group's eps is set to ``adam_eps`` of the new world (the
+        saved state carries the old world's).  A resharded resume continues the run; it is not bit-identical to any
+        run, since frame seqs, record positions and the set of streams of each shard change."""
+        from .dist import adam_eps
+        pg = self.pg
+        if rank is None:
+            rank = torch.distributed.get_rank(pg) if pg is not None else 0
+        if world is None:
+            world = torch.distributed.get_world_size(pg) if pg is not None else 1
+        files = _replay_files(directory)
+        G = len(files)
+        rp = self.replay
+        own = rp.checkpoint_info(files[rank]) if rank < G else None
+        same = own is not None and G == world and (own["N"], own["NF"], own["F"], own["n_step"], own["age_limit"]) == \
+            (rp.size, rp.index.NF, rp.F, rp.index.n, rp.index.age_limit)
+        if same:
+            rp.load(files[rank])
+        else:
+            ids = [rp.checkpoint_info(f)["streams"] for f in files]
+            parts = reshard_assignment(G, world, ids)[rank]
+            rp.load_merged([files[f] for f, _ in parts], [m for _, m in parts])
         state = torch.load(os.path.join(directory, "learner.pt"), map_location=self.replay.device, weights_only=False)
         ln = self.learner
         ln.model.load_state_dict(state["model"])
@@ -215,4 +240,41 @@ class Trainer:
         torch.set_rng_state(state["rng_cpu"].cpu())
         torch.cuda.set_rng_state(state["rng_cuda"].cpu(), dev)
         np.random.set_state(state["rng_numpy"])
+        if not same:
+            for g in ln.optimizer.param_groups:
+                g["eps"] = adam_eps(self.cfg.learner.batch_size, world)
         self._graphed = None
+
+
+def _replay_files(directory):
+    """The shard files of a saved run: [replay.a0ckpt] or [replay.rank0.a0ckpt, ..., replay.rank{G-1}.a0ckpt]."""
+    one = os.path.join(directory, "replay.a0ckpt")
+    if os.path.exists(one):
+        return [one]
+    files = []
+    while os.path.exists(os.path.join(directory, f"replay.rank{len(files)}.a0ckpt")):
+        files.append(os.path.join(directory, f"replay.rank{len(files)}.a0ckpt"))
+    if not files:
+        raise FileNotFoundError(f"{directory} holds no replay.a0ckpt or replay.rank0.a0ckpt")
+    return files
+
+
+def reshard_assignment(G, G_new, stream_ids_per_file):
+    """Which streams of G shard files each of G_new ranks takes: a list over the new ranks of [(file, {old id: new
+    id})].  G_new <= G: rank r' takes the whole files r with r % G_new == r', the ids of its j-th file offset by j * S
+    (S = 1 + the largest id of its files; ReplayDataset.load_merged's default).  G_new > G: rank r' takes file
+    r' % G, and of that file's streams in ascending id order (ordinal t) those with t % c == r' // G, where c new ranks
+    share the file; ids are kept.  Every (file, stream) goes to exactly one rank."""
+    ids = [sorted(int(x) for x in f) for f in stream_ids_per_file]
+    assert len(ids) == G and G >= 1 and G_new >= 1
+    out = []
+    for r2 in range(G_new):
+        if G_new <= G:
+            mine = [f for f in range(G) if f % G_new == r2]
+            S = 1 + max((max(ids[f]) for f in mine if ids[f]), default=-1)
+            out.append([(f, {sid: sid + j * S for sid in ids[f]}) for j, f in enumerate(mine)])
+        else:
+            f = r2 % G
+            c = len(range(f, G_new, G))
+            out.append([(f, {sid: sid for t, sid in enumerate(ids[f]) if t % c == r2 // G})])
+    return out

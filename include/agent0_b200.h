@@ -306,11 +306,65 @@ int a0_ckpt_save(a0_replay_t* h, a0_index_t* ix, a0_extend_t* ex, const char* pa
                  int64_t user_len, a0_stream_t stream);
 int a0_ckpt_load(a0_replay_t* h, a0_index_t* ix, a0_extend_t* ex, const char* path, uint8_t* user_out,
                  int64_t user_cap, int64_t* user_len_out, a0_stream_t stream);
-/* Phases of the last a0_ckpt_save / a0_ckpt_load of the process.  Save: {total us, K7 device us (CUDA events),
- * blob compaction + device-to-host copy device us (CUDA events), file write us, raw frame bytes, blob bytes, host
- * wait for the copies us, 0}.  Load: {total us, header + small sections + validation us, blob file read us,
- * decode + hash check + restore us (host clock, K6a included), raw frame bytes, blob bytes, 0, 0}.               */
+/* Phases of the last a0_ckpt_save / a0_ckpt_load / a0_ckpt_merge of the process.  Save: {total us, K7 device us
+ * (CUDA events), blob compaction + device-to-host copy device us (CUDA events), file write us, raw frame bytes, blob
+ * bytes, host wait for the copies us, 0}.  Load: {total us, header + small sections + validation us, blob file read
+ * us, decode + hash check + restore us (host clock, K6a included), raw frame bytes, blob bytes, 0, 0}.  Merge: {total
+ * us, header + small sections + validation us of all files, host merge plan (a0_ix_merge) us, decode + place device
+ * us (CUDA events around K6a and K1), records + leaves + scalars + tails us, bytes decoded, bytes placed, blob file
+ * read + hash us}.                                                                                               */
 int a0_ckpt_last_timing(double* out8);
+
+/* ---- merging shard checkpoints into a shard of another capacity or world size ----------------------------------
+ * a0_ix_merge (host code only) fills the EMPTY index `target` (any record capacity, frame capacity and age limit;
+ * the same n_step) from k checkpoint files, given each file's index (a0_ix_deserialize of its INDEX section), its
+ * RECORDS and LEAVES sections and, optionally, its TAILS ids and seq[8] (tail_count[k], tail_ids and tail_seq[][8]
+ * concatenated over the files; tail_count NULL = none).  The rule (specification: agent0_b200/ring_index.py, merge):
+ *   1. from each file the live records of the kept streams; a record's stream is found by walking the link words
+ *      backwards from the stream's last record;
+ *   2. ages head_q - 1 - q inside each file; all records oldest first, ties by file index;
+ *   3. fed to a0_ix_plan in chunks of the target's max_chunk; a frame is (file, source seq) and reuses its newest
+ *      target seq t when t is resident and next_fs - t < age_limit, otherwise it takes the next new seq in (record,
+ *      slot) order; the target's eviction rule keeps the newest suffix;
+ *   4. a record sampleable in the target keeps its source leaf bit for bit; a record stale in its file (live,
+ *      neither sampleable nor pending) enters the target's stale set and stays unsampleable;
+ *   5. map_len[j] < 0: every stream of file j, id + j * S (S = 1 + the largest id of any file); otherwise the
+ *      map_len[j] pairs (map_old, map_new; concatenated over such files) name the streams taken and their new ids.
+ *      Two kept streams with one new id fail the call before the target is touched;
+ *   6. stacks whose frames are resident in their file are placed after the records (frames-only plans, ascending new
+ *      id, the rule of 3); a tail takes the newest target seq of each of its frames and is dropped when one of them is
+ *      not resident in the target at the end.
+ * records_out receives the target's RECORDS (N'*48 bytes: what K1 writes for the plans on a freshly reset shard),
+ * leaves_out f32[N'] its leaves (0 where not sampleable).  *out: arrays owned by the target index until its next
+ * merge.  Every target ring slot receives at most one placement, so they may run in any order.                    */
+typedef struct {
+  int64_t n_place;
+  const int64_t* place;           /* [n_place][3] {file, source frame seq, target ring slot}                    */
+  int64_t n_rec;
+  const int64_t* record_map;      /* [n_rec][3] {file, source position, target position or -1 if evicted}     */
+  int64_t n_tail;
+  const int64_t* tails;           /* [n_tail][11] {new id, file, TAILS entry, target seq[8]}, ascending new id   */
+  int64_t stride_hint;            /* K3's successor stride after the target's records (as the ingest sets it)  */
+} a0_merge_t;
+int a0_ix_merge(a0_index_t* target, int32_t k, a0_index_t* const* src, const uint8_t* const* records,
+                const float* const* leaves, const int64_t* map_old, const int64_t* map_new, const int64_t* map_len,
+                const int64_t* tail_count, const int64_t* tail_ids, const int64_t* tail_seq, uint8_t* records_out,
+                float* leaves_out, a0_merge_t* out);
+/* a0_ckpt_info reads only the header and the INDEX section of a checkpoint: out8 = {N, NF, F, n_step, age_limit,
+ * live records, sampleable records, streams}; ids_out[ids_cap] receives the stream ids in ascending order.       */
+int a0_ckpt_info(const char* path, int64_t* out8, int64_t* ids_out, int64_t ids_cap);
+/* a0_ckpt_merge fills the shard h + index ix (+ ex, or NULL) from k checkpoint files of the same F and n_step by
+ * the rule of a0_ix_merge (map_old / map_new / map_len as there).  Every file is validated as a0_ckpt_load
+ * validates it before anything is touched; then the shard is reset, records, leaves (inner nodes fl32(left +
+ * right)), max_p (the maximum over the files), the sampler's call counter (the maximum), dyn {top, file 0's beta,
+ * 0} and the stride hint are written, and the frames are placed file by file: the BLOBS section is read once,
+ * hashed whole, and only the groups that hold a placed frame are decoded by K6a (at most 1024 groups at a time,
+ * every decoded frame's hash compared with the saved one) and copied to their target slots by K1.  A failure from
+ * the reset on leaves shard, index and tails as freshly created.  user_out[user_cap] receives the files' USER
+ * bytes back to back, user_len_out[k] their lengths.                                                            */
+int a0_ckpt_merge(a0_replay_t* h, a0_index_t* ix, a0_extend_t* ex, const char* const* paths, int32_t k,
+                  const int64_t* map_old, const int64_t* map_new, const int64_t* map_len, uint8_t* user_out,
+                  int64_t user_cap, int64_t* user_len_out, a0_stream_t stream);
 
 /* ---- staged ingest: execute a plan on the device ------------------------------------------------
  * One pinned H2D copy of {frames, positions, record metadata, marks} from a double-buffered
