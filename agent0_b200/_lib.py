@@ -119,6 +119,7 @@ SIGNATURES = {
     "a0_loss_dqn": (_i32, [C.POINTER(LossCommon), _vp, _vp, _vp, _vp, _vp]),
     "a0_loss_mdqn": (_i32, [C.POINTER(LossCommon), _vp, _vp, _vp, _f32, _f32, _vp, _vp]),
     "a0_loss_c51": (_i32, [C.POINTER(LossCommon), _vp, _vp, _vp, _vp, _i32, _f32, _f32, _vp, _vp, _vp]),
+    "a0_c51_div_check": (_i32, [_f32, _f32, _i32, _vp, _vp]),
     "a0_loss_quantile": (_i32, [C.POINTER(LossCommon), _i32, _vp, _vp, _vp, _vp, _i32, _i32, _vp,
                                 _vp, _vp, _vp, _vp, _vp]),
     "a0_act_epsilon_greedy": (_i32, [_vp, _i32, _i32, _f64, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),

@@ -407,22 +407,58 @@ a0_k4_c51(const A0Common c, const float* __restrict__ logits, const float* __res
 // chain (device timeline, tools/trace_step.py: 3.5 us of a 3.9 us launch-to-launch period, 20 of them
 // per Trainer.step), so what counts is instructions on that chain, not throughput:
 //   * arg-max over the A selection values computed by every lane from broadcast loads (no shuffles);
-//   * the two row maxima reduced together, then the two sum-exps together: 10 shuffle steps, not 15;
+//   * each row maximum is one warp-reduction instruction (redux.sync.max.f32), the two sum-exps are
+//     reduced together: 5 shuffle steps before the projection, not 15;
 //   * u = l + 1 always holds after the reference's two adjustments (agent.py:246-250), so
 //     l = max(ceil(b) - 1, 0) and one key per atom drives the scan of both terms;
-//   * bins are written by read-modify-write in four fixed phases (one writer per bin and phase by
-//     construction) instead of shared-memory atomics (CAS loops);
-//   * cross-entropy and mass reduced together; the zeros of the sample's [A, M] gradient block (every
-//     row but the taken action's) are stored as soon as the action is known, under the latency of the
-//     input loads, so only row a is left after the arithmetic.
+//   * everything of the projection that does not depend on the softmax -- the bin positions b_j (a
+//     division without IEEE division's slow path, a0_c51_div_delta), the keys, the scan's run masks,
+//     the fractions of both terms -- is computed under the latency of the sum-exp reduction, so after
+//     it only p_j / sum, two multiplies and the scan of the values are left;
+//   * each term of a bin goes to its own shared-memory row (one writer per row and bin by construction)
+//     and a bin is then the sum of its four rows in the order of a0_k4_c51's four phases: one store /
+//     load round trip instead of four read-modify-writes;
+//   * log-sum-exp of the online row and the gradient's softmax are computed as soon as its sum is
+//     known; cross-entropy and mass reduced together; the zeros of the sample's [A, M] gradient block
+//     (every row but the taken action's) are stored as soon as the action is known, under the latency
+//     of the input loads, so only row a is left after the arithmetic.
 // ------------------------------------------------------------------------------------------------
+
+// Maximum over the warp in one instruction.  Without .NaN a NaN operand is ignored, as fmaxf does, so this is the
+// fmaxf butterfly's result whatever the order of the lanes.
+__device__ __forceinline__ float a0_warp_max_redux(float v) {
+  float m;
+  asm("redux.sync.max.f32 %0, %1, 0xffffffff;" : "=f"(m) : "f"(v));
+  return m;
+}
+
+// fl32(nu / delta) for 0 <= nu <= fl32(vmax - vmin), equal to __fdiv_rn(nu, delta) and without its slow-path call:
+// a float64 quotient by one Markstein correction from rdelta = RN64(1/delta), then rounded to float32.  Every float32
+// operand is a normal float64, so the correction step's premises hold (q0 = RN64(nu * rdelta) is within one ulp of
+// nu/delta, the remainder is exact) and the float64 quotient is correctly rounded; rounding that to float32 is exact
+// too, because a quotient of 24-bit operands is never within 2^-53 relative of a float32 rounding boundary without
+// being on it (53 >= 2 * 24 + 2).  tests/test_gpu_c51_chain.py checks every float32 nu of the tested supports.
+__device__ __forceinline__ float a0_c51_div_delta(float nu, float delta, double rdelta) {
+  const double q0 = __dmul_rn((double)nu, rdelta);
+  const double rem = __fma_rn(-q0, (double)delta, (double)nu);
+  return __double2float_rn(__fma_rn(rem, rdelta, q0));
+}
+
+// delta and 1/delta of a launch: delta is the same float division the kernels' rule uses (oracle/losses.py).
+static void a0_c51_delta(float vmin, float vmax, int32_t M, float* delta, double* rdelta) {
+  *delta = (vmax - vmin) / (float)(M - 1);
+  *rdelta = 1.0 / (double)*delta;
+}
+
 template <int WARPS>
 __global__ void __launch_bounds__(WARPS * 32)
 a0_k4_c51_fast(const A0Common c, const float* __restrict__ logits, const float* __restrict__ tgt_logits,
                const float* __restrict__ qsel, const float* __restrict__ atoms, int32_t M, float vmin, float vmax,
-               float delta, float* __restrict__ grad, float* __restrict__ target_prob) {
-  __shared__ float s_m[WARPS][72];       // projected distribution (bin M may be touched when b rounds above M-1: that
-                                             // upper term is dropped, as in a0_k4_c51 and oracle.losses.c51_project)
+               float delta, double rdelta, float* __restrict__ grad, float* __restrict__ target_prob) {
+  // the four terms of the projection, one row each: lower terms of atoms lane and lane + 32, then upper terms.  Index
+  // M may be written when b rounds above M-1 (never read: that upper term is dropped, as in a0_k4_c51 and
+  // oracle.losses.c51_project)
+  __shared__ float s_t[WARPS][4][72];
   A0_T0();
   A0_PDL_PROLOGUE();
   A0_TMID();
@@ -452,8 +488,12 @@ a0_k4_c51_fast(const A0Common c, const float* __restrict__ logits, const float* 
   const int a = (int)c.action[b];
   const float r = c.reward[b], d = c.done[b], w = c.weight[b];
   const float z0 = in0 ? atoms[lane] : 0.0f, z1 = in1 ? atoms[lane + 32] : 0.0f;
-  s_m[wid][lane] = 0.0f;
-  s_m[wid][lane + 32] = 0.0f;
+  float(*terms)[72] = s_t[wid];
+#pragma unroll
+  for (int t = 0; t < 4; ++t) {
+    terms[t][lane] = 0.0f;
+    terms[t][lane + 32] = 0.0f;
+  }
   // The gradient block [A, M] of the sample is zero outside row a: those stores depend on nothing but
   // `a`, so they go out now, under the latency of the loads above, and only row a is left for the end.
   const int AM = A * M, r0 = a * M;
@@ -473,20 +513,36 @@ a0_k4_c51_fast(const A0Common c, const float* __restrict__ logits, const float* 
     if (a2 == a_star) { p0 = tg_all[a2][0]; p1 = tg_all[a2][1]; }
   }
   A0_TX(0);
-  // ---- both softmaxes: maxima together, then sum-exps together -----------------------------------------
-  float omx = fmaxf(l0, l1), mx = fmaxf(p0, p1);
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    const float a_ = __shfl_xor_sync(0xffffffffu, omx, o);
-    const float b_ = __shfl_xor_sync(0xffffffffu, mx, o);
-    omx = fmaxf(omx, a_);
-    mx = fmaxf(mx, b_);
-  }
+  // ---- both softmaxes: the maxima, then the sum-exps together --------------------------------------------
+  const float omx = a0_warp_max_redux(fmaxf(l0, l1)), mx = a0_warp_max_redux(fmaxf(p0, p1));
   A0_TX(1);
-  const float eo0 = in0 ? expf(l0 - omx) : 0.0f, eo1 = in1 ? expf(l1 - omx) : 0.0f;
-  p0 = in0 ? expf(p0 - mx) : 0.0f;
-  p1 = in1 ? expf(p1 - mx) : 0.0f;
+  // an idle atom's exponential is expf(-inf) = +0: the arguments are selected, the calls are not branched around
+  const float eo0 = expf(in0 ? l0 - omx : -INFINITY), eo1 = expf(in1 ? l1 - omx : -INFINITY);
+  p0 = expf(in0 ? p0 - mx : -INFINITY);
+  p1 = expf(in1 ? p1 - mx : -INFINITY);
   float ose = eo0 + eo1, se = p0 + p1;
+  // The projection's geometry (agent.py:230-250) needs neither softmax: bin positions, keys of the segmented scan
+  // and its run masks, fractions of the lower and upper terms.
+  const float gm = __fmul_rn(c.gamma_n, __fsub_rn(1.0f, d));
+  const float tz0 = fminf(fmaxf(__fadd_rn(r, __fmul_rn(gm, z0)), vmin), vmax);
+  const float tz1 = fminf(fmaxf(__fadd_rn(r, __fmul_rn(gm, z1)), vmin), vmax);
+  const float bs0 = a0_c51_div_delta(__fsub_rn(tz0, vmin), delta, rdelta);
+  const float bs1 = a0_c51_div_delta(__fsub_rn(tz1, vmin), delta, rdelta);
+  const int c0 = max((int)ceilf(bs0) - 1, 0), c1 = max((int)ceilf(bs1) - 1, 0);
+  const int k0 = in0 ? c0 : -1, k1 = in1 ? c1 : -1;   // lower bin of atoms lane and lane + 32; the upper one is k + 1
+  const float fl0 = __fsub_rn((float)(c0 + 1), bs0), fu0 = __fsub_rn(bs0, (float)c0);
+  const float fl1 = __fsub_rn((float)(c1 + 1), bs1), fu1 = __fsub_rn(bs1, (float)c1);
+  // segmented inclusive scan over the lanes, keyed by the lower bin (bins are non-decreasing in the atom index, so
+  // the sources of one bin are adjacent lanes); step s adds the partial sum 2^s lanes up where the keys agree
+  unsigned join0 = 0, join1 = 0;
+#pragma unroll
+  for (int s = 0; s < 5; ++s) {
+    const int q0 = __shfl_up_sync(0xffffffffu, k0, 1 << s), q1 = __shfl_up_sync(0xffffffffu, k1, 1 << s);
+    if (lane >= (1 << s) && q0 == k0) join0 |= 1u << s;
+    if (lane >= (1 << s) && q1 == k1) join1 |= 1u << s;
+  }
+  const int n0 = __shfl_down_sync(0xffffffffu, k0, 1), n1 = __shfl_down_sync(0xffffffffu, k1, 1);
+  const bool tail0 = k0 >= 0 && (lane == 31 || n0 != k0), tail1 = k1 >= 0 && (lane == 31 || n1 != k1);
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) {
     const float a_ = __shfl_xor_sync(0xffffffffu, ose, o);
@@ -494,54 +550,46 @@ a0_k4_c51_fast(const A0Common c, const float* __restrict__ logits, const float* 
     ose += a_;
     se += b_;
   }
-  A0_TX(2);
-  // ---- projection (agent.py:230-264) ---------------------------------------------------------------------
-  // The warp pays for IEEE division's slow path (a subroutine) if ANY lane's operands need it -- a zero
-  // numerator does: the idle lanes of the second atom chunk (p = 0), an atom clamped onto vmin.  Those
-  // lanes divide a harmless stand-in instead and select the exact answer (0) afterwards: same bits.
-  const float gm = __fmul_rn(c.gamma_n, __fsub_rn(1.0f, d));
-  int k0 = -1, k1 = -1;                       // lower bin of atoms lane and lane + 32; the upper one is k + 1
-  float wl0 = 0.0f, wu0 = 0.0f, wl1 = 0.0f, wu1 = 0.0f;
-  {
-    const float pj0 = p0 != 0.0f ? __fdiv_rn(p0, se) : 0.0f, pj1 = p1 != 0.0f ? __fdiv_rn(p1, se) : 0.0f;
-    const float tz0 = fminf(fmaxf(__fadd_rn(r, __fmul_rn(gm, z0)), vmin), vmax);
-    const float tz1 = fminf(fmaxf(__fadd_rn(r, __fmul_rn(gm, z1)), vmin), vmax);
-    const float nu0 = __fsub_rn(tz0, vmin), nu1 = __fsub_rn(tz1, vmin);
-    const float bs0 = nu0 != 0.0f ? __fdiv_rn(nu0, delta) : 0.0f, bs1 = nu1 != 0.0f ? __fdiv_rn(nu1, delta) : 0.0f;
-    const int c0 = max((int)ceilf(bs0) - 1, 0), c1 = max((int)ceilf(bs1) - 1, 0);
-    if (in0) { k0 = c0; wl0 = __fmul_rn(pj0, __fsub_rn((float)(c0 + 1), bs0)); wu0 = __fmul_rn(pj0, __fsub_rn(bs0, (float)c0)); }
-    if (in1) { k1 = c1; wl1 = __fmul_rn(pj1, __fsub_rn((float)(c1 + 1), bs1)); wu1 = __fmul_rn(pj1, __fsub_rn(bs1, (float)c1)); }
-  }
-  A0_TX(3);
-  // segmented inclusive scan over the lanes, keyed by the lower bin (bins are non-decreasing in the atom
-  // index, so the sources of one bin are adjacent lanes); the same combination order as a0_c51_scatter
-#pragma unroll
-  for (int dd = 1; dd < 32; dd <<= 1) {
-    const int q0 = __shfl_up_sync(0xffffffffu, k0, dd), q1 = __shfl_up_sync(0xffffffffu, k1, dd);
-    const float a0_ = __shfl_up_sync(0xffffffffu, wl0, dd), b0_ = __shfl_up_sync(0xffffffffu, wu0, dd);
-    const float a1_ = __shfl_up_sync(0xffffffffu, wl1, dd), b1_ = __shfl_up_sync(0xffffffffu, wu1, dd);
-    if (lane >= dd && q0 == k0) { wl0 = __fadd_rn(wl0, a0_); wu0 = __fadd_rn(wu0, b0_); }
-    if (lane >= dd && q1 == k1) { wl1 = __fadd_rn(wl1, a1_); wu1 = __fadd_rn(wu1, b1_); }
-  }
-  const int n0 = __shfl_down_sync(0xffffffffu, k0, 1), n1 = __shfl_down_sync(0xffffffffu, k1, 1);
-  const bool tail0 = k0 >= 0 && (lane == 31 || n0 != k0), tail1 = k1 >= 0 && (lane == 31 || n1 != k1);
-  float* bins = s_m[wid];
-  __syncwarp();                                // the zeros above are visible
-  // four phases in the order of a0_k4_c51 (lower terms of both chunks, then upper terms): within a
-  // phase every bin has at most one writer, so a plain read-modify-write is exact and deterministic
-  if (tail0) bins[k0] = __fadd_rn(bins[k0], wl0);
-  __syncwarp();
-  if (tail1) bins[k1] = __fadd_rn(bins[k1], wl1);
-  __syncwarp();
-  if (tail0) bins[k0 + 1] = __fadd_rn(bins[k0 + 1], wu0);
-  __syncwarp();
-  if (tail1) bins[k1 + 1] = __fadd_rn(bins[k1 + 1], wu1);
-  __syncwarp();
-  const float m0 = bins[lane], m1 = bins[lane + 32];
-  A0_TX(4);
-  // ---- cross-entropy with the online row, gradient through log_softmax (agent.py:266-268) -----------------
+  // log-softmax of the online row and its exponential (the gradient's softmax, agent.py:266-268)
   const float lse = logf(ose);
   const float ls0 = (l0 - omx) - lse, ls1 = (l1 - omx) - lse;
+  float sm0 = expf(ls0), sm1 = expf(ls1);
+  A0_TX(2);
+  // ---- projection (agent.py:252-264) -------------------------------------------------------------------
+  // The warp pays for IEEE division's slow path (a subroutine) if ANY lane's operands need it -- a zero
+  // numerator does: the idle lanes of the second atom chunk (p = 0).  Those lanes divide a harmless
+  // stand-in (1) instead and select the exact answer (0) afterwards: same bits.
+  float wl0 = 0.0f, wu0 = 0.0f, wl1 = 0.0f, wu1 = 0.0f;
+  {
+    const float q0 = __fdiv_rn(p0 != 0.0f ? p0 : 1.0f, se), q1 = __fdiv_rn(p1 != 0.0f ? p1 : 1.0f, se);
+    const float pj0 = p0 != 0.0f ? q0 : 0.0f, pj1 = p1 != 0.0f ? q1 : 0.0f;
+    if (in0) { wl0 = __fmul_rn(pj0, fl0); wu0 = __fmul_rn(pj0, fu0); }
+    if (in1) { wl1 = __fmul_rn(pj1, fl1); wu1 = __fmul_rn(pj1, fu1); }
+  }
+  A0_TX(3);
+  // the same combination order as a0_c51_scatter
+#pragma unroll
+  for (int s = 0; s < 5; ++s) {
+    const float a0_ = __shfl_up_sync(0xffffffffu, wl0, 1 << s), b0_ = __shfl_up_sync(0xffffffffu, wu0, 1 << s);
+    const float a1_ = __shfl_up_sync(0xffffffffu, wl1, 1 << s), b1_ = __shfl_up_sync(0xffffffffu, wu1, 1 << s);
+    if (join0 >> s & 1u) { wl0 = __fadd_rn(wl0, a0_); wu0 = __fadd_rn(wu0, b0_); }
+    if (join1 >> s & 1u) { wl1 = __fadd_rn(wl1, a1_); wu1 = __fadd_rn(wu1, b1_); }
+  }
+  // sm0 and sm1 are needed only by the last stores: without this the compiler would compute them there, after the
+  // cross-entropy reduction, instead of under the latency of the scan
+  asm volatile("" : "+f"(sm0), "+f"(sm1));
+  // A run tail holds its run's total; every row has at most one writer per bin.  a0_k4_c51 adds the four terms of
+  // a bin into a zeroed bin in this order (lower terms of both chunks, then upper terms); the absent ones are +0
+  // here and there (every term is >= +0), so the sum below has the same bits.
+  __syncwarp();                                // the zeros above are visible
+  if (tail0) { terms[0][k0] = wl0; terms[2][k0 + 1] = wu0; }
+  if (tail1) { terms[1][k1] = wl1; terms[3][k1 + 1] = wu1; }
+  __syncwarp();
+  const float m0 = __fadd_rn(__fadd_rn(__fadd_rn(terms[0][lane], terms[1][lane]), terms[2][lane]), terms[3][lane]);
+  const float m1 = __fadd_rn(__fadd_rn(__fadd_rn(terms[0][lane + 32], terms[1][lane + 32]), terms[2][lane + 32]),
+                             terms[3][lane + 32]);
+  A0_TX(4);
+  // ---- cross-entropy with the online row, gradient through log_softmax (agent.py:266-268) -----------------
   float ce = 0.0f, msum = 0.0f;
   if (in0) { ce += m0 * ls0; msum += m0; }
   if (in1) { ce += m1 * ls1; msum += m1; }
@@ -554,7 +602,7 @@ a0_k4_c51_fast(const A0Common c, const float* __restrict__ logits, const float* 
   }
   A0_TX(5);
   if (lane == 0) a0_emit(c, b, -ce);           // loss / priority / max_p leave before the gradient block does
-  const float g0 = w * (expf(ls0) * msum - m0), g1 = w * (expf(ls1) * msum - m1);
+  const float g0 = w * (sm0 * msum - m0), g1 = w * (sm1 * msum - m1);
   if (in0) gb[r0 + lane] = g0;
   if (in1) gb[r0 + lane + 32] = g1;
   if (target_prob) {
@@ -588,8 +636,11 @@ extern "C" int a0_loss_c51(const a0_loss_common_t* c, const float* logits, const
   A0_REQUIRE(M >= 2 && M <= C51_MAXR * 32, "a0_loss_c51: num_atoms %d outside [2,%d]", M, C51_MAXR * 32);
   A0_REQUIRE(vmax > vmin, "a0_loss_c51: vmax must exceed vmin");
   if (c->B == 0) return A0_OK;
-  if (qsel && c->A <= C51_SPEC_A && M <= 64 && a0_option_c51_fast()) {
-    const float delta = (vmax - vmin) / (float)(M - 1);      // the same float division the kernels do
+  float delta;
+  double rdelta;
+  a0_c51_delta(vmin, vmax, M, &delta, &rdelta);
+  // a0_c51_div_delta needs a finite, nonzero delta (not so when vmax - vmin overflows or underflows)
+  if (qsel && c->A <= C51_SPEC_A && M <= 64 && delta > 0.0f && delta < INFINITY && a0_option_c51_fast()) {
     static int warps = 0;                                     // samples (= warps) per CTA: A0_C51_WARPS, measured default
     if (!warps) {
       const char* e = getenv("A0_C51_WARPS");
@@ -599,7 +650,7 @@ extern "C" int a0_loss_c51(const a0_loss_common_t* c, const float* logits, const
     const unsigned grid = (unsigned)((c->B + warps - 1) / warps);
 #define A0_C51_FAST_LAUNCH(W)                                                                                              \
     A0_LAUNCH(a0_k4_c51_fast<W>, grid, W * 32, 0, (cudaStream_t)stream, 1, A0_PDL_K4, a0_unpack(c), logits, tgt_logits, qsel,   \
-              atoms, M, vmin, vmax, delta, grad, target_prob)
+              atoms, M, vmin, vmax, delta, rdelta, grad, target_prob)
     if (warps == 1) A0_C51_FAST_LAUNCH(1);
     else if (warps == 2) A0_C51_FAST_LAUNCH(2);
     else if (warps == 4) A0_C51_FAST_LAUNCH(4);
@@ -611,6 +662,40 @@ extern "C" int a0_loss_c51(const a0_loss_common_t* c, const float* logits, const
   }
   A0_LAUNCH(a0_k4_c51, (unsigned)((c->B + C51_WARPS - 1) / C51_WARPS), C51_WARPS * 32, 0, (cudaStream_t)stream, 1, A0_PDL_K4,
             a0_unpack(c), logits, tgt_logits, qsel, atoms, M, vmin, vmax, grad, target_prob);
+  return A0_OK;
+}
+
+// Every float32 nu in [0, hi] (by bit pattern): a0_c51_div_delta against __fdiv_rn.  out[0] += mismatches,
+// out[1] = min(bit pattern of a mismatching nu).
+__global__ void a0_c51_div_check_kernel(uint32_t hi, float delta, double rdelta, unsigned long long* out) {
+  unsigned long long bad = 0, first = ~0ull;
+  for (unsigned long long u = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; u <= hi;
+       u += (unsigned long long)gridDim.x * blockDim.x) {
+    const float nu = __uint_as_float((uint32_t)u);
+    if (__float_as_uint(a0_c51_div_delta(nu, delta, rdelta)) != __float_as_uint(__fdiv_rn(nu, delta))) {
+      ++bad;
+      first = min(first, u);
+    }
+  }
+  if (bad) {
+    atomicAdd(out, bad);
+    atomicMin(out + 1, first);
+  }
+}
+
+extern "C" int a0_c51_div_check(float vmin, float vmax, int32_t M, unsigned long long* out, a0_stream_t stream) {
+  A0_REQUIRE(out != nullptr, "a0_c51_div_check: NULL output");
+  A0_REQUIRE(M >= 2 && vmax > vmin, "a0_c51_div_check: M %d, vmin %g, vmax %g", M, (double)vmin, (double)vmax);
+  float delta;
+  double rdelta;
+  a0_c51_delta(vmin, vmax, M, &delta, &rdelta);
+  A0_REQUIRE(delta > 0.0f && delta < INFINITY, "a0_c51_div_check: delta %g is zero or infinite", (double)delta);
+  const float hi = vmax - vmin;
+  A0_REQUIRE(hi < INFINITY, "a0_c51_div_check: vmax - vmin overflows");
+  uint32_t hb;
+  memcpy(&hb, &hi, sizeof(hb));
+  a0_c51_div_check_kernel<<<148 * 8, 256, 0, (cudaStream_t)stream>>>(hb, delta, rdelta, out);
+  A0_LAUNCH_CHECK();
   return A0_OK;
 }
 

@@ -75,7 +75,8 @@ const char* a0_last_error(void);
  * a0_pt_mark followed by a0_rb_append.  Same shard state either way.                              */
 #define A0_OPT_FUSED_INGEST 4
 /* A0_OPT_C51_FAST (default 1; A0_C51_FAST in the environment): a0_loss_c51 with qsel given, at most 6
- * actions and at most 64 atoms runs the short-dependent-chain kernel; 0 forces the general kernel.
+ * actions, at most 64 atoms and a finite, nonzero fl32(vmax - vmin) / (M - 1) runs the
+ * short-dependent-chain kernel; 0 forces the general kernel.
  * Bit-identical outputs.                                                                         */
 #define A0_OPT_C51_FAST 5
 /* A0_OPT_K3_L2 (A0_K3_L2 in the environment): L2 eviction hints of the default gather's bulk copies.
@@ -602,6 +603,10 @@ int a0_loss_mdqn(const a0_loss_common_t* c, const float* q, const float* qt_next
 int a0_loss_c51(const a0_loss_common_t* c, const float* logits, const float* tgt_logits,
                 const float* qsel, const float* atoms, int32_t M, float vmin, float vmax,
                 float* grad, float* target_prob, a0_stream_t stream);
+/* Test hook of a0_loss_c51's bin arithmetic: for every float32 nu in [0, fl32(vmax - vmin)], the division
+ * nu / delta of the short-chain kernel against the correctly rounded one, delta = fl32(vmax - vmin) / (M - 1).
+ * out: 2 device words; out[0] += the number of mismatches, out[1] = min(out[1], bit pattern of the first). */
+int a0_c51_div_check(float vmin, float vmax, int32_t M, unsigned long long* out, a0_stream_t stream);
 /* Quantile-Huber family.  layout 0: q f32[B,A,Nj], qt f32[B,A,Ni], taus implicit (2j+1)/2Nj (QR).
  * layout 1: q f32[B,Nj,A], qt f32[B,Ni,A], taus f32[B,Nj] (IQN, FQF).
  * FQF fraction term (optional, layout 1, Ni == Nj == F): q_bar f32[B,F-1,A] = quantile values at the

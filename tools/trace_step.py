@@ -94,8 +94,8 @@ if m4.any():
     c0 = rec[sel][:, 2][m4]
     pts = np.concatenate([c0[:, None], xs[m4]], 1)
     d = np.median(np.diff(pts, axis=1), 0)
-    lab = ["loads land", "arg-max | online max", "target softmax | online sum-exp", "projection arithmetic", "segmented scan + bins",
-           "CE | mass reductions", "gradient stores", "emit loss / priority / max_p"]
+    lab = ["loads land", "arg-max | row maxima", "sum-exps | bin geometry | log-softmax", "p / sum + term weights", "segmented scan + bins",
+           "CE | mass reductions", "emit loss / priority / max_p + gradient stores", "-"]
     print("K4 (C51) warp-0 phases after griddepcontrol.wait, median SM cycles over", int(m4.sum()), "CTAs (1965 cycles = 1 us):")
     print("   " + " | ".join(f"{l} {int(v)}" for l, v in zip(lab, d)) + f" | total {int(d.sum())}")
 m3 = kid == 3
