@@ -19,6 +19,7 @@ PTR_FRAMES, PTR_REC_SLOTS, PTR_REC_INFO, PTR_TREE, PTR_MAX_P = range(5)
 OPT_PDL = 1          # include/agent0_b200.h: A0_OPT_PDL (mask of kernel classes launched programmatically; bit 0 = K4)
 K2B_PLAN_MAX = 1024  # include/agent0_b200.h: A0_K2B_PLAN_MAX (largest index count of a0_pt_update_plan / _apply)
 K2B_PLAN_BYTES = 90176  # A0_K2B_PLAN_BYTES (the plan buffer)
+C51_EARLY = 1        # include/agent0_b200.h: A0_C51_EARLY (a0_loss_c51_linked: batch-side work before the wait)
 
 
 def lz4_stride(frame_bytes):
@@ -119,6 +120,7 @@ SIGNATURES = {
     "a0_loss_dqn": (_i32, [C.POINTER(LossCommon), _vp, _vp, _vp, _vp, _vp]),
     "a0_loss_mdqn": (_i32, [C.POINTER(LossCommon), _vp, _vp, _vp, _f32, _f32, _vp, _vp]),
     "a0_loss_c51": (_i32, [C.POINTER(LossCommon), _vp, _vp, _vp, _vp, _i32, _f32, _f32, _vp, _vp, _vp]),
+    "a0_loss_c51_linked": (_i32, [C.POINTER(LossCommon), _vp, _vp, _vp, _vp, _i32, _f32, _f32, _vp, _vp, _i32, _vp]),
     "a0_c51_div_check": (_i32, [_f32, _f32, _i32, _vp, _vp]),
     "a0_loss_quantile": (_i32, [C.POINTER(LossCommon), _i32, _vp, _vp, _vp, _vp, _i32, _i32, _vp,
                                 _vp, _vp, _vp, _vp, _vp]),

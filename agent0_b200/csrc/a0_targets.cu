@@ -450,7 +450,13 @@ static void a0_c51_delta(float vmin, float vmax, int32_t M, float* delta, double
   *rdelta = 1.0 / (double)*delta;
 }
 
-template <int WARPS>
+// EARLY (a0_loss_c51_linked, A0_C51_EARLY): one link of a chain of dependent launches whose batch-side inputs were
+// complete before the link ahead of it passed its own wait.  The CTAs of such a link are resident for the whole
+// dependent chain of that link (it lets this one launch right after its wait), so everything that reads only the
+// batch side -- action, reward, done, weight, atoms, the projection's geometry, the zeros of the gradient block --
+// runs before griddepcontrol.wait; the network outputs are still read after it, and of the online rows only the
+// taken action's (known by then).  launch_dependents stays after the wait, so the chain stays one launch deep.
+template <int WARPS, bool EARLY>
 __global__ void __launch_bounds__(WARPS * 32)
 a0_k4_c51_fast(const A0Common c, const float* __restrict__ logits, const float* __restrict__ tgt_logits,
                const float* __restrict__ qsel, const float* __restrict__ atoms, int32_t M, float vmin, float vmax,
@@ -460,56 +466,115 @@ a0_k4_c51_fast(const A0Common c, const float* __restrict__ logits, const float* 
   // oracle.losses.c51_project)
   __shared__ float s_t[WARPS][4][72];
   A0_T0();
-  A0_PDL_PROLOGUE();
-  A0_TMID();
 #ifdef A0_TRACE
-  const long long _c0 = clock64();
+  _tx[7] = (unsigned long long)clock64();      // entry: with EARLY, the batch-side phase is x[7] .. the wait
+#endif
+  if (!EARLY) {
+    A0_PDL_PROLOGUE();
+    A0_TMID();
+  }
+#ifdef A0_TRACE
+  long long _c0 = clock64();
 #endif
   const int lane = threadIdx.x & 31;
   const int wid = threadIdx.x >> 5;
   const int b = blockIdx.x * WARPS + wid;
-  if (b >= c.B) return;
+  if (b >= c.B) return;       // never the whole CTA: warp 0 always has a sample, and it waits
   const int A = c.A;
   const bool in0 = lane < M, in1 = lane + 32 < M;
-  // ---- every global load of the sample, issued up front ----------------------------------------------
+  float(*terms)[72] = s_t[wid];
+  // ---- the batch side: scalars of the sample, atoms, zeros of the shared rows and of the gradient block ----
+  int a, r0;
+  float r, d, w, z0, z1;
+  float* gb;
+  auto batch_side = [&] {
+    a = (int)c.action[b];
+    r = c.reward[b], d = c.done[b], w = c.weight[b];
+    z0 = in0 ? atoms[lane] : 0.0f, z1 = in1 ? atoms[lane + 32] : 0.0f;
+#pragma unroll
+    for (int t = 0; t < 4; ++t) {
+      terms[t][lane] = 0.0f;
+      terms[t][lane + 32] = 0.0f;
+    }
+    // The gradient block [A, M] of the sample is zero outside row a: those stores depend on nothing but
+    // `a`, so they go out now, under the latency of the loads, and only row a is left for the end.
+    const int AM = A * M;
+    r0 = a * M;
+    gb = grad + (size_t)b * AM;
+    for (int e = lane; e < AM; e += 32)
+      if (e < r0 || e >= r0 + M) gb[e] = 0.0f;
+  };
+  // ---- the projection's geometry (agent.py:230-250), which needs neither softmax: bin positions, keys of the
+  // segmented scan and its run masks, fractions of the lower and upper terms --------------------------------------
+  int k0, k1;
+  float fl0, fu0, fl1, fu1;
+  unsigned join0 = 0, join1 = 0;
+  unsigned tail0, tail1;       // run tails (0 / 1)
+  auto geometry = [&] {
+    const float gm = __fmul_rn(c.gamma_n, __fsub_rn(1.0f, d));
+    const float tz0 = fminf(fmaxf(__fadd_rn(r, __fmul_rn(gm, z0)), vmin), vmax);
+    const float tz1 = fminf(fmaxf(__fadd_rn(r, __fmul_rn(gm, z1)), vmin), vmax);
+    const float bs0 = a0_c51_div_delta(__fsub_rn(tz0, vmin), delta, rdelta);
+    const float bs1 = a0_c51_div_delta(__fsub_rn(tz1, vmin), delta, rdelta);
+    const int c0 = max((int)ceilf(bs0) - 1, 0), c1 = max((int)ceilf(bs1) - 1, 0);
+    k0 = in0 ? c0 : -1, k1 = in1 ? c1 : -1;   // lower bin of atoms lane and lane + 32; the upper one is k + 1
+    fl0 = __fsub_rn((float)(c0 + 1), bs0), fu0 = __fsub_rn(bs0, (float)c0);
+    fl1 = __fsub_rn((float)(c1 + 1), bs1), fu1 = __fsub_rn(bs1, (float)c1);
+    // segmented inclusive scan over the lanes, keyed by the lower bin (bins are non-decreasing in the atom index, so
+    // the sources of one bin are adjacent lanes); step s adds the partial sum 2^s lanes up where the keys agree
+#pragma unroll
+    for (int s = 0; s < 5; ++s) {
+      const int q0 = __shfl_up_sync(0xffffffffu, k0, 1 << s), q1 = __shfl_up_sync(0xffffffffu, k1, 1 << s);
+      if (lane >= (1 << s) && q0 == k0) join0 |= 1u << s;
+      if (lane >= (1 << s) && q1 == k1) join1 |= 1u << s;
+    }
+    const int n0 = __shfl_down_sync(0xffffffffu, k0, 1), n1 = __shfl_down_sync(0xffffffffu, k1, 1);
+    tail0 = k0 >= 0 && (lane == 31 || n0 != k0), tail1 = k1 >= 0 && (lane == 31 || n1 != k1);
+  };
+  if (EARLY) {
+    batch_side();
+    geometry();
+    // the wait orders memory accesses only: without this the compiler would sink the geometry's arithmetic below it
+    asm volatile("" : "+r"(k0), "+r"(k1), "+f"(fl0), "+f"(fu0), "+f"(fl1), "+f"(fu1), "+r"(join0), "+r"(join1),
+                 "+r"(tail0), "+r"(tail1), "+r"(a), "+f"(w));
+    A0_PDL_PROLOGUE();        // from here on the network outputs are read
+    A0_TMID();
+#ifdef A0_TRACE
+    _c0 = clock64();
+#endif
+  }
+  // ---- every global load of the network outputs, issued up front ---------------------------------------
   float lo_all[C51_SPEC_A][2], tg_all[C51_SPEC_A][2], qs[C51_SPEC_A];
+  float l0 = -INFINITY, l1 = -INFINITY, p0 = -INFINITY, p1 = -INFINITY;
   const float* lrow = logits + (size_t)b * A * M + lane;
   const float* trow = tgt_logits + (size_t)b * A * M + lane;
   const float* qrow = qsel + (size_t)b * A;
+  if (EARLY) {                // the action is known: only its online row (an action outside [0, A) selects none)
+    const bool on = a >= 0 && a < A;
+    l0 = (on && in0) ? lrow[a * M] : -INFINITY;
+    l1 = (on && in1) ? lrow[a * M + 32] : -INFINITY;
+  }
 #pragma unroll
   for (int a2 = 0; a2 < C51_SPEC_A; ++a2) {
     const bool on = a2 < A;
-    lo_all[a2][0] = (on && in0) ? lrow[a2 * M] : -INFINITY;
-    lo_all[a2][1] = (on && in1) ? lrow[a2 * M + 32] : -INFINITY;
+    if (!EARLY) {
+      lo_all[a2][0] = (on && in0) ? lrow[a2 * M] : -INFINITY;
+      lo_all[a2][1] = (on && in1) ? lrow[a2 * M + 32] : -INFINITY;
+    }
     tg_all[a2][0] = (on && in0) ? trow[a2 * M] : -INFINITY;
     tg_all[a2][1] = (on && in1) ? trow[a2 * M + 32] : -INFINITY;
     qs[a2] = on ? qrow[a2] : -INFINITY;                 // same address in every lane: one broadcast transaction
   }
-  const int a = (int)c.action[b];
-  const float r = c.reward[b], d = c.done[b], w = c.weight[b];
-  const float z0 = in0 ? atoms[lane] : 0.0f, z1 = in1 ? atoms[lane + 32] : 0.0f;
-  float(*terms)[72] = s_t[wid];
-#pragma unroll
-  for (int t = 0; t < 4; ++t) {
-    terms[t][lane] = 0.0f;
-    terms[t][lane + 32] = 0.0f;
-  }
-  // The gradient block [A, M] of the sample is zero outside row a: those stores depend on nothing but
-  // `a`, so they go out now, under the latency of the loads above, and only row a is left for the end.
-  const int AM = A * M, r0 = a * M;
-  float* gb = grad + (size_t)b * AM;
-  for (int e = lane; e < AM; e += 32)
-    if (e < r0 || e >= r0 + M) gb[e] = 0.0f;
+  if (!EARLY) batch_side();
   // ---- action selection: first maximum, as torch.argmax (agent.py:224) ---------------------------------
   int a_star = 0;
   float best = qs[0];
 #pragma unroll
   for (int a2 = 1; a2 < C51_SPEC_A; ++a2)
     if (qs[a2] > best) { best = qs[a2]; a_star = a2; }
-  float l0 = -INFINITY, l1 = -INFINITY, p0 = -INFINITY, p1 = -INFINITY;
 #pragma unroll
   for (int a2 = 0; a2 < C51_SPEC_A; ++a2) {
-    if (a2 == a) { l0 = lo_all[a2][0]; l1 = lo_all[a2][1]; }
+    if (!EARLY && a2 == a) { l0 = lo_all[a2][0]; l1 = lo_all[a2][1]; }
     if (a2 == a_star) { p0 = tg_all[a2][0]; p1 = tg_all[a2][1]; }
   }
   A0_TX(0);
@@ -521,28 +586,7 @@ a0_k4_c51_fast(const A0Common c, const float* __restrict__ logits, const float* 
   p0 = expf(in0 ? p0 - mx : -INFINITY);
   p1 = expf(in1 ? p1 - mx : -INFINITY);
   float ose = eo0 + eo1, se = p0 + p1;
-  // The projection's geometry (agent.py:230-250) needs neither softmax: bin positions, keys of the segmented scan
-  // and its run masks, fractions of the lower and upper terms.
-  const float gm = __fmul_rn(c.gamma_n, __fsub_rn(1.0f, d));
-  const float tz0 = fminf(fmaxf(__fadd_rn(r, __fmul_rn(gm, z0)), vmin), vmax);
-  const float tz1 = fminf(fmaxf(__fadd_rn(r, __fmul_rn(gm, z1)), vmin), vmax);
-  const float bs0 = a0_c51_div_delta(__fsub_rn(tz0, vmin), delta, rdelta);
-  const float bs1 = a0_c51_div_delta(__fsub_rn(tz1, vmin), delta, rdelta);
-  const int c0 = max((int)ceilf(bs0) - 1, 0), c1 = max((int)ceilf(bs1) - 1, 0);
-  const int k0 = in0 ? c0 : -1, k1 = in1 ? c1 : -1;   // lower bin of atoms lane and lane + 32; the upper one is k + 1
-  const float fl0 = __fsub_rn((float)(c0 + 1), bs0), fu0 = __fsub_rn(bs0, (float)c0);
-  const float fl1 = __fsub_rn((float)(c1 + 1), bs1), fu1 = __fsub_rn(bs1, (float)c1);
-  // segmented inclusive scan over the lanes, keyed by the lower bin (bins are non-decreasing in the atom index, so
-  // the sources of one bin are adjacent lanes); step s adds the partial sum 2^s lanes up where the keys agree
-  unsigned join0 = 0, join1 = 0;
-#pragma unroll
-  for (int s = 0; s < 5; ++s) {
-    const int q0 = __shfl_up_sync(0xffffffffu, k0, 1 << s), q1 = __shfl_up_sync(0xffffffffu, k1, 1 << s);
-    if (lane >= (1 << s) && q0 == k0) join0 |= 1u << s;
-    if (lane >= (1 << s) && q1 == k1) join1 |= 1u << s;
-  }
-  const int n0 = __shfl_down_sync(0xffffffffu, k0, 1), n1 = __shfl_down_sync(0xffffffffu, k1, 1);
-  const bool tail0 = k0 >= 0 && (lane == 31 || n0 != k0), tail1 = k1 >= 0 && (lane == 31 || n1 != k1);
+  if (!EARLY) geometry();     // under the latency of the sum-exp reduction
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) {
     const float a_ = __shfl_xor_sync(0xffffffffu, ose, o);
@@ -610,7 +654,6 @@ a0_k4_c51_fast(const A0Common c, const float* __restrict__ logits, const float* 
     if (in1) target_prob[(size_t)b * M + lane + 32] = m1;
   }
   A0_TX(6);
-  A0_TX(7);
 #ifdef A0_TRACE
   _t2 = _t2 * 0 + (unsigned long long)_c0;
 #endif
@@ -627,14 +670,14 @@ static bool a0_option_c51_fast() {
 }
 void a0_set_c51_fast(int on) { g_c51_fast = on != 0; }
 
-extern "C" int a0_loss_c51(const a0_loss_common_t* c, const float* logits, const float* tgt_logits,
-                           const float* qsel, const float* atoms, int32_t M, float vmin, float vmax, float* grad,
-                           float* target_prob, a0_stream_t stream) {
-  int rc = a0_check_common(c, "a0_loss_c51");
+static int a0_loss_c51_launch(const char* fn, const a0_loss_common_t* c, const float* logits, const float* tgt_logits,
+                              const float* qsel, const float* atoms, int32_t M, float vmin, float vmax, float* grad,
+                              float* target_prob, bool early, a0_stream_t stream) {
+  int rc = a0_check_common(c, fn);
   if (rc) return rc;
-  A0_REQUIRE(logits && tgt_logits && atoms && grad, "a0_loss_c51: NULL tensor");
-  A0_REQUIRE(M >= 2 && M <= C51_MAXR * 32, "a0_loss_c51: num_atoms %d outside [2,%d]", M, C51_MAXR * 32);
-  A0_REQUIRE(vmax > vmin, "a0_loss_c51: vmax must exceed vmin");
+  A0_REQUIRE(logits && tgt_logits && atoms && grad, "%s: NULL tensor", fn);
+  A0_REQUIRE(M >= 2 && M <= C51_MAXR * 32, "%s: num_atoms %d outside [2,%d]", fn, M, C51_MAXR * 32);
+  A0_REQUIRE(vmax > vmin, "%s: vmax must exceed vmin", fn);
   if (c->B == 0) return A0_OK;
   float delta;
   double rdelta;
@@ -649,20 +692,39 @@ extern "C" int a0_loss_c51(const a0_loss_common_t* c, const float* logits, const
     }
     const unsigned grid = (unsigned)((c->B + warps - 1) / warps);
 #define A0_C51_FAST_LAUNCH(W)                                                                                              \
-    A0_LAUNCH(a0_k4_c51_fast<W>, grid, W * 32, 0, (cudaStream_t)stream, 1, A0_PDL_K4, a0_unpack(c), logits, tgt_logits, qsel,   \
-              atoms, M, vmin, vmax, delta, rdelta, grad, target_prob)
-    if (warps == 1) A0_C51_FAST_LAUNCH(1);
-    else if (warps == 2) A0_C51_FAST_LAUNCH(2);
-    else if (warps == 4) A0_C51_FAST_LAUNCH(4);
-    else if (warps == 8) A0_C51_FAST_LAUNCH(8);
-    else if (warps == 16) A0_C51_FAST_LAUNCH(16);
-    else A0_C51_FAST_LAUNCH(32);
+    if (early)                                                                                                             \
+      A0_LAUNCH(a0_k4_c51_fast<W, true>, grid, W * 32, 0, (cudaStream_t)stream, 1, A0_PDL_K4, a0_unpack(c), logits,         \
+                tgt_logits, qsel, atoms, M, vmin, vmax, delta, rdelta, grad, target_prob);                                 \
+    else                                                                                                                   \
+      A0_LAUNCH(a0_k4_c51_fast<W, false>, grid, W * 32, 0, (cudaStream_t)stream, 1, A0_PDL_K4, a0_unpack(c), logits,        \
+                tgt_logits, qsel, atoms, M, vmin, vmax, delta, rdelta, grad, target_prob)
+    if (warps == 1) { A0_C51_FAST_LAUNCH(1); }
+    else if (warps == 2) { A0_C51_FAST_LAUNCH(2); }
+    else if (warps == 4) { A0_C51_FAST_LAUNCH(4); }
+    else if (warps == 8) { A0_C51_FAST_LAUNCH(8); }
+    else if (warps == 16) { A0_C51_FAST_LAUNCH(16); }
+    else { A0_C51_FAST_LAUNCH(32); }
 #undef A0_C51_FAST_LAUNCH
     return A0_OK;
   }
   A0_LAUNCH(a0_k4_c51, (unsigned)((c->B + C51_WARPS - 1) / C51_WARPS), C51_WARPS * 32, 0, (cudaStream_t)stream, 1, A0_PDL_K4,
             a0_unpack(c), logits, tgt_logits, qsel, atoms, M, vmin, vmax, grad, target_prob);
   return A0_OK;
+}
+
+extern "C" int a0_loss_c51(const a0_loss_common_t* c, const float* logits, const float* tgt_logits,
+                           const float* qsel, const float* atoms, int32_t M, float vmin, float vmax, float* grad,
+                           float* target_prob, a0_stream_t stream) {
+  return a0_loss_c51_launch("a0_loss_c51", c, logits, tgt_logits, qsel, atoms, M, vmin, vmax, grad, target_prob, false,
+                            stream);
+}
+
+extern "C" int a0_loss_c51_linked(const a0_loss_common_t* c, const float* logits, const float* tgt_logits,
+                                  const float* qsel, const float* atoms, int32_t M, float vmin, float vmax, float* grad,
+                                  float* target_prob, int32_t flags, a0_stream_t stream) {
+  A0_REQUIRE((flags & ~A0_C51_EARLY) == 0, "a0_loss_c51_linked: unknown flags 0x%x", (unsigned)flags);
+  return a0_loss_c51_launch("a0_loss_c51_linked", c, logits, tgt_logits, qsel, atoms, M, vmin, vmax, grad, target_prob,
+                            (flags & A0_C51_EARLY) != 0, stream);
 }
 
 // Every float32 nu in [0, hi] (by bit pattern): a0_c51_div_delta against __fdiv_rn.  out[0] += mismatches,

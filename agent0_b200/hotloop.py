@@ -60,6 +60,21 @@ def wave_plan(L, B, frame_bytes, spec="auto"):
     return plan
 
 
+def early_links(L, waves, plan_join=None):
+    """The K4 links of a waved step that may run their batch-side work before griddepcontrol.wait (a0_loss_c51_linked,
+    A0_C51_EARLY): those whose sole predecessor is the previous K4.  A link launches once the link ahead of it has
+    passed its own wait, so everything that link joined -- the wave that holds this batch, the draw before it -- is
+    complete.  A link that itself joins a wave (the first batch of each) or the write-back plan (``plan_join``) has a
+    second predecessor and reads nothing before its wait.  waves: wave_plan's rows; None (the single gather launch):
+    no link."""
+    if not waves:
+        return frozenset()
+    joins = {b0 for b0, _, _, _ in waves}
+    if plan_join is not None:
+        joins.add(plan_join)
+    return frozenset(k for k in range(L) if k not in joins)
+
+
 class ReplayTargetLoop:
     def __init__(self, replay, algo, batch_size, learner_steps, action_dim, outputs, n_step=None, double_q=True,
                  per=None, variant=0, discount=None, alpha=0.5, eps=0.01, c51=(51, -10.0, 10.0), mdqn=(0.03, -1.0),
@@ -164,7 +179,7 @@ class ReplayTargetLoop:
             self.plan = torch.empty(_lib.K2B_PLAN_BYTES, dtype=torch.uint8, device=dev)
             self.plan_ev = torch.cuda.Event()
         self.launches_per_step = 1 + n_gather + self.L + (1 if self.per else 0)     # our kernels (uniform_ is torch's)
-        self._k4 = None
+        self._k4 = self._k4_early = None
         self._k4_all = None
         self.graph = None
         self.report = []          # pinned host (indices, losses) pairs filled by K2b: bind_report()
@@ -244,9 +259,10 @@ class ReplayTargetLoop:
                                # appends heavier than earlier ones (leaf = max_p^alpha) and the draw non-uniform
                                max_p=self.rp.max_p_tensor.data_ptr() if self.per else None), s
 
-    def _bind(self, lo, count):
+    def _bind(self, lo, count, early=False):
         """(function, argument tuple) of the K4 launch over rows [lo, lo+count): the a0_loss_common_t block
-        and the sliced device pointers are built once, so a launch is a single ctypes call."""
+        and the sliced device pointers are built once, so a launch is a single ctypes call.  early: a link of
+        ``early_links`` (C51 only)."""
         lib, o, algo = self.lib, self.o, self.algo
         c, s = self._common(lo, count)
         p = lambda t: t[s].data_ptr()
@@ -258,8 +274,12 @@ class ReplayTargetLoop:
                                     p(self.grad)))
         elif algo == "c51":
             M, vmin, vmax = self.c51
-            a = (lib.a0_loss_c51, (C.byref(c), p(o["online"]), p(o["tgt_next"]), qsel, o["atoms"].data_ptr(), M, vmin, vmax,
-                                   p(self.grad), None))
+            if early:
+                a = (lib.a0_loss_c51_linked, (C.byref(c), p(o["online"]), p(o["tgt_next"]), qsel, o["atoms"].data_ptr(), M, vmin,
+                                              vmax, p(self.grad), None, _lib.C51_EARLY))
+            else:
+                a = (lib.a0_loss_c51, (C.byref(c), p(o["online"]), p(o["tgt_next"]), qsel, o["atoms"].data_ptr(), M, vmin, vmax,
+                                       p(self.grad), None))
         elif algo == "qr":
             N = o["online"].shape[2]
             a = (lib.a0_loss_quantile, (C.byref(c), 0, p(o["online"]), p(o["tgt_next"]), None, qsel, o["tgt_next"].shape[2], N,
@@ -273,11 +293,13 @@ class ReplayTargetLoop:
                                         p(self.grad), p(o["q_bar"]), p(o["taus"]), p(self.frac), p(self.gtau)))
         return c, a
 
-    def target_loss(self, k):
-        """K4 for batch k: per-sample loss, gradient w.r.t. the online output, new priorities."""
+    def target_loss(self, k, early=False):
+        """K4 for batch k: per-sample loss, gradient w.r.t. the online output, new priorities.  early: batch k's link is
+        one of ``early_links`` (its inputs but the network outputs are read before its wait; C51's short-chain kernel)."""
         if self._k4 is None:
             self._k4 = [self._bind(k_ * self.B, self.B) for k_ in range(self.L)]
-        fn, args = self._k4[k][1]
+            self._k4_early = [self._bind(k_ * self.B, self.B, early=True) for k_ in range(self.L)] if self.algo == "c51" else None
+        fn, args = (self._k4_early if early and self._k4_early else self._k4)[k][1]
         rc = fn(*args, self._st())
         if rc:
             _lib.check(rc, "a0_loss_" + self.algo)
@@ -344,6 +366,7 @@ class ReplayTargetLoop:
             if update:
                 self.update(slot, after_k4=True)
             return
+        early = early_links(self.L, self.waves, self._plan_join if planned else None)
         for k in range(self.L):
             j = self._join.get(k)
             join_plan = planned and k == self._plan_join
@@ -352,7 +375,7 @@ class ReplayTargetLoop:
             if (j is None and not join_plan) or self.pdl_at_joins:
                 if j is not None:
                     self._wait_wave(j)
-                self.target_loss(k)
+                self.target_loss(k, early=k in early)
             else:
                 # the K4 that joins wave j (or the plan) has more than one predecessor: launched without the
                 # programmatic attribute unless pdl_at_joins

@@ -603,6 +603,19 @@ int a0_loss_mdqn(const a0_loss_common_t* c, const float* q, const float* qt_next
 int a0_loss_c51(const a0_loss_common_t* c, const float* logits, const float* tgt_logits,
                 const float* qsel, const float* atoms, int32_t M, float vmin, float vmax,
                 float* grad, float* target_prob, a0_stream_t stream);
+/* a0_loss_c51 as one link of a chain of dependent launches on one stream (hotloop.ReplayTargetLoop: one launch per
+ * batch, each behind the previous one).  flags = 0: a0_loss_c51 exactly.  A0_C51_EARLY: the short-chain kernel (qsel
+ * given, A <= 6, M <= 64) reads action, reward, done, weight and atoms, computes the projection's geometry and stores
+ * the zeros of the sample's gradient block outside the taken action's row BEFORE it waits for its stream predecessor
+ * (griddepcontrol.wait); logits, tgt_logits and qsel are still read after the wait.  The caller guarantees: those
+ * batch-side inputs and atoms are complete, and no kernel that can still run once this launch's stream predecessor
+ * has passed its own wait writes them or reads this batch's gradient rows.  That holds when the stream predecessor
+ * is the previous link of the chain and its own only predecessor joined every writer of this batch's inputs; a link
+ * that itself joins another stream or event must not set the flag.  Other kernels ignore it.  Same results.     */
+#define A0_C51_EARLY 1
+int a0_loss_c51_linked(const a0_loss_common_t* c, const float* logits, const float* tgt_logits,
+                       const float* qsel, const float* atoms, int32_t M, float vmin, float vmax,
+                       float* grad, float* target_prob, int32_t flags, a0_stream_t stream);
 /* Test hook of a0_loss_c51's bin arithmetic: for every float32 nu in [0, fl32(vmax - vmin)], the division
  * nu / delta of the short-chain kernel against the correctly rounded one, delta = fl32(vmax - vmin) / (M - 1).
  * out: 2 device words; out[0] += the number of mismatches, out[1] = min(out[1], bit pattern of the first). */

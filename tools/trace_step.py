@@ -91,13 +91,34 @@ rows.sort(key=lambda r: r[2])
 m4 = kid == 4
 if m4.any():
     # K4 stores clock64 (SM cycles) at the wait's return in t2 and at eight points after it
+    # x[7] holds the cycle at entry: entry -> wait returned is the batch-side phase plus the wait on an early link
     c0 = rec[sel][:, 2][m4]
-    pts = np.concatenate([c0[:, None], xs[m4]], 1)
-    d = np.median(np.diff(pts, axis=1), 0)
+    pts = np.concatenate([c0[:, None], xs[m4][:, :7]], 1)
+    dd = np.diff(pts, axis=1)
     lab = ["loads land", "arg-max | row maxima", "sum-exps | bin geometry | log-softmax", "p / sum + term weights", "segmented scan + bins",
-           "CE | mass reductions", "emit loss / priority / max_p + gradient stores", "-"]
-    print("K4 (C51) warp-0 phases after griddepcontrol.wait, median SM cycles over", int(m4.sum()), "CTAs (1965 cycles = 1 us):")
-    print("   " + " | ".join(f"{l} {int(v)}" for l, v in zip(lab, d)) + f" | total {int(d.sum())}")
+           "CE | mass reductions", "emit loss / priority / max_p + gradient stores"]
+    from agent0_b200.hotloop import early_links
+    early = early_links(L, hp.waves, hp._plan_join if hp._use_plan else None)
+    t0_4, t1_4 = t0[m4], t1[m4]
+    o4 = np.argsort(t0_4)
+    per4 = max(1, int(m4.sum()) // L)
+    link = np.empty(int(m4.sum()), np.int64)
+    for i in range(L):
+        link[o4[i * per4:(i + 1) * per4]] = i
+    print("K4 (C51) warp-0 phases after griddepcontrol.wait, median SM cycles (1965 cycles = 1 us):")
+    for name, ks in (("all links", range(L)), ("early links", sorted(early)), ("join / other links", sorted(set(range(L)) - early))):
+        mk = np.isin(link, list(ks))
+        if mk.any():
+            d = np.median(dd[mk], 0)
+            print(f"   {name} ({int(mk.sum())} CTAs): " + " | ".join(f"{l} {int(v)}" for l, v in zip(lab, d)) +
+                  f" | total {int(np.median(dd[mk].sum(1)))}")
+    # the link-to-link period: last exit of link i-1 -> last exit of link i, by the kind of link i
+    ex = np.array([t1_4[link == i].max() for i in range(L)])
+    pre = np.array([np.median(c0[link == i] - xs[m4][link == i, 7]) for i in range(L)])
+    for name, ks in (("early links", sorted(early)), ("join / other links", sorted(set(range(1, L)) - early))):
+        if ks:
+            print(f"   {name}: link-to-link period (exit to exit) median {np.median(np.diff(ex)[np.array(ks) - 1]) / 1e3:.2f} us; "
+                  f"entry -> wait returned median {int(np.median(pre[ks]))} cycles; links {ks}")
 m3 = kid == 3
 if m3.any():
     q = [0, 10, 50, 90, 100]
