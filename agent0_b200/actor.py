@@ -37,10 +37,12 @@ class ActorPolicy:
         self.A = int(cfg.action_dim)
         self.norm_mode = int(norm_mode)
         self.rng = rng if rng is not None else np.random
-        self._E = -1
+        self._key = None
 
     def _buffers(self, E, obs_shape):
-        if E == self._E:
+        # keyed on the whole shape: a call with the same E and other frames needs other buffers
+        key = (E,) + tuple(obs_shape)
+        if key == self._key:
             return
         dev = self.device
         n = int(np.prod(obs_shape))
@@ -53,7 +55,7 @@ class ActorPolicy:
         self._res_dev = torch.zeros(E + 1, dtype=torch.int64, device=dev)          # [actions | mean (f32 bits)]
         self._res_host = torch.empty(E + 1, dtype=torch.int64).pin_memory()
         self._scratch = torch.zeros(2, dtype=torch.float32, device=dev)
-        self._E = E
+        self._key = key
 
     @torch.no_grad()
     def act(self, obs, epsilon):

@@ -264,7 +264,7 @@ a0_k4_c51(const A0Common c, const float* __restrict__ logits, const float* __res
       const float ov = __shfl_xor_sync(0xffffffffu, v, o);
       const int oi = __shfl_xor_sync(0xffffffffu, vi, o);
       const float om = __shfl_xor_sync(0xffffffffu, omx, o);
-      if (ov > v || (ov == v && oi < vi)) { v = ov; vi = oi; }
+      if (a0_argmax_before(ov, oi, v, vi)) { v = ov; vi = oi; }
       omx = fmaxf(omx, om);
     }
     a_star = vi;
@@ -290,7 +290,7 @@ a0_k4_c51(const A0Common c, const float* __restrict__ logits, const float* __res
 #pragma unroll
       for (int k = 0; k < C51_MAXR; ++k) ev += __fdiv_rn(v[k], se) * z[k];
       ev = a0_warp_sum(ev);
-      if (ev > best) { best = ev; a_star = a2; }
+      if (a0_argmax_takes(ev, best)) { best = ev; a_star = a2; }
     }
   }
 
@@ -566,12 +566,8 @@ a0_k4_c51_fast(const A0Common c, const float* __restrict__ logits, const float* 
     qs[a2] = on ? qrow[a2] : -INFINITY;                 // same address in every lane: one broadcast transaction
   }
   if (!EARLY) batch_side();
-  // ---- action selection: first maximum, as torch.argmax (agent.py:224) ---------------------------------
-  int a_star = 0;
-  float best = qs[0];
-#pragma unroll
-  for (int a2 = 1; a2 < C51_SPEC_A; ++a2)
-    if (qs[a2] > best) { best = qs[a2]; a_star = a2; }
+  // ---- action selection: torch.argmax's rule (agent.py:224) ---------------------------------------------
+  const int a_star = a0_argmax_regs(qs);
 #pragma unroll
   for (int a2 = 0; a2 < C51_SPEC_A; ++a2) {
     if (!EARLY && a2 == a) { l0 = lo_all[a2][0]; l1 = lo_all[a2][1]; }
@@ -825,11 +821,7 @@ a0_k4_quantile(const A0Common c, int32_t layout, const float* __restrict__ q, co
       qv[a2] = (on && tid < Nj) ? qb[(size_t)tid * A + a2] : 0.0f;
     }
     if (tid < Nj) tau = taus[(size_t)b * Nj + tid];
-    int a_star = 0;
-    float best = qs[0];
-#pragma unroll
-    for (int a2 = 1; a2 < QH_SPEC_A; ++a2)
-      if (qs[a2] > best) { best = qs[a2]; a_star = a2; }       // first maximum, as torch.argmax
+    const int a_star = a0_argmax_regs(qs);
     float tsel = 0.0f;
 #pragma unroll
     for (int a2 = 0; a2 < QH_SPEC_A; ++a2) {
@@ -1025,11 +1017,7 @@ a0_k4_quantile_sorted(const A0Common c, int32_t layout, const float* __restrict_
     w = c.weight[b];
     if (tid < Nj) tau = taus ? taus[(size_t)b * Nj + tid] : __fdiv_rn((float)(2 * tid + 1), 2.0f * (float)Nj);
     for (int i = tid; i < A * Nj; i += nthreads) gb[i] = 0.0f;      // the taken action's entries are rewritten after the barriers below
-    int a_star = 0;
-    float best = qs[0];
-#pragma unroll
-    for (int a2 = 1; a2 < AMAX; ++a2)
-      if (qs[a2] > best) { best = qs[a2]; a_star = a2; }       // first maximum, as torch.argmax
+    const int a_star = a0_argmax_regs(qs);
     float tsel = 0.0f;
 #pragma unroll
     for (int a2 = 0; a2 < AMAX; ++a2) {
@@ -1217,7 +1205,7 @@ a0_k4_quantile_warp(const A0Common c, int32_t layout, const float* __restrict__ 
       float s = 0.0f;
       for (int i = lane; i < Ni; i += 32) s += tb[a2 * sA_t + i * sN_t];
       s = __fdiv_rn(a0_warp_sum(s), (float)Ni);
-      if (s > best) { best = s; a_star = a2; }       // first maximum, as torch.argmax
+      if (a0_argmax_takes(s, best)) { best = s; a_star = a2; }
     }
   }
   a_star = __shfl_sync(0xffffffffu, a_star, 0);
@@ -1393,8 +1381,10 @@ a0_k5_act(const float* __restrict__ q, int32_t E, int32_t A, double epsilon, con
       if (qmax_out) qmax_out[e] = q[(size_t)e * A + arg];
     }
   }
-  // The last CTA to finish computes mean_e max_a q[e,a] in a fixed order (thread-strided partial sums,
+  // The last CTA to finish computes mean_e q[e, a*_e] in a fixed order (thread-strided partial sums,
   // shuffle tree, warps in order), so the result does not depend on scheduling; it then re-arms the ticket.
+  // a*_e is found again by the scan form of the same rule, so each term is the value qmax_out holds (a NaN row
+  // makes the mean NaN, as qt_max.mean() does).
   __syncthreads();
   if (threadIdx.x == 0) is_last = (atomicAdd(ticket, 1u) == gridDim.x - 1);
   __syncthreads();
@@ -1402,7 +1392,10 @@ a0_k5_act(const float* __restrict__ q, int32_t E, int32_t A, double epsilon, con
   float s = 0.0f;
   for (int i = threadIdx.x; i < E; i += K5_WARPS * 32) {
     float m = -INFINITY;
-    for (int a2 = 0; a2 < A; ++a2) m = fmaxf(m, q[(size_t)i * A + a2]);
+    for (int a2 = 0; a2 < A; ++a2) {
+      const float v = q[(size_t)i * A + a2];
+      if (a0_argmax_takes(v, m)) m = v;
+    }
     s += m;
   }
   s = a0_warp_sum(s);

@@ -633,7 +633,10 @@ int a0_loss_quantile(const a0_loss_common_t* c, int32_t layout, const float* q, 
 /* ---- K5: actor-side helpers (SURVEY 8f: actor inference batching) ----------------------------------
  * a0_act_epsilon_greedy replaces the tail of Actor.act (agent.py:30-39): per env e,
  *   action[e] = u[e] > epsilon ? argmax_a q[e,a] : action_random[e]   (np.where(rand > eps, greedy, random))
- *   qmax_out[e] = max_a q[e,a] (optional), *qmax_mean = mean_e qmax (qt_max.mean()).
+ *   qmax_out[e] = q[e, argmax_a q[e,a]] (optional), *qmax_mean = mean_e of that value (qt_max.mean()).
+ * The arg-max is torch's (qt.max(dim=-1)): NaN is greater than every number, and among equal maxima
+ * (+0 == -0) or among NaNs the first index wins.  So action, qmax_out and the mean agree: a row with a
+ * NaN picks its first NaN, stores NaN and makes the mean NaN.
  * q f32[E,A] = model.qval(obs); u f64[E] and action_random i64[E] are the caller's draws (numpy's
  * generator in the reference: randint first, then rand).  scratch: 8 bytes of device memory, zero
  * before the first call (the kernel re-arms it).  The mean is summed in a fixed order: the same

@@ -6,12 +6,14 @@ a0_k4_c51_fast computes the bin positions b = (tz - vmin) / delta with a float64
 fmaxf butterfly.  The first test checks the division against __fdiv_rn for every float32 numerator the kernel can see
 (every nu in [0, fl32(vmax - vmin)]) on every support and atom count of tests/test_gpu_loss_shapes.py; the second checks
 both kernels bit for bit on adversarial samples: exact ties, rows of equal values, +-0 maxima, -inf and NaN entries,
-huge offsets, terminal and clamped returns, and returns that put tz exactly on vmin, vmax or a bin edge."""
+huge offsets, terminal and clamped returns, returns that put tz exactly on vmin, vmax or a bin edge, and NaN selection
+values, where both must pick torch.argmax's action (the first NaN) in every lane, as oracle/losses64.py does."""
 import numpy as np
 import pytest
 import torch
 
-from tests.test_gpu_loss_shapes import G3, OPT_C51_FAST, SUPPORTS, dev, launch, same_bits
+from oracle import losses64 as O64
+from tests.test_gpu_loss_shapes import G3, OPT_C51_FAST, SUPPORTS, bound64, dev, launch, nan_selection_rows, same_bits
 
 pytestmark = pytest.mark.gpu
 
@@ -40,7 +42,8 @@ def test_bin_division_is_correctly_rounded_for_every_numerator(lib, vmin, vmax):
                           f"{np.array(first & 0xffffffff, np.uint32).view(f32)!r}")
 
 
-N_CASES = 21
+N_CASES = 27
+SEL_CASES = 21                         # cases SEL_CASES.. are NaN selection values (nan_selection_rows)
 
 
 def _adversarial(M, A, B, vmin, vmax, seed):
@@ -98,6 +101,8 @@ def _adversarial(M, A, B, vmin, vmax, seed):
             r[b] = -1000.0
         elif c == 19:                                  # shifted by whole bins (with gamma_n = 1: tz = z + 3 delta)
             r[b], d[b] = f32(3 * delta), 0.0
+        elif c >= SEL_CASES:                           # random rows, NaN selection values
+            qs[b] = nan_selection_rows(A)[c - SEL_CASES]
         else:
             r[b], d[b] = 0.0, 0.0
     return a, r, d, w, atoms, lg, tg, qs
@@ -122,3 +127,7 @@ def test_fast_kernel_matches_general_on_adversarial_samples(lib, M, A):
             fast = launch(*args)
             same_bits(f"c51 fast vs general, adversarial M={M} A={A} ({vmin},{vmax}) G={G}", fast, general)
             same_bits(f"c51 fast, second launch M={M} A={A}", launch(*args), fast)
+            sel = np.arange(B) % N_CASES >= SEL_CASES
+            ref64 = O64.c51(lg[sel], tg[sel], qs[sel], a[sel], r[sel], d[sel], w[sel], G, atoms, vmin, vmax)
+            for k in ("loss", "target_prob", "grad"):
+                bound64(f"c51 NaN selection M={M} A={A} ({vmin},{vmax}) G={G}.{k}", fast[k][sel], ref64[k])

@@ -10,7 +10,9 @@ and checks
   (d) two launches bit-identical (a race shows up here);
   (e) bit-identity between the paths that are the same arithmetic: a0_k4_c51_fast and a0_k4_c51 (A0_OPT_C51_FAST),
       the quantile kernels with and without the all-action fetch (A0_OPT_QH_SPEC);
-and the sorted quantile kernels against their specification oracle.losses.huber_qr_sorted to 1e-6."""
+and the sorted quantile kernels against their specification oracle.losses.huber_qr_sorted to 1e-6.  Where a reference
+value is NaN or infinite (a NaN selection value picks its action, as torch.argmax does, so its row's outputs are NaN),
+the kernel's value must be the same."""
 import ctypes as C
 
 import numpy as np
@@ -74,20 +76,61 @@ def same_bits(name, x, y):
         assert np.array_equal(x[k].view(np.uint32), y[k].view(np.uint32)), f"{name}: {k} differs"
 
 
+def finite_part(name, got, want):
+    """Where ``want`` is NaN or infinite, ``got`` must be the same (any NaN for NaN).  Returns the mask of the rest."""
+    got, want = np.asarray(got), np.asarray(want)
+    odd = ~np.isfinite(want) | ~np.isfinite(got)
+    same = (np.isnan(got) & np.isnan(want)) | (got == want)
+    bad = odd & ~same
+    assert not bad.any(), (f"{name}: {int(bad.sum())} non-finite elements differ, e.g. index {np.argwhere(bad)[0].tolist()}: "
+                           f"got {got[bad][0]!r}, reference {want[bad][0]!r}")
+    return ~odd
+
+
+def bound64(name, got, r):
+    """(b) of the module docstring for one output against its losses64.R."""
+    ok = finite_part(name, got, r.v)
+    got = np.asarray(got, np.float64)
+    err = np.abs(got - r.v)
+    tol = (r.n + 16) * 2.0 ** -24 * r.s + np.where(r.s > 0, TINY, 0.0)
+    bad = ok & ~(err <= tol)
+    assert not bad.any(), (f"{name}: {int(bad.sum())} elements outside the float64 bound, e.g. index "
+                           f"{np.argwhere(bad)[0].tolist()}: got {got[bad][0]!r}, float64 {r.v[bad][0]!r}, bound {tol[bad][0]:.3g}")
+
+
 def check(name, out, ref32, ref64, alpha, scales=None):
     """(a), (b) and (c) of the module docstring.  ref32: {key: fp32 oracle}; ref64: {key: losses64.R}."""
     for k, r in ref64.items():
-        got = out[k].astype(np.float64)
-        err = np.abs(got - r.v)
-        tol = (r.n + 16) * 2.0 ** -24 * r.s + np.where(r.s > 0, TINY, 0.0)
-        bad = ~(err <= tol)
-        assert not bad.any(), (f"{name}.{k}: {int(bad.sum())} elements outside the float64 bound, e.g. index "
-                               f"{np.argwhere(bad)[0].tolist()}: got {got[bad][0]!r}, float64 {r.v[bad][0]!r}, bound {tol[bad][0]:.3g}")
+        bound64(f"{name}.{k}", out[k], r)
     for k, want in ref32.items():
-        parity.close(f"{name}.{k}", out[k], want, scale=(scales or {}).get(k))
+        ok = finite_part(f"{name}.{k}", out[k], want)
+        parity.close(f"{name}.{k}", out[k][ok], want[ok], scale=(scales or {}).get(k))
     loss = out["loss"]
-    assert out["max_p"][0] == max(0.0, float(loss[np.isfinite(loss)].max())), f"{name}: max_p"
-    parity.close(f"{name}.prio[alpha={alpha}]", out["prio"], O64.priority(loss, PRIO_EPS, alpha))
+    fin = loss[np.isfinite(loss)]
+    assert out["max_p"][0] == max(0.0, float(fin.max()) if fin.size else 0.0), f"{name}: max_p"
+    prio = O64.priority(loss, PRIO_EPS, alpha)
+    ok = finite_part(f"{name}.prio", out["prio"], prio)
+    parity.close(f"{name}.prio[alpha={alpha}]", out["prio"][ok], prio[ok])
+
+
+def nan_selection_rows(A):
+    """Selection values (qsel) whose arg-max depends on NaN being the largest value, the first NaN winning: NaN first, in
+    the middle, last; the row a '>' butterfly split three ways; all NaN; NaN next to +inf."""
+    n, inf = f32(np.nan), f32(np.inf)
+    base = np.linspace(-1.0, 1.0, A, dtype=f32)
+    rows = []
+    for j in (0, A // 2, A - 1):
+        r = base.copy(); r[j] = n; rows.append(r)
+    r = np.full(A, -2.0, f32); r[:4] = [1.0, n, 5.0, 9.0][:A]; rows.append(r)
+    rows.append(np.full(A, n, f32))
+    r = base.copy(); r[max(A - 2, 0)] = inf; r[A - 1] = n; rows.append(r)
+    return rows
+
+
+def put_rows(x, rows, start):
+    """x[start + i] = rows[i] where x has room."""
+    for i, row in enumerate(rows[:max(0, len(x) - start)]):
+        x[start + i] = row
 
 
 def _batch(rng, B, A, rewards=(-1.0, 0.0, 1.0, 2.5)):
@@ -110,6 +153,7 @@ def test_dqn_and_mdqn(lib, A, B):
     q, tn, tc, qs = [(rng.randn(B, A) * 3).astype(f32) for _ in range(4)]
     tn[1::4] *= 27; tc[2::4] *= 27; q[3::4] *= 27
     qs[::2] = np.round(qs[::2] / 3); tn[::5] = np.round(tn[::5] / 3)
+    put_rows(qs, nan_selection_rows(A), 7)          # B = 1000: each target row has distinct values, so a* shows
     ag, rg, dg, wg, qg, tng, tcg, qsg = map(dev, (a, r, d, w, q, tn, tc, qs))
     # the gradient w * clamp(q - T) is a difference of operands of magnitude max(|q|, |T|), which is its error scale
     sc = float(max(np.abs(q).max(), np.abs(tn).max() + np.abs(r).max() + 1.0) * w.max())
@@ -148,6 +192,8 @@ def _c51_inputs(M, A, B, vmin, vmax, seed):
     tg[4] = -200.0; tg[4, :, 1] = 0.0          # one-hot target logits: exact zeros in p
     qs = (rng.randn(B, A) * 3).astype(f32)
     qs[5] = 1.0                                # ties: the first maximum wins
+    put_rows(qs, nan_selection_rows(A), 6)     # NaN selection values: samples 6-11
+    tg[12, A - 1, M // 3] = np.nan             # without qsel the last action's expected value is NaN: it is selected
     return a, r, d, w, atoms, lg, tg, qs
 
 
@@ -173,7 +219,7 @@ def _c51_case(lib, M, A, B, vmin, vmax, qsel, fast_too, seed):
     # is up to 9e-6 off the float64 value under this scale (2.6e-5 under the default floor), so the gradient is held to
     # the contract against the float64 value
     wm = np.abs(w)[:, None] * ref64["target_prob"].v
-    sc = float((np.abs(ref64["grad"].v[np.arange(B), a] + wm) + wm).max())
+    sc = float(np.nanmax(np.abs(ref64["grad"].v[np.arange(B), a] + wm) + wm))   # NaN rows: the NaN-selection samples
     ref32 = {"grad": ref64["grad"].v}
     # the reference's delta is fl32 of a float64 division, the kernels' an fp32 division of fl32(vmax - vmin): where the two
     # differ in the last bit (vmax = 0.7) so do the bins, and only the float64 evaluation of the kernels' rule applies
@@ -181,7 +227,9 @@ def _c51_case(lib, M, A, B, vmin, vmax, qsel, fast_too, seed):
         loss, _, m = OL.c51(lg, tg, sel, a, r, d, w, G3, 1, atoms, vmin, vmax)
         ref32.update(loss=loss, target_prob=m)
     check(tag, out, ref32, ref64, alpha, {"grad": sc})
-    assert (out["target_prob"].sum(-1) <= 1.0 + 1e-5).all()
+    tp = out["target_prob"]
+    tp = tp[np.isfinite(tp).all(-1)]              # the NaN rows were matched to the references above
+    assert (tp.sum(-1) <= 1.0 + 1e-5).all()
 
 
 @pytest.mark.parametrize("A", [1, 5, 6])
@@ -272,8 +320,13 @@ def _quantile_call(lib, layout, qg, qtg, tg, qsg, Ni, Nj):
 def test_quantile_pair_loop(lib, Ni, Nj, A, layout, qsel):
     """a0_k4_quantile<true | false>: at most 64 targets or at most 64 online quantiles, Ni != Nj, up to 256 threads."""
     rng = np.random.RandomState(Ni * 1000 + Nj * 10 + A + layout)
-    B, G = 6, 0.5
+    B, G = 12, 0.5
     a, r, d, w, q, qt, taus, qs = _quantile_inputs(rng, B, A, Ni, Nj, layout)
+    put_rows(qs, nan_selection_rows(A), B - 6)                   # NaN selection values: the last six samples
+    if not qsel:
+        # the last action's row mean is NaN (+inf and -inf targets): it is selected and the targets are +-inf
+        qt[B - 1, A - 1, 0] = np.inf
+        qt[B - 1, A - 1, Ni - 1] = -np.inf if Ni > 1 else np.inf
     ag, rg, dg, wg, qg, qtg, qsg = map(dev, (a, r, d, w, q, qt, qs))
     tg = dev(taus) if taus is not None else None
     alpha = ALPHAS[(Ni + Nj + A) % 3]
@@ -293,11 +346,17 @@ def test_quantile_pair_loop(lib, Ni, Nj, A, layout, qsel):
 def test_quantile_sorted_forms(lib, Ni, Nj, A, layout, qsel):
     """a0_k4_quantile_sorted<true,4>, <true,8>, <false,1> and a0_k4_quantile_warp, QR and IQN (layout 1, per-sample tau),
     with the quantiles offset by up to 1e6: the float64 prefix sums must stay within the contract at any magnitude."""
-    B, G = 4, 0.5
-    gshape = (B, A, Nj) if layout == 0 else (B, Nj, A)
+    G = 0.5
     for k, c in enumerate((0.0, 1e3, 1e5, 1e6)):
         rng = np.random.RandomState(Ni * 1000 + Nj * 10 + A + layout + k)
-        a, r, d, w, q, qt, taus, qs = _quantile_inputs(rng, B, A, Ni, Nj, layout, c=c, spread=2.0)
+        a, r, d, w, q, qt, taus, qs = _quantile_inputs(rng, 4, A, Ni, Nj, layout, c=c, spread=2.0)
+        if k == 0:
+            # six more samples with NaN selection values
+            more = _quantile_inputs(np.random.RandomState(Ni * 1000 + Nj * 10 + A + layout + 99), 6, A, Ni, Nj, layout)
+            put_rows(more[-1], nan_selection_rows(A), 0)
+            a, r, d, w, q, qt, taus, qs = [None if x is None else np.concatenate((x, y)) for x, y in zip((a, r, d, w, q, qt, taus, qs), more)]
+        B = len(a)
+        gshape = (B, A, Nj) if layout == 0 else (B, Nj, A)
         ag, rg, dg, wg, qg, qtg, qsg = map(dev, (a, r, d, w, q, qt, qs))
         tg = dev(taus) if taus is not None else None
         alpha = ALPHAS[k % 3]
