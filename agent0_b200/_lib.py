@@ -126,6 +126,15 @@ SIGNATURES = {
                                 _vp, _vp, _vp, _vp, _vp]),
     "a0_act_epsilon_greedy": (_i32, [_vp, _i32, _i32, _f64, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "a0_u8_to_f32": (_i32, [_vp, _vp, _i64, _i32, _vp]),
+    "a0_wp_create": (_i32, [C.POINTER(_vp), _i64, C.c_uint64, _i32]),
+    "a0_wp_destroy": (_i32, [_vp]),
+    "a0_wp_handle": (_i32, [_vp, _vp]),
+    "a0_wp_ctl": (_vp, [_vp]),
+    "a0_wp_publish": (_i32, [_vp, _vp, _vp, _i32, _vp]),
+    "a0_ws_open": (_i32, [C.POINTER(_vp), _vp, C.c_uint64, _i64, _i32]),
+    "a0_ws_attach": (_i32, [C.POINTER(_vp), _vp]),
+    "a0_ws_fetch": (_i32, [_vp, _vp, _vp, _i32, _vp, _vp]),
+    "a0_ws_close": (_i32, [_vp]),
 }
 
 _lib = None

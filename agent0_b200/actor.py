@@ -23,13 +23,19 @@ from .replay import NORM_RECIP
 
 
 class ActorPolicy:
-    def __init__(self, cfg, model, device=None, norm_mode=NORM_RECIP, rng=None):
+    def __init__(self, cfg, model, device=None, norm_mode=NORM_RECIP, rng=None, weights=None):
         """model: the learner's DeepQNet (shared, as trainer.py:42-43 shares it with the Actors).
         norm_mode: NORM_RECIP reproduces torch's CUDA ``.div(255.0)`` bit for bit, NORM_DIV the CPU one.
-        rng: a numpy RandomState-like object (default: numpy's global generator, as the reference)."""
+        rng: a numpy RandomState-like object (default: numpy's global generator, as the reference).
+        weights: a weights.WeightSubscriber whose model is ``model`` (an actor with its own copy of the net, e.g. in
+        another process): ``pull_weights`` refreshes it, and ``ShardActor.sample`` does so at the start of every call,
+        the cadence of the reference's actor node (launch.py:56-61)."""
         if not torch.cuda.is_available():
             raise RuntimeError("agent0_b200.ActorPolicy needs a CUDA device (no CPU fallback)")
+        if weights is not None and weights.model is not model:
+            raise ValueError("ActorPolicy(weights=): the subscriber must write into this policy's model")
         self.cfg, self.model, self.lib = cfg, model, _lib.load()
+        self.weights = weights
         dv = device if device is not None else next(model.parameters()).device
         self.device = torch.device(dv)
         if self.device.type != "cuda":
@@ -56,6 +62,13 @@ class ActorPolicy:
         self._res_host = torch.empty(E + 1, dtype=torch.int64).pin_memory()
         self._scratch = torch.zeros(2, dtype=torch.float32, device=dev)
         self._key = key
+
+    def pull_weights(self):
+        """The newest complete snapshot of the learner's weights into the model (WeightSubscriber.pull): the version
+        applied, or 0 when there was nothing new (or the pull was torn and left the model as it was)."""
+        if self.weights is None:
+            raise RuntimeError("ActorPolicy.pull_weights: construct the policy with weights=WeightSubscriber(...)")
+        return self.weights.pull()
 
     @torch.no_grad()
     def act(self, obs, epsilon):
@@ -118,8 +131,11 @@ class ShardActor:
 
     def sample(self, epsilon):
         """Runs ``cfg.actor.sample_steps`` vector steps.  Returns (transitions appended, episode returns,
-        per-step mean max-q), i.e. the reference's (data, rs, qs) with the data already in the shard."""
+        per-step mean max-q), i.e. the reference's (data, rs, qs) with the data already in the shard.  A policy with a
+        weight subscriber first pulls the learner's newest weights (launch.py:56-61)."""
         cfg = self.cfg
+        if getattr(self.policy, "weights", None) is not None:
+            self.policy.pull_weights()
         rs, qs, count = [], [], 0
         for _ in range(cfg.actor.sample_steps):
             if cfg.learner.noisy_net and self.steps % cfg.learner.reset_noise_freq == 0:

@@ -36,9 +36,12 @@ class GraphedUpdates:
     At batch 32 the eager loop is bound by ~150 kernel launches per update; the replay is not."""
 
     def __init__(self, learner, replay, batch_size, learner_steps, normalized=None, sampler_seed=None, obs_dtype=None,
-                 replacement=True):
+                 replacement=True, publisher=None):
+        """publisher (weights.WeightPublisher, optional): publishes the model after the L updates, as the last node of
+        the graph."""
         import torch
         assert learner.capturable, "construct the learner with capturable=True"
+        self.publisher = publisher
         freq = learner.cfg.learner.target_update_freq
         assert freq % learner_steps == 0, "target_update_freq must be a multiple of learner_steps for graphed updates"
         self.torch, self.learner, self.replay = torch, learner, replay
@@ -58,6 +61,8 @@ class GraphedUpdates:
             result = self.learner.update(_learner_data(b))
             self.replay.update_priority(result["indices"], result["q_loss"])
             outs.append((result["q_loss"], result["fraction_loss"]))
+        if self.publisher is not None:
+            self.publisher.publish()
         return outs
 
     def run(self):
@@ -81,7 +86,7 @@ class GraphedUpdates:
 
 class Trainer:
     def __init__(self, cfg, process_group=None, native_nstep=False, graph=False, fused_input=False, sampler_seed=None,
-                 global_is_max=False, amp=False, channels_last=None, replacement=True, **replay_kw):
+                 global_is_max=False, amp=False, channels_last=None, replacement=True, publish_weights=False, **replay_kw):
         """graph=True: the learner updates of a step run as one CUDA-graph replay (GraphedUpdates).
         fused_input=True: K3 writes the learner's normalised f32 obs / next_obs directly
         (a0_rb_gather_f32) instead of u8 frames that torch then casts, divides and splits
@@ -99,7 +104,10 @@ class Trainer:
         GLOBAL batch of all ranks (one all-reduce(MAX) of learner_steps floats per draw) instead of per shard.
         replacement=False: every batch holds B distinct records, with the law of the reference's
         torch.multinomial(priority[:top], B, replacement=False) (replay.py:41-43; ReplayDataset.sample), eagerly and
-        in the graphed updates."""
+        in the graphed updates.
+        publish_weights=True: ``learn`` publishes the online model once after its L updates (weights.WeightPublisher; with
+        graph=True the publish is the last node of the captured graph), and ``weight_handle()`` gives what actor
+        processes subscribe with (weights.WeightSubscriber).  Off by default: the captured step is then unchanged."""
         self.pg = process_group
         self.global_is_max = bool(global_is_max) and process_group is not None
         self.cfg = cfg
@@ -114,6 +122,10 @@ class Trainer:
                                     max_p=None, capturable=self.graph, amp_dtype=torch.bfloat16 if self.amp else None,
                                     channels_last=self.amp if channels_last is None else bool(channels_last))
         self._graphed = None
+        self.publisher = None
+        if publish_weights:
+            from .weights import WeightPublisher
+            self.publisher = WeightPublisher(self.learner.model)
         self.num_transitions = cfg.actor.sample_steps * cfg.actor.num_envs
         self.frame_count = 0
         # the reference keeps every value ever logged (trainer.py:45-47) but only ever reads the last 20 / 100:
@@ -132,7 +144,7 @@ class Trainer:
             if self._graphed is None or self._graphed.L != L:
                 self._graphed = GraphedUpdates(self.learner, self.replay, B, L, normalized=self.normalized,
                                                sampler_seed=self.sampler_seed, obs_dtype=self.obs_dtype,
-                                               replacement=self.replacement)
+                                               replacement=self.replacement, publisher=self.publisher)
             return self._graphed.run()
         out = []
         drawn = self.replay.sample(B, k_batches=L, normalized=self.normalized, seed=self.sampler_seed, obs_dtype=self.obs_dtype,
@@ -143,7 +155,15 @@ class Trainer:
             result = self.learner.train(_learner_data(b))
             self.replay.update_priority(result["indices"], result["q_loss"])
             out.append((result["q_loss"], result["fraction_loss"]))
+        if self.publisher is not None:
+            self.publisher.publish()
         return out
+
+    def weight_handle(self):
+        """The handle actor processes subscribe to the learner's weights with (``publish_weights=True`` only)."""
+        if self.publisher is None:
+            raise RuntimeError("construct the Trainer with publish_weights=True to serve weights to actors")
+        return self.publisher.handle()
 
     def step(self, transitions, returns=(), qmax=()):
         """trainer.py:74-119 with the same argument list: new transitions from the actor (reference

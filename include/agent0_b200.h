@@ -29,6 +29,7 @@
  *   agent0/deepq/agent.py:110-114,273-327 huber_qr_loss, QR/IQN    -> a0_loss_quantile
  *   agent0/deepq/agent.py:340-388  FQFLearner.train_step           -> a0_loss_quantile (+fraction)
  *   agent0/deepq/agent.py:25-39    Actor.act (actor side, "next")  -> a0_u8_to_f32 + a0_act_epsilon_greedy
+ *   agent0/deepq/launch.py:33-36   state_dict() fetch per Actor.sample -> a0_wp_publish / a0_ws_fetch
  */
 #ifndef AGENT0_B200_H
 #define AGENT0_B200_H
@@ -649,6 +650,41 @@ int a0_act_epsilon_greedy(const float* q /* dev */, int32_t E, int32_t A, double
                           a0_stream_t stream);
 int a0_u8_to_f32(const uint8_t* in /* dev */, float* out /* dev */, int64_t count, int32_t norm_mode,
                  a0_stream_t stream);
+
+/* ---- K8: versioned weight snapshots for actor processes (agent0/deepq/launch.py:33-36,56-61) --------------------
+ * A publisher owns ONE device allocation (one CUDA IPC handle covers it): a 256-byte control block {magic, format,
+ * layout hash u64, word count u64, latest u64 (0 = nothing published), seq[2] u64, ...} and two snapshot buffers of
+ * n_words 4-byte words, each 256-byte aligned.  Version v goes into buffer v & 1; seq[b] is 2v - 1 while v is written
+ * and 2v once it is complete; latest advances after every word of v is visible at system scope.
+ * A state is a table of n_seg device segments: seg_ptr u64[n_seg] (4-byte aligned addresses, any offset) and
+ * seg_words i64[n_seg + 1] (word-count prefix sums, seg_words[n_seg] == n_words), both in device memory, prepared once.
+ * a0_wp_publish  copies the segments into the next buffer in ONE launch.  The version is read and advanced on the
+ *                device: every replay of a captured CUDA graph publishes latest + 1.  Publishes on one region must be
+ *                stream-ordered.
+ * a0_wp_handle   the region's cudaIpcMemHandle_t (64 bytes) for a subscriber in another process.
+ * a0_ws_open     maps a handle (cudaIpcOpenMemHandle, peer access enabled lazily: a subscriber on another GPU reads
+ *                over NVLink) and checks magic, layout hash and word count with one copy; a mismatch is A0_EINVAL.
+ * a0_ws_attach   the same subscriber on a publisher of this process (CUDA refuses to open a process's own handle).
+ * a0_ws_fetch    copies the newest complete version into the subscriber's private staging buffer, checking seq
+ *                before and after every chunk, then scatters it into the segments only when nothing was torn and it
+ *                is newer than the version applied last.  Two launches, never waits for the writer (no spin): the
+ *                caller decides whether to retry.  *status_out (device-visible u64, optional) = the version applied,
+ *                or 0 (nothing published, nothing new, or torn: the segments are left exactly as they were).
+ * a0_wp_ctl      TEST HOOK: device address of the control block.                                              */
+typedef struct a0_wpub a0_wpub_t;
+typedef struct a0_wsub a0_wsub_t;
+int a0_wp_create(a0_wpub_t** out, int64_t n_words, uint64_t layout_hash, int32_t device);
+int a0_wp_destroy(a0_wpub_t* wp);
+int a0_wp_handle(a0_wpub_t* wp, uint8_t* out64 /* host [64] */);
+void* a0_wp_ctl(a0_wpub_t* wp);
+int a0_wp_publish(a0_wpub_t* wp, const uint64_t* seg_ptr /* dev */, const int64_t* seg_words /* dev */, int32_t n_seg,
+                  a0_stream_t stream);
+int a0_ws_open(a0_wsub_t** out, const uint8_t* handle64 /* host [64] */, uint64_t layout_hash, int64_t n_words,
+               int32_t device);
+int a0_ws_attach(a0_wsub_t** out, a0_wpub_t* wp);
+int a0_ws_fetch(a0_wsub_t* ws, const uint64_t* seg_ptr /* dev */, const int64_t* seg_words /* dev */, int32_t n_seg,
+                uint64_t* status_out /* dev-visible */, a0_stream_t stream);
+int a0_ws_close(a0_wsub_t* ws);
 
 #ifdef __cplusplus
 }
