@@ -20,6 +20,7 @@ OPT_PDL = 1          # include/agent0_b200.h: A0_OPT_PDL (mask of kernel classes
 K2B_PLAN_MAX = 1024  # include/agent0_b200.h: A0_K2B_PLAN_MAX (largest index count of a0_pt_update_plan / _apply)
 K2B_PLAN_BYTES = 90176  # A0_K2B_PLAN_BYTES (the plan buffer)
 C51_EARLY = 1        # include/agent0_b200.h: A0_C51_EARLY (a0_loss_c51_linked: batch-side work before the wait)
+TX_COMMITTED, TX_FULL = 1, 2   # include/agent0_b200.h: A0_TX_COMMITTED / A0_TX_FULL (a0_tw_commit's status)
 
 
 def lz4_stride(frame_bytes):
@@ -135,6 +136,20 @@ SIGNATURES = {
     "a0_ws_attach": (_i32, [C.POINTER(_vp), _vp]),
     "a0_ws_fetch": (_i32, [_vp, _vp, _vp, _i32, _vp, _vp]),
     "a0_ws_close": (_i32, [_vp]),
+    "a0_tx_layout": (_i32, [_i64, _i64, _i64, _i32, _i32, _vp]),
+    "a0_tx_create": (_i32, [C.POINTER(_vp), _i32, _i32, _i64, _i64, _i64, _i32, _i32, _i32]),
+    "a0_tx_destroy": (_i32, [_vp]),
+    "a0_tx_handle": (_i32, [_vp, _vp]),
+    "a0_tx_scan": (_i32, [_vp, _i32, _vp]),
+    "a0_tx_scan_host": (_vp, [_vp]),
+    "a0_tx_slot_frames": (_vp, [_vp, _i32, _i32]),
+    "a0_tx_release": (_i32, [_vp, _vp]),
+    "a0_tx_unclaim": (_i32, [_vp, _i32]),
+    "a0_tx_ctl": (_vp, [_vp]),
+    "a0_tw_open": (_i32, [C.POINTER(_vp), _vp, _i32, _i64, _i64, _i64, _i32]),
+    "a0_tw_attach": (_i32, [C.POINTER(_vp), _vp, _i32]),
+    "a0_tw_commit": (_i32, [_vp, _vp, _i64, _i64, _i64, _vp, _vp]),
+    "a0_tw_close": (_i32, [_vp]),
 }
 
 _lib = None

@@ -132,7 +132,8 @@ class ShardActor:
     def sample(self, epsilon):
         """Runs ``cfg.actor.sample_steps`` vector steps.  Returns (transitions appended, episode returns,
         per-step mean max-q), i.e. the reference's (data, rs, qs) with the data already in the shard.  A policy with a
-        weight subscriber first pulls the learner's newest weights (launch.py:56-61)."""
+        weight subscriber first pulls the learner's newest weights (launch.py:56-61).  A sink with ``flush`` (an
+        inbox.TransitionWriter in an actor process) is flushed at the end, so the call's steps reach the learner."""
         cfg = self.cfg
         if getattr(self.policy, "weights", None) is not None:
             self.policy.pull_weights()
@@ -154,6 +155,8 @@ class ShardActor:
             if "final_info" in info:
                 for stat in info["final_info"][info["_final_info"]]:
                     rs.append(stat["episode"]["r"][0])
+        if getattr(self.replay, "flush", None) is not None:      # a TransitionWriter sink commits the call's steps
+            self.replay.flush()
         return count, rs, qs
 
     def close(self):

@@ -8,7 +8,7 @@ PKG = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG, "csrc")
 LIB = os.path.join(PKG, "libagent0_b200.so")
 SOURCES = ["a0_replay.cu", "a0_sumtree.cu", "a0_targets.cu", "a0_ingest.cu", "a0_extend.cu", "a0_lz4enc.cu", "a0_ckpt.cu",
-           "a0_weights.cu"]
+           "a0_weights.cu", "a0_inbox.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "--use_fast_math=false", "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=default",
               "--fmad=true", "-shared", "-cudart", "static"]

@@ -86,7 +86,8 @@ class GraphedUpdates:
 
 class Trainer:
     def __init__(self, cfg, process_group=None, native_nstep=False, graph=False, fused_input=False, sampler_seed=None,
-                 global_is_max=False, amp=False, channels_last=None, replacement=True, publish_weights=False, **replay_kw):
+                 global_is_max=False, amp=False, channels_last=None, replacement=True, publish_weights=False, inbox_lanes=0,
+                 inbox_kw=None, **replay_kw):
         """graph=True: the learner updates of a step run as one CUDA-graph replay (GraphedUpdates).
         fused_input=True: K3 writes the learner's normalised f32 obs / next_obs directly
         (a0_rb_gather_f32) instead of u8 frames that torch then casts, divides and splits
@@ -107,7 +108,11 @@ class Trainer:
         in the graphed updates.
         publish_weights=True: ``learn`` publishes the online model once after its L updates (weights.WeightPublisher; with
         graph=True the publish is the last node of the captured graph), and ``weight_handle()`` gives what actor
-        processes subscribe with (weights.WeightSubscriber).  Off by default: the captured step is then unchanged."""
+        processes subscribe with (weights.WeightSubscriber).  Off by default: the captured step is then unchanged.
+        inbox_lanes=k (with native_nstep=True): the trainer owns an inbox.TransitionInbox of k lanes (``inbox_kw``: its
+        slots, slot_transitions, slot_frames); ``inbox_handle(lane)`` gives what an actor process opens a
+        TransitionWriter with, and ``step`` drains the inbox into the shard (eagerly, before the updates) where it
+        otherwise calls ``extend``.  Off by default."""
         self.pg = process_group
         self.global_is_max = bool(global_is_max) and process_group is not None
         self.cfg = cfg
@@ -126,6 +131,12 @@ class Trainer:
         if publish_weights:
             from .weights import WeightPublisher
             self.publisher = WeightPublisher(self.learner.model)
+        self.inbox = None
+        if inbox_lanes:
+            if not native_nstep:
+                raise ValueError("an inbox feeds the native ingest: construct the Trainer with native_nstep=True")
+            from .inbox import TransitionInbox
+            self.inbox = TransitionInbox(self.replay, inbox_lanes, **(inbox_kw or {}))
         self.num_transitions = cfg.actor.sample_steps * cfg.actor.num_envs
         self.frame_count = 0
         # the reference keeps every value ever logged (trainer.py:45-47) but only ever reads the last 20 / 100:
@@ -165,13 +176,23 @@ class Trainer:
             raise RuntimeError("construct the Trainer with publish_weights=True to serve weights to actors")
         return self.publisher.handle()
 
-    def step(self, transitions, returns=(), qmax=()):
+    def inbox_handle(self, lane):
+        """The handle an actor process opens lane ``lane`` of the trainer's inbox with (``inbox_lanes`` only)."""
+        if self.inbox is None:
+            raise RuntimeError("construct the Trainer with inbox_lanes=k to take transitions from actor processes")
+        return self.inbox.handle(lane)
+
+    def step(self, transitions=(), returns=(), qmax=()):
         """trainer.py:74-119 with the same argument list: new transitions from the actor (reference
-        tuples), episode returns and mean q-values for logging."""
+        tuples), episode returns and mean q-values for logging.  With an inbox, the transitions drained from it are
+        ingested here and counted into ``frames``."""
         self.Qs.extend(qmax)
         self.Rs.extend(returns)
         self.replay.extend(transitions)
-        self.frame_count += self.num_transitions
+        if self.inbox is not None:
+            self.frame_count += self.inbox.drain()
+        else:
+            self.frame_count += self.num_transitions
         if len(self.replay) > self.cfg.trainer.training_start_steps:
             for q_loss, fraction_loss in self.learn():
                 if q_loss is not None:

@@ -686,6 +686,53 @@ int a0_ws_fetch(a0_wsub_t* ws, const uint64_t* seg_ptr /* dev */, const int64_t*
                 uint64_t* status_out /* dev-visible */, a0_stream_t stream);
 int a0_ws_close(a0_wsub_t* ws);
 
+/* ---- K9: a transition inbox for actor processes (agent0/deepq/launch.py:45-63) ----------------------------------
+ * The learner owns ONE device allocation (one CUDA IPC handle covers it): a 256-byte control block {magic, format,
+ * frame bytes, lanes, slots, slot capacity in transitions and frames, streams per lane, n_gather, slot and lane bytes},
+ * then per lane a 512-byte header (claimed, committed, consumed, each on its own 128-byte line) and `slots` slots.
+ * A slot: a 256-byte header {n_transitions, n_steps, n_frames} (i64), the arrays step_count i64[T], step_reset u8[T],
+ * stream i64[T], n_new i64[T], action i64[T], reward f64[T], done u8[T] (each 16-byte aligned), then u8[SF][F] frames
+ * (256-byte aligned) in allocation order: per vector step the 4-frame stacks of a reset step, then the new frames.
+ * a0_tx_layout      the byte offsets: out[0..6] the arrays, [7] the frames (= header + metadata bytes), [8] slot
+ *                   bytes, [9] lane bytes, [10] region bytes, [11] the metadata copies in the scan buffer, [12] scan
+ *                   buffer bytes, [13] control block bytes, [14] lane header bytes.  Needs no GPU.
+ * a0_tx_scan        K9b: per lane, slots [consumed, committed) (at most max_slots_per_lane): headers and the used
+ *                   prefix of every array into the page-locked mapped scan buffer (a0_tx_scan_host: per lane i64
+ *                   {consumed, committed, taken, 0}, then at out[11] + (lane * slots + j) * out[7] the copy of slot
+ *                   consumed + j).  The caller synchronises before it reads the buffer.
+ * a0_tx_slot_frames device address of a slot's frames, for a0_rb_ingest_* with A0_INGEST_FRAMES_ON_DEVICE.
+ * a0_tx_release     K9c: consumed += taken of the last scan, for every lane (stream-ordered after the ingest).
+ * a0_tx_unclaim     hands the lane of a dead writer to a new one.
+ * a0_tx_ctl         TEST HOOK: device address of the region.
+ * a0_tw_open        maps a handle (peer access enabled lazily), checks magic, format and the slot layout, and claims
+ *                   the lane (atomicCAS on `claimed`): a claimed lane fails with A0_EINVAL.  a0_tw_attach: the same
+ *                   writer on an inbox of this process.  a0_tw_close hands the lane back.
+ * a0_tw_commit      K9a: copies the device staging (the slot's layout) into the next slot and commits it, in one
+ *                   launch that never waits; *status_out (device-visible u64) = A0_TX_COMMITTED, or A0_TX_FULL when
+ *                   every slot of the lane is committed and not yet consumed (nothing is copied; retry later).  */
+#define A0_TX_COMMITTED 1
+#define A0_TX_FULL 2
+typedef struct a0_txbox a0_txbox_t;
+typedef struct a0_txwriter a0_twriter_t;
+int a0_tx_layout(int64_t slot_transitions, int64_t slot_frames, int64_t frame_bytes, int32_t lanes, int32_t slots,
+                 int64_t* out /* host [15] */);
+int a0_tx_create(a0_txbox_t** out, int32_t lanes, int32_t slots, int64_t slot_transitions, int64_t slot_frames,
+                 int64_t frame_bytes, int32_t streams_per_lane, int32_t n_gather, int32_t device);
+int a0_tx_destroy(a0_txbox_t* tx);
+int a0_tx_handle(a0_txbox_t* tx, uint8_t* out64 /* host [64] */);
+int a0_tx_scan(a0_txbox_t* tx, int32_t max_slots_per_lane, a0_stream_t stream);
+void* a0_tx_scan_host(a0_txbox_t* tx);
+void* a0_tx_slot_frames(a0_txbox_t* tx, int32_t lane, int32_t slot);
+int a0_tx_release(a0_txbox_t* tx, a0_stream_t stream);
+int a0_tx_unclaim(a0_txbox_t* tx, int32_t lane);
+void* a0_tx_ctl(a0_txbox_t* tx);
+int a0_tw_open(a0_twriter_t** out, const uint8_t* handle64 /* host [64] */, int32_t lane, int64_t frame_bytes,
+               int64_t slot_transitions, int64_t slot_frames, int32_t device);
+int a0_tw_attach(a0_twriter_t** out, a0_txbox_t* tx, int32_t lane);
+int a0_tw_commit(a0_twriter_t* tw, const uint8_t* staging_dev, int64_t n_transitions, int64_t n_steps,
+                 int64_t n_frames, uint64_t* status_out /* dev-visible */, a0_stream_t stream);
+int a0_tw_close(a0_twriter_t* tw);
+
 #ifdef __cplusplus
 }
 #endif
