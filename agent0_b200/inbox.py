@@ -138,7 +138,9 @@ def _pci_bus_id(index):
 class TransitionInbox:
     """The learner's side: ``lanes`` lanes of ``slots`` slots next to ``replay`` (a native_nstep=True shard).  Lane ``l``
     owns the shard's streams [l * E, (l + 1) * E), E = ``cfg.actor.num_envs``.  The default slot holds one
-    ``ShardActor.sample`` call: num_envs * sample_steps transitions and 2 * transitions + 4 * num_envs frames."""
+    ``ShardActor.sample`` call: num_envs * sample_steps transitions and max(2 * transitions + 4 * num_envs,
+    8 * num_envs) frames.  A slot must take any one vector step, so ``slot_transitions`` >= E and ``slot_frames`` >= 8E
+    (a writer's first step carries the E reset stacks and up to 4 new frames per stream); a smaller one is refused."""
 
     def __init__(self, replay, lanes, slots=4, slot_transitions=None, slot_frames=None):
         cfg = replay.cfg
@@ -146,7 +148,12 @@ class TransitionInbox:
         self.E = int(cfg.actor.num_envs)
         self.lanes, self.slots = int(lanes), int(slots)
         self.T = int(slot_transitions or self.E * int(cfg.actor.sample_steps))
-        self.SF = int(slot_frames or 2 * self.T + 4 * self.E)
+        self.SF = int(slot_frames or max(2 * self.T + 4 * self.E, 8 * self.E))
+        if self.T < self.E:
+            raise ValueError(f"slot_transitions {self.T} is below one vector step of {self.E} streams")
+        if self.SF < 8 * self.E:
+            raise ValueError(f"slot_frames {self.SF} is below the {8 * self.E} frames a writer's first vector step of "
+                             f"{self.E} streams can carry")
         self.F = replay.F
         self.layout = slot_layout(self.T, self.SF, self.F, self.lanes, self.slots)
         h = C.c_void_p()
