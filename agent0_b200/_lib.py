@@ -231,6 +231,13 @@ def ptr(t, dtype=None):
     return t.data_ptr()
 
 
+def pci_bus_id(index):
+    """PCI bus id (domain:bus:device.function) of CUDA device ``index``: names the GPU of a region in the handle an
+    actor process receives."""
+    p = torch.cuda.get_device_properties(index)
+    return f"{p.pci_domain_id:04x}:{p.pci_bus_id:02x}:{p.pci_device_id:02x}.0"
+
+
 def host_map(t):
     """Device-visible address of a pinned CPU tensor (a0_host_map), for kernels that write results
     straight into host memory."""

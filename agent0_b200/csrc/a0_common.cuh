@@ -340,6 +340,90 @@ __device__ __forceinline__ void a0_bulk_store_hint(void* gdst, uint32_t smem_src
                ::"l"(gdst), "r"(smem_src), "r"(bytes), "l"(pol) : "memory");
 }
 
+// ---- system-scope memory order: the words of a region shared with other processes and peer GPUs (K8, K9) ---------
+__device__ __forceinline__ void a0_sys_fence() { asm volatile("fence.acq_rel.sys;" ::: "memory"); }
+__device__ __forceinline__ uint64_t a0_sys_ld_acquire(const uint64_t* p) {
+  uint64_t v;
+  asm volatile("ld.acquire.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
+  return v;
+}
+__device__ __forceinline__ uint64_t a0_sys_ld_relaxed(const uint64_t* p) {
+  uint64_t v;
+  asm volatile("ld.relaxed.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
+  return v;
+}
+__device__ __forceinline__ void a0_sys_st_relaxed(uint64_t* p, uint64_t v) {
+  asm volatile("st.relaxed.sys.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
+}
+__device__ __forceinline__ void a0_sys_st_release(uint64_t* p, uint64_t v) {
+  asm volatile("st.release.sys.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
+}
+__device__ __forceinline__ uint4 a0_sys_ld4_relaxed(const uint4* p) {
+  uint4 v;
+  asm volatile("ld.relaxed.sys.global.v4.u32 {%0, %1, %2, %3}, [%4];"
+               : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p) : "memory");
+  return v;
+}
+__device__ __forceinline__ void a0_sys_st4_relaxed(uint4* p, uint4 v) {
+  asm volatile("st.relaxed.sys.global.v4.u32 [%0], {%1, %2, %3, %4};" ::"l"(p), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w)
+               : "memory");
+}
+
+// ---- a device region shared with other processes through CUDA IPC (K8 weight snapshots, K9 transition inbox) -----
+// ONE cudaMalloc allocation, so one cudaIpcMemHandle_t covers it, starting with a control block whose first two words
+// are {uint32_t magic, format}: what a0_ipc_map checks before the caller reads anything else of the block.  The
+// caller sets the device.
+// A zeroed region of `bytes` starting with the control block `ctl`; a failed allocation is A0_ENOMEM.
+inline int a0_ipc_create(const char* who, size_t bytes, const void* ctl, size_t ctl_bytes, uint8_t** region) {
+  void* p = nullptr;
+  cudaError_t e = cudaMalloc(&p, bytes);
+  if (e != cudaSuccess) {
+    a0_set_error("%s: cudaMalloc of %zu bytes failed: %s", who, bytes, cudaGetErrorString(e));
+    return e == cudaErrorMemoryAllocation ? A0_ENOMEM : (int)e;
+  }
+  e = cudaMemset(p, 0, bytes);
+  if (e == cudaSuccess) e = cudaMemcpy(p, ctl, ctl_bytes, cudaMemcpyHostToDevice);
+  if (e != cudaSuccess) {
+    cudaFree(p);
+    a0_set_error("%s: initialising the region failed: %s", who, cudaGetErrorString(e));
+    return (int)e;
+  }
+  *region = static_cast<uint8_t*>(p);
+  return A0_OK;
+}
+inline int a0_ipc_handle(uint8_t* region, uint8_t* out64) {
+  static_assert(sizeof(cudaIpcMemHandle_t) == 64, "cudaIpcMemHandle_t is 64 bytes");
+  cudaIpcMemHandle_t h;
+  A0_CUDA(cudaIpcGetMemHandle(&h, region));
+  memcpy(out64, &h, 64);
+  return A0_OK;
+}
+inline void a0_ipc_unmap(uint8_t* region) { cudaIpcCloseMemHandle(region); }
+// Maps another process's region (peer access enabled lazily: a peer GPU's region is read over NVLink) and copies its
+// control block to `ctl`; a block of another kind (`kind`: the owner named in the error) is A0_EINVAL.  A failed
+// mapping's error names cudaIpcOpenMemHandle: callers tell "this machine refuses CUDA IPC" by it.
+inline int a0_ipc_map(const char* who, const uint8_t* handle64, uint32_t magic, uint32_t format, const char* kind,
+                      void* ctl, size_t ctl_bytes, uint8_t** region) {
+  cudaIpcMemHandle_t h;
+  memcpy(&h, handle64, 64);
+  void* p = nullptr;
+  A0_CUDA(cudaIpcOpenMemHandle(&p, h, cudaIpcMemLazyEnablePeerAccess));
+  const cudaError_t e = cudaMemcpy(ctl, p, ctl_bytes, cudaMemcpyDeviceToHost);
+  if (e != cudaSuccess) {
+    a0_ipc_unmap(static_cast<uint8_t*>(p));
+    a0_set_error("%s: reading the control block failed: %s", who, cudaGetErrorString(e));
+    return (int)e;
+  }
+  const uint32_t* w = static_cast<const uint32_t*>(ctl);
+  if (w[0] != magic || w[1] != format) {
+    a0_ipc_unmap(static_cast<uint8_t*>(p));
+    a0_set_error("%s: the handle's region is not a %s region (magic %08x format %u)", who, kind, w[0], w[1]);
+    return A0_EINVAL;
+  }
+  *region = static_cast<uint8_t*>(p);
+  return A0_OK;
+}
+
 // ---- 64-bit frame content hash of K6a / K7 ---------------------------------------------------------
 __device__ __forceinline__ uint32_t a0_k6_rotl(uint32_t x, int r) { return (x << r) | (x >> (32 - r)); }
 __device__ __forceinline__ uint32_t a0_k6_mix32(uint32_t h) {

@@ -108,34 +108,6 @@ A0XLayout a0x_layout(int64_t T, int64_t SF, int64_t F, int64_t lanes, int64_t sl
   return L;
 }
 
-__device__ __forceinline__ void a0x_fence_sys() { asm volatile("fence.acq_rel.sys;" ::: "memory"); }
-__device__ __forceinline__ uint64_t a0x_ld_acquire(const uint64_t* p) {
-  uint64_t v;
-  asm volatile("ld.acquire.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ uint64_t a0x_ld_relaxed(const uint64_t* p) {
-  uint64_t v;
-  asm volatile("ld.relaxed.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ void a0x_st_relaxed(uint64_t* p, uint64_t v) {
-  asm volatile("st.relaxed.sys.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
-}
-__device__ __forceinline__ void a0x_st_release(uint64_t* p, uint64_t v) {
-  asm volatile("st.release.sys.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
-}
-__device__ __forceinline__ uint4 a0x_ld4_relaxed(const uint4* p) {
-  uint4 v;
-  asm volatile("ld.relaxed.sys.global.v4.u32 {%0, %1, %2, %3}, [%4];"
-               : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ void a0x_st4_relaxed(uint4* p, uint4 v) {
-  asm volatile("st.relaxed.sys.global.v4.u32 [%0], {%1, %2, %3, %4};" ::"l"(p), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w)
-               : "memory");
-}
-
 // K9a.  The staging buffer has the slot's layout; bytes [256, 256 + n16 * 16) (metadata and frames) are copied, the
 // header is written from the arguments.
 __global__ void __launch_bounds__(A0X_THREADS) a0x_commit_kernel(A0XLane* lane, uint8_t* slot0, int64_t slot_bytes,
@@ -146,26 +118,26 @@ __global__ void __launch_bounds__(A0X_THREADS) a0x_commit_kernel(A0XLane* lane, 
   __shared__ uint64_t s_c;
   __shared__ int s_full;
   if (threadIdx.x == 0) {
-    const uint64_t c = a0x_ld_relaxed(&lane->committed);    // this writer's own word
-    const uint64_t d = a0x_ld_acquire(&lane->consumed);
+    const uint64_t c = a0_sys_ld_relaxed(&lane->committed);  // this writer's own word
+    const uint64_t d = a0_sys_ld_acquire(&lane->consumed);
     s_c = c;
     s_full = c - d >= (uint64_t)S;
   }
   __syncthreads();
   const uint64_t c = s_c;
   if (!s_full) {
-    a0x_fence_sys();                                         // the acquire above before this thread's stores
+    a0_sys_fence();                                          // the acquire above before this thread's stores
     uint8_t* slot = slot0 + (int64_t)(c % S) * slot_bytes;
     uint4* dst = reinterpret_cast<uint4*>(slot + 256);
     const int64_t g0 = (int64_t)blockIdx.x * (A0X_CHUNK / 16), g1 = min(g0 + A0X_CHUNK / 16, n16);
-    for (int64_t g = g0 + threadIdx.x; g < g1; g += A0X_THREADS) a0x_st4_relaxed(dst + g, __ldg(staging + g));
+    for (int64_t g = g0 + threadIdx.x; g < g1; g += A0X_THREADS) a0_sys_st4_relaxed(dst + g, __ldg(staging + g));
     if (blockIdx.x == 0 && threadIdx.x == 0) {
       uint64_t* hdr = reinterpret_cast<uint64_t*>(slot);
-      a0x_st_relaxed(hdr + 0, (uint64_t)n_transitions);
-      a0x_st_relaxed(hdr + 1, (uint64_t)n_steps);
-      a0x_st_relaxed(hdr + 2, (uint64_t)n_frames);
+      a0_sys_st_relaxed(hdr + 0, (uint64_t)n_transitions);
+      a0_sys_st_relaxed(hdr + 1, (uint64_t)n_steps);
+      a0_sys_st_relaxed(hdr + 2, (uint64_t)n_frames);
     }
-    a0x_fence_sys();                                         // close: this thread's stores before the ticket
+    a0_sys_fence();                                          // close: this thread's stores before the ticket
   }
   __syncthreads();
   if (threadIdx.x == 0) {
@@ -175,8 +147,8 @@ __global__ void __launch_bounds__(A0X_THREADS) a0x_commit_kernel(A0XLane* lane, 
       __threadfence();
       const bool full = atomicAdd(&w->full, 0u) != 0u;
       if (!full) {
-        a0x_fence_sys();
-        a0x_st_release(&lane->committed, c + 1);
+        a0_sys_fence();
+        a0_sys_st_release(&lane->committed, c + 1);
       }
       *reinterpret_cast<volatile unsigned long long*>(status_out) = full ? A0_TX_FULL : A0_TX_COMMITTED;
       __threadfence_system();
@@ -198,8 +170,8 @@ __global__ void __launch_bounds__(A0X_THREADS) a0x_scan_kernel(const uint8_t* re
   __shared__ int64_t s_n;
   __shared__ int64_t s_first;
   if (threadIdx.x == 0) {
-    const uint64_t c = a0x_ld_acquire(&lane->committed);
-    const uint64_t d = a0x_ld_relaxed(&lane->consumed);     // stored only by K9c on this stream
+    const uint64_t c = a0_sys_ld_acquire(&lane->committed);
+    const uint64_t d = a0_sys_ld_relaxed(&lane->consumed);  // stored only by K9c on this stream
     const int64_t avail = (int64_t)(c - d);
     const int64_t n = avail < 0 ? 0 : min(min(avail, max_slots), (int64_t)S);
     s_n = n;
@@ -217,8 +189,8 @@ __global__ void __launch_bounds__(A0X_THREADS) a0x_scan_kernel(const uint8_t* re
     uint8_t* out = scan_meta + ((int64_t)l * S + j) * L.frames;
     if (threadIdx.x == 0) {
       const uint64_t* hdr = reinterpret_cast<const uint64_t*>(slot);
-      s_cnt[0] = (int64_t)min(a0x_ld_relaxed(hdr + 0), (uint64_t)T);   // transitions (bounded: the host validates)
-      s_cnt[1] = (int64_t)min(a0x_ld_relaxed(hdr + 1), (uint64_t)T);   // steps
+      s_cnt[0] = (int64_t)min(a0_sys_ld_relaxed(hdr + 0), (uint64_t)T);  // transitions (bounded: the host validates)
+      s_cnt[1] = (int64_t)min(a0_sys_ld_relaxed(hdr + 1), (uint64_t)T);  // steps
     }
     __syncthreads();
     // the header, then the used prefix of every array, 16 bytes at a time
@@ -229,7 +201,7 @@ __global__ void __launch_bounds__(A0X_THREADS) a0x_scan_kernel(const uint8_t* re
       const int64_t bytes = k < 0 ? 256 : a0x_up(esz * s_cnt[k < 2 ? 1 : 0], 16);
       const uint4* src = reinterpret_cast<const uint4*>(slot + off);
       uint4* dst = reinterpret_cast<uint4*>(out + off);
-      for (int64_t g = threadIdx.x; g < bytes / 16; g += A0X_THREADS) dst[g] = a0x_ld4_relaxed(src + g);
+      for (int64_t g = threadIdx.x; g < bytes / 16; g += A0X_THREADS) dst[g] = a0_sys_ld4_relaxed(src + g);
     }
     __syncthreads();
   }
@@ -241,9 +213,9 @@ __global__ void a0x_release_kernel(uint8_t* region, int64_t lane_bytes, int32_t 
     const int64_t n = taken[l];
     if (n == 0) continue;
     A0XLane* lane = reinterpret_cast<A0XLane*>(region + sizeof(A0XCtl) + (int64_t)l * lane_bytes);
-    const uint64_t d = a0x_ld_relaxed(&lane->consumed);
-    a0x_fence_sys();
-    a0x_st_release(&lane->consumed, d + (uint64_t)n);
+    const uint64_t d = a0_sys_ld_relaxed(&lane->consumed);
+    a0_sys_fence();
+    a0_sys_st_release(&lane->consumed, d + (uint64_t)n);
     taken[l] = 0;
   }
 }
@@ -256,13 +228,13 @@ __global__ void a0x_claim_kernel(A0XLane* lane, unsigned long long token, unsign
 }
 
 __global__ void a0x_hand_back_kernel(A0XLane* lane, unsigned long long token) {
-  a0x_fence_sys();                                 // the writer's earlier stores before the lane is free
+  a0_sys_fence();                                  // the writer's earlier stores before the lane is free
   atomicCAS_system(&lane->claimed, token, 0ull);
 }
 
 __global__ void a0x_unclaim_kernel(A0XLane* lane) {
-  a0x_fence_sys();
-  a0x_st_release(reinterpret_cast<uint64_t*>(&lane->claimed), 0ull);
+  a0_sys_fence();
+  a0_sys_st_release(reinterpret_cast<uint64_t*>(&lane->claimed), 0ull);
 }
 
 int a0x_check_shape(const char* who, int64_t T, int64_t SF, int64_t F) {
@@ -292,7 +264,7 @@ struct a0_txwriter {
   int64_t T, SF, F;
   A0XLayout L;
   uint8_t* region;               // IPC mapping or (attach) the inbox's own pointer
-  bool ipc;
+  bool mapped;                   // region came from a0_ipc_map
   A0XWriter* w;
   unsigned long long* claim;     // device word for the claim's result; NULL when the lane was not claimed
   unsigned long long token;      // this writer's value of `claimed`
@@ -340,30 +312,7 @@ extern "C" int a0_tx_create(a0_txbox_t** out, int32_t lanes, int32_t slots, int6
              A0_MAX_NSTEP);
   A0_REQUIRE(device >= 0, "a0_tx_create: device %d is negative", device);
   A0DeviceGuard guard(device);
-  a0_txbox* tx = new a0_txbox();
-  tx->device = device;
-  tx->lanes = lanes;
-  tx->slots = slots;
-  tx->streams_per_lane = streams_per_lane;
-  tx->n_gather = n_gather;
-  tx->T = slot_transitions;
-  tx->SF = slot_frames;
-  tx->F = frame_bytes;
-  tx->L = a0x_layout(slot_transitions, slot_frames, frame_bytes, lanes, slots);
-  tx->region = nullptr;
-  tx->scan_host = nullptr;
-  tx->scan_dev = nullptr;
-  tx->taken = nullptr;
-  const size_t bytes = (size_t)tx->L.region_bytes;
-  cudaError_t e = cudaMalloc((void**)&tx->region, bytes);
-  if (e == cudaSuccess) e = cudaMalloc((void**)&tx->taken, (size_t)lanes * 8);
-  if (e == cudaSuccess) e = cudaHostAlloc((void**)&tx->scan_host, (size_t)tx->L.scan_bytes, cudaHostAllocMapped);
-  if (e == cudaSuccess) e = cudaHostGetDevicePointer((void**)&tx->scan_dev, tx->scan_host, 0);
-  if (e != cudaSuccess) {
-    a0_tx_destroy(tx);
-    a0_set_error("a0_tx_create: allocating %zu bytes failed: %s", bytes, cudaGetErrorString(e));
-    return e == cudaErrorMemoryAllocation ? A0_ENOMEM : (int)e;
-  }
+  const A0XLayout L = a0x_layout(slot_transitions, slot_frames, frame_bytes, lanes, slots);
   A0XCtl ctl;
   memset(&ctl, 0, sizeof(ctl));
   ctl.magic = A0X_MAGIC;
@@ -375,17 +324,22 @@ extern "C" int a0_tx_create(a0_txbox_t** out, int32_t lanes, int32_t slots, int6
   ctl.slot_frames = (uint32_t)slot_frames;
   ctl.streams_per_lane = (uint32_t)streams_per_lane;
   ctl.n_gather = (uint32_t)n_gather;
-  ctl.slot_bytes = (uint64_t)tx->L.slot_bytes;
-  ctl.lane_bytes = (uint64_t)tx->L.lane_bytes;
-  e = cudaMemset(tx->region, 0, bytes);
+  ctl.slot_bytes = (uint64_t)L.slot_bytes;
+  ctl.lane_bytes = (uint64_t)L.lane_bytes;
+  uint8_t* region = nullptr;
+  { int rc = a0_ipc_create("a0_tx_create", (size_t)L.region_bytes, &ctl, sizeof(ctl), &region); if (rc) return rc; }
+  a0_txbox* tx = new a0_txbox{device, lanes, slots, streams_per_lane, n_gather, slot_transitions, slot_frames,
+                              frame_bytes, L, region, nullptr, nullptr, nullptr};
+  cudaError_t e = cudaMalloc((void**)&tx->taken, (size_t)lanes * 8);
   if (e == cudaSuccess) e = cudaMemset(tx->taken, 0, (size_t)lanes * 8);
-  if (e == cudaSuccess) e = cudaMemcpy(tx->region, &ctl, sizeof(ctl), cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) e = cudaHostAlloc((void**)&tx->scan_host, (size_t)L.scan_bytes, cudaHostAllocMapped);
+  if (e == cudaSuccess) e = cudaHostGetDevicePointer((void**)&tx->scan_dev, tx->scan_host, 0);
   if (e != cudaSuccess) {
     a0_tx_destroy(tx);
-    a0_set_error("a0_tx_create: initialising the region failed: %s", cudaGetErrorString(e));
-    return (int)e;
+    a0_set_error("a0_tx_create: allocating the scan buffers failed: %s", cudaGetErrorString(e));
+    return e == cudaErrorMemoryAllocation ? A0_ENOMEM : (int)e;
   }
-  memset(tx->scan_host, 0, (size_t)tx->L.scan_bytes);
+  memset(tx->scan_host, 0, (size_t)L.scan_bytes);
   *out = tx;
   return A0_OK;
 }
@@ -393,10 +347,7 @@ extern "C" int a0_tx_create(a0_txbox_t** out, int32_t lanes, int32_t slots, int6
 extern "C" int a0_tx_handle(a0_txbox_t* tx, uint8_t* out64) {
   A0_REQUIRE(tx != nullptr && out64 != nullptr, "a0_tx_handle: NULL argument");
   A0DeviceGuard guard(tx->device);
-  cudaIpcMemHandle_t h;
-  A0_CUDA(cudaIpcGetMemHandle(&h, tx->region));
-  memcpy(out64, &h, 64);
-  return A0_OK;
+  return a0_ipc_handle(tx->region, out64);
 }
 
 extern "C" void* a0_tx_ctl(a0_txbox_t* tx) { return tx ? tx->region : nullptr; }
@@ -442,12 +393,12 @@ extern "C" int a0_tx_unclaim(a0_txbox_t* tx, int32_t lane) {
 extern "C" int a0_tw_close(a0_twriter_t* tw) {
   if (!tw) return A0_OK;
   A0DeviceGuard guard(tw->device);
-  if (tw->region && tw->claim) {                 // the lane is handed back if this writer still holds it
+  if (tw->claim) {                               // the lane is handed back if this writer still holds it
     a0x_hand_back_kernel<<<1, 1>>>(
         reinterpret_cast<A0XLane*>(tw->region + sizeof(A0XCtl) + (int64_t)tw->lane * tw->L.lane_bytes), tw->token);
     cudaStreamSynchronize(nullptr);
   }
-  if (tw->ipc && tw->region) cudaIpcCloseMemHandle(tw->region);
+  if (tw->mapped) a0_ipc_unmap(tw->region);
   cudaFree(tw->w);
   cudaFree(tw->claim);
   delete tw;
@@ -480,6 +431,16 @@ static int a0x_writer_init(a0_txwriter* tw, const char* who) {
   return A0_OK;
 }
 
+// A writer of lane `lane` of `region` (mapped: closing it unmaps the region); what is taken is given back on failure.
+static int a0x_writer_new(a0_twriter_t** out, const char* who, int32_t device, int32_t lane, uint32_t slots, int64_t T,
+                          int64_t SF, int64_t F, const A0XLayout& L, uint8_t* region, bool mapped) {
+  a0_txwriter* tw = new a0_txwriter{device, lane, slots, T, SF, F, L, region, mapped, nullptr, nullptr, 0};
+  const int rc = a0x_writer_init(tw, who);
+  if (rc != A0_OK) { a0_tw_close(tw); return rc; }
+  *out = tw;
+  return A0_OK;
+}
+
 extern "C" int a0_tw_open(a0_twriter_t** out, const uint8_t* handle64, int32_t lane, int64_t frame_bytes,
                           int64_t slot_transitions, int64_t slot_frames, int32_t device) {
   A0_REQUIRE(out != nullptr && handle64 != nullptr, "a0_tw_open: NULL argument");
@@ -487,72 +448,34 @@ extern "C" int a0_tw_open(a0_twriter_t** out, const uint8_t* handle64, int32_t l
   A0_REQUIRE(lane >= 0, "a0_tw_open: lane %d is negative", lane);
   A0_REQUIRE(device >= 0, "a0_tw_open: device %d is negative", device);
   A0DeviceGuard guard(device);
-  cudaIpcMemHandle_t h;
-  memcpy(&h, handle64, 64);
-  void* region = nullptr;
-  A0_CUDA(cudaIpcOpenMemHandle(&region, h, cudaIpcMemLazyEnablePeerAccess));
   A0XCtl ctl;
-  cudaError_t e = cudaMemcpy(&ctl, region, sizeof(ctl), cudaMemcpyDeviceToHost);
-  if (e != cudaSuccess) {
-    cudaIpcCloseMemHandle(region);
-    a0_set_error("a0_tw_open: reading the control block failed: %s", cudaGetErrorString(e));
-    return (int)e;
-  }
+  uint8_t* region = nullptr;
+  const int rc = a0_ipc_map("a0_tw_open", handle64, A0X_MAGIC, A0X_FORMAT, "transition inbox's", &ctl, sizeof(ctl), &region);
+  if (rc != A0_OK) return rc;
   const A0XLayout L = a0x_layout(slot_transitions, slot_frames, frame_bytes, ctl.lanes, ctl.slots);
-  const char* bad = ctl.magic != A0X_MAGIC || ctl.format != A0X_FORMAT ? "is not a transition inbox's region"
-                    : ctl.frame_bytes != (uint64_t)frame_bytes         ? "holds frames of another size"
+  const char* bad = ctl.frame_bytes != (uint64_t)frame_bytes ? "holds frames of another size"
                     : ctl.slot_transitions != (uint64_t)slot_transitions || ctl.slot_frames != (uint64_t)slot_frames ||
                             ctl.slot_bytes != (uint64_t)L.slot_bytes || ctl.lane_bytes != (uint64_t)L.lane_bytes
                         ? "has slots of another layout"
                     : lane >= (int32_t)ctl.lanes ? "has fewer lanes"
                                                  : nullptr;
   if (bad) {
-    cudaIpcCloseMemHandle(region);
+    a0_ipc_unmap(region);
     a0_set_error("a0_tw_open: the handle's region %s (frame bytes %llu vs %lld, slot %u x %u vs %lld x %lld, lane %d of %u)",
                  bad, (unsigned long long)ctl.frame_bytes, (long long)frame_bytes, ctl.slot_transitions, ctl.slot_frames,
                  (long long)slot_transitions, (long long)slot_frames, lane, ctl.lanes);
     return A0_EINVAL;
   }
-  a0_txwriter* tw = new a0_txwriter();
-  tw->device = device;
-  tw->lane = lane;
-  tw->slots = ctl.slots;
-  tw->T = slot_transitions;
-  tw->SF = slot_frames;
-  tw->F = frame_bytes;
-  tw->L = L;
-  tw->region = static_cast<uint8_t*>(region);
-  tw->ipc = true;
-  tw->w = nullptr;
-  tw->claim = nullptr;
-  tw->token = 0;
-  const int rc = a0x_writer_init(tw, "a0_tw_open");
-  if (rc != A0_OK) { a0_tw_close(tw); return rc; }
-  *out = tw;
-  return A0_OK;
+  return a0x_writer_new(out, "a0_tw_open", device, lane, ctl.slots, slot_transitions, slot_frames, frame_bytes, L,
+                        region, true);
 }
 
 extern "C" int a0_tw_attach(a0_twriter_t** out, a0_txbox_t* tx, int32_t lane) {
   A0_REQUIRE(out != nullptr && tx != nullptr, "a0_tw_attach: NULL argument");
   A0_REQUIRE(lane >= 0 && lane < tx->lanes, "a0_tw_attach: lane %d outside [0, %d)", lane, tx->lanes);
   A0DeviceGuard guard(tx->device);
-  a0_txwriter* tw = new a0_txwriter();
-  tw->device = tx->device;
-  tw->lane = lane;
-  tw->slots = (uint32_t)tx->slots;
-  tw->T = tx->T;
-  tw->SF = tx->SF;
-  tw->F = tx->F;
-  tw->L = tx->L;
-  tw->region = tx->region;
-  tw->ipc = false;
-  tw->w = nullptr;
-  tw->claim = nullptr;
-  tw->token = 0;
-  const int rc = a0x_writer_init(tw, "a0_tw_attach");
-  if (rc != A0_OK) { a0_tw_close(tw); return rc; }
-  *out = tw;
-  return A0_OK;
+  return a0x_writer_new(out, "a0_tw_attach", tx->device, lane, (uint32_t)tx->slots, tx->T, tx->SF, tx->F, tx->L,
+                        tx->region, false);
 }
 
 extern "C" int a0_tw_commit(a0_twriter_t* tw, const uint8_t* staging_dev, int64_t n_transitions, int64_t n_steps,

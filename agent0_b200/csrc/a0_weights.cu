@@ -39,6 +39,7 @@
 namespace {
 
 constexpr uint32_t A0W_MAGIC = 0x57304130u;     // "0A0W"
+constexpr uint32_t A0W_FORMAT = 1;
 constexpr int A0W_THREADS = 256;
 constexpr int A0W_ITERS = 8;                     // 16-byte groups per thread per chunk
 constexpr int64_t A0W_CHUNK = (int64_t)A0W_THREADS * A0W_ITERS * 4;   // words per CTA (32 KB)
@@ -47,7 +48,7 @@ constexpr int32_t A0W_MAX_SEGMENTS = 1 << 24;
 
 struct A0WCtl {                  // 256 B at the start of the region
   uint32_t magic;
-  uint32_t format;               // 1
+  uint32_t format;               // A0W_FORMAT
   uint64_t layout_hash;
   uint64_t n_words;
   uint64_t latest;               // newest complete version, 0 = none
@@ -68,34 +69,6 @@ struct A0WSub {                  // subscriber-private device words
 static_assert(sizeof(A0WSub) == 256, "subscriber words are 256 bytes");
 
 int64_t a0w_buf_bytes(int64_t n_words) { return (n_words * 4 + 255) / 256 * 256; }
-
-__device__ __forceinline__ void a0w_fence_sys() { asm volatile("fence.acq_rel.sys;" ::: "memory"); }
-__device__ __forceinline__ uint64_t a0w_ld_acquire(const uint64_t* p) {
-  uint64_t v;
-  asm volatile("ld.acquire.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ uint64_t a0w_ld_relaxed(const uint64_t* p) {
-  uint64_t v;
-  asm volatile("ld.relaxed.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ void a0w_st_relaxed(uint64_t* p, uint64_t v) {
-  asm volatile("st.relaxed.sys.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
-}
-__device__ __forceinline__ void a0w_st_release(uint64_t* p, uint64_t v) {
-  asm volatile("st.release.sys.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
-}
-__device__ __forceinline__ uint4 a0w_ld4_relaxed(const uint4* p) {
-  uint4 v;
-  asm volatile("ld.relaxed.sys.global.v4.u32 {%0, %1, %2, %3}, [%4];"
-               : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ void a0w_st4_relaxed(uint4* p, uint4 v) {
-  asm volatile("st.relaxed.sys.global.v4.u32 [%0], {%1, %2, %3, %4};" ::"l"(p), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w)
-               : "memory");
-}
 
 // The segment holding flat word i: the largest s in [lo, hi] with pre[s] <= i (pre = word-count prefix sums).
 __device__ __forceinline__ int a0w_seg_find(const int64_t* __restrict__ pre, int lo, int hi, int64_t i) {
@@ -140,12 +113,12 @@ __global__ void __launch_bounds__(A0W_THREADS) a0w_publish_kernel(A0WCtl* ctl, u
                                                                   const int64_t* __restrict__ pre, int n_seg) {
   __shared__ uint64_t s_v;
   if (threadIdx.x == 0) {
-    const uint64_t v = a0w_ld_relaxed(&ctl->latest) + 1;   // the previous publish on this stream has completed
+    const uint64_t v = a0_sys_ld_relaxed(&ctl->latest) + 1;  // the previous publish on this stream has completed
     s_v = v;
-    a0w_st_relaxed(&ctl->seq[v & 1], 2 * v - 1);             // open
+    a0_sys_st_relaxed(&ctl->seq[v & 1], 2 * v - 1);          // open
   }
   __syncthreads();
-  a0w_fence_sys();
+  a0_sys_fence();
   const uint64_t v = s_v;
   uint4* dst = reinterpret_cast<uint4*>(buf0 + (v & 1) * buf_words);
   const int64_t c0 = (int64_t)blockIdx.x * A0W_CHUNK, c1 = min(c0 + A0W_CHUNK, n_words);
@@ -162,15 +135,15 @@ __global__ void __launch_bounds__(A0W_THREADS) a0w_publish_kernel(A0WCtl* ctl, u
     x.y = w[1] ? *w[1] : 0u;
     x.z = w[2] ? *w[2] : 0u;
     x.w = w[3] ? *w[3] : 0u;
-    a0w_st4_relaxed(dst + (i >> 2), x);
+    a0_sys_st4_relaxed(dst + (i >> 2), x);
   }
-  a0w_fence_sys();                                           // close
+  a0_sys_fence();                                            // close
   __syncthreads();
   if (threadIdx.x == 0) {
     if (atomicAdd(&ctl->ticket, 1u) == gridDim.x - 1) {
-      a0w_fence_sys();
-      a0w_st_release(&ctl->seq[v & 1], 2 * v);
-      a0w_st_release(&ctl->latest, v);
+      a0_sys_fence();
+      a0_sys_st_release(&ctl->seq[v & 1], 2 * v);
+      a0_sys_st_release(&ctl->latest, v);
       ctl->ticket = 0u;
     }
   }
@@ -182,8 +155,8 @@ __global__ void __launch_bounds__(A0W_THREADS) a0w_fetch_kernel(const A0WCtl* ct
   __shared__ uint64_t s_v, s_seq;
   __shared__ int s_copy;
   if (threadIdx.x == 0) {
-    const uint64_t v = a0w_ld_acquire(&ctl->latest);
-    const uint64_t s1 = v ? a0w_ld_acquire(&ctl->seq[v & 1]) : 0;
+    const uint64_t v = a0_sys_ld_acquire(&ctl->latest);
+    const uint64_t s1 = v ? a0_sys_ld_acquire(&ctl->seq[v & 1]) : 0;
     s_v = v;
     s_seq = s1;
     s_copy = v != 0 && v != sub->applied && s1 == 2 * v;
@@ -197,13 +170,13 @@ __global__ void __launch_bounds__(A0W_THREADS) a0w_fetch_kernel(const A0WCtl* ct
 #pragma unroll 4
     for (int it = 0; it < A0W_ITERS; ++it) {
       const int64_t g = g0 + (int64_t)it * A0W_THREADS + threadIdx.x;
-      if (g < g1) dst[g] = a0w_ld4_relaxed(src + g);
+      if (g < g1) dst[g] = a0_sys_ld4_relaxed(src + g);
     }
-    a0w_fence_sys();                                         // the loads above before the re-read below
+    a0_sys_fence();                                          // the loads above before the re-read below
   }
   __syncthreads();
   if (threadIdx.x == 0) {
-    bool ok = !s_copy || a0w_ld_relaxed(&ctl->seq[v & 1]) == s_seq;
+    bool ok = !s_copy || a0_sys_ld_relaxed(&ctl->seq[v & 1]) == s_seq;
     if (v != 0 && v != sub->applied && s_seq != 2 * v) ok = false;   // a version in flight or overtaken at the start
     atomicMin(&sub->vmin, (unsigned long long)v);
     atomicMax(&sub->vmax, (unsigned long long)v);
@@ -274,7 +247,7 @@ struct a0_wsub {
   int32_t device;
   int64_t n_words, buf_words;
   uint8_t* region;               // the publisher's region: IPC mapping or (attach) its own pointer
-  bool ipc;                      // region came from cudaIpcOpenMemHandle
+  bool mapped;                   // region came from a0_ipc_map
   uint32_t* staging;             // [buf_words] private
   A0WSub* sub;
 };
@@ -284,34 +257,17 @@ extern "C" int a0_wp_create(a0_wpub_t** out, int64_t n_words, uint64_t layout_ha
   A0_REQUIRE(n_words >= 1 && n_words <= A0W_MAX_WORDS, "a0_wp_create: n_words %lld outside [1, 2^34]", (long long)n_words);
   A0_REQUIRE(device >= 0, "a0_wp_create: device %d is negative", device);
   A0DeviceGuard guard(device);
-  a0_wpub* wp = new a0_wpub();
-  wp->device = device;
-  wp->n_words = n_words;
-  wp->buf_words = a0w_buf_bytes(n_words) / 4;
-  wp->layout_hash = layout_hash;
-  wp->region = nullptr;
-  const size_t bytes = sizeof(A0WCtl) + 2 * (size_t)a0w_buf_bytes(n_words);
-  cudaError_t e = cudaMalloc((void**)&wp->region, bytes);
-  if (e != cudaSuccess) {
-    delete wp;
-    a0_set_error("a0_wp_create: cudaMalloc of %zu bytes failed: %s", bytes, cudaGetErrorString(e));
-    return e == cudaErrorMemoryAllocation ? A0_ENOMEM : (int)e;
-  }
   A0WCtl ctl;
   memset(&ctl, 0, sizeof(ctl));
   ctl.magic = A0W_MAGIC;
-  ctl.format = 1;
+  ctl.format = A0W_FORMAT;
   ctl.layout_hash = layout_hash;
   ctl.n_words = (uint64_t)n_words;
-  e = cudaMemset(wp->region, 0, bytes);
-  if (e == cudaSuccess) e = cudaMemcpy(wp->region, &ctl, sizeof(ctl), cudaMemcpyHostToDevice);
-  if (e != cudaSuccess) {
-    cudaFree(wp->region);
-    delete wp;
-    a0_set_error("a0_wp_create: initialising the region failed: %s", cudaGetErrorString(e));
-    return (int)e;
-  }
-  *out = wp;
+  uint8_t* region = nullptr;
+  const int rc = a0_ipc_create("a0_wp_create", sizeof(A0WCtl) + 2 * (size_t)a0w_buf_bytes(n_words), &ctl, sizeof(ctl),
+                               &region);
+  if (rc != A0_OK) return rc;
+  *out = new a0_wpub{device, n_words, a0w_buf_bytes(n_words) / 4, layout_hash, region};
   return A0_OK;
 }
 
@@ -325,12 +281,8 @@ extern "C" int a0_wp_destroy(a0_wpub_t* wp) {
 
 extern "C" int a0_wp_handle(a0_wpub_t* wp, uint8_t* out64) {
   A0_REQUIRE(wp != nullptr && out64 != nullptr, "a0_wp_handle: NULL argument");
-  static_assert(sizeof(cudaIpcMemHandle_t) == 64, "cudaIpcMemHandle_t is 64 bytes");
   A0DeviceGuard guard(wp->device);
-  cudaIpcMemHandle_t h;
-  A0_CUDA(cudaIpcGetMemHandle(&h, wp->region));
-  memcpy(out64, &h, 64);
-  return A0_OK;
+  return a0_ipc_handle(wp->region, out64);
 }
 
 extern "C" void* a0_wp_ctl(a0_wpub_t* wp) { return wp ? wp->region : nullptr; }
@@ -348,11 +300,11 @@ extern "C" int a0_wp_publish(a0_wpub_t* wp, const uint64_t* seg_ptr, const int64
   return A0_OK;
 }
 
-static int a0w_sub_alloc(a0_wsub* ws) {
+static int a0w_sub_alloc(a0_wsub* ws, const char* who) {
   cudaError_t e = cudaMalloc((void**)&ws->staging, (size_t)ws->buf_words * 4);
   if (e == cudaSuccess) e = cudaMalloc((void**)&ws->sub, sizeof(A0WSub));
   if (e != cudaSuccess) {
-    a0_set_error("a0_ws_open: cudaMalloc failed: %s", cudaGetErrorString(e));
+    a0_set_error("%s: cudaMalloc failed: %s", who, cudaGetErrorString(e));
     return e == cudaErrorMemoryAllocation ? A0_ENOMEM : (int)e;
   }
   a0w_init_sub<<<1, 1>>>(ws->sub);
@@ -364,10 +316,19 @@ static int a0w_sub_alloc(a0_wsub* ws) {
 extern "C" int a0_ws_close(a0_wsub_t* ws) {
   if (!ws) return A0_OK;
   A0DeviceGuard guard(ws->device);
-  if (ws->ipc && ws->region) cudaIpcCloseMemHandle(ws->region);
+  if (ws->mapped) a0_ipc_unmap(ws->region);
   cudaFree(ws->staging);
   cudaFree(ws->sub);
   delete ws;
+  return A0_OK;
+}
+
+// A subscriber of `region` (mapped: closing it unmaps the region); what is taken is given back on failure.
+static int a0w_sub_new(a0_wsub_t** out, const char* who, int32_t device, int64_t n_words, uint8_t* region, bool mapped) {
+  a0_wsub* ws = new a0_wsub{device, n_words, a0w_buf_bytes(n_words) / 4, region, mapped, nullptr, nullptr};
+  const int rc = a0w_sub_alloc(ws, who);
+  if (rc != A0_OK) { a0_ws_close(ws); return rc; }
+  *out = ws;
   return A0_OK;
 }
 
@@ -377,57 +338,27 @@ extern "C" int a0_ws_open(a0_wsub_t** out, const uint8_t* handle64, uint64_t lay
   A0_REQUIRE(n_words >= 1 && n_words <= A0W_MAX_WORDS, "a0_ws_open: n_words %lld outside [1, 2^34]", (long long)n_words);
   A0_REQUIRE(device >= 0, "a0_ws_open: device %d is negative", device);
   A0DeviceGuard guard(device);
-  cudaIpcMemHandle_t h;
-  memcpy(&h, handle64, 64);
-  void* region = nullptr;
-  A0_CUDA(cudaIpcOpenMemHandle(&region, h, cudaIpcMemLazyEnablePeerAccess));
   A0WCtl ctl;
-  cudaError_t e = cudaMemcpy(&ctl, region, sizeof(ctl), cudaMemcpyDeviceToHost);
-  if (e != cudaSuccess) {
-    cudaIpcCloseMemHandle(region);
-    a0_set_error("a0_ws_open: reading the control block failed: %s", cudaGetErrorString(e));
-    return (int)e;
-  }
-  const char* bad = ctl.magic != A0W_MAGIC || ctl.format != 1 ? "is not a weight publisher's region"
-                    : ctl.layout_hash != layout_hash           ? "has another state layout (names, shapes, dtypes or strides differ)"
-                    : ctl.n_words != (uint64_t)n_words         ? "holds another number of words"
-                                                                : nullptr;
+  uint8_t* region = nullptr;
+  const int rc = a0_ipc_map("a0_ws_open", handle64, A0W_MAGIC, A0W_FORMAT, "weight publisher's", &ctl, sizeof(ctl), &region);
+  if (rc != A0_OK) return rc;
+  const char* bad = ctl.layout_hash != layout_hash   ? "has another state layout (names, shapes, dtypes or strides differ)"
+                    : ctl.n_words != (uint64_t)n_words ? "holds another number of words"
+                                                       : nullptr;
   if (bad) {
-    cudaIpcCloseMemHandle(region);
+    a0_ipc_unmap(region);
     a0_set_error("a0_ws_open: the handle's region %s (hash %016llx vs %016llx, %llu vs %lld words)", bad,
                  (unsigned long long)ctl.layout_hash, (unsigned long long)layout_hash, (unsigned long long)ctl.n_words,
                  (long long)n_words);
     return A0_EINVAL;
   }
-  a0_wsub* ws = new a0_wsub();
-  ws->device = device;
-  ws->n_words = n_words;
-  ws->buf_words = a0w_buf_bytes(n_words) / 4;
-  ws->region = static_cast<uint8_t*>(region);
-  ws->ipc = true;
-  ws->staging = nullptr;
-  ws->sub = nullptr;
-  const int rc = a0w_sub_alloc(ws);
-  if (rc != A0_OK) { a0_ws_close(ws); return rc; }
-  *out = ws;
-  return A0_OK;
+  return a0w_sub_new(out, "a0_ws_open", device, n_words, region, true);
 }
 
 extern "C" int a0_ws_attach(a0_wsub_t** out, a0_wpub_t* wp) {
   A0_REQUIRE(out != nullptr && wp != nullptr, "a0_ws_attach: NULL argument");
   A0DeviceGuard guard(wp->device);
-  a0_wsub* ws = new a0_wsub();
-  ws->device = wp->device;
-  ws->n_words = wp->n_words;
-  ws->buf_words = wp->buf_words;
-  ws->region = wp->region;
-  ws->ipc = false;
-  ws->staging = nullptr;
-  ws->sub = nullptr;
-  const int rc = a0w_sub_alloc(ws);
-  if (rc != A0_OK) { a0_ws_close(ws); return rc; }
-  *out = ws;
-  return A0_OK;
+  return a0w_sub_new(out, "a0_ws_attach", wp->device, wp->n_words, wp->region, false);
 }
 
 extern "C" int a0_ws_fetch(a0_wsub_t* ws, const uint64_t* seg_ptr, const int64_t* seg_words, int32_t n_seg,

@@ -130,11 +130,6 @@ def parse_slot(meta, layout, slot_transitions, slot_frames, streams_per_lane, wh
     return steps
 
 
-def _pci_bus_id(index):
-    p = torch.cuda.get_device_properties(index)
-    return f"{p.pci_domain_id:04x}:{p.pci_bus_id:02x}:{p.pci_device_id:02x}.0"
-
-
 class TransitionInbox:
     """The learner's side: ``lanes`` lanes of ``slots`` slots next to ``replay`` (a native_nstep=True shard).  Lane ``l``
     owns the shard's streams [l * E, (l + 1) * E), E = ``cfg.actor.num_envs``.  The default slot holds one
@@ -175,7 +170,7 @@ class TransitionInbox:
         return dict(ipc=bytes(buf), lane=int(lane), lanes=self.lanes, slots=self.slots, slot_transitions=self.T,
                     slot_frames=self.SF, frame_bytes=self.F, frame_shape=tuple(self.replay.frame_shape),
                     streams_per_lane=self.E, n_gather=self.replay.n_gather, layout=dict(self.layout),
-                    pci_bus_id=_pci_bus_id(self.device.index))
+                    pci_bus_id=_lib.pci_bus_id(self.device.index))
 
     def drain(self):
         """Ingests every committed slot of every lane (up to ``slots`` per lane) into the shard and releases them.

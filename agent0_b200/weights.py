@@ -76,11 +76,6 @@ def _cuda_device(model, device):
     return torch.device("cuda", dev.index if dev.index is not None else torch.cuda.current_device())
 
 
-def _pci_bus_id(index):
-    p = torch.cuda.get_device_properties(index)
-    return f"{p.pci_domain_id:04x}:{p.pci_bus_id:02x}:{p.pci_device_id:02x}.0"
-
-
 class WeightPublisher:
     """Publishes ``model``'s state (the learner's online network) as versions 1, 2, ... into a device region that
     subscribers map.  ``publish`` enqueues one kernel on the current stream and can be captured in a CUDA graph."""
@@ -108,7 +103,7 @@ class WeightPublisher:
         buf = (C.c_uint8 * 64)()
         _lib.check(self.lib.a0_wp_handle(self._h, buf), "a0_wp_handle")
         return dict(ipc=bytes(buf), n_words=self.n_words, layout_hash=self.hash,
-                    pci_bus_id=_pci_bus_id(self.device.index))
+                    pci_bus_id=_lib.pci_bus_id(self.device.index))
 
     def control_words(self):
         """TEST HOOK: the region's control block as a u64[32] device view (magic | format, hash, n_words, latest,

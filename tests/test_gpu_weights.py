@@ -1,7 +1,8 @@
 """K8 on the B200: weight snapshots published by the learner and pulled by actors (agent0_b200/weights.py,
 csrc/a0_weights.cu).  Bit-exact round trips of every learner's state, segment tables of every shape and alignment, a
 torn fetch that must leave the actor's weights alone, the publish as a node of the Trainer's captured graph, an actor
-policy fed by a subscriber, and subscribers in another process (same GPU, and a peer GPU when there are two)."""
+policy fed by a subscriber, subscribers in another process (same GPU, and a peer GPU when there are two), and handles of
+a publisher and of a transition inbox each refused by the other kind's open."""
 import multiprocessing as mp
 import pickle
 import time
@@ -246,6 +247,15 @@ def _child(handle, device, n_last, ready, results, deadline_s):
             pass
 
 
+def _stop(p):
+    if p.is_alive():
+        p.terminate()
+        p.join(timeout=10)
+    if p.is_alive():
+        p.kill()
+        p.join(timeout=10)
+
+
 def _cross_process(device):
     N = 200
     state = _State({f"t{i}": torch.zeros(s, device="cuda:0") for i, s in enumerate(SHAPES)})
@@ -270,12 +280,7 @@ def _cross_process(device):
         out = results.get(timeout=90)
         p.join(timeout=30)
     finally:
-        if p.is_alive():
-            p.terminate()
-            p.join(timeout=10)
-        if p.is_alive():
-            p.kill()
-            p.join(timeout=10)
+        _stop(p)
     assert not p.is_alive()
     if out["ipc_refused"]:
         pytest.skip(f"this machine refuses to map another process's CUDA IPC handle: {out['ipc_refused']}")
@@ -294,3 +299,58 @@ def test_cross_process_subscriber_on_a_peer_gpu():
         pytest.skip("needs two GPUs")
     seen = _cross_process(1)
     assert len(seen) >= 2
+
+
+def _cross_kind_child(weights_handle, inbox_handle, results):
+    """Opens the inbox's handle with the publisher's region in it as a TransitionWriter, and the inbox's region as a
+    WeightSubscriber whose model passes the Python-side layout check: the region's control block must refuse both."""
+    out = dict(error=None, ipc_refused=None, writer=None, subscriber=None)
+    try:
+        import torch
+        from agent0_b200.inbox import TransitionWriter
+        from agent0_b200.weights import WeightSubscriber, layout_hash
+        torch.cuda.set_device(0)
+        state = _State({"t0": torch.zeros(1000, device="cuda:0")})
+        opens = dict(
+            writer=lambda: TransitionWriter(dict(inbox_handle, ipc=weights_handle["ipc"]), device=torch.device("cuda", 0)),
+            subscriber=lambda: WeightSubscriber(dict(ipc=inbox_handle["ipc"], n_words=1000, layout_hash=layout_hash(state),
+                                                     pci_bus_id=inbox_handle["pci_bus_id"]), state))
+        for kind, open_ in opens.items():
+            try:
+                open_().close()
+                out[kind] = "opened"
+            except RuntimeError as e:
+                if "cudaIpcOpenMemHandle" in str(e):
+                    out["ipc_refused"] = str(e)
+                    return
+                out[kind] = str(e)
+    except Exception as e:                                          # reported, never raised past the queue
+        out["error"] = repr(e)
+    finally:
+        try:
+            results.put(out, timeout=10)
+        except Exception:
+            pass
+
+
+def test_a_handle_of_the_other_kind_is_refused_in_another_process():
+    from agent0_b200.inbox import TransitionInbox
+    from agent0_b200.replay import ReplayDataset
+    cfg = make_config("c51", per=True, n_step=3, batch_size=32, replay_size=2048, num_envs=16)
+    inbox = TransitionInbox(ReplayDataset(cfg, native_nstep=True), 1, slots=2)
+    pub = WeightPublisher(_State({"t0": torch.zeros(1000, device="cuda:0")}))
+    ctx = mp.get_context("spawn")
+    results = ctx.Queue()
+    p = ctx.Process(target=_cross_kind_child, args=(pub.handle(), inbox.handle(0), results), daemon=True)
+    p.start()
+    try:
+        out = results.get(timeout=180)
+        p.join(timeout=30)
+    finally:
+        _stop(p)
+    assert not p.is_alive()
+    if out["ipc_refused"]:
+        pytest.skip(f"this machine refuses to map another process's CUDA IPC handle: {out['ipc_refused']}")
+    assert out["error"] is None, out["error"]
+    assert "is not a transition inbox's region" in out["writer"], out["writer"]
+    assert "is not a weight publisher's region" in out["subscriber"], out["subscriber"]
