@@ -60,6 +60,9 @@ SIGNATURES = {
     "a0_last_error": (C.c_char_p, []),
     "a0_set_option": (_i32, [_i32, _i64]),
     "a0_get_option": (_i32, [_i32, C.POINTER(C.c_int64)]),
+    "a0_capture_node": (_i32, [_vp, C.POINTER(_vp)]),
+    "a0_capture_join": (_i32, [_vp, _vp]),
+    "a0_graph_edges": (_i32, [_vp, _vp, _vp, _vp, _vp, _i64, C.POINTER(_i64)]),
     "a0_rb_create": (_i32, [C.POINTER(_vp), _i64, _i64, _i32, _i32]),
     "a0_rb_destroy": (_i32, [_vp]),
     "a0_rb_reset": (_i32, [_vp, _vp]),

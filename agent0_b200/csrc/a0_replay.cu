@@ -170,6 +170,62 @@ extern "C" int a0_set_option(int32_t option, int64_t value) {
 }
 
 // ------------------------------------------------------------------------------------------------
+// typed joins of a captured step (hotloop.ReplayTargetLoop)
+// ------------------------------------------------------------------------------------------------
+// A kernel launched with the programmatic attribute after a cross-stream event wait gets programmatic edges from
+// every predecessor, so it may start before the other stream's work is complete.  Instead the joining kernel is
+// launched with its stream predecessor alone, and the edge from the other stream's node is added to the graph
+// afterwards as a full edge: its type is then the one set here, whatever the launch attribute does to the others.
+static int a0_capture_tail(cudaStream_t stream, cudaGraph_t* graph, cudaGraphNode_t* node) {
+  cudaStreamCaptureStatus st = cudaStreamCaptureStatusNone;
+  const cudaGraphNode_t* deps = nullptr;
+  size_t n = 0;
+  A0_CUDA(cudaStreamGetCaptureInfo_v3(stream, &st, nullptr, graph, &deps, nullptr, &n));
+  A0_REQUIRE(st == cudaStreamCaptureStatusActive && n == 1,
+             "the stream is not capturing (status %d) or its last captured work is not one node (%zu)", (int)st, n);
+  *node = deps[0];
+  return A0_OK;
+}
+
+extern "C" int a0_capture_node(a0_stream_t stream, void** node) {
+  A0_REQUIRE(node != nullptr, "a0_capture_node: node is NULL");
+  cudaGraphNode_t n;
+  int rc = a0_capture_tail((cudaStream_t)stream, nullptr, &n);
+  if (rc) return rc;
+  *node = n;
+  return A0_OK;
+}
+
+extern "C" int a0_capture_join(a0_stream_t stream, void* from) {
+  A0_REQUIRE(from != nullptr, "a0_capture_join: from is NULL");
+  cudaGraph_t g;
+  cudaGraphNode_t to, f = (cudaGraphNode_t)from;
+  int rc = a0_capture_tail((cudaStream_t)stream, &g, &to);
+  if (rc) return rc;
+  cudaGraphEdgeData full = {};      // cudaGraphDependencyTypeDefault from cudaGraphKernelNodePortDefault: on completion
+  A0_CUDA(cudaGraphAddDependencies_v2(g, &f, &to, &full, 1));
+  return A0_OK;
+}
+
+extern "C" int a0_graph_edges(void* graph, void** from, void** to, int32_t* type, int32_t* from_port, int64_t capacity,
+                              int64_t* count) {
+  A0_REQUIRE(graph != nullptr && count != nullptr && capacity >= 0, "a0_graph_edges: bad graph, count or capacity");
+  size_t n = 0;
+  A0_CUDA(cudaGraphGetEdges_v2((cudaGraph_t)graph, nullptr, nullptr, nullptr, &n));
+  *count = (int64_t)n;
+  if (n == 0 || capacity == 0) return A0_OK;
+  A0_REQUIRE((int64_t)n <= capacity && from && to && type && from_port, "a0_graph_edges: %zu edges, room for %lld", n,
+             (long long)capacity);
+  std::vector<cudaGraphNode_t> f(n), t(n);
+  std::vector<cudaGraphEdgeData> d(n);
+  A0_CUDA(cudaGraphGetEdges_v2((cudaGraph_t)graph, f.data(), t.data(), d.data(), &n));
+  for (size_t i = 0; i < n; ++i) {
+    from[i] = f[i]; to[i] = t[i]; type[i] = d[i].type; from_port[i] = d[i].from_port;
+  }
+  return A0_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
 // lifetime
 // ------------------------------------------------------------------------------------------------
 __global__ void a0_fill_i32(int32_t* p, int64_t n, int32_t v) {
@@ -675,6 +731,9 @@ __device__ __forceinline__ void a0_k3_gather_body(const A0GatherArgs& g) {
     const unsigned int old = atomicAdd(g.progress, 1u);
     if (old == (unsigned int)g.gtotal - 1u) *reinterpret_cast<volatile unsigned int*>(g.progress) = 0u;   // every draw done: nobody polls any more
   }
+#ifdef A0_TRACE
+  _tx[0] = (unsigned long long)g.gbase + 1;     // which launch (gather wave) the record belongs to: its first draw + 1
+#endif
   A0_TEND(3);
   if (g.mail) asm volatile("griddepcontrol.wait;" ::: "memory");
 }

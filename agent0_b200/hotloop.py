@@ -75,6 +75,19 @@ def early_links(L, waves, plan_join=None):
     return frozenset(k for k in range(L) if k not in joins)
 
 
+def captured_early_links(L, waves):
+    """The early links of a CAPTURED waved step.  There a link that joins a wave can take that wave through a full
+    graph edge of its own (a0_capture_join) while the edge from the previous link stays programmatic: it then starts
+    only once its wave is complete, still under its predecessor link, and reads before its wait like any early link.
+    The write-back plan joins the apply the same way, so no link joins it.  K4[0] has no programmatic predecessor
+    to overlap and stays an ordinary join.  With one wave per batch every link is gated by its wave and a full edge
+    could only add the launch latency that a resident programmatic launch hides: that plan keeps ``early_links``'s
+    ordinary joins.  waves: wave_plan's rows; None: no link."""
+    if not waves or all(n == 1 for _, n, _, _ in waves):
+        return early_links(L, waves)
+    return frozenset(range(1, L))
+
+
 class ReplayTargetLoop:
     def __init__(self, replay, algo, batch_size, learner_steps, action_dim, outputs, n_step=None, double_q=True,
                  per=None, variant=0, discount=None, alpha=0.5, eps=0.01, c51=(51, -10.0, 10.0), mdqn=(0.03, -1.0),
@@ -111,7 +124,8 @@ class ReplayTargetLoop:
         ``step()`` issues the single gather launch unless this is set (the tests set it).
         pdl_at_joins: the K4 that waits for a wave keeps its programmatic-launch attribute (it executes griddepcontrol.wait
         before it reads anything, so every predecessor is complete whichever way the edge is typed): 67.2 against 68.2 us
-        per batch-32 step.  False: those K4 launches are plain stream-ordered launches.
+        per batch-32 step.  False: those K4 launches are plain stream-ordered launches.  Neither applies to the typed
+        joins of a captured C51 step (``captured_early_links``), which take their wave through a full graph edge.
         replacement=False: every batch holds B distinct records, drawn by a0_pt_sample_unique (the law of the
         reference's torch.multinomial(priority[:top], B, replacement=False), replay.py:41-43) from the sampler's own
         Philox stream (``rng_seed``; drawn from torch's default generator when None), and gathered by one plain K3
@@ -181,6 +195,7 @@ class ReplayTargetLoop:
         self.launches_per_step = 1 + n_gather + self.L + (1 if self.per else 0)     # our kernels (uniform_ is torch's)
         self._k4 = self._k4_early = None
         self._k4_all = None
+        self.nodes = None         # the last captured step's graph nodes: waves, plan, k4 (one per link), apply
         self.graph = None
         self.report = []          # pinned host (indices, losses) pairs filled by K2b: bind_report()
         self._report_dev = []
@@ -232,6 +247,8 @@ class ReplayTargetLoop:
         first half of the write-back (a0_pt_update_plan) on the same stream, and ``plan_ev`` after it."""
         rp, lib = self.rp, self.lib
         main = torch.cuda.current_stream(self.dev)
+        capturing = torch.cuda.is_current_stream_capturing()
+        self.nodes = {"waves": [], "plan": None, "k4": [], "apply": None} if capturing else None
         self.side.wait_stream(main)           # everything before this step (the previous write-back, the ingest)
         with torch.cuda.stream(self.side):
             st = self._st()
@@ -243,12 +260,26 @@ class ReplayTargetLoop:
                                                  self.r64.data_ptr(), self.r32.data_ptr(), self.d8.data_ptr(), self.d32.data_ptr(),
                                                  self.boot.data_ptr(), st), "a0_rb_gather_mail")
                 self.wave_ev[j].record(self.side)
+                if capturing:
+                    self.nodes["waves"].append(self._captured())
             if plan:
                 _lib.check(lib.a0_pt_update_plan(rp.h, self.idx.data_ptr(), self.total, self.plan.data_ptr(), st), "a0_pt_update_plan")
                 self.plan_ev.record(self.side)
+                if capturing:
+                    self.nodes["plan"] = self._captured()
 
     def _wait_wave(self, j):
         torch.cuda.current_stream(self.dev).wait_event(self.wave_ev[j])
+
+    def _captured(self):
+        """The node just captured on the current stream (a0_capture_node)."""
+        node = C.c_void_p()
+        _lib.check(self.lib.a0_capture_node(self._st(), C.byref(node)), "a0_capture_node")
+        return node.value
+
+    def _join_full(self, node):
+        """A full (default-typed) edge from ``node`` to the node just captured on the current stream (a0_capture_join)."""
+        _lib.check(self.lib.a0_capture_join(self._st(), node), "a0_capture_join")
 
     def _common(self, lo, count):
         s = slice(lo, lo + count)
@@ -357,8 +388,10 @@ class ReplayTargetLoop:
     # ------------------------------------------------------------------ whole steps
     def _targets_and_update(self, fused_k4, slot, update=True, planned=False):
         """The K4 launches of a step whose gather runs in waves (each waits for the wave that holds its batch), then K2b.
-        planned: the K4 ``_plan_join`` also waits for the plan (it executes griddepcontrol.wait before anything else, so the
-        plan is complete when the apply, launched under the last K4, starts), and the apply is the write-back."""
+        planned: the apply is the write-back.  Captured, the plan joins the apply through a full edge, and so do the waves
+        the links of ``captured_early_links`` join.  Issued eagerly, every join is a stream wait: the K4 ``_plan_join``
+        also waits for the plan (it executes griddepcontrol.wait before anything else, so the plan is complete when the
+        apply, launched under the last K4, starts)."""
         if fused_k4:
             for j in range(len(self.waves)):
                 self._wait_wave(j)
@@ -366,13 +399,20 @@ class ReplayTargetLoop:
             if update:
                 self.update(slot, after_k4=True)
             return
-        early = early_links(self.L, self.waves, self._plan_join if planned else None)
+        typed = self.nodes is not None
+        early = captured_early_links(self.L, self.waves) if typed else \
+            early_links(self.L, self.waves, self._plan_join if planned else None)
         for k in range(self.L):
             j = self._join.get(k)
-            join_plan = planned and k == self._plan_join
+            join_plan = planned and not typed and k == self._plan_join
             if join_plan:
                 torch.cuda.current_stream(self.dev).wait_event(self.plan_ev)
-            if (j is None and not join_plan) or self.pdl_at_joins:
+            if j is not None and typed and k in early and self.algo == "c51":
+                # a typed join: programmatic edge from the previous link (the launch attribute), full edge from the wave.
+                # (The other algorithms' K4 read nothing before their wait: a full edge could only delay them.)
+                self.target_loss(k, early=True)
+                self._join_full(self.nodes["waves"][j])
+            elif (j is None and not join_plan) or self.pdl_at_joins:
                 if j is not None:
                     self._wait_wave(j)
                 self.target_loss(k, early=k in early)
@@ -388,10 +428,19 @@ class ReplayTargetLoop:
                     self.target_loss(k)
                 finally:
                     self.lib.a0_set_option(_lib.OPT_PDL, mask.value)
+            if typed:
+                self.nodes["k4"].append(self._captured())
         if planned:
             self._apply(slot)
+            if typed:
+                self.nodes["apply"] = self._captured()
+                self._join_full(self.nodes["plan"])
         elif update:
             self.update(slot, after_k4=True)
+        if typed:
+            # the typed joins are graph edges that stream capture does not track: join the side stream's last node (the
+            # plan, or the last wave) through the stream as well; it precedes the apply or a link already
+            torch.cuda.current_stream(self.dev).wait_stream(self.side)
 
     def step(self, fused_k4=False, slot=None, update=True):
         """update=False: everything but the priority write-back (StaleByOneLoop issues it during the next step)."""

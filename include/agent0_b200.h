@@ -134,6 +134,20 @@ int a0_set_option(int32_t option, int64_t value);
  * the K4 that joins a gather wave from another stream -- restores the mask it found).                     */
 int a0_get_option(int32_t option, int64_t* value);
 
+/* ---- typed joins in a captured graph ---------------------------------------------------------
+ * A kernel launched with the programmatic attribute after waiting for another stream's event gets programmatic
+ * edges from all its predecessors, so it may start before that other work is complete.  A captured step joins such
+ * work through a full edge of its own instead: launch the kernel after its stream predecessor alone, then
+ * a0_capture_join(stream, node) adds a default-typed edge (on completion) from `node` -- taken with a0_capture_node
+ * right after it was captured -- to the stream's last captured node.  Both need a stream that is capturing and whose
+ * last captured work is one node.
+ * a0_graph_edges: the edges of a graph (cudaGraph_t) with their cudaGraphDependencyType and outgoing port, for
+ * reading a captured step back; `count` receives the number of edges (call with capacity 0 to size the arrays). */
+int a0_capture_node(a0_stream_t stream, void** node);
+int a0_capture_join(a0_stream_t stream, void* from);
+int a0_graph_edges(void* graph, void** from, void** to, int32_t* type, int32_t* from_port, int64_t capacity,
+                   int64_t* count);
+
 /* ---- shard lifetime -------------------------------------------------------------------------
  * rec_capacity   transitions kept (cfg.replay.size); indices returned by a0_pt_sample are record
  *                ring positions in [0, rec_capacity)

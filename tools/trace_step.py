@@ -1,6 +1,8 @@
 """Device-side timeline of one replay+target step (the -DA0_TRACE build): per kernel launch, when its
-CTAs entered, passed griddepcontrol.wait / received their input, and finished (%globaltimer).
-Usage: A0_LIB=agent0_b200/libagent0_b200_trace.so python tools/trace_step.py [B] [L] [overlap 0/1]"""
+CTAs entered, passed griddepcontrol.wait / received their input, and finished (%globaltimer); the edge types of the
+captured graph, and for each K4 link which of its predecessors finished last.
+Usage: A0_LIB=agent0_b200/libagent0_b200_trace.so python tools/trace_step.py [B] [L] [overlap 0/1]
+A0_UNTYPED_JOINS=1,2,4: those links join their wave through the stream wait (programmatic edge) instead of a typed join."""
 import ctypes as C
 import json
 import os
@@ -13,7 +15,7 @@ import numpy as np
 import torch
 
 import bench as BN
-from agent0_b200 import _lib
+from agent0_b200 import _lib, hotloop
 from agent0_b200.config import make_config
 from agent0_b200.replay import ReplayDataset
 
@@ -43,7 +45,35 @@ if k4_only:
         for k in range(L):
             hp.target_loss(k)
 else:
-    g = BN.capture_step(hp, torch)
+    if os.environ.get("A0_UNTYPED_JOINS"):
+        _untyped = {int(x) for x in os.environ["A0_UNTYPED_JOINS"].split(",")}
+        _typed = hotloop.captured_early_links
+        hotloop.captured_early_links = lambda L_, w_: _typed(L_, w_) - _untyped
+    hp.rp.push_dynamic()
+    for _ in range(3):
+        hp.step()
+    torch.cuda.synchronize()
+    g = torch.cuda.CUDAGraph(keep_graph=True)
+    with torch.cuda.graph(g):
+        hp.step()
+    if hp.nodes:
+        nE = C.c_int64()
+        assert lib.a0_graph_edges(g.raw_cuda_graph(), None, None, None, None, 0, C.byref(nE)) == 0
+        cap = nE.value
+        ef, et, ety, eport = (C.c_void_p * cap)(), (C.c_void_p * cap)(), (C.c_int32 * cap)(), (C.c_int32 * cap)()
+        assert lib.a0_graph_edges(g.raw_cuda_graph(), ef, et, ety, eport, cap, C.byref(nE)) == 0
+        E = {(ef[i], et[i]): ("programmatic" if ety[i] else "full") for i in range(nE.value)}
+        nd = hp.nodes
+        name = {n: f"K4[{k}]" for k, n in enumerate(nd["k4"])}
+        name.update({n: f"wave {j}" for j, n in enumerate(nd["waves"])})
+        if nd["plan"]:
+            name[nd["plan"]] = "plan"
+        if nd["apply"]:
+            name[nd["apply"]] = "apply"
+        print("edges into the K4 links and the apply (captured graph):")
+        for n in nd["k4"] + ([nd["apply"]] if nd["apply"] else []):
+            print(f"   {name[n]:8s} <- " + ", ".join(f"{name.get(a, 'other')} {t}" for (a, b), t in E.items() if b == n))
+    g.instantiate()
 for _ in range(5):
     g.replay()
 torch.cuda.synchronize()
@@ -97,8 +127,8 @@ if m4.any():
     dd = np.diff(pts, axis=1)
     lab = ["loads land", "arg-max | row maxima", "sum-exps | bin geometry | log-softmax", "p / sum + term weights", "segmented scan + bins",
            "CE | mass reductions", "emit loss / priority / max_p + gradient stores"]
-    from agent0_b200.hotloop import early_links
-    early = early_links(L, hp.waves, hp._plan_join if hp._use_plan else None)
+    early = hotloop.captured_early_links(L, hp.waves) if hp.nodes else \
+        hotloop.early_links(L, hp.waves, hp._plan_join if hp._use_plan else None)
     t0_4, t1_4 = t0[m4], t1[m4]
     o4 = np.argsort(t0_4)
     per4 = max(1, int(m4.sum()) // L)
@@ -119,6 +149,26 @@ if m4.any():
         if ks:
             print(f"   {name}: link-to-link period (exit to exit) median {np.median(np.diff(ex)[np.array(ks) - 1]) / 1e3:.2f} us; "
                   f"entry -> wait returned median {int(np.median(pre[ks]))} cycles; links {ks}")
+    # which predecessor finished last: the previous link, or the gather wave the link joins (a K3 record carries the
+    # first draw of its launch + 1 in x[0])
+    wave_exit = {}
+    for b0, _, lo, _ in hp.waves or []:
+        mw = (kid == 3) & (xs[:, 0] == lo + 1)
+        if mw.any():
+            wave_exit[b0] = t1[mw].max()
+    en = np.array([t0_4[link == i].min() for i in range(L)])
+    f_ = lambda v: f"{(v - base) / 1e3:7.2f}" if v is not None else "      -"
+    print("   per link, us from the first traced entry: entry | previous link's exit | its wave's exit | exit | link to link"
+          " | last predecessor")
+    for i in range(L):
+        pe, we = (ex[i - 1] if i else None), wave_exit.get(i)
+        last = "wave" if we is not None and (pe is None or we > pe) else ("previous link" if pe is not None else "-")
+        print(f"   K4[{i:2d}] {'early' if i in early else 'join '} {f_(en[i])} | {f_(pe)} | {f_(we)} | {f_(ex[i])} | "
+              f"{(ex[i] - pe) / 1e3 if pe is not None else 0.0:5.2f} | {last}")
+m7, m8 = kid == 7, kid == 8
+if m7.any() and m8.any() and m4.any():
+    print(f"apply: plan exit {(t1[m7].max() - base) / 1e3:.2f} us, last K4 exit {(t1[m4].max() - base) / 1e3:.2f} us: last predecessor "
+          f"{'plan' if t1[m7].max() > t1[m4].max() else 'K4[L-1]'}")
 m3 = kid == 3
 if m3.any():
     q = [0, 10, 50, 90, 100]
